@@ -10,9 +10,14 @@ same GPU and the CPU baseline beside it.
 One "step" = one pass of the hot path over one batch of synthetic
 nuScenes-shaped input: BASELINE.json configs[1] (6 cams 16x44 feats, D=88,
 C=64, batch 8 per GPU; weak scaling: every rank lifts its own 8 samples, no
-data-path collective).  The K-step region is repeated until at least one
-second of GPU time has been measured; `value` is the median repeat.  Prints
-ONE JSON line on rank 0.
+data-path collective).  Exactly K steps are timed after W warm-up steps
+(--min-seconds S repeats the K-step region until S seconds of GPU time have
+been measured and reports the median repeat).  Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes what the last timed step returned to its caller --
+the pooled volume and the gradients of depth and features -- as float32 .npy
+files (see dump_outputs); the inputs depend on the arguments only, so two
+builds can be compared output for output.
 
 Secondary objects of the line (all device-timed with CUDA events):
   workloads        C3 (C=512), C4 (C=768, D=118, B=16) lift fwd+bwd and the real VEON neck
@@ -45,22 +50,52 @@ VOX = 640000
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    # 1300 C2 steps of 0.76 ms (one B200): the default timed region lasts about a second
+    ap.add_argument("--steps", type=int, default=1300, help="timed steps K")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C2", help="veon_b200.synthetic.CONFIGS key")
     ap.add_argument("--batch", type=int, default=0, help="override samples per GPU per step")
     ap.add_argument("--cpu-seconds", type=float, default=15.0,
                     help="budget of the cpu_baseline leg (rank 0, N=1 only)")
-    ap.add_argument("--min-seconds", type=float, default=1.0,
-                    help="the K-step region is repeated until this much GPU time is measured")
+    ap.add_argument("--min-seconds", type=float, default=0.0,
+                    help="repeat the K-step region until this much GPU time is measured and "
+                         "report the median (default 0: one region, exactly K timed steps)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true",
                     help="headline + e2e only (no workloads / comparator / pipeline / tail legs)")
     ap.add_argument("--host-sync", type=int, default=0,
                     help="1: read the point / interval counts back every step (the reference's "
                          "empty-input check); default 0 = LSSViewTransformer(sync_free=True)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy "
+                         "(rank 0's outputs when several GPUs run)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computes: it needs --impl ours")
+    return args
+
+
+DUMP_MAX_ELEMENTS = 4 << 20      # 16 MB of float32 per array, three arrays: under 64 MB in all
+
+
+def dump_outputs(directory, arrays):
+    """Writes each tensor of `arrays` as float32 `directory/<name>.npy`.  A tensor of more than
+    DUMP_MAX_ELEMENTS elements is stored as `<name>_sample.npy`: its elements at a fixed set of
+    flat indices (drawn with seed 0 from its size alone, sorted), so two runs of the same
+    arguments store the same positions."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), DUMP_MAX_ELEMENTS))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+            name += "_sample"
+        np.save(os.path.join(directory, name + ".npy"), t.float().cpu().numpy())
 
 
 def workload_dict(cfg, batch, extra=None):
@@ -705,7 +740,19 @@ def run_ours(args):
         feat = feat.detach().requires_grad_()
         bev = neck.voxel_pooling_v2(coor, depth, feat)
         bev.backward(out_grad)
-        return depth.grad, feat.grad
+        return bev, depth.grad, feat.grad
+
+    # --dump-outputs: the outputs of the last step of the final timed region only, so that no
+    # earlier region runs with a step's outputs held alive
+    last, capture = {}, {"on": False}
+
+    def step_headline(i):
+        out = step_device(i)
+        if capture["on"] and i == K - 1:
+            last.update(zip(("bev", "depth_grad", "feat_grad"), out))
+
+    def final_region_of_headline():
+        capture["on"] = bool(args.dump_outputs) and rank == 0
 
     def step_device_lookahead(i):
         """The same step with the index preparation of step i+1 queued on the neck's side stream
@@ -832,18 +879,22 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps, warmup, whole_loop=False, min_seconds=0.0, max_repeats=400):
+    def timed(fn, steps, warmup, whole_loop=False, min_seconds=0.0, max_repeats=400,
+              before_final=None):
         """W warm-up steps, then the K-step region (barrier + synchronize on both sides, CUDA
-        events, max over ranks) repeated until `min_seconds` of GPU time: returns the MEDIAN
-        region in ms, the launches of one region, the number of repeats and the total time."""
+        events, max over ranks), once or, with `min_seconds` > 0, repeated until that much GPU
+        time: returns the MEDIAN region in ms, the launches of one region, the number of repeats
+        and the total time.  `before_final` is called before the last region starts."""
         if whole_loop:
             fn(warmup)
         else:
             for i in range(warmup):
                 fn(i)
 
-        def region():
+        def region(final):
             barrier()
+            if final and before_final is not None:
+                before_final()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             l0 = lib.veon_kernel_launch_count()
             e0.record()
@@ -859,26 +910,31 @@ def run_ours(args):
             if world > 1:
                 dist.all_reduce(ms, op=dist.ReduceOp.MAX)
             return float(ms.item()), launches
-        ms0, launches = region()
-        repeats = max(3, min(max_repeats, int(min_seconds * 1e3 / max(ms0, 1e-3)) + 1))
+        ms0, launches = region(final=min_seconds <= 0)
+        repeats = 1 if min_seconds <= 0 else \
+            max(3, min(max_repeats, int(min_seconds * 1e3 / max(ms0, 1e-3)) + 1))
         if world > 1:      # every rank must run the same number of regions (collectives inside)
             r = torch.tensor([repeats], device=dev)
             dist.broadcast(r, 0)
             repeats = int(r.item())
-        all_ms = [ms0] + [region()[0] for _ in range(repeats - 1)]
+        all_ms = [ms0] + [region(final=k == repeats - 2)[0] for k in range(repeats - 1)]
         s = sorted(all_ms)
         return s[len(s) // 2], launches, len(all_ms), sum(all_ms) * 1e-3, s[0], s[-1]
 
-    K, Wm = max(args.steps, 1), max(args.warmup, 3)
+    K, Wm = args.steps, max(args.warmup, 3)
     with ClockSampler(local) as clocks:
-        ms_total, launches, reps, total_s, ms_min, ms_max = timed(step_device, K, Wm,
-                                                                  min_seconds=args.min_seconds)
+        ms_total, launches, reps, total_s, ms_min, ms_max = timed(
+            step_headline, K, Wm, min_seconds=args.min_seconds,
+            before_final=final_region_of_headline)
+        if last:
+            dump_outputs(args.dump_outputs, last)
+            last.clear()
         ms_look, _, reps_look, _, _, _ = timed(step_device_lookahead, K, Wm,
                                                min_seconds=args.min_seconds / 2)
     ms_e2e, _, reps_e2e, total_e2e, _, _ = timed(run_e2e, K, max(3, Wm // 2), whole_loop=True,
                                                  min_seconds=args.min_seconds / 2)
     ms_copy, _, _, _, _, _ = timed(lambda n: run_e2e(n, compute=False), K, 3, whole_loop=True,
-                                   min_seconds=0.2)
+                                   min_seconds=args.min_seconds)
 
     # live per-call device times (CUDA events on the launching stream) over K more steps
     BP.enable_kernel_timing(True)
@@ -922,7 +978,8 @@ def run_ours(args):
             "host_sync_per_step": 0 if sync_free else 1,
             "numa": numa,
             "n_kept": n_kept, "n_intervals": n_int}),
-        "timing": {"what": f"median of {reps} repeats of the {K}-step region "
+        "timing": {"what": (f"one {K}-step region " if reps == 1 else
+                            f"median of {reps} repeats of the {K}-step region ") +
                            "(barrier + synchronize on both sides, CUDA events, max over ranks)",
                    "repeats": reps, "timed_region_s_total": round(total_s, 3),
                    "ms_per_step_min": ms_min / K, "ms_per_step_max": ms_max / K},

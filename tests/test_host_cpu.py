@@ -411,3 +411,34 @@ def test_prepare_vocabulary_matches_the_reference_expression():
     # loss-side grouping (no background row): occ3d_nuscenes.py:249-265
     assert class_of_prompt([0, 0, 1, 2, 2], background=False).tolist() == [0, 0, 1, 2, 2]
     assert class_of_prompt([0, 0, 1, 2, 2]).tolist() == [0, 0, 1, 2, 2, 3]
+
+
+# ---- bench.py --dump-outputs ----------------------------------------------------------------------
+def test_bench_dump_outputs_stores_a_fixed_sample_of_large_arrays(tmp_path):
+    """Arrays up to DUMP_MAX_ELEMENTS are stored whole with their shape, larger ones at flat indices
+    that depend on their size alone (seed 0), so two runs store the same positions; the three
+    outputs of a step stay under 64 MB."""
+    import bench
+    cap = bench.DUMP_MAX_ELEMENTS
+    assert 3 * cap * 4 <= 64 << 20
+    n = cap + 1000                                  # < 2^24: float32 holds every index exactly
+    big = torch.arange(n, dtype=torch.float32)      # element value == its flat index
+    small = torch.randn(5, 4, dtype=torch.float64).t()          # non-contiguous, float64
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"bev": big.view(2, -1), "feat_grad": small})
+    assert sorted(os.listdir(tmp_path / "a")) == ["bev_sample.npy", "feat_grad.npy"]
+    a = np.load(tmp_path / "a" / "bev_sample.npy")
+    want = np.unique(np.random.default_rng(0).integers(0, n, cap)).astype(np.float32)
+    assert a.dtype == np.float32 and np.array_equal(a, want)
+    assert np.array_equal(a, np.load(tmp_path / "b" / "bev_sample.npy"))
+    f = np.load(tmp_path / "a" / "feat_grad.npy")
+    assert f.dtype == np.float32 and f.shape == (4, 5)
+    np.testing.assert_array_equal(f, small.float().numpy())
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "d"]])
+def test_bench_refuses_arguments_it_cannot_honour(monkeypatch, argv):
+    import bench
+    monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+    with pytest.raises(SystemExit):
+        bench.parse()
