@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define VEON_ABI_VERSION 8
+#define VEON_ABI_VERSION 9
 
 #define VEON_E_BADARG    (-1)  /* NULL pointer / non-positive dimension          */
 #define VEON_E_WORKSPACE (-2)  /* workspace smaller than *_workspace_bytes()     */
@@ -271,6 +271,29 @@ int veon_bev_pool_v2_fwd_planar(const float* depth, const float* feat,
                                 float* out, void* workspace, size_t workspace_bytes,
                                 void* stream);
 
+/* The same pooling into a CHANNELS-LAST volume: out is [B,Z,Y,X,C] (the reference kernel's own
+ * layout, bev_pool_cuda.cu:46), every element written exactly once (zero rows for empty voxels),
+ * no workspace.  The sums are the same bits as veon_bev_pool_v2_fwd_planar's, only their order in
+ * memory differs: torch's channels_last_3d view of [B,C,Z,Y,X] has exactly this storage.
+ * Requires a valid plan; any C >= 1, any V (ragged x-runs), B >= 1.  Kernel selection: rows of at
+ * most 32 channels (C % 4 == 0, tile_heavy given, V % 32 == 0, B*V <= 2^24, 16-byte aligned feat
+ * and out) take the lane-per-voxel kernel; everything else the lane-per-channel kernel, which
+ * stages a tile's rows in shared memory and writes them as contiguous rows.  Tiles listed in
+ * tile_heavy get a thread block each, queued behind the main grid as a programmatic dependent
+ * that completes only after it: the next kernel in the stream, or the next node of a captured
+ * graph, sees the whole volume.  VEON_E_RANGE when B*V, B or the 32-bit feature row offsets
+ * overflow (as veon_bev_pool_v2_fwd_planar). */
+int veon_bev_pool_v2_fwd_planar_cl(const float* depth, const float* feat,
+                                   const int32_t* ranks_depth,
+                                   const int32_t* ranks_feat,
+                                   const int32_t* ranks_bev,
+                                   const int32_t* tile_start,
+                                   const int32_t* tile_heavy /* may be NULL */,
+                                   int64_t tile_heavy_ints /* its size in int32 */,
+                                   int B, int C, int64_t voxels_per_sample,
+                                   int64_t n_feat_rows /* B*N*H*W rows of feat */,
+                                   float* out, void* stream);
+
 /* Pooling fused with the 2x2x2 max-downsample VEON's neck applies next
  * (view_transformer_raw.py:549-553), forward only: out is [B, C, Z/2, Y/2, X/2], bit-identical
  * to that maximum over the volume veon_bev_pool_v2_fwd_planar would write (never materialised).
@@ -303,6 +326,15 @@ int veon_maxdown2_fwd_mask(const float* in, int64_t BC, int Z, int Y, int X, flo
                            uint8_t* mask, void* stream);
 int veon_maxdown2_bwd(const float* in, const float* out, const float* grad_out,
                       int64_t BC, int Z, int Y, int X, float* grad_in, void* stream);
+/* The same two operations on CHANNELS-LAST volumes: in / grad_in [B,Z,Y,X,C], out / grad_out
+ * [B,Z/2,Y/2,X/2,C], float32, contiguous, any alignment.  Same reduction tree, NaN rule, -0/+0
+ * result and first-arg-max gradient as veon_maxdown2_fwd / _bwd, so the values are the same
+ * bits in the other layout.  Z, Y, X even, else VEON_E_UNSUPPORTED; VEON_E_RANGE when the output
+ * has 2^32 voxels or more. */
+int veon_maxdown2_cl_fwd(const float* in, int B, int C, int Z, int Y, int X, float* out,
+                         void* stream);
+int veon_maxdown2_cl_bwd(const float* in, const float* out, const float* grad_out,
+                         int B, int C, int Z, int Y, int X, float* grad_in, void* stream);
 
 /* QuickCumsumCuda.backward (bev_pool.py:43-83) for a [B,C,Z,Y,X] out_grad.
  *   rows_ws      float scratch of at least veon_bev_pool_v2_bwd_workspace_floats() elements
@@ -324,6 +356,24 @@ int veon_bev_pool_v2_bwd_planar(const float* out_grad,
                                 float* rows_ws, int64_t rows_ws_floats,
                                 float* depth_grad, float* feat_grad,
                                 void* stream);
+
+/* QuickCumsumCuda.backward for a CHANNELS-LAST out_grad [B,Z,Y,X,C] in ONE launch: an occupied
+ * voxel's gradient is already one contiguous row there, so the pixel pass reads it in place --
+ * no row pass and no rows_ws scratch.  The row of a kept point is that of its voxel,
+ * ranks_bev[interval_starts[point_interval[...]]]; only intervals named by point_interval are
+ * read, so a capacity-sized interval_starts (the sync-free prepare outputs) is never read beyond
+ * the device-side interval count.  depth_grad / feat_grad as in veon_bev_pool_v2_bwd_planar and
+ * the same bits (same rows, same order of operations).  Requires a valid plan.  VEON_E_RANGE when
+ * B*V >= 2^31; VEON_E_UNSUPPORTED when D is too large for the per-warp point lists (as the
+ * channels-first pixel pass). */
+int veon_bev_pool_v2_bwd_planar_cl(const float* out_grad,
+                                   const float* depth, const float* feat,
+                                   const int32_t* ranks_bev,
+                                   const int32_t* interval_starts,
+                                   const int32_t* point_interval,
+                                   int B, int N, int D, int H, int W, int C,
+                                   int64_t voxels_per_sample,
+                                   float* depth_grad, float* feat_grad, void* stream);
 
 /* QuickCumsumCuda.backward for a gradient that arrives BEHIND the 2x2x2 max-downsample:
  * grad_ds [B,C,Z/2,Y/2,X/2] and the mask of veon_maxdown2_fwd_mask replace out_grad; the

@@ -46,6 +46,8 @@ _SIGNATURES = {
                                                c_int, c_int, c_int, c_int, c_int, c_int,
                                                c_int, c_int, c_int, _P, _P, _P, _P]),
     "veon_maxdown2_bwd": (c_int, [_P, _P, _P, c_int64, c_int, c_int, c_int, _P, _P]),
+    "veon_maxdown2_cl_fwd": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
+    "veon_maxdown2_cl_bwd": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     "veon_prepare_v2_voxel_start_offset": (c_size_t, [c_int, c_int, c_int, c_int, c_int, _P]),
     "veon_bev_pool_v2_ds_fwd": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
                                         c_int64, _P, _P]),
@@ -66,6 +68,10 @@ _SIGNATURES = {
     "veon_bev_pool_v2_fwd_workspace_bytes": (c_size_t, [c_int, c_int, c_int64]),
     "veon_bev_pool_v2_fwd_planar": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, c_int64,
                                             c_int, c_int, c_int64, c_int64, _P, _P, c_size_t, _P]),
+    "veon_bev_pool_v2_fwd_planar_cl": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64,
+                                               c_int, c_int, c_int64, c_int64, _P, _P]),
+    "veon_bev_pool_v2_bwd_planar_cl": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int,
+                                               c_int, c_int, c_int64, _P, _P, _P]),
     "veon_bev_pool_v2_bwd_workspace_floats": (c_size_t, [c_int64, c_int, c_int, c_int, c_int, c_int,
                                                          c_int, c_int64]),
     "veon_bev_pool_v2_bwd_planar": (c_int, [_P, _P, _P, _P, _P, _P, c_int64,

@@ -16,6 +16,11 @@ What differs underneath (DESIGN.md): the volume is produced channels-first
 in one pass (no memset, no permute copy), the backward needs no argsort, and a
 "plan" (tile tables + point->interval table) rides along with the rank
 tensors.  Everything runs in CUDA through the C ABI; there is no CPU path.
+
+`memory_format=torch.channels_last_3d` (bev_pool_v2 / pool_prepared) returns the
+same [B,C,Z,Y,X] values stored channels-last ([B,Z,Y,X,C] underneath), written
+that way by the kernels; a channels-last gradient is consumed in place by a
+single-pass backward, whichever layout the forward produced.
 """
 import collections
 import weakref
@@ -32,6 +37,17 @@ __all__ = ["bev_pool_v2", "QuickCumsumCuda", "TRTBEVPoolv2",
 LAYOUT_BZYXC, LAYOUT_BCZYX = 0, 1
 PLAN_OUT_OF_RANGE = 8       # VEON_PLAN_OUT_OF_RANGE
 TILE_VOXELS = 32
+
+
+_MEMORY_FORMATS = (torch.contiguous_format, torch.channels_last_3d)
+
+
+def _channels_last(memory_format):
+    """True for torch.channels_last_3d, False for torch.contiguous_format; ValueError otherwise."""
+    if memory_format not in _MEMORY_FORMATS:
+        raise ValueError("memory_format must be torch.contiguous_format or torch.channels_last_3d, "
+                         f"got {memory_format!r}")
+    return memory_format is torch.channels_last_3d
 
 
 def _stream_ptr(device):
@@ -477,17 +493,33 @@ def two_hot_depth(depths, depth_cfg, D, gamma=4.0, downsample=0):
 class MaxDown2x2x2(torch.autograd.Function):
     """The neck's 2x2x2 reduction, `rearrange(... '(dz dh dw)') -> torch.max(dim=-1).values`
     (view_transformer_raw.py:549-553), and its gradient (all of it to the first arg-max of a
-    block, as max(dim) does) as two streaming kernels."""
+    block, as max(dim) does) as two streaming kernels.  A channels-last-3d input (even Z, Y, X)
+    goes through the channels-last kernels and gives a channels-last-3d result."""
 
     @staticmethod
     def supports(x):
-        return (x.is_cuda and x.dtype == torch.float32 and x.dim() == 5 and x.is_contiguous()
-                and x.shape[2] % 2 == 0 and x.shape[3] % 2 == 0 and x.shape[4] % 4 == 0)
+        if not (x.is_cuda and x.dtype == torch.float32 and x.dim() == 5
+                and x.shape[2] % 2 == 0 and x.shape[3] % 2 == 0):
+            return False
+        if x.is_contiguous():
+            return x.shape[4] % 4 == 0
+        return x.shape[4] % 2 == 0 and x.is_contiguous(memory_format=torch.channels_last_3d)
 
     @staticmethod
     def forward(ctx, x):
         lib = _lib.load()
         B, C, Z, Y, X = x.shape
+        ctx.channels_last = not x.is_contiguous()
+        if ctx.channels_last:
+            with torch.cuda.device(x.device):
+                out = torch.empty((B, Z // 2, Y // 2, X // 2, C), dtype=torch.float32,
+                                  device=x.device).permute(0, 4, 1, 2, 3)
+                with _timed("maxdown_cl_fwd", x.device):
+                    rc = lib.veon_maxdown2_cl_fwd(_ptr(x), B, C, Z, Y, X, _ptr(out),
+                                                  _stream_ptr(x.device))
+            _lib.check(rc, "veon_maxdown2_cl_fwd")
+            ctx.save_for_backward(x, out)
+            return out
         with torch.cuda.device(x.device):
             out = torch.empty((B, C, Z // 2, Y // 2, X // 2), dtype=torch.float32, device=x.device)
             with _timed("maxdown_fwd", x.device):
@@ -501,6 +533,15 @@ class MaxDown2x2x2(torch.autograd.Function):
         x, out = ctx.saved_tensors
         lib = _lib.load()
         B, C, Z, Y, X = x.shape
+        if ctx.channels_last:
+            g = grad_out.float().contiguous(memory_format=torch.channels_last_3d)
+            with torch.cuda.device(x.device):
+                grad_in = torch.empty_like(x)          # channels-last, like x
+                with _timed("maxdown_cl_bwd", x.device):
+                    rc = lib.veon_maxdown2_cl_bwd(_ptr(x), _ptr(out), _ptr(g), B, C, Z, Y, X,
+                                                  _ptr(grad_in), _stream_ptr(x.device))
+            _lib.check(rc, "veon_maxdown2_cl_bwd")
+            return grad_in
         g = grad_out.contiguous().float()
         with torch.cuda.device(x.device):
             grad_in = torch.empty_like(x)
@@ -651,6 +692,20 @@ def _fwd_planar(depth, feat, rd, rf, rb, plan, B, C, V, shape5):
     return out
 
 
+def _fwd_planar_cl(depth, feat, rd, rf, rb, plan, B, C, V, shape5):
+    lib = _lib.load()
+    dev = feat.device
+    with torch.cuda.device(dev):
+        out = torch.empty(shape5, dtype=torch.float32, device=dev)  # [B,Z,Y,X,C]
+        with _timed("pool_fwd_cl", dev):
+            rc = lib.veon_bev_pool_v2_fwd_planar_cl(
+                _ptr(depth), _ptr(feat), _ptr(rd), _ptr(rf), _ptr(rb), _ptr(plan.tile_start),
+                _ptr(plan.tile_heavy), plan.tile_heavy.numel(), B, C, V, feat.numel() // C,
+                _ptr(out), _stream_ptr(dev))
+    _lib.check(rc, "veon_bev_pool_v2_fwd_planar_cl")
+    return out
+
+
 def _need_backward_tables(plan):
     if plan.point_interval is None:
         raise RuntimeError("these ranks were prepared with backward_tables=False (inference): "
@@ -677,18 +732,44 @@ def _bwd_planar(grad_planar, depth, feat, rb, ist, plan, C):
     return depth_grad, feat_grad
 
 
+def _bwd_planar_cl(grad_cl, depth, feat, rb, ist, plan, C):
+    """Single pass on a channels-last [B,Z,Y,X,C] gradient (no row pass, no scratch)."""
+    _need_backward_tables(plan)
+    lib = _lib.load()
+    dev = feat.device
+    B, N, D, H, W = plan.dims
+    with torch.cuda.device(dev):
+        depth_grad = torch.empty_like(depth)
+        feat_grad = torch.empty_like(feat)
+        with _timed("pool_bwd_cl", dev):
+            rc = lib.veon_bev_pool_v2_bwd_planar_cl(
+                _ptr(grad_cl), _ptr(depth), _ptr(feat), _ptr(rb), _ptr(ist),
+                _ptr(plan.point_interval), B, N, D, H, W, C, plan.V, _ptr(depth_grad),
+                _ptr(feat_grad), _stream_ptr(dev))
+    _lib.check(rc, "veon_bev_pool_v2_bwd_planar_cl")
+    return depth_grad, feat_grad
+
+
 class QuickCumsumCuda(torch.autograd.Function):
     """Same signature and result as the reference Function (bev_pool.py:11-83):
     returns the pooled volume shaped [B,Z,Y,X,C].  It is a permuted VIEW of a
     channels-first buffer, so the `.permute(0,4,1,2,3).contiguous()` that
-    `bev_pool_v2` applies next (bev_pool.py:91) is free."""
+    `bev_pool_v2` applies next (bev_pool.py:91) is free.  With the extra
+    `channels_last` argument it is a contiguous [B,Z,Y,X,C] tensor instead.
+
+    The backward takes the gradient in the layout it arrives in: channels-first
+    storage -> the two-pass kernels; channels-last storage (a contiguous
+    [B,Z,Y,X,C] gradient) with a valid plan -> the single-pass kernel, which reads
+    the gradient rows in place; anything else is copied to channels-first first.
+    All routes give the same bits."""
 
     @staticmethod
     def forward(ctx, depth, feat, ranks_depth, ranks_feat, ranks_bev,
                 bev_feat_shape, interval_starts, interval_lengths, *extra):
-        # `extra` = (PoolPlan,) when called from this package; the reference's
-        # 8-argument call is accepted unchanged
+        # `extra` = (PoolPlan or None[, channels_last]) when called from this package; the
+        # reference's 8-argument call is accepted unchanged
         plan = extra[0] if extra else None
+        channels_last = bool(extra[1]) if len(extra) > 1 else False
         ctx.n_extra = len(extra)
         _require_cuda(depth, feat, ranks_depth, ranks_feat, ranks_bev,
                       interval_starts, interval_lengths)
@@ -723,7 +804,21 @@ class QuickCumsumCuda(torch.autograd.Function):
             # bev_pool.cpp has no CHECK_* macros); so would the unchecked generic kernels
             raise ValueError("bev_pool_v2: a rank lies outside its tensor (ranks_depth >= "
                              "depth.numel(), ranks_feat >= feat rows or ranks_bev >= B*Z*Y*X)")
-        if plan.ok:
+        if channels_last:
+            if plan.ok:
+                out = _fwd_planar_cl(depth, feat, ranks_depth, ranks_feat, ranks_bev, plan,
+                                     B, C, V, (B, Z, Y, X, C))
+            else:
+                lib = _lib.load()
+                out = feat.new_zeros((B, Z, Y, X, C))
+                with torch.cuda.device(feat.device):
+                    rc = lib.veon_bev_pool_v2_generic(
+                        C, interval_starts.numel(), LAYOUT_BZYXC, V, _ptr(depth), _ptr(feat),
+                        _ptr(ranks_depth), _ptr(ranks_feat), _ptr(ranks_bev),
+                        _ptr(interval_starts), _ptr(interval_lengths), _ptr(out),
+                        _stream_ptr(feat.device))
+                _lib.check(rc, "veon_bev_pool_v2_generic")
+        elif plan.ok:
             out = _fwd_planar(depth, feat, ranks_depth, ranks_feat, ranks_bev, plan,
                               B, C, V, (B, C, Z, Y, X))
         else:
@@ -739,7 +834,7 @@ class QuickCumsumCuda(torch.autograd.Function):
         ctx.save_for_backward(ranks_bev, depth, feat, ranks_feat, ranks_depth, interval_starts)
         ctx.plan = plan
         ctx.vol = (B, C, Z, Y, X)
-        return out.permute(0, 2, 3, 4, 1)
+        return out if channels_last else out.permute(0, 2, 3, 4, 1)
 
     @staticmethod
     def backward(ctx, out_grad):
@@ -747,9 +842,15 @@ class QuickCumsumCuda(torch.autograd.Function):
         B, C, Z, Y, X = ctx.vol
         plan = ctx.plan
         g = out_grad.permute(0, 4, 1, 2, 3)  # back to the channels-first storage order
-        if g.dtype != torch.float32 or not g.is_contiguous():
+        cl_grad = (out_grad.dtype == torch.float32 and not g.is_contiguous()
+                   and out_grad.is_contiguous() and plan.ok)
+        if not cl_grad and (g.dtype != torch.float32 or not g.is_contiguous()):
             g = g.float().contiguous()
-        if plan.ok:
+        if cl_grad:
+            # channels-last storage: the single pass reads its rows in place
+            depth_grad, feat_grad = _bwd_planar_cl(out_grad, depth, feat, ranks_bev,
+                                                   interval_starts, plan, C)
+        elif plan.ok:
             depth_grad, feat_grad = _bwd_planar(g, depth, feat, ranks_bev, interval_starts,
                                                 plan, C)
         else:
@@ -770,26 +871,34 @@ class QuickCumsumCuda(torch.autograd.Function):
 
 
 def bev_pool_v2(depth, feat, ranks_depth, ranks_feat, ranks_bev,
-                bev_feat_shape, interval_starts, interval_lengths):
+                bev_feat_shape, interval_starts, interval_lengths, *,
+                memory_format=torch.contiguous_format):
     """Drop-in for the reference `bev_pool_v2` (bev_pool.py:86-92).
 
     depth [B,N,D,H,W]; feat [B,N,H,W,C] (any strides); int32 rank / interval
-    tensors; bev_feat_shape = (B,Z,Y,X,C).  Returns [B,C,Z,Y,X] float32
-    contiguous, differentiable w.r.t. depth and feat."""
+    tensors; bev_feat_shape = (B,Z,Y,X,C).  Returns [B,C,Z,Y,X] float32,
+    differentiable w.r.t. depth and feat: contiguous, or with
+    memory_format=torch.channels_last_3d the same values stored channels-last
+    (written so by the kernels, not copied)."""
+    cl = _channels_last(memory_format)
+    extra = (None, True) if cl else ()
     x = QuickCumsumCuda.apply(depth, feat, ranks_depth, ranks_feat, ranks_bev,
-                              bev_feat_shape, interval_starts, interval_lengths)
-    x = x.permute(0, 4, 1, 2, 3).contiguous()  # no copy: already channels-first
-    return x
+                              bev_feat_shape, interval_starts, interval_lengths, *extra)
+    x = x.permute(0, 4, 1, 2, 3)
+    # no copy either way: the storage already has the requested order
+    return x if cl else x.contiguous()
 
 
-def pool_prepared(depth, feat, prep, bev_feat_shape):
+def pool_prepared(depth, feat, prep, bev_feat_shape, memory_format=torch.contiguous_format):
     """bev_pool_v2 on a `PreparedRanks` without any host synchronisation in the
     forward (the counts are only needed, and by then long available, when the
-    backward sizes its scratch)."""
+    backward sizes its scratch).  memory_format as in bev_pool_v2."""
+    cl = _channels_last(memory_format)
+    extra = (prep.plan, True) if cl else (prep.plan,)
     x = QuickCumsumCuda.apply(depth, feat, prep.ranks_depth, prep.ranks_feat, prep.ranks_bev,
-                              bev_feat_shape, prep.interval_starts, prep.interval_lengths,
-                              prep.plan)
-    return x.permute(0, 4, 1, 2, 3).contiguous()
+                              bev_feat_shape, prep.interval_starts, prep.interval_lengths, *extra)
+    x = x.permute(0, 4, 1, 2, 3)
+    return x if cl else x.contiguous()
 
 
 def lift_classify_prepared(depth, pix, prep, Q, prompt_class, grid_zyx, free_label=17):

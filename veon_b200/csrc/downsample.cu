@@ -96,6 +96,82 @@ k_maxdown2_bwd(const float* __restrict__ in, const float* __restrict__ out,
   }
 }
 
+// ---- channels-last volumes: in [B][Z][Y][X][C], out [B][Z/2][Y/2][X/2][C] ----------------------
+// A thread owns one output element (b, zo, yo, xo, c); consecutive threads are consecutive
+// channels, so each of its eight loads is a full coalesced line across the warp.  The same
+// reduction tree, NaN rule and first-arg-max order (dz, dy, dx) as the channels-first kernels.
+__device__ __forceinline__ void cl_block(int64_t e, int C, int Zh, int Yh, int Xh, int Y, int X,
+                                         int64_t& ibase, int64_t step[4]) {
+  const int64_t vo = e / C;
+  const int c = (int)(e - vo * C);
+  uint32_t r = (uint32_t)vo;   // output voxels < 2^32 (checked by the launcher)
+  const int xo = (int)(r % (uint32_t)Xh);
+  r /= (uint32_t)Xh;
+  const int yo = (int)(r % (uint32_t)Yh);
+  r /= (uint32_t)Yh;
+  const int zo = (int)(r % (uint32_t)Zh);
+  const int64_t b = r / (uint32_t)Zh;
+  const int64_t row = (int64_t)X * C;   // one y step
+  ibase = (((b * (2 * Zh) + 2 * zo) * Y + 2 * yo) * (int64_t)X + 2 * xo) * C + c;
+  step[0] = 0;
+  step[1] = row;
+  step[2] = (int64_t)Y * row;
+  step[3] = (int64_t)Y * row + row;
+}
+
+__global__ void __launch_bounds__(256)
+k_maxdown2_cl_fwd(const float* __restrict__ in, int64_t n_out, int C, int Zh, int Yh, int Xh, int Y,
+                  int X, float* __restrict__ out) {
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n_out;
+       e += (int64_t)gridDim.x * blockDim.x) {
+    int64_t ib, st[4];
+    cl_block(e, C, Zh, Yh, Xh, Y, X, ib, st);
+    float a[4][2];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      a[k][0] = __ldcs(in + ib + st[k]);
+      a[k][1] = __ldcs(in + ib + st[k] + C);
+    }
+    out[e] = max_nan(max_nan(max_nan(a[0][0], a[0][1]), max_nan(a[1][0], a[1][1])),
+                     max_nan(max_nan(a[2][0], a[2][1]), max_nan(a[3][0], a[3][1])));
+  }
+}
+
+__global__ void __launch_bounds__(256)
+k_maxdown2_cl_bwd(const float* __restrict__ in, const float* __restrict__ out,
+                  const float* __restrict__ grad_out, int64_t n_out, int C, int Zh, int Yh, int Xh,
+                  int Y, int X, float* __restrict__ grad_in) {
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n_out;
+       e += (int64_t)gridDim.x * blockDim.x) {
+    int64_t ib, st[4];
+    cl_block(e, C, Zh, Yh, Xh, Y, X, ib, st);
+    float v[4][2];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      v[k][0] = __ldcs(in + ib + st[k]);
+      v[k][1] = __ldcs(in + ib + st[k] + C);
+    }
+    const float m = out[e], g = grad_out[e];
+    bool open = true;   // the whole gradient to the FIRST maximum in (dz, dy, dx) order
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+#pragma unroll
+      for (int dx = 0; dx < 2; ++dx) {
+        const bool hit = open && is_max(v[k][dx], m);
+        open = open && !is_max(v[k][dx], m);
+        st_stream(grad_in + ib + st[k] + dx * C, hit ? g : 0.f);
+      }
+    }
+  }
+}
+
+static int check_cl(const void* a, const void* b, int B, int C, int Z, int Y, int X) {
+  if (!a || !b || B <= 0 || C <= 0 || Z <= 0 || Y <= 0 || X <= 0) return VEON_E_BADARG;
+  if ((Z & 1) || (Y & 1) || (X & 1)) return VEON_E_UNSUPPORTED;
+  if ((int64_t)B * (Z / 2) * (Y / 2) * (X / 2) > 0xffffffffLL) return VEON_E_RANGE;
+  return 0;
+}
+
 static int check(const void* a, const void* b, int64_t BC, int Z, int Y, int X) {
   if (!a || !b || BC <= 0 || Z <= 0 || Y <= 0 || X <= 0) return VEON_E_BADARG;
   if ((Z & 1) || (Y & 1) || (X & 3) || ((uintptr_t)a & 15) || ((uintptr_t)b & 7))
@@ -146,6 +222,34 @@ extern "C" int veon_maxdown2_bwd(const float* in, const float* out, const float*
   if (blocks > 148 * 64) blocks = 148 * 64;
   k_maxdown2_bwd<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(
       in, out, grad_out, n_quads, Z / 2, Y / 2, X / 4, Y, X, grad_in);
+  VEON_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int veon_maxdown2_cl_fwd(const float* in, int B, int C, int Z, int Y, int X, float* out,
+                                    void* stream_) {
+  int rc = check_cl(in, out, B, C, Z, Y, X);
+  if (rc) return rc;
+  const int64_t n_out = (int64_t)B * (Z / 2) * (Y / 2) * (X / 2) * C;
+  int64_t blocks = ceil_div64(n_out, 256);
+  if (blocks > 148 * 64) blocks = 148 * 64;
+  k_maxdown2_cl_fwd<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(
+      in, n_out, C, Z / 2, Y / 2, X / 2, Y, X, out);
+  VEON_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int veon_maxdown2_cl_bwd(const float* in, const float* out, const float* grad_out,
+                                    int B, int C, int Z, int Y, int X, float* grad_in,
+                                    void* stream_) {
+  int rc = check_cl(in, out, B, C, Z, Y, X);
+  if (rc) return rc;
+  if (!grad_out || !grad_in) return VEON_E_BADARG;
+  const int64_t n_out = (int64_t)B * (Z / 2) * (Y / 2) * (X / 2) * C;
+  int64_t blocks = ceil_div64(n_out, 256);
+  if (blocks > 148 * 64) blocks = 148 * 64;
+  k_maxdown2_cl_bwd<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(
+      in, out, grad_out, n_out, C, Z / 2, Y / 2, X / 2, Y, X, grad_in);
   VEON_LAUNCH_CHECK();
   return 0;
 }

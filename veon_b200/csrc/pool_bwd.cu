@@ -23,6 +23,8 @@
 //                 densely (zeros for dropped points), so no memset either.
 // Every output element has exactly one writer and a fixed summation order
 // (ascending depth bin) => bitwise run-to-run deterministic.
+// A channels-last out_grad [B,Z,Y,X,C] already holds every occupied voxel's gradient as one
+// contiguous row: k_bwd_pixels<KCH, true> reads those rows in place (no row pass, no scratch).
 #include "common.cuh"
 
 namespace veon {
@@ -391,17 +393,22 @@ __device__ __forceinline__ float reduce_many(float (&d)[U], int lane, int& which
 // one warp: feature pixel `pix`; wsm = 4*D floats of per-warp shared memory.
 // COHERENT: true when `rows` was written earlier in the SAME kernel (fused path): the
 // read-only (.nc) path may then not be used.
-template <int KCH, bool COHERENT>
+// CL: `rows` is a channels-last out_grad [B*V, C] itself; a kept point's row is that of its
+// voxel, ranks_bev[interval_starts[interval]] (only intervals a kept point names are read, so a
+// capacity-sized interval_starts is never read past the device-side interval count).
+template <int KCH, bool COHERENT, bool CL = false>
 __device__ __forceinline__ void pixel_warp(float* wsm, int lane, const float* __restrict__ rows,
                                            const float* __restrict__ depth,
                                            const float* __restrict__ feat,
                                            const int32_t* __restrict__ point_interval,
+                                           const int32_t* __restrict__ ranks_bev,
+                                           const int32_t* __restrict__ interval_starts,
                                            int64_t pix, int D, int HW, int C,
                                            float* __restrict__ depth_grad,
                                            float* __restrict__ feat_grad) {
   constexpr int CC = 32 * KCH;
   constexpr int U = (KCH <= 2) ? 8 : 4;  // gradient rows in flight per warp
-  // per warp: dots[D] | dep[D] | iis[D] | kd[D]
+  // per warp: dots[D] | dep[D] | iis[D] (row index: interval, CL: voxel) | kd[D]
   float* dots = wsm;
   float* dep = dots + D;
   int* iis = reinterpret_cast<int*>(dep + D);
@@ -418,6 +425,7 @@ __device__ __forceinline__ void pixel_warp(float* wsm, int lane, const float* __
     if (d < D) {
       ii = __ldg(point_interval + pix * D + d);
       dv = __ldg(depth + dbase + (int64_t)d * HW);
+      if (CL && ii >= 0) ii = __ldg(ranks_bev + __ldg(interval_starts + ii));
       dots[d] = 0.f;
     }
     const uint32_t m = __ballot_sync(0xffffffffu, ii >= 0);
@@ -481,18 +489,22 @@ __device__ __forceinline__ void pixel_warp(float* wsm, int lane, const float* __
   for (int d = lane; d < D; d += 32) depth_grad[dbase + (int64_t)d * HW] = dots[d];
 }
 
-template <int KCH>
-__global__ void __launch_bounds__(kBwdWarps * 32)
+// CL: the single-pass channels-last backward (rows = out_grad [B,Z,Y,X,C], no row pass).  (Its
+// KCH = 8 instance spills 24 bytes at the register count ptxas picks on its own; the minimum of
+// one CTA per SM lets it keep everything in registers.)
+template <int KCH, bool CL = false>
+__global__ void __launch_bounds__(kBwdWarps * 32, CL ? 1 : 0)
 k_bwd_pixels(const float* __restrict__ rows, const float* __restrict__ depth,
              const float* __restrict__ feat, const int32_t* __restrict__ point_interval,
+             const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ interval_starts,
              int64_t pix_begin, int64_t pix_end, int D, int HW, int C,
              float* __restrict__ depth_grad, float* __restrict__ feat_grad) {
   extern __shared__ float smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t pix = pix_begin + (int64_t)blockIdx.x * kBwdWarps + warp;
   if (pix >= pix_end) return;
-  pixel_warp<KCH, false>(smem + (size_t)warp * 4 * D, lane, rows, depth, feat, point_interval, pix,
-                         D, HW, C, depth_grad, feat_grad);
+  pixel_warp<KCH, false, CL>(smem + (size_t)warp * 4 * D, lane, rows, depth, feat, point_interval,
+                             ranks_bev, interval_starts, pix, D, HW, C, depth_grad, feat_grad);
 }
 
 // (Round 2 measured a single-launch variant of this -- one persistent cooperative kernel whose row
@@ -542,9 +554,10 @@ static int launch_rows(const float* out_grad, const int32_t* tile_istart, const 
   return 0;
 }
 
-template <int KCH>
+template <int KCH, bool CL>
 static int launch_pixels(const float* rows, const float* depth, const float* feat,
-                         const int32_t* point_interval, int64_t pix_begin, int64_t pix_end,
+                         const int32_t* point_interval, const int32_t* ranks_bev,
+                         const int32_t* interval_starts, int64_t pix_begin, int64_t pix_end,
                          int D, int HW, int C, float* depth_grad, float* feat_grad,
                          cudaStream_t stream) {
   const size_t smem = sizeof(float) * kBwdWarps * 4 * (size_t)D;
@@ -553,28 +566,34 @@ static int launch_pixels(const float* rows, const float* depth, const float* fea
   const int dev = current_device();
   if (attr_smem[dev] == 0) attr_smem[dev] = 48 * 1024;
   if (smem > attr_smem[dev]) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_pixels<KCH>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_pixels<KCH, CL>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_smem[dev] = smem;
   }
   const int64_t blocks = ceil_div64(pix_end - pix_begin, kBwdWarps);
   if (blocks <= 0) return 0;
   if (blocks > 0x7fffffffLL) return VEON_E_RANGE;
-  k_bwd_pixels<KCH><<<(unsigned)blocks, kBwdWarps * 32, smem, stream>>>(
-      rows, depth, feat, point_interval, pix_begin, pix_end, D, HW, C, depth_grad, feat_grad);
+  k_bwd_pixels<KCH, CL><<<(unsigned)blocks, kBwdWarps * 32, smem, stream>>>(
+      rows, depth, feat, point_interval, ranks_bev, interval_starts, pix_begin, pix_end, D, HW, C,
+      depth_grad, feat_grad);
   VEON_LAUNCH_CHECK();
   return 0;
 }
 
+// ranks_bev / interval_starts: the channels-last pass (rows = out_grad), else NULL
+template <bool CL = false>
 static int pixel_pass(int pk, const float* rows, const float* depth, const float* feat,
                       const int32_t* point_interval, int64_t pixels, int D, int HW, int C,
-                      float* depth_grad, float* feat_grad, cudaStream_t stream) {
+                      float* depth_grad, float* feat_grad, cudaStream_t stream,
+                      const int32_t* ranks_bev = nullptr, const int32_t* interval_starts = nullptr) {
+#define VEON_PIX(K_) launch_pixels<K_, CL>(rows, depth, feat, point_interval, ranks_bev, interval_starts, 0, pixels, D, HW, C, depth_grad, feat_grad, stream)
   switch (pk) {
-    case 1: return launch_pixels<1>(rows, depth, feat, point_interval, 0, pixels, D, HW, C, depth_grad, feat_grad, stream);
-    case 2: return launch_pixels<2>(rows, depth, feat, point_interval, 0, pixels, D, HW, C, depth_grad, feat_grad, stream);
-    case 4: return launch_pixels<4>(rows, depth, feat, point_interval, 0, pixels, D, HW, C, depth_grad, feat_grad, stream);
-    default: return launch_pixels<8>(rows, depth, feat, point_interval, 0, pixels, D, HW, C, depth_grad, feat_grad, stream);
+    case 1: return VEON_PIX(1);
+    case 2: return VEON_PIX(2);
+    case 4: return VEON_PIX(4);
+    default: return VEON_PIX(8);
   }
+#undef VEON_PIX
 }
 
 }  // namespace veon
@@ -614,6 +633,24 @@ extern "C" int veon_bev_pool_v2_bwd_planar(
   if (rc) return rc;
   return pixel_pass(pk, rows_ws, depth, feat, point_interval, B * pix_per_sample, D, HW, C,
                     depth_grad, feat_grad, stream);
+}
+
+// Single pass for a channels-last out_grad [B,Z,Y,X,C]: its occupied rows are already contiguous,
+// so the pixel pass reads them in place -- no row pass, no scratch.  Same rows, same order of
+// operations: the same bits as veon_bev_pool_v2_bwd_planar on the channels-first copy.
+extern "C" int veon_bev_pool_v2_bwd_planar_cl(
+    const float* out_grad, const float* depth, const float* feat, const int32_t* ranks_bev,
+    const int32_t* interval_starts, const int32_t* point_interval, int B, int N, int D, int H,
+    int W, int C, int64_t V, float* depth_grad, float* feat_grad, void* stream_) {
+  if (!out_grad || !depth || !feat || !ranks_bev || !interval_starts || !point_interval ||
+      !depth_grad || !feat_grad || B <= 0 || N <= 0 || D <= 0 || H <= 0 || W <= 0 || C <= 0 ||
+      V <= 0)
+    return VEON_E_BADARG;
+  if ((int64_t)B * V > 0x7fffffffLL) return VEON_E_RANGE;
+  const int pk = C <= 32 ? 1 : (C <= 64 ? 2 : (C <= 256 ? 4 : 8));
+  return pixel_pass<true>(pk, out_grad, depth, feat, point_interval, (int64_t)B * N * H * W, D,
+                          H * W, C, depth_grad, feat_grad, (cudaStream_t)stream_, ranks_bev,
+                          interval_starts);
 }
 
 extern "C" int veon_bev_pool_v2_bwd_planar_ds(

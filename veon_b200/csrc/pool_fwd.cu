@@ -27,6 +27,8 @@
 //   k_pool_fwd_narrow  C <= 32 (C % 4 == 0): a LANE per voxel instead of a lane per channel, all
 //                      channels of the voxel in registers, same fma order; heavy grid first
 //   k_pool_ds_fwd      opt-in: pooling fused with the neck's 2x2x2 max-downsample
+// The first three also write channels-last volumes out[B,Z,Y,X,C] (template flag CL,
+// veon_bev_pool_v2_fwd_planar_cl): same sums, rows instead of channel planes.
 #include "common.cuh"
 #include "pool_fwd.cuh"
 
@@ -68,6 +70,26 @@ __device__ __forceinline__ void cp_async_wait_dist() {
   asm volatile("cp.async.wait_group %0;" ::"n"(kDist - 1) : "memory");
 }
 
+// Channels-last zeros: voxels [va, vb) of the tile whose first voxel has the global index g0,
+// channels [c0, c0 + cw) of each row.  Whole rows are one contiguous span (16-byte stores when
+// aligned); a channel chunk of a row is one span per voxel.  Warp-wide.
+__device__ __forceinline__ void zero_rows_cl(float* __restrict__ out, int64_t g0, int va, int vb,
+                                             int c0, int cw, int C, int lane) {
+  auto span = [&](float* p, int64_t n) {
+    if ((((uintptr_t)p | (uintptr_t)(n * 4)) & 15) == 0) {
+      for (int64_t i = 4 * lane; i < n; i += 128) st_stream4(p + i, make_float4(0.f, 0.f, 0.f, 0.f));
+    } else {
+      for (int64_t i = lane; i < n; i += 32) st_stream(p + i, 0.f);
+    }
+  };
+  if (va >= vb) return;
+  if (cw == C) {
+    span(out + (g0 + va) * C, (int64_t)(vb - va) * C);
+  } else {
+    for (int v = va; v < vb; ++v) span(out + (g0 + v) * C + c0, cw);
+  }
+}
+
 // Persistent: every warp strides over (tile, channel-chunk) items.
 //  * index prefetch: tile bounds -> rank triple -> depth value run 3 / 2 / 1 x kDist
 //    items ahead as 4-byte cp.async copies into a per-warp ring (no registers held;
@@ -90,7 +112,13 @@ __device__ __forceinline__ void cp_async_wait_dist() {
 // LOOPC (rows wider than one chunk): an item is a whole TILE and the channel chunks are looped
 // inside it -- the index work (ring, fix-up, the records of the points past the first 32, kept
 // in `ext`) is done once per tile instead of once per (tile, chunk).
-template <int KCH, bool FULLC, bool LOOPC = false>
+// CL: channels-last output out[B,Z,Y,X,C].  The shared tile is then ROW-major, [voxel][CC + 4]:
+// a finished voxel sum (lanes = channels) is one conflict-free row store, and the write-out
+// moves the tile's rows -- one contiguous 32 * C * 4-byte block when a chunk holds every
+// channel -- with 16-byte loads and stores (vec_ok: C % 4 == 0 and a 16-byte aligned volume).
+// Nothing is transposed.  (Storing the rows straight from the registers, with zeros for the
+// empty voxels between them, was measured at 578 us at C2: short scattered stores.)
+template <int KCH, bool FULLC, bool LOOPC = false, bool CL = false>
 __global__ void __launch_bounds__(kFwdWarps * 32)
 k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
            const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
@@ -100,7 +128,8 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
            uint32_t loop_chunks) {
   constexpr int CC = 32 * KCH;
   constexpr int U = (KCH <= 2) ? 16 : 8;  // feature rows in flight per warp
-  constexpr int kTileFloats = CC * kRowPitch;
+  constexpr int kClPitch = CC + 4;   // CL: row pitch of the [voxel][channel] tile
+  constexpr int kTileFloats = CL ? kTileVoxels * kClPitch : CC * kRowPitch;
   // records of the points past the first 32 of a tile (a tile of the main grid has fewer points
   // than the plan's heavy threshold)
   constexpr int kExtInts = LOOPC ? ((kHeavyDefaultThreshold + 31) / 32 - 1) * 128 : 0;
@@ -212,8 +241,15 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
     const uint32_t b = (uint32_t)h.w >> 16;
     const bool fast = vec_ok && (whole_tiles || (uint32_t)g0 - b * Vu + kTileVoxels <= Vu);
     const uint32_t n_loop = LOOPC ? loop_chunks : 1u;
+    // CL: voxels of this tile inside the volume (a ragged sample end has fewer than 32)
+    const int v_end = CL ? (int)min((uint32_t)kTileVoxels, Vu - ((uint32_t)g0 - b * Vu)) : 0;
 
-    if (e0 <= s0 && fast) {  // empty tile
+    if (CL && e0 <= s0) {  // empty tile
+      const int c_lo = LOOPC ? 0 : (h.w & 0xffff) * CC;
+      zero_rows_cl(out, g0, 0, v_end, c_lo, LOOPC ? C : min(CC, C - c_lo), C, lane);
+      continue;
+    }
+    if (!CL && e0 <= s0 && fast) {  // empty tile
       const int c_lo = LOOPC ? 0 : (h.w & 0xffff) * CC;
       const int c_hi = LOOPC ? C : min(c_lo + CC, C);
       float* o = out + (int64_t)(b * (uint32_t)(C - 1) + (uint32_t)(c_lo + r)) * V + g0 + q4;
@@ -271,6 +307,14 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
       float acc[KCH];
       int acc_vl = -1;
       const bool full_chunk = FULLC || (cmax == CC);
+      // one finished voxel into the tile: CL row acc_vl, else column acc_vl
+      auto flush = [&]() {
+#pragma unroll
+        for (int k = 0; k < KCH; ++k) {
+          if constexpr (CL) tile[acc_vl * kClPitch + lane + 32 * k] = acc[k];
+          else tlane[32 * k * kRowPitch + acc_vl] = acc[k];
+        }
+      };
       int blk = 0;
       for (int32_t base = s0; base < e0; base += 32, ++blk) {
         const int cnt = min(32, e0 - base);
@@ -316,10 +360,7 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
                 if (j0 + u < cnt) {
                   const float dj = __int_as_float(p[u].w);
                   if (p[u].z & 0x100) {  // first point of its voxel (warp-uniform)
-                    if (acc_vl >= 0) {
-#pragma unroll
-                      for (int k = 0; k < KCH; ++k) tlane[32 * k * kRowPitch + acc_vl] = acc[k];
-                    }
+                    if (acc_vl >= 0) flush();
                     acc_vl = p[u].z & 0xff;
 #pragma unroll
                     for (int k = 0; k < KCH; ++k) acc[k] = fmaf(f[u][k], dj, 0.f);
@@ -333,11 +374,27 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
           }
         }
       }
-      if (acc_vl >= 0) {
-#pragma unroll
-        for (int k = 0; k < KCH; ++k) tlane[32 * k * kRowPitch + acc_vl] = acc[k];
-      }
+      if (acc_vl >= 0) flush();
       __syncwarp();
+
+      if constexpr (CL) {
+        // rows v < v_end, channels [cbase, cbase + cmax): element (or 16-byte piece) j of the
+        // flat [v][q] index space per lane and step, (v, q) advanced without a division
+        const int w = vec_ok ? 4 : 1;
+        const int per_row = cmax / w;
+        int v = 0, q = lane;
+        while (q >= per_row) { q -= per_row; ++v; }
+        float* const obase = out + (int64_t)g0 * C + cbase;
+        for (; v < v_end;) {
+          const float* t = tile + v * kClPitch + q * w;
+          float* o = obase + (int64_t)v * C + q * w;
+          if (vec_ok) st_stream4(o, *reinterpret_cast<const float4*>(t));
+          else st_stream(o, *t);
+          q += 32;
+          while (q >= per_row) { q -= per_row; ++v; }
+        }
+        continue;   // (the __syncwarp before the next zero-fill protects the tile reuse)
+      }
 
       // Write-out: lane (r = lane/8, q = lane%8) moves voxels 4q..4q+3 of channel
       // 4*it + r with four LDS.32 + one 16-byte streaming store.
@@ -397,7 +454,8 @@ __device__ __forceinline__ void store_label(const ClsArgs& ca, uint32_t b, uint3
   ca.labels[(((int64_t)b * ca.X + x) * ca.Y + y) * ca.Z + z] = (uint8_t)label;
 }
 
-template <int KCH, bool CLS = false>
+// CL: channels-last write-out (warp = voxel, lanes = channels), see k_pool_fwd
+template <int KCH, bool CLS = false, bool CL = false>
 __global__ void __launch_bounds__(kHeavyThreads)
 k_pool_fwd_heavy(const float* __restrict__ depth, const float* __restrict__ feat,
                  const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
@@ -525,6 +583,11 @@ k_pool_fwd_heavy(const float* __restrict__ depth, const float* __restrict__ feat
         for (int q = 0; q < ca.Q; ++q) m.push(__ldg(ca.cls + q), tile[(2 + q) * kRowPitch + lane]);
         store_label(ca, b, (uint32_t)(v0 + lane),
                     m.label(tile[lane], tile[kRowPitch + lane], ca.free_label));
+      }
+    } else if constexpr (CL) {  // rows of the empty voxels are the tile's zeros
+      for (int v = warp; v < kTileVoxels && v0 + v < V; v += kHeavyThreads / 32) {
+        float* o = out + ((int64_t)g0 + v) * C + cbase;
+        for (int c = lane; c < cmax; c += 32) st_stream(o + c, tile[c * kRowPitch + v]);
       }
     } else {  // write-out: thread (row = tid/8, q = tid%8) moves voxels 4q..4q+3 of channel row (+32j)
       const int q4 = (tid & 7) * 4;
@@ -753,7 +816,9 @@ constexpr int kNarrowHeavyMin = 512;
 // Fused lift + classify (CLS): NP passes of 4*NV channels each over the tile's points; the
 // class-merge state lives in registers between the passes (the merge is a scan over the prompt
 // rows in order), so Q + 2 <= 96 channels need no more registers than 32 do.
-template <int NV, bool CLS = false, int NP = 1>  // 16-byte pieces per pass: C = 4 * NV * NP
+// CL: channels-last output; a lane's voxel row is NV 16-byte stores and the warp's 32 rows are one
+// contiguous 32 * C * 4-byte block.
+template <int NV, bool CLS = false, int NP = 1, bool CL = false>  // 16-byte pieces per pass: C = 4 * NV * NP
 __global__ void __launch_bounds__(kNarrowWarps * 32, (NV <= 5) ? 3 : 2)
 k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ feat,
                   const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
@@ -925,6 +990,11 @@ k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ fea
           cur = head ? logit : fmaxf(cur, logit);
           cur_q = head ? q : cur_q;
         }
+      } else if constexpr (CL) {
+        float* o = out + ((int64_t)g0 + lane) * C;
+#pragma unroll
+        for (int k = 0; k < NV; ++k)
+          st_stream4(o + 4 * k, make_float4(acc[4 * k], acc[4 * k + 1], acc[4 * k + 2], acc[4 * k + 3]));
       } else {
         float* o = out + (int64_t)b * C * V + v0 + lane;
 #pragma unroll
@@ -945,17 +1015,17 @@ k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ fea
 
 
 // ---- launchers ---------------------------------------------------------------------------------
-template <int KCH, bool CLS = false>
+template <int KCH, bool CLS = false, bool CL = false>
 static int heavy_config(size_t& smem, int& ctas_per_sm) {
   constexpr int CC = 32 * KCH;
   smem = sizeof(float) * (kHeavyChunk * CC + CC * kRowPitch + 2 * kHeavyChunk + 128);
   static int cached[kMaxDevices] = {};
   const int dev = current_device();
   if (cached[dev] == 0) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd_heavy<KCH, CLS>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd_heavy<KCH, CLS, CL>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_heavy<KCH, CLS>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_heavy<KCH, CLS, CL>,
                                                                 kHeavyThreads, smem));
     cached[dev] = n < 1 ? 1 : (n > 8 ? 8 : n);
   }
@@ -964,7 +1034,7 @@ static int heavy_config(size_t& smem, int& ctas_per_sm) {
 }
 
 // the heavy-tile grid; pdl: queued as a programmatic dependent of the previous launch (joins it)
-template <int KCH, bool CLS = false>
+template <int KCH, bool CLS = false, bool CL = false>
 static int launch_heavy(const float* depth, const float* feat, const int32_t* rd, const int32_t* rf,
                         const int32_t* rb, const int32_t* tile_start, const int32_t* heavy,
                         int64_t heavy_ints, int B, int C, int64_t V, float* out, bool pdl,
@@ -972,7 +1042,7 @@ static int launch_heavy(const float* depth, const float* feat, const int32_t* rd
   constexpr int CC = 32 * KCH;
   size_t smem;
   int per_sm;
-  int rc = heavy_config<KCH, CLS>(smem, per_sm);
+  int rc = heavy_config<KCH, CLS, CL>(smem, per_sm);
   if (rc) return rc;
   const int64_t tps = ceil_div64(V, kTileVoxels);
   const int n_chunks = (C + CC - 1) / CC;
@@ -982,11 +1052,11 @@ static int launch_heavy(const float* depth, const float* feat, const int32_t* rd
   if (blocks > (int64_t)per_sm * sm_count()) blocks = (int64_t)per_sm * sm_count();
   if (blocks <= 0) return 0;
   if (pdl) {
-    VEON_CUDA_TRY(launch_pdl(k_pool_fwd_heavy<KCH, CLS>, dim3((unsigned)blocks), dim3(kHeavyThreads),
+    VEON_CUDA_TRY(launch_pdl(k_pool_fwd_heavy<KCH, CLS, CL>, dim3((unsigned)blocks), dim3(kHeavyThreads),
                              smem, stream, depth, feat, rd, rf, rb, tile_start, heavy, heavy_cap,
                              (uint32_t)tps, V, C, (uint32_t)n_chunks, vec_ok, out, 1, min_points, ca));
   } else {
-    k_pool_fwd_heavy<KCH, CLS><<<(unsigned)blocks, kHeavyThreads, smem, stream>>>(
+    k_pool_fwd_heavy<KCH, CLS, CL><<<(unsigned)blocks, kHeavyThreads, smem, stream>>>(
         depth, feat, rd, rf, rb, tile_start, heavy, heavy_cap, (uint32_t)tps, V, C,
         (uint32_t)n_chunks, vec_ok, out, 0, min_points, ca);
   }
@@ -1007,21 +1077,22 @@ int launch_heavy_behind(const float* depth, const float* feat, const int32_t* rd
 }
 
 // general route: k_pool_fwd over every (tile, channel chunk), the heavy tiles queued behind it
-template <int KCH, bool FULLC, bool LOOPC>
+template <int KCH, bool FULLC, bool LOOPC, bool CL>
 static int launch_fwd_impl(const float* depth, const float* feat, const int32_t* rd,
                            const int32_t* rf, const int32_t* rb, const int32_t* tile_start,
                            const int32_t* heavy, int64_t heavy_ints, int B, int C, int64_t V,
                            bool feat_rows_fit_32bit, float* out, cudaStream_t stream) {
   constexpr int CC = 32 * KCH;
   constexpr int kExtInts = LOOPC ? ((kHeavyDefaultThreshold + 31) / 32 - 1) * 128 : 0;
-  const size_t smem = sizeof(float) * kFwdWarps * (CC * kRowPitch + kRingSlots * kSlotInts + kExtInts);
+  const size_t smem = sizeof(float) * kFwdWarps *
+                      ((CL ? kTileVoxels * (CC + 4) : CC * kRowPitch) + kRingSlots * kSlotInts + kExtInts);
   static int ctas_per_sm[kMaxDevices] = {};
   const int dev = current_device();
   if (ctas_per_sm[dev] == 0) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd<KCH, FULLC, LOOPC>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd<KCH, FULLC, LOOPC, CL>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd<KCH, FULLC, LOOPC>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd<KCH, FULLC, LOOPC, CL>,
                                                                 kFwdWarps * 32, smem));
     ctas_per_sm[dev] = n < 1 ? 1 : n;
   }
@@ -1029,14 +1100,16 @@ static int launch_fwd_impl(const float* depth, const float* feat, const int32_t*
   const int n_chunks = (C + CC - 1) / CC;
   if (n_tiles * n_chunks > 0x7fffffffLL || (int64_t)B * V > 0x7fffffffLL) return VEON_E_RANGE;
   if (!feat_rows_fit_32bit) return VEON_E_RANGE;   // the gather uses 32-bit byte offsets
-  const int vec_ok = ((V & 3) == 0) && (((uintptr_t)out & 15) == 0);
+  // 16-byte stores: channel planes of 4-voxel pieces (channels-first) or rows of 4-channel
+  // pieces (channels-last)
+  const int vec_ok = (((CL ? C : V) & 3) == 0) && (((uintptr_t)out & 15) == 0);
   const int64_t n_items = LOOPC ? n_tiles : n_tiles * n_chunks;   // LOOPC: chunks looped per tile
   int64_t blocks = ceil_div64(n_items, kFwdWarps);
   const int64_t resident = (int64_t)ctas_per_sm[dev] * sm_count();  // persistent grid
   if (blocks > resident) blocks = resident;
   // the heavy-tile kernel stages feature rows with 16-byte copies
   if (heavy && ((C & 3) != 0 || ((uintptr_t)feat & 15) != 0)) heavy = nullptr;
-  k_pool_fwd<KCH, FULLC, LOOPC><<<(unsigned)blocks, kFwdWarps * 32, smem, stream>>>(
+  k_pool_fwd<KCH, FULLC, LOOPC, CL><<<(unsigned)blocks, kFwdWarps * 32, smem, stream>>>(
       depth, feat, rd, rf, rb, tile_start, heavy, (uint32_t)n_items, (uint32_t)tps,
       V, C, (uint32_t)(LOOPC ? 1 : n_chunks), vec_ok, out, (uint32_t)n_chunks);
   VEON_LAUNCH_CHECK();
@@ -1045,13 +1118,13 @@ static int launch_fwd_impl(const float* depth, const float* feat, const int32_t*
   // grid before they complete.
 #ifndef VEON_FWD_X_NOHEAVY
   if (heavy)
-    return launch_heavy<(KCH > 2 ? 2 : KCH)>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints,
+    return launch_heavy<(KCH > 2 ? 2 : KCH), false, CL>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints,
                                              B, C, V, out, true, 0, stream);
 #endif
   return 0;
 }
 
-template <int KCH>
+template <int KCH, bool CL = false>
 static int launch_fwd(const float* depth, const float* feat, const int32_t* rd,
                       const int32_t* rf, const int32_t* rb, const int32_t* tile_start,
                       const int32_t* heavy, int64_t heavy_ints, int B, int C, int64_t V,
@@ -1063,7 +1136,7 @@ static int launch_fwd(const float* depth, const float* feat, const int32_t* rd,
   const bool loopc = false;
 #endif
 #define VEON_FWD_GO(FULLC_, LOOPC_)                                                            \
-  return launch_fwd_impl<KCH, FULLC_, LOOPC_>(depth, feat, rd, rf, rb, tile_start, heavy,      \
+  return launch_fwd_impl<KCH, FULLC_, LOOPC_, CL>(depth, feat, rd, rf, rb, tile_start, heavy,      \
                                               heavy_ints, B, C, V, feat_rows_fit_32bit, out, stream)
   if (C % (32 * KCH) == 0) {
     if (loopc) VEON_FWD_GO(true, true);
@@ -1078,7 +1151,7 @@ static int launch_fwd(const float* depth, const float* feat, const int32_t* rd,
 // CTA works ~100 us on one 1 000-point tile at C3 density: behind the persistent main grid the
 // two nearly serialise, 344 vs 295 us); k_pool_fwd_narrow moves in beside it as its programmatic
 // dependent and joins it at the end
-template <int NV, bool CLS = false, int NP = 1>
+template <int NV, bool CLS = false, int NP = 1, bool CL = false>
 static int launch_fwd_narrow(const float* depth, const float* feat, const int32_t* rd,
                              const int32_t* rf, const int32_t* rb, const int32_t* tile_start,
                              const int32_t* heavy, int64_t heavy_ints, int B, int64_t V,
@@ -1090,16 +1163,16 @@ static int launch_fwd_narrow(const float* depth, const float* feat, const int32_
   const int dev = current_device();
   if (ctas_per_sm[dev] == 0) {
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_narrow<NV, CLS, NP>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_narrow<NV, CLS, NP, CL>,
                                                                 kNarrowWarps * 32, 0));
     ctas_per_sm[dev] = n < 1 ? 1 : n;
   }
   int64_t blocks = ceil_div64(n_tiles, kNarrowWarps);
   if (blocks > (int64_t)ctas_per_sm[dev] * sm_count()) blocks = (int64_t)ctas_per_sm[dev] * sm_count();
-  int rc = launch_heavy<KCH, CLS>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C, V,
+  int rc = launch_heavy<KCH, CLS, CL>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C, V,
                                   out, false, kNarrowHeavyMin, stream, ca);
   if (rc) return rc;
-  VEON_CUDA_TRY(launch_pdl(k_pool_fwd_narrow<NV, CLS, NP>, dim3((unsigned)blocks),
+  VEON_CUDA_TRY(launch_pdl(k_pool_fwd_narrow<NV, CLS, NP, CL>, dim3((unsigned)blocks),
                            dim3(kNarrowWarps * 32), 0, stream, depth, feat, rd, rf, rb, tile_start,
                            heavy, (uint32_t)n_tiles, (uint32_t)tps, V, out, 0u, kNarrowHeavyMin, 1,
                            ca));
@@ -1168,6 +1241,43 @@ extern "C" int veon_bev_pool_v2_fwd_planar(const float* depth, const float* feat
                          tile_heavy_ints, B, C, V, fit32, out, stream);
   return launch_fwd<2>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy,
                        tile_heavy_ints, B, C, V, fit32, out, stream);
+}
+
+// Channels-last volume out[B,Z,Y,X,C]: the same kernels with a row write-out (the streaming
+// two-role kernel is channels-first only).  Same sums, same bits, another layout.
+extern "C" int veon_bev_pool_v2_fwd_planar_cl(const float* depth, const float* feat,
+                                              const int32_t* ranks_depth,
+                                              const int32_t* ranks_feat,
+                                              const int32_t* ranks_bev,
+                                              const int32_t* tile_start,
+                                              const int32_t* tile_heavy, int64_t tile_heavy_ints,
+                                              int B, int C, int64_t V, int64_t n_feat_rows,
+                                              float* out, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  if (!depth || !feat || !ranks_depth || !ranks_feat || !ranks_bev || !tile_start || !out ||
+      B <= 0 || C <= 0 || V <= 0 || n_feat_rows <= 0 || (tile_heavy && tile_heavy_ints < 2))
+    return VEON_E_BADARG;
+  const bool fit32 = n_feat_rows * (int64_t)C <= 0x3fffffffLL && B < 65536 &&
+                     (int64_t)C <= 65535LL * 32;
+  {  // narrow rows: lane-per-voxel kernel (conditions as in veon_bev_pool_v2_fwd_planar)
+    const bool ok = C <= 32 && (C & 3) == 0 && tile_heavy && fit32 && V % kTileVoxels == 0 &&
+                    (int64_t)B * V <= (1 << 24) &&
+                    (((uintptr_t)feat | (uintptr_t)out) & 15) == 0;
+    if (ok) {
+#define VEON_NARROW_CASE(NV_) case NV_: return launch_fwd_narrow<NV_, false, 1, true>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy, tile_heavy_ints, B, V, out, stream);
+      switch (C / 4) {
+        VEON_NARROW_CASE(1) VEON_NARROW_CASE(2) VEON_NARROW_CASE(3) VEON_NARROW_CASE(4)
+        VEON_NARROW_CASE(5) VEON_NARROW_CASE(6) VEON_NARROW_CASE(7) VEON_NARROW_CASE(8)
+        default: break;
+      }
+#undef VEON_NARROW_CASE
+    }
+  }
+  if (C <= 32)
+    return launch_fwd<1, true>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
+                               tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
+  return launch_fwd<2, true>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
+                             tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
 }
 
 // Fused lift + classify: pools the [gate 0, gate 1, logit 0..Q-1, pad] rows and ends every tile

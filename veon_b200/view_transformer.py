@@ -32,12 +32,21 @@ class LSSViewTransformer(nn.Module):
     that an input with no point inside the grid yields an all-zero volume of
     the regular shape instead of the reference's warning + dummy tensor
     (:179-189).
+
+    Extra: `memory_format` -- torch.channels_last_3d makes every pooling route
+    (fused geometry, voxel_pooling_v2, accelerate) return the same values stored
+    channels-last, written that way by the pooling kernels (the layout a
+    channels-last 3D encoder wants; its channels-last gradient is consumed
+    without a copy).  The default, torch.contiguous_format, is the reference's.
     """
 
     def __init__(self, grid_config, input_size, downsample=16, in_channels=512,
                  out_channels=64, accelerate=False, sid=False, collapse_z=True,
-                 sync_free=False, rank_cache=0, depth_eps=None):
+                 sync_free=False, rank_cache=0, depth_eps=None,
+                 memory_format=torch.contiguous_format):
         super().__init__()
+        _bp._channels_last(memory_format)     # ValueError for anything but the two formats
+        self.memory_format = memory_format
         self.grid_config = grid_config
         self.downsample = downsample
         self.create_grid_infos(**grid_config)
@@ -248,7 +257,7 @@ class LSSViewTransformer(nn.Module):
         prep.plan.sync_free = self.sync_free   # the backward then sizes its scratch by a bound
         if self.prepared_hook is not None:
             self.prepared_hook()               # see __init__: lets a caller time its transfers
-        bev_feat = _bp.pool_prepared(depth, feat_last, prep, shape)
+        bev_feat = _bp.pool_prepared(depth, feat_last, prep, shape, self.memory_format)
         if not self.sync_free and prep.plan.n_intervals == 0:
             return self._no_points_dummy(feat)
         if self.collapse_z:
@@ -278,7 +287,8 @@ class LSSViewTransformer(nn.Module):
             depth = depth.view(B, N, self.D, H, W)
             bev_feat = _bp.bev_pool_v2(depth, feat, self.ranks_depth, self.ranks_feat,
                                        self.ranks_bev, self._bev_shape(depth, feat.shape[-1]),
-                                       self.interval_starts, self.interval_lengths)
+                                       self.interval_starts, self.interval_lengths,
+                                       memory_format=self.memory_format)
             bev_feat = bev_feat.squeeze(2)
         elif self.fuse_geometry and input[1].is_cuda:
             # get_lidar_coor folded into the index preparation: same ranks, no coor tensor
@@ -309,7 +319,10 @@ class LSSViewTransformer(nn.Module):
 class LSSViewTransformerRaw(LSSViewTransformer):
     """VEON's neck entry (reference view_transformer_raw.py:537-555): takes
     ready-made features and a depth distribution, lifts, then (use_ds)
-    max-pools the volume 2x2x2."""
+    max-pools the volume 2x2x2.  With memory_format=torch.channels_last_3d it
+    pools channels-last and reduces with the channels-last 2x2x2 kernels (the
+    fused `fuse_ds` kernel and the one-node PoolMaxDown training route are
+    channels-first only and are not taken); the result is channels-last-3d."""
 
     def __init__(self, *args, use_ds=True, ds=(2, 2, 2), fuse_ds=False, **kwargs):
         kwargs.setdefault("collapse_z", False)
@@ -376,6 +389,7 @@ class LSSViewTransformerRaw(LSSViewTransformer):
         forms the full-resolution gradient (bev_pool.PoolMaxDown).  None -> plain route."""
         tran_feat = input[0]
         if (not self.use_ds or self.ds != (2, 2, 2) or self.accelerate or self.collapse_z
+                or self.memory_format is not torch.contiguous_format
                 or not tran_feat.is_cuda or not torch.is_grad_enabled()
                 or not (tran_feat.requires_grad or depth.requires_grad)):
             return None
@@ -400,7 +414,7 @@ class LSSViewTransformerRaw(LSSViewTransformer):
         taken: gradients wanted, cached ranks (`accelerate`), other `ds`, odd grids, ..."""
         tran_feat = input[0]
         if (not self.fuse_ds or not self.use_ds or self.ds != (2, 2, 2) or self.accelerate
-                or self.collapse_z
+                or self.collapse_z or self.memory_format is not torch.contiguous_format
                 or (torch.is_grad_enabled() and (tran_feat.requires_grad or depth.requires_grad))
                 or not tran_feat.is_cuda):
             return None
