@@ -33,7 +33,8 @@ def ptr(t, off=0):
 
 
 def reference():
-    return BP._bwd_planar(og, depth, feat, prep.ranks_bev, prep.interval_starts, plan, C)
+    return BP._pool_bwd(og.permute(0, 2, 3, 4, 1), depth, feat, prep.ranks_depth,
+                        prep.ranks_feat, prep.ranks_bev, prep.interval_starts, plan)
 
 
 want_dg, want_fg = reference()

@@ -15,7 +15,8 @@ og = torch.randn(shape, device="cuda")
 a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 for i in range(iters):
     a.record()
-    dg, fg = BP._bwd_planar(og, depth, feat, prep.ranks_bev, prep.interval_starts, prep.plan, C)
+    dg, fg = BP._pool_bwd(og.permute(0, 2, 3, 4, 1), depth, feat, prep.ranks_depth,
+                          prep.ranks_feat, prep.ranks_bev, prep.interval_starts, prep.plan)
     b.record()
 torch.cuda.synchronize()
 print("ok", float(dg.abs().sum()), float(fg.abs().sum()), f"last call {a.elapsed_time(b) * 1e3:.1f} us")

@@ -102,14 +102,16 @@ def pool_group(name, cfg, B, C, region_s, rounds, dev):
     def fwd_cf_convert():
         return fwd_cf().contiguous(memory_format=CL)
 
+    # _pool_bwd takes the gradient of the [B,Z,Y,X,C] volume QuickCumsumCuda returns
     def bwd_cf():
-        return BP._bwd_planar(g_cf, depth, feat, rb, ist, plan, C)
+        return BP._pool_bwd(g_cf.permute(0, 2, 3, 4, 1), depth, feat, rd, rf, rb, ist, plan)
 
     def bwd_cl():
-        return BP._bwd_planar_cl(g_cl, depth, feat, rb, ist, plan, C)
+        return BP._pool_bwd(g_cl, depth, feat, rd, rf, rb, ist, plan)
 
     def bwd_copy():
-        return BP._bwd_planar(g_cl_view.contiguous(), depth, feat, rb, ist, plan, C)
+        return BP._pool_bwd(g_cl_view.contiguous().permute(0, 2, 3, 4, 1), depth, feat, rd, rf,
+                            rb, ist, plan)
 
     # bit-for-bit checks at the timed sizes, outside the timed regions
     a, b = fwd_cf(), fwd_cl()

@@ -7,6 +7,8 @@ import ctypes
 import os
 from ctypes import c_char_p, c_int, c_int32, c_int64, c_size_t, c_void_p
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libveonlift.so")
 
@@ -137,3 +139,21 @@ def check(code, what):
 def float3(values):
     """[host] float32[3] argument."""
     return (ctypes.c_float * 3)(*[float(v) for v in values])
+
+
+def ptr(t):
+    """A tensor's data as a pointer argument."""
+    return ctypes.c_void_p(t.data_ptr())
+
+
+def stream_ptr(device):
+    """torch's current stream on `device` as a cudaStream_t argument."""
+    return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+def require_cuda(*tensors):
+    for t in tensors:
+        if not t.is_cuda:
+            raise RuntimeError(
+                "veon_b200 runs on CUDA tensors only (there is no CPU fallback); "
+                f"got a tensor on {t.device}")

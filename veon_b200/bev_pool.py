@@ -23,12 +23,14 @@ that way by the kernels; a channels-last gradient is consumed in place by a
 single-pass backward, whichever layout the forward produced.
 """
 import collections
+import functools
 import weakref
 import ctypes
 
 import torch
 
 from . import _lib
+from ._lib import ptr as _ptr, require_cuda as _require_cuda, stream_ptr as _stream_ptr
 
 __all__ = ["bev_pool_v2", "QuickCumsumCuda", "TRTBEVPoolv2",
            "voxel_pooling_prepare_v2", "prepare_ranks", "PreparedRanks",
@@ -48,14 +50,6 @@ def _channels_last(memory_format):
         raise ValueError("memory_format must be torch.contiguous_format or torch.channels_last_3d, "
                          f"got {memory_format!r}")
     return memory_format is torch.channels_last_3d
-
-
-def _stream_ptr(device):
-    return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-
-
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr())
 
 
 # Opt-in device timing of the library calls (bench.py / profiling only): CUDA
@@ -91,14 +85,6 @@ class _timed:
         return False
 
 
-def _require_cuda(*tensors):
-    for t in tensors:
-        if not t.is_cuda:
-            raise RuntimeError(
-                "veon_b200 runs on CUDA tensors only (there is no CPU fallback); "
-                f"got a tensor on {t.device}")
-
-
 def lidar_coor(frustum, sensor2ego, cam2imgs, post_rots, post_trans, bda):
     """get_lidar_coor (view_transformer.py:114-152) as one fused CUDA pass.
     frustum [D,H,W,3]; returns coor [B,N,D,H,W,3] float32."""
@@ -127,14 +113,19 @@ class PoolPlan:
                  "flags", "_n_intervals", "_n_points", "counts_dev", "counts_host",
                  "counts_event", "keepalive", "sync_free")
 
-    def __init__(self):
-        self.flags = 0
-        self._n_intervals = None
-        self._n_points = None
-        self.counts_dev = self.counts_host = self.counts_event = None
+    def __init__(self, tiles, heavy, point_interval, dims, V, flags=0, voxel_start=None,
+                 counts=(None, None, None), n_points=None, n_intervals=None):
+        """tiles: the [3, n_tiles + 1] start / interval-start / occupancy table; counts: the
+        (device, pinned host, event) of counts still in flight, else n_points / n_intervals."""
+        self.tile_start, self.tile_istart, self.tile_occ = tiles[0], tiles[1], tiles[2]
+        self.tile_heavy = heavy
+        self.point_interval = point_interval
+        self.voxel_start = voxel_start
+        self.dims, self.V, self.flags = dims, V, flags
+        self.counts_dev, self.counts_host, self.counts_event = counts
+        self._n_points, self._n_intervals = n_points, n_intervals
         self.keepalive = None
         self.sync_free = False
-        self.voxel_start = None
 
     def _resolve(self):
         if self._n_intervals is None:
@@ -310,11 +301,11 @@ def _prepare(coor, calib, dims, dev, grid_lower_bound, grid_interval, grid_size,
         n_tiles = lib.veon_pool_num_tiles(B, V)
         if len(_GEOMETRY_CACHE) > 64:
             _GEOMETRY_CACHE.clear()
-        geo = (None, None, None, _lib.float3(lower), _lib.float3(interval), c_size, V, ws_bytes,
-               n_tiles, lib.veon_pool_heavy_list_ints(P, n_tiles),
+        geo = (_lib.float3(lower), _lib.float3(interval), c_size, V, ws_bytes, n_tiles,
+               lib.veon_pool_heavy_list_ints(P, n_tiles),
                lib.veon_prepare_v2_voxel_start_offset(B, N, D, H, W, c_size))
         _GEOMETRY_CACHE[key] = geo
-    _, _, _, c_lower, c_interval, c_size, V, ws_bytes, n_tiles, nh, vs_off = geo
+    c_lower, c_interval, c_size, V, ws_bytes, n_tiles, nh, vs_off = geo
     with torch.cuda.device(dev):
         # one allocation for every int32 output + the kernel workspace (fewer allocator
         # round-trips per call); the pieces below are views of it
@@ -361,16 +352,11 @@ def _prepare(coor, calib, dims, dev, grid_lower_bound, grid_interval, grid_size,
         _lib.check(rc, "veon_prepare_v2")
         ev = torch.cuda.Event()
         ev.record(launch_on)
-    plan = PoolPlan()
-    plan.tile_start, plan.tile_istart, plan.tile_occ = tiles[0], tiles[1], tiles[2]
-    plan.tile_heavy = heavy
     # first point of every voxel: lives in the preparation workspace (kept alive by this view)
-    if B * V < (1 << 24) and vs_off % 4 == 0:
-        plan.voxel_start = ws[vs_off // 4: vs_off // 4 + B * V + 1]
-    plan.point_interval = point_interval if backward_tables else None
-    plan.dims = (B, N, D, H, W)
-    plan.V = V
-    plan.counts_dev, plan.counts_host, plan.counts_event = counts, counts_host, ev
+    voxel_start = (ws[vs_off // 4: vs_off // 4 + B * V + 1]
+                   if B * V < (1 << 24) and vs_off % 4 == 0 else None)
+    plan = PoolPlan(tiles, heavy, point_interval if backward_tables else None, (B, N, D, H, W), V,
+                    voxel_start=voxel_start, counts=(counts, counts_host, ev))
     _COUNTS_RING[dev.index][1][slot] = (ev, weakref.ref(plan))
     out = PreparedRanks()
     out.ranks_bev, out.ranks_depth, out.ranks_feat = ranks[0], ranks[1], ranks[2]
@@ -422,13 +408,9 @@ def _plan_for(rd, rf, rb, ist, iln, dims, V):
             B, N, D, H, W, V, _ptr(tiles[0]), _ptr(tiles[1]), _ptr(tiles[2]), _ptr(heavy),
             _ptr(point_interval), _ptr(flags), _stream_ptr(dev))
         _lib.check(rc, "veon_pool_plan_build")
-        plan = PoolPlan()
-        plan.flags = int(flags.item())  # one sync per distinct rank set
-    plan.tile_start, plan.tile_istart, plan.tile_occ = tiles[0], tiles[1], tiles[2]
-    plan.tile_heavy = heavy
-    plan.point_interval = point_interval
-    plan.dims, plan.V = dims, V
-    plan._n_points, plan._n_intervals = rd.numel(), ist.numel()
+        plan = PoolPlan(tiles, heavy, point_interval, dims, V,
+                        flags=int(flags.item()),  # one sync per distinct rank set
+                        n_points=rd.numel(), n_intervals=ist.numel())
     _remember_plan(key, plan, (rd, rf, rb, ist, iln))
     return plan
 
@@ -448,13 +430,7 @@ def pool_prepared_downsampled(depth, feat, prep, bev_feat_shape):
     lib = _lib.load()
     dev = feat.device
     depth = depth.detach().contiguous().float()
-    feat = feat.detach()
-    if (feat.dtype == torch.float32 and not feat.is_contiguous()
-            and feat.permute(0, 1, 4, 2, 3).is_contiguous()):
-        feat = _transpose_batched(feat.permute(0, 1, 4, 2, 3), feat.shape[0] * feat.shape[1],
-                                  feat.shape[4], feat.shape[2] * feat.shape[3], tuple(feat.shape))
-    else:
-        feat = feat.contiguous().float()
+    feat, _ = _feat_rows(feat.detach())
     with torch.cuda.device(dev):
         out = torch.empty((B, C, Z // 2, Y // 2, X // 2), dtype=torch.float32, device=dev)
         with _timed("pool_ds_fwd", dev):
@@ -566,14 +542,7 @@ class PoolMaxDown(torch.autograd.Function):
         B, Z, Y, X, C = (int(v) for v in bev_feat_shape)
         plan = prep.plan
         depth = depth.contiguous().float()
-        ctx.feat_channels_first = (feat.dtype == torch.float32 and not feat.is_contiguous()
-                                   and feat.permute(0, 1, 4, 2, 3).is_contiguous())
-        if ctx.feat_channels_first:
-            feat = _transpose_batched(feat.permute(0, 1, 4, 2, 3), feat.shape[0] * feat.shape[1],
-                                      feat.shape[4], feat.shape[2] * feat.shape[3],
-                                      tuple(feat.shape))
-        else:
-            feat = feat.contiguous().float()
+        feat, ctx.feat_transposed = _feat_rows(feat)
         vol = _fwd_planar(depth, feat, prep.ranks_depth, prep.ranks_feat, prep.ranks_bev, plan,
                           B, C, Z * Y * X, (B, C, Z, Y, X))
         dev = vol.device
@@ -598,23 +567,18 @@ class PoolMaxDown(torch.autograd.Function):
         C = feat.shape[-1]
         dev = feat.device
         g = grad_ds.contiguous().float()
-        n_int = plan.interval_capacity()
         _need_backward_tables(plan)
         with torch.cuda.device(dev):
             depth_grad = torch.empty_like(depth)
             feat_grad = torch.empty_like(feat)
-            rows = torch.empty(max(n_int, 1) * C, dtype=torch.float32, device=dev)
+            n_int, rows = _bwd_rows(lib, plan, C, dev)
             with _timed("pool_bwd_ds", dev):
                 rc = lib.veon_bev_pool_v2_bwd_planar_ds(
                     _ptr(g), _ptr(mask), _ptr(depth), _ptr(feat), _ptr(plan.tile_istart),
                     _ptr(plan.tile_occ), _ptr(plan.point_interval), n_int, B, N, D, H, W, C,
                     Z, Y, X, _ptr(rows), _ptr(depth_grad), _ptr(feat_grad), _stream_ptr(dev))
         _lib.check(rc, "veon_bev_pool_v2_bwd_planar_ds")
-        if ctx.feat_channels_first:
-            Bf, Nf, Hf, Wf, Cf = feat_grad.shape
-            feat_grad = _transpose_batched(feat_grad, Bf * Nf, Hf * Wf, Cf,
-                                           (Bf, Nf, Cf, Hf, Wf)).permute(0, 1, 3, 4, 2)
-        return depth_grad, feat_grad, None, None
+        return depth_grad, _feat_grad_back(feat_grad, ctx.feat_transposed), None, None
 
 
 def pool_prepared_maxdown(depth, feat, prep, bev_feat_shape):
@@ -657,6 +621,27 @@ def _transpose_batched(src, batch, R, S, out_shape):
     return dst
 
 
+def _feat_rows(feat):
+    """feat [B,N,H,W,C] as contiguous float32 rows, and whether they were transposed: the necks
+    hand over a channels-last VIEW of channels-first maps, which our own transpose kernel turns
+    into rows instead of a strided copy."""
+    if (feat.dtype == torch.float32 and not feat.is_contiguous()
+            and feat.permute(0, 1, 4, 2, 3).is_contiguous()):
+        B, N, H, W, C = feat.shape
+        return _transpose_batched(feat.permute(0, 1, 4, 2, 3), B * N, C, H * W,
+                                  (B, N, H, W, C)), True
+    return feat.contiguous().float(), False
+
+
+def _feat_grad_back(feat_grad, transposed):
+    """The gradient of `_feat_rows`' rows, transposed back to channels-first storage (as a
+    [B,N,H,W,C] view) when the rows were transposed."""
+    if not transposed:
+        return feat_grad
+    B, N, H, W, C = feat_grad.shape
+    return _transpose_batched(feat_grad, B * N, H * W, C, (B, N, C, H, W)).permute(0, 1, 3, 4, 2)
+
+
 # Scratch of the streaming forward (control block + the L2-resident ring of compact rows):
 # one buffer per (device, stream) -- calls on one stream are ordered, calls on different
 # streams may overlap and must not share it.  FWD_RING_BYTES: None = the library's default size
@@ -676,34 +661,34 @@ def _fwd_workspace(lib, dev, B, C, V):
     return ws
 
 
-def _fwd_planar(depth, feat, rd, rf, rb, plan, B, C, V, shape5):
+def _fwd_planar(depth, feat, rd, rf, rb, plan, B, C, V, shape5, channels_last=False):
+    """Planar forward of a valid plan into a new volume `shape5`: [B,C,Z,Y,X], or [B,Z,Y,X,C]
+    with channels_last (the streaming kernel and its workspace are channels-first only)."""
     lib = _lib.load()
     dev = feat.device
     with torch.cuda.device(dev):
-        out = torch.empty(shape5, dtype=torch.float32, device=dev)  # [B,C,Z,Y,X]
-        ws = _fwd_workspace(lib, dev, B, C, V)
-        with _timed("pool_fwd", dev):
-            rc = lib.veon_bev_pool_v2_fwd_planar(
-                _ptr(depth), _ptr(feat), _ptr(rd), _ptr(rf), _ptr(rb), _ptr(plan.tile_start),
-                _ptr(plan.tile_istart), _ptr(plan.tile_occ),
-                _ptr(plan.tile_heavy), plan.tile_heavy.numel(),
-                B, C, V, feat.numel() // C, _ptr(out), _ptr(ws), ws.numel(), _stream_ptr(dev))
-    _lib.check(rc, "veon_bev_pool_v2_fwd_planar")
+        out = torch.empty(shape5, dtype=torch.float32, device=dev)
+        if channels_last:
+            what = "veon_bev_pool_v2_fwd_planar_cl"
+            with _timed("pool_fwd_cl", dev):
+                rc = lib.veon_bev_pool_v2_fwd_planar_cl(
+                    _ptr(depth), _ptr(feat), _ptr(rd), _ptr(rf), _ptr(rb), _ptr(plan.tile_start),
+                    _ptr(plan.tile_heavy), plan.tile_heavy.numel(), B, C, V, feat.numel() // C,
+                    _ptr(out), _stream_ptr(dev))
+        else:
+            what = "veon_bev_pool_v2_fwd_planar"
+            ws = _fwd_workspace(lib, dev, B, C, V)
+            with _timed("pool_fwd", dev):
+                rc = lib.veon_bev_pool_v2_fwd_planar(
+                    _ptr(depth), _ptr(feat), _ptr(rd), _ptr(rf), _ptr(rb), _ptr(plan.tile_start),
+                    _ptr(plan.tile_istart), _ptr(plan.tile_occ),
+                    _ptr(plan.tile_heavy), plan.tile_heavy.numel(),
+                    B, C, V, feat.numel() // C, _ptr(out), _ptr(ws), ws.numel(), _stream_ptr(dev))
+    _lib.check(rc, what)
     return out
 
 
-def _fwd_planar_cl(depth, feat, rd, rf, rb, plan, B, C, V, shape5):
-    lib = _lib.load()
-    dev = feat.device
-    with torch.cuda.device(dev):
-        out = torch.empty(shape5, dtype=torch.float32, device=dev)  # [B,Z,Y,X,C]
-        with _timed("pool_fwd_cl", dev):
-            rc = lib.veon_bev_pool_v2_fwd_planar_cl(
-                _ptr(depth), _ptr(feat), _ptr(rd), _ptr(rf), _ptr(rb), _ptr(plan.tile_start),
-                _ptr(plan.tile_heavy), plan.tile_heavy.numel(), B, C, V, feat.numel() // C,
-                _ptr(out), _stream_ptr(dev))
-    _lib.check(rc, "veon_bev_pool_v2_fwd_planar_cl")
-    return out
+_fwd_planar_cl = functools.partial(_fwd_planar, channels_last=True)
 
 
 def _need_backward_tables(plan):
@@ -712,41 +697,56 @@ def _need_backward_tables(plan):
                            "no gradient can flow through the pooling")
 
 
-def _bwd_planar(grad_planar, depth, feat, rb, ist, plan, C):
-    _need_backward_tables(plan)
-    lib = _lib.load()
-    dev = feat.device
+def _bwd_rows(lib, plan, C, dev):
+    """The intervals a row pass covers (a bound while a sync-free plan's count is still in
+    flight) and its scratch: one C-float row per interval."""
     B, N, D, H, W = plan.dims
     n_int = plan.interval_capacity()
-    with torch.cuda.device(dev):
-        depth_grad = torch.empty_like(depth)
-        feat_grad = torch.empty_like(feat)
-        n_rows = lib.veon_bev_pool_v2_bwd_workspace_floats(n_int, B, N, D, H, W, C, plan.V)
-        rows = torch.empty(max(n_rows, 1), dtype=torch.float32, device=dev)
-        with _timed("pool_bwd", dev):
-            rc = lib.veon_bev_pool_v2_bwd_planar(
-                _ptr(grad_planar), _ptr(depth), _ptr(feat), _ptr(plan.tile_istart),
-                _ptr(plan.tile_occ), _ptr(plan.point_interval), n_int, B, N, D, H, W, C, plan.V,
-                _ptr(rows), rows.numel(), _ptr(depth_grad), _ptr(feat_grad), _stream_ptr(dev))
-    _lib.check(rc, "veon_bev_pool_v2_bwd_planar")
-    return depth_grad, feat_grad
+    n_rows = lib.veon_bev_pool_v2_bwd_workspace_floats(n_int, B, N, D, H, W, C, plan.V)
+    return n_int, torch.empty(max(n_rows, 1), dtype=torch.float32, device=dev)
 
 
-def _bwd_planar_cl(grad_cl, depth, feat, rb, ist, plan, C):
-    """Single pass on a channels-last [B,Z,Y,X,C] gradient (no row pass, no scratch)."""
-    _need_backward_tables(plan)
+def _pool_bwd(out_grad, depth, feat, rd, rf, rb, ist, plan):
+    """(depth_grad, feat_grad) for the gradient of a [B,Z,Y,X,C] volume, routed by its storage:
+    float32 channels-last (out_grad contiguous, its [B,C,Z,Y,X] view not) with a valid plan ->
+    the single pass, which reads the gradient rows in place; otherwise a valid plan -> the two
+    passes on a float32 channels-first copy; a rejected plan -> the generic kernel."""
     lib = _lib.load()
     dev = feat.device
-    B, N, D, H, W = plan.dims
+    _, Z, Y, X, C = out_grad.shape
+    g = out_grad.permute(0, 4, 1, 2, 3)  # back to the channels-first storage order
+    single = (out_grad.dtype == torch.float32 and not g.is_contiguous()
+              and out_grad.is_contiguous() and plan.ok)
+    if not single:
+        g = g.float().contiguous()
     with torch.cuda.device(dev):
-        depth_grad = torch.empty_like(depth)
-        feat_grad = torch.empty_like(feat)
-        with _timed("pool_bwd_cl", dev):
-            rc = lib.veon_bev_pool_v2_bwd_planar_cl(
-                _ptr(grad_cl), _ptr(depth), _ptr(feat), _ptr(rb), _ptr(ist),
-                _ptr(plan.point_interval), B, N, D, H, W, C, plan.V, _ptr(depth_grad),
-                _ptr(feat_grad), _stream_ptr(dev))
-    _lib.check(rc, "veon_bev_pool_v2_bwd_planar_cl")
+        if not plan.ok:
+            what = "veon_bev_pool_v2_grad_generic"
+            depth_grad, feat_grad = torch.zeros_like(depth), torch.zeros_like(feat)
+            rc = lib.veon_bev_pool_v2_grad_generic(
+                C, rb.numel(), LAYOUT_BCZYX, Z * Y * X, _ptr(g), _ptr(depth), _ptr(feat), _ptr(rd),
+                _ptr(rf), _ptr(rb), _ptr(depth_grad), _ptr(feat_grad), _stream_ptr(dev))
+        else:
+            _need_backward_tables(plan)
+            B, N, D, H, W = plan.dims
+            depth_grad, feat_grad = torch.empty_like(depth), torch.empty_like(feat)
+            if single:
+                what = "veon_bev_pool_v2_bwd_planar_cl"
+                with _timed("pool_bwd_cl", dev):
+                    rc = lib.veon_bev_pool_v2_bwd_planar_cl(
+                        _ptr(out_grad), _ptr(depth), _ptr(feat), _ptr(rb), _ptr(ist),
+                        _ptr(plan.point_interval), B, N, D, H, W, C, plan.V, _ptr(depth_grad),
+                        _ptr(feat_grad), _stream_ptr(dev))
+            else:
+                what = "veon_bev_pool_v2_bwd_planar"
+                n_int, rows = _bwd_rows(lib, plan, C, dev)
+                with _timed("pool_bwd", dev):
+                    rc = lib.veon_bev_pool_v2_bwd_planar(
+                        _ptr(g), _ptr(depth), _ptr(feat), _ptr(plan.tile_istart),
+                        _ptr(plan.tile_occ), _ptr(plan.point_interval), n_int, B, N, D, H, W, C,
+                        plan.V, _ptr(rows), rows.numel(), _ptr(depth_grad), _ptr(feat_grad),
+                        _stream_ptr(dev))
+    _lib.check(rc, what)
     return depth_grad, feat_grad
 
 
@@ -772,21 +772,12 @@ class QuickCumsumCuda(torch.autograd.Function):
         channels_last = bool(extra[1]) if len(extra) > 1 else False
         ctx.n_extra = len(extra)
         _require_cuda(depth, feat, ranks_depth, ranks_feat, ranks_bev,
-                      interval_starts, interval_lengths)
+                     interval_starts, interval_lengths)
         if depth.dim() != 5 or feat.dim() != 5:
             raise ValueError("depth must be [B,N,D,H,W] and feat [B,N,H,W,C]")
         ranks_bev = ranks_bev.int().contiguous()
         depth = depth.contiguous().float()
-        # the neck hands over a channels-last VIEW of channels-first maps: transpose it
-        # with our own kernel (and feat_grad back the same way) instead of a strided copy
-        ctx.feat_channels_first = (feat.dtype == torch.float32 and not feat.is_contiguous()
-                                   and feat.permute(0, 1, 4, 2, 3).is_contiguous())
-        if ctx.feat_channels_first:
-            feat = _transpose_batched(feat.permute(0, 1, 4, 2, 3), feat.shape[0] * feat.shape[1],
-                                      feat.shape[4], feat.shape[2] * feat.shape[3],
-                                      tuple(feat.shape))
-        else:
-            feat = feat.contiguous().float()
+        feat, ctx.feat_transposed = _feat_rows(feat)
         ranks_depth = ranks_depth.contiguous().int()
         ranks_feat = ranks_feat.contiguous().int()
         interval_lengths = interval_lengths.contiguous().int()
@@ -804,69 +795,31 @@ class QuickCumsumCuda(torch.autograd.Function):
             # bev_pool.cpp has no CHECK_* macros); so would the unchecked generic kernels
             raise ValueError("bev_pool_v2: a rank lies outside its tensor (ranks_depth >= "
                              "depth.numel(), ranks_feat >= feat rows or ranks_bev >= B*Z*Y*X)")
-        if channels_last:
-            if plan.ok:
-                out = _fwd_planar_cl(depth, feat, ranks_depth, ranks_feat, ranks_bev, plan,
-                                     B, C, V, (B, Z, Y, X, C))
-            else:
-                lib = _lib.load()
-                out = feat.new_zeros((B, Z, Y, X, C))
-                with torch.cuda.device(feat.device):
-                    rc = lib.veon_bev_pool_v2_generic(
-                        C, interval_starts.numel(), LAYOUT_BZYXC, V, _ptr(depth), _ptr(feat),
-                        _ptr(ranks_depth), _ptr(ranks_feat), _ptr(ranks_bev),
-                        _ptr(interval_starts), _ptr(interval_lengths), _ptr(out),
-                        _stream_ptr(feat.device))
-                _lib.check(rc, "veon_bev_pool_v2_generic")
-        elif plan.ok:
-            out = _fwd_planar(depth, feat, ranks_depth, ranks_feat, ranks_bev, plan,
-                              B, C, V, (B, C, Z, Y, X))
+        shape5 = (B, Z, Y, X, C) if channels_last else (B, C, Z, Y, X)
+        if plan.ok:
+            out = _fwd_planar(depth, feat, ranks_depth, ranks_feat, ranks_bev, plan, B, C, V,
+                              shape5, channels_last)
         else:
+            # the interval-driven generic kernel adds into a zeroed volume
             lib = _lib.load()
-            out = feat.new_zeros((B, C, Z, Y, X))
+            out = feat.new_zeros(shape5)
             with torch.cuda.device(feat.device):
                 rc = lib.veon_bev_pool_v2_generic(
-                    C, interval_starts.numel(), LAYOUT_BCZYX, V, _ptr(depth), _ptr(feat),
-                    _ptr(ranks_depth), _ptr(ranks_feat), _ptr(ranks_bev),
+                    C, interval_starts.numel(), LAYOUT_BZYXC if channels_last else LAYOUT_BCZYX, V,
+                    _ptr(depth), _ptr(feat), _ptr(ranks_depth), _ptr(ranks_feat), _ptr(ranks_bev),
                     _ptr(interval_starts), _ptr(interval_lengths), _ptr(out),
                     _stream_ptr(feat.device))
             _lib.check(rc, "veon_bev_pool_v2_generic")
         ctx.save_for_backward(ranks_bev, depth, feat, ranks_feat, ranks_depth, interval_starts)
         ctx.plan = plan
-        ctx.vol = (B, C, Z, Y, X)
         return out if channels_last else out.permute(0, 2, 3, 4, 1)
 
     @staticmethod
     def backward(ctx, out_grad):
         ranks_bev, depth, feat, ranks_feat, ranks_depth, interval_starts = ctx.saved_tensors
-        B, C, Z, Y, X = ctx.vol
-        plan = ctx.plan
-        g = out_grad.permute(0, 4, 1, 2, 3)  # back to the channels-first storage order
-        cl_grad = (out_grad.dtype == torch.float32 and not g.is_contiguous()
-                   and out_grad.is_contiguous() and plan.ok)
-        if not cl_grad and (g.dtype != torch.float32 or not g.is_contiguous()):
-            g = g.float().contiguous()
-        if cl_grad:
-            # channels-last storage: the single pass reads its rows in place
-            depth_grad, feat_grad = _bwd_planar_cl(out_grad, depth, feat, ranks_bev,
-                                                   interval_starts, plan, C)
-        elif plan.ok:
-            depth_grad, feat_grad = _bwd_planar(g, depth, feat, ranks_bev, interval_starts,
-                                                plan, C)
-        else:
-            lib = _lib.load()
-            depth_grad = torch.zeros_like(depth)
-            feat_grad = torch.zeros_like(feat)
-            with torch.cuda.device(feat.device):
-                rc = lib.veon_bev_pool_v2_grad_generic(
-                    C, ranks_bev.numel(), LAYOUT_BCZYX, Z * Y * X, _ptr(g), _ptr(depth),
-                    _ptr(feat), _ptr(ranks_depth), _ptr(ranks_feat), _ptr(ranks_bev),
-                    _ptr(depth_grad), _ptr(feat_grad), _stream_ptr(feat.device))
-            _lib.check(rc, "veon_bev_pool_v2_grad_generic")
-        if ctx.feat_channels_first:
-            Bf, Nf, Hf, Wf, Cf = feat_grad.shape
-            feat_grad = _transpose_batched(feat_grad, Bf * Nf, Hf * Wf, Cf,
-                                           (Bf, Nf, Cf, Hf, Wf)).permute(0, 1, 3, 4, 2)
+        depth_grad, feat_grad = _pool_bwd(out_grad, depth, feat, ranks_depth, ranks_feat,
+                                          ranks_bev, interval_starts, ctx.plan)
+        feat_grad = _feat_grad_back(feat_grad, ctx.feat_transposed)
         return (depth_grad, feat_grad, None, None, None, None, None, None) + (None,) * ctx.n_extra
 
 

@@ -17,25 +17,18 @@ kernels go to torch's current stream.  A reference checkout uses it with
 before `mmdet3d.ops.bev_pool_v2.bev_pool` is imported; its own QuickCumsumCuda (memset,
 permute, argsort and all) then runs unchanged on our kernels.
 """
-import ctypes
-
 import torch
 
 from . import _lib
+from ._lib import ptr, require_cuda, stream_ptr
 
 __all__ = ["bev_pool_v2_forward", "bev_pool_v2_backward"]
 
 
-def _p(t):
-    return ctypes.c_void_p(t.data_ptr())
-
-
 def _check(*tensors):
-    for t in tensors:
-        if not t.is_cuda:
-            raise RuntimeError("bev_pool_v2_ext: CUDA tensors only (no CPU fallback)")
-        if not t.is_contiguous():
-            raise RuntimeError("bev_pool_v2_ext: tensors must be contiguous")
+    require_cuda(*tensors)
+    if not all(t.is_contiguous() for t in tensors):
+        raise RuntimeError("bev_pool_v2_ext: tensors must be contiguous")
 
 
 def bev_pool_v2_forward(depth, feat, out, ranks_depth, ranks_feat, ranks_bev,
@@ -43,10 +36,10 @@ def bev_pool_v2_forward(depth, feat, out, ranks_depth, ranks_feat, ranks_bev,
     _check(depth, feat, out, ranks_depth, ranks_feat, ranks_bev, interval_lengths, interval_starts)
     lib = _lib.load()
     with torch.cuda.device(depth.device):                    # OptionalCUDAGuard, bev_pool.cpp:42
-        rc = lib.veon_bev_pool_v2(int(feat.size(4)), int(interval_lengths.size(0)), _p(depth),
-                                  _p(feat), _p(ranks_depth), _p(ranks_feat), _p(ranks_bev),
-                                  _p(interval_starts), _p(interval_lengths), _p(out),
-                                  ctypes.c_void_p(torch.cuda.current_stream().cuda_stream))
+        rc = lib.veon_bev_pool_v2(int(feat.size(4)), int(interval_lengths.size(0)), ptr(depth),
+                                  ptr(feat), ptr(ranks_depth), ptr(ranks_feat), ptr(ranks_bev),
+                                  ptr(interval_starts), ptr(interval_lengths), ptr(out),
+                                  stream_ptr(depth.device))
     _lib.check(rc, "veon_bev_pool_v2")
 
 
@@ -57,8 +50,8 @@ def bev_pool_v2_backward(out_grad, depth_grad, feat_grad, depth, feat, ranks_dep
     lib = _lib.load()
     with torch.cuda.device(out_grad.device):                 # bev_pool.cpp:88
         rc = lib.veon_bev_pool_v2_grad(int(out_grad.size(4)), int(interval_lengths.size(0)),
-                                       _p(out_grad), _p(depth), _p(feat), _p(ranks_depth),
-                                       _p(ranks_feat), _p(ranks_bev), _p(interval_starts),
-                                       _p(interval_lengths), _p(depth_grad), _p(feat_grad),
-                                       ctypes.c_void_p(torch.cuda.current_stream().cuda_stream))
+                                       ptr(out_grad), ptr(depth), ptr(feat), ptr(ranks_depth),
+                                       ptr(ranks_feat), ptr(ranks_bev), ptr(interval_starts),
+                                       ptr(interval_lengths), ptr(depth_grad), ptr(feat_grad),
+                                       stream_ptr(out_grad.device))
     _lib.check(rc, "veon_bev_pool_v2_grad")

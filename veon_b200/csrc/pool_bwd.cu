@@ -580,14 +580,22 @@ static int launch_pixels(const float* rows, const float* depth, const float* fea
   return 0;
 }
 
+// the compact rows of tiles [0, n_tiles)
+static int row_pass(const float* out_grad, const int32_t* tile_istart, const uint32_t* tile_occ,
+                    int64_t n_tiles, int64_t tps, int64_t V, int C, float* rows,
+                    cudaStream_t stream) {
+  return C <= 32 ? launch_rows<1>(out_grad, tile_istart, tile_occ, 0, n_tiles, tps, V, C, rows, stream)
+                 : launch_rows<2>(out_grad, tile_istart, tile_occ, 0, n_tiles, tps, V, C, rows, stream);
+}
+
 // ranks_bev / interval_starts: the channels-last pass (rows = out_grad), else NULL
 template <bool CL = false>
-static int pixel_pass(int pk, const float* rows, const float* depth, const float* feat,
+static int pixel_pass(const float* rows, const float* depth, const float* feat,
                       const int32_t* point_interval, int64_t pixels, int D, int HW, int C,
                       float* depth_grad, float* feat_grad, cudaStream_t stream,
                       const int32_t* ranks_bev = nullptr, const int32_t* interval_starts = nullptr) {
 #define VEON_PIX(K_) launch_pixels<K_, CL>(rows, depth, feat, point_interval, ranks_bev, interval_starts, 0, pixels, D, HW, C, depth_grad, feat_grad, stream)
-  switch (pk) {
+  switch (C <= 32 ? 1 : (C <= 64 ? 2 : (C <= 256 ? 4 : 8))) {   // channels per lane
     case 1: return VEON_PIX(1);
     case 2: return VEON_PIX(2);
     case 4: return VEON_PIX(4);
@@ -624,14 +632,11 @@ extern "C" int veon_bev_pool_v2_bwd_planar(
   const int64_t tps = ceil_div64(V, kTileVoxels);
   const int HW = H * W;
   const int64_t pix_per_sample = (int64_t)N * HW;
-  const int rk = C <= 32 ? 1 : 2;
-  const int pk = C <= 32 ? 1 : (C <= 64 ? 2 : (C <= 256 ? 4 : 8));
   // general route: one row launch + one pixel launch over all samples (launch ramps cost more
   // than keeping the rows L2-resident by sample groups saves: 456 vs 593 us at C2, round 1)
-  int rc = rk == 1 ? launch_rows<1>(out_grad, tile_istart, tile_occ, 0, B * tps, tps, V, C, rows_ws, stream)
-                   : launch_rows<2>(out_grad, tile_istart, tile_occ, 0, B * tps, tps, V, C, rows_ws, stream);
+  const int rc = row_pass(out_grad, tile_istart, tile_occ, B * tps, tps, V, C, rows_ws, stream);
   if (rc) return rc;
-  return pixel_pass(pk, rows_ws, depth, feat, point_interval, B * pix_per_sample, D, HW, C,
+  return pixel_pass(rows_ws, depth, feat, point_interval, B * pix_per_sample, D, HW, C,
                     depth_grad, feat_grad, stream);
 }
 
@@ -647,9 +652,8 @@ extern "C" int veon_bev_pool_v2_bwd_planar_cl(
       V <= 0)
     return VEON_E_BADARG;
   if ((int64_t)B * V > 0x7fffffffLL) return VEON_E_RANGE;
-  const int pk = C <= 32 ? 1 : (C <= 64 ? 2 : (C <= 256 ? 4 : 8));
-  return pixel_pass<true>(pk, out_grad, depth, feat, point_interval, (int64_t)B * N * H * W, D,
-                          H * W, C, depth_grad, feat_grad, (cudaStream_t)stream_, ranks_bev,
+  return pixel_pass<true>(out_grad, depth, feat, point_interval, (int64_t)B * N * H * W, D, H * W,
+                          C, depth_grad, feat_grad, (cudaStream_t)stream_, ranks_bev,
                           interval_starts);
 }
 
@@ -680,8 +684,7 @@ extern "C" int veon_bev_pool_v2_bwd_planar_ds(
     k_bwd_rows_ds<<<(unsigned)blocks, 256, 0, stream>>>(grad_ds, mask, tile_istart, tile_occ,
                                                         n_tiles, tps, Z, Y, X, C, rows_ws);
   VEON_LAUNCH_CHECK();
-  const int pk = C <= 32 ? 1 : (C <= 64 ? 2 : (C <= 256 ? 4 : 8));
-  return pixel_pass(pk, rows_ws, depth, feat, point_interval, (int64_t)B * N * H * W, D, H * W, C,
+  return pixel_pass(rows_ws, depth, feat, point_interval, (int64_t)B * N * H * W, D, H * W, C,
                     depth_grad, feat_grad, stream);
 }
 
@@ -691,14 +694,12 @@ extern "C" int veon_bev_pool_v2_bwd_planar_ds(
 extern "C" int veon_internal_bwd_rows(const float* out_grad, const int32_t* tile_istart,
                                       const uint32_t* tile_occ, int64_t n_tiles, int64_t tps,
                                       int64_t V, int C, float* rows, void* stream) {
-  return C <= 32 ? launch_rows<1>(out_grad, tile_istart, tile_occ, 0, n_tiles, tps, V, C, rows, (cudaStream_t)stream)
-                 : launch_rows<2>(out_grad, tile_istart, tile_occ, 0, n_tiles, tps, V, C, rows, (cudaStream_t)stream);
+  return row_pass(out_grad, tile_istart, tile_occ, n_tiles, tps, V, C, rows, (cudaStream_t)stream);
 }
 extern "C" int veon_internal_bwd_pixels(const float* rows, const float* depth, const float* feat,
                                         const int32_t* point_interval, int64_t pixels, int D, int HW,
                                         int C, float* depth_grad, float* feat_grad, void* stream) {
-  const int pk = C <= 32 ? 1 : (C <= 64 ? 2 : (C <= 256 ? 4 : 8));
-  return pixel_pass(pk, rows, depth, feat, point_interval, pixels, D, HW, C, depth_grad, feat_grad,
+  return pixel_pass(rows, depth, feat, point_interval, pixels, D, HW, C, depth_grad, feat_grad,
                     (cudaStream_t)stream);
 }
 extern "C" int veon_internal_l2_window(void* stream, void* base, size_t bytes, float hit_ratio,

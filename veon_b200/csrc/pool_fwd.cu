@@ -1195,18 +1195,16 @@ extern "C" size_t veon_bev_pool_v2_fwd_workspace_bytes(int B, int C, int64_t V) 
   return fwd_stream_workspace_bytes(C);
 }
 
-extern "C" int veon_bev_pool_v2_fwd_planar(const float* depth, const float* feat,
-                                           const int32_t* ranks_depth,
-                                           const int32_t* ranks_feat,
-                                           const int32_t* ranks_bev,
-                                           const int32_t* tile_start,
-                                           const int32_t* tile_istart,
-                                           const uint32_t* tile_occ,
-                                           const int32_t* tile_heavy, int64_t tile_heavy_ints,
-                                           int B, int C, int64_t V, int64_t n_feat_rows,
-                                           float* out, void* workspace, size_t workspace_bytes,
-                                           void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
+// Both planar entry points: out is [B,C,Z,Y,X], or [B,Z,Y,X,C] with CL (the same kernels with a
+// row write-out: same sums, same bits, another layout).  Routes in order: narrow rows, the
+// streaming kernel (channels-first only; needs tile_occ and a workspace), the general kernel.
+template <bool CL>
+static int fwd_planar(const float* depth, const float* feat, const int32_t* ranks_depth,
+                      const int32_t* ranks_feat, const int32_t* ranks_bev,
+                      const int32_t* tile_start, const uint32_t* tile_occ,
+                      const int32_t* tile_heavy, int64_t tile_heavy_ints, int B, int C, int64_t V,
+                      int64_t n_feat_rows, float* out, void* workspace, size_t workspace_bytes,
+                      cudaStream_t stream) {
   if (!depth || !feat || !ranks_depth || !ranks_feat || !ranks_bev || !tile_start || !out ||
       B <= 0 || C <= 0 || V <= 0 || n_feat_rows <= 0 || (tile_heavy && tile_heavy_ints < 2))
     return VEON_E_BADARG;
@@ -1220,7 +1218,7 @@ extern "C" int veon_bev_pool_v2_fwd_planar(const float* depth, const float* feat
                     (int64_t)B * V <= (1 << 24) &&
                     (((uintptr_t)feat | (uintptr_t)out) & 15) == 0;
     if (ok) {
-#define VEON_NARROW_CASE(NV_) case NV_: return launch_fwd_narrow<NV_>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy, tile_heavy_ints, B, V, out, stream);
+#define VEON_NARROW_CASE(NV_) case NV_: return launch_fwd_narrow<NV_, false, 1, CL>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy, tile_heavy_ints, B, V, out, stream);
       switch (C / 4) {
         VEON_NARROW_CASE(1) VEON_NARROW_CASE(2) VEON_NARROW_CASE(3) VEON_NARROW_CASE(4)
         VEON_NARROW_CASE(5) VEON_NARROW_CASE(6) VEON_NARROW_CASE(7) VEON_NARROW_CASE(8)
@@ -1230,21 +1228,38 @@ extern "C" int veon_bev_pool_v2_fwd_planar(const float* depth, const float* feat
     }
   }
   // aligned volumes, whole 64-channel chunks: the two-role streaming kernel
-  if (workspace && tile_occ && tile_heavy && fwd_stream_supported(B, C, V, feat, out, n_feat_rows)) {
-    const int rc = launch_fwd_stream(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
-                                     tile_occ, tile_heavy, tile_heavy_ints, B, C, V, out,
-                                     workspace, workspace_bytes, stream);
-    if (rc != VEON_E_UNSUPPORTED && rc != VEON_E_WORKSPACE) return rc;
+  if constexpr (!CL) {
+    if (workspace && tile_occ && tile_heavy &&
+        fwd_stream_supported(B, C, V, feat, out, n_feat_rows)) {
+      const int rc = launch_fwd_stream(depth, feat, ranks_depth, ranks_feat, ranks_bev,
+                                       tile_start, tile_occ, tile_heavy, tile_heavy_ints, B, C, V,
+                                       out, workspace, workspace_bytes, stream);
+      if (rc != VEON_E_UNSUPPORTED && rc != VEON_E_WORKSPACE) return rc;
+    }
   }
   if (C <= 32)
-    return launch_fwd<1>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy,
-                         tile_heavy_ints, B, C, V, fit32, out, stream);
-  return launch_fwd<2>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy,
-                       tile_heavy_ints, B, C, V, fit32, out, stream);
+    return launch_fwd<1, CL>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
+                             tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
+  return launch_fwd<2, CL>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
+                           tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
 }
 
-// Channels-last volume out[B,Z,Y,X,C]: the same kernels with a row write-out (the streaming
-// two-role kernel is channels-first only).  Same sums, same bits, another layout.
+extern "C" int veon_bev_pool_v2_fwd_planar(const float* depth, const float* feat,
+                                           const int32_t* ranks_depth,
+                                           const int32_t* ranks_feat,
+                                           const int32_t* ranks_bev,
+                                           const int32_t* tile_start,
+                                           const int32_t* tile_istart,
+                                           const uint32_t* tile_occ,
+                                           const int32_t* tile_heavy, int64_t tile_heavy_ints,
+                                           int B, int C, int64_t V, int64_t n_feat_rows,
+                                           float* out, void* workspace, size_t workspace_bytes,
+                                           void* stream) {
+  return fwd_planar<false>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_occ,
+                           tile_heavy, tile_heavy_ints, B, C, V, n_feat_rows, out, workspace,
+                           workspace_bytes, (cudaStream_t)stream);
+}
+
 extern "C" int veon_bev_pool_v2_fwd_planar_cl(const float* depth, const float* feat,
                                               const int32_t* ranks_depth,
                                               const int32_t* ranks_feat,
@@ -1252,32 +1267,10 @@ extern "C" int veon_bev_pool_v2_fwd_planar_cl(const float* depth, const float* f
                                               const int32_t* tile_start,
                                               const int32_t* tile_heavy, int64_t tile_heavy_ints,
                                               int B, int C, int64_t V, int64_t n_feat_rows,
-                                              float* out, void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  if (!depth || !feat || !ranks_depth || !ranks_feat || !ranks_bev || !tile_start || !out ||
-      B <= 0 || C <= 0 || V <= 0 || n_feat_rows <= 0 || (tile_heavy && tile_heavy_ints < 2))
-    return VEON_E_BADARG;
-  const bool fit32 = n_feat_rows * (int64_t)C <= 0x3fffffffLL && B < 65536 &&
-                     (int64_t)C <= 65535LL * 32;
-  {  // narrow rows: lane-per-voxel kernel (conditions as in veon_bev_pool_v2_fwd_planar)
-    const bool ok = C <= 32 && (C & 3) == 0 && tile_heavy && fit32 && V % kTileVoxels == 0 &&
-                    (int64_t)B * V <= (1 << 24) &&
-                    (((uintptr_t)feat | (uintptr_t)out) & 15) == 0;
-    if (ok) {
-#define VEON_NARROW_CASE(NV_) case NV_: return launch_fwd_narrow<NV_, false, 1, true>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy, tile_heavy_ints, B, V, out, stream);
-      switch (C / 4) {
-        VEON_NARROW_CASE(1) VEON_NARROW_CASE(2) VEON_NARROW_CASE(3) VEON_NARROW_CASE(4)
-        VEON_NARROW_CASE(5) VEON_NARROW_CASE(6) VEON_NARROW_CASE(7) VEON_NARROW_CASE(8)
-        default: break;
-      }
-#undef VEON_NARROW_CASE
-    }
-  }
-  if (C <= 32)
-    return launch_fwd<1, true>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
-                               tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
-  return launch_fwd<2, true>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
-                             tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
+                                              float* out, void* stream) {
+  return fwd_planar<true>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, nullptr,
+                          tile_heavy, tile_heavy_ints, B, C, V, n_feat_rows, out, nullptr, 0,
+                          (cudaStream_t)stream);
 }
 
 // Fused lift + classify: pools the [gate 0, gate 1, logit 0..Q-1, pad] rows and ends every tile

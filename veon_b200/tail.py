@@ -16,6 +16,7 @@ import ctypes
 import torch
 
 from . import _lib
+from ._lib import require_cuda, stream_ptr
 
 __all__ = ["class_of_prompt", "voxel_text_argmax", "semantic_inference_3d", "classify_logits",
            "upsample_classify", "voxel_text_argmax_lowres", "prepare_vocabulary",
@@ -76,9 +77,7 @@ def voxel_text_argmax(feat_occ, ov_classifier_weight, prompt_class, bin_occ, fre
     """feat_occ [B,C,Z,Y,X] f32, ov_classifier_weight [Q,C] f32, prompt_class
     [Q] int32 (from `class_of_prompt`), bin_occ [B,2,Z,Y,X] f32 ->
     uint8 occupancy labels [B,X,Y,Z] (free voxels = `free_label`)."""
-    for t in (feat_occ, ov_classifier_weight, prompt_class, bin_occ):
-        if not t.is_cuda:
-            raise RuntimeError("veon_b200 runs on CUDA tensors only (no CPU fallback)")
+    require_cuda(feat_occ, ov_classifier_weight, prompt_class, bin_occ)
     lib = _lib.load()
     feat_occ = feat_occ.detach().contiguous().float()
     w = ov_classifier_weight.detach().contiguous().float()
@@ -95,20 +94,9 @@ def voxel_text_argmax(feat_occ, ov_classifier_weight, prompt_class, bin_occ, fre
             ctypes.c_void_p(feat_occ.data_ptr()), ctypes.c_void_p(w.data_ptr()),
             ctypes.c_void_p(cls.data_ptr()), ctypes.c_void_p(bin_occ.data_ptr()),
             B, C, Q, Z, Y, X, int(free_label), ctypes.c_void_p(labels.data_ptr()),
-            _classifier_image(lib, w, dev),
-            ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+            _classifier_image(lib, w, dev), stream_ptr(dev))
     _lib.check(rc, "veon_voxel_text_argmax")
     return labels
-
-
-def _cuda_only(*tensors):
-    for t in tensors:
-        if not t.is_cuda:
-            raise RuntimeError("veon_b200 runs on CUDA tensors only (no CPU fallback)")
-
-
-def _stream(dev):
-    return ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
 
 
 _IMAGE_BUFFERS = {}
@@ -140,7 +128,7 @@ def semantic_inference_3d(ov_classifier_weight, mask_pred):
     einsum("qc,bczhw->bqzhw") of the [Q,C] classifier and a [B,C,Z,Y,X] volume -> [B,Q,Z,Y,X]
     f32 (no gradient: the reference's weight is a detached constant and this entry serves the
     inference route)."""
-    _cuda_only(ov_classifier_weight, mask_pred)
+    require_cuda(ov_classifier_weight, mask_pred)
     lib = _lib.load()
     w = ov_classifier_weight.detach().contiguous().float()
     feat = mask_pred.detach().contiguous().float()
@@ -153,7 +141,7 @@ def semantic_inference_3d(ov_classifier_weight, mask_pred):
         sem = torch.empty((B, Q, Z, Y, X), dtype=torch.float32, device=dev)
         rc = lib.veon_semantic_inference_3d(
             ctypes.c_void_p(w.data_ptr()), ctypes.c_void_p(feat.data_ptr()), B, C, Q, Z, Y, X,
-            ctypes.c_void_p(sem.data_ptr()), _classifier_image(lib, w, dev), _stream(dev))
+            ctypes.c_void_p(sem.data_ptr()), _classifier_image(lib, w, dev), stream_ptr(dev))
     _lib.check(rc, "veon_semantic_inference_3d")
     return sem
 
@@ -178,7 +166,7 @@ def classify_logits(sem_occ, bin_occ, prompt_class, free_label=17):
     (san_in_veon_entry_temporal.py:273-297, veon_temporal.py:223-229,240): sem_occ [B,Q,Z,Y,X],
     bin_occ [B,2,Z,Y,X] -> uint8 [B,X,Y,Z].  Channel slices of a larger volume are taken as
     they are (no copy)."""
-    _cuda_only(sem_occ, bin_occ, prompt_class)
+    require_cuda(sem_occ, bin_occ, prompt_class)
     lib = _lib.load()
     sem = _sample_contiguous(sem_occ)
     gate = _sample_contiguous(bin_occ)
@@ -192,7 +180,7 @@ def classify_logits(sem_occ, bin_occ, prompt_class, free_label=17):
         rc = lib.veon_classify_logits(
             ctypes.c_void_p(sem.data_ptr()), sem.stride(0), ctypes.c_void_p(gate.data_ptr()),
             gate.stride(0), ctypes.c_void_p(cls.data_ptr()), B, Q, Z, Y, X, int(free_label),
-            ctypes.c_void_p(labels.data_ptr()), _stream(dev))
+            ctypes.c_void_p(labels.data_ptr()), stream_ptr(dev))
     _lib.check(rc, "veon_classify_logits")
     return labels
 
@@ -200,7 +188,7 @@ def classify_logits(sem_occ, bin_occ, prompt_class, free_label=17):
 def upsample_classify(sem_occ_lr, bin_occ_lr, prompt_class, occ_size, free_label=17):
     """Low-resolution logits [B,Q,Zi,Yi,Xi] and gate [B,2,Zi,Yi,Xi] -> trilinear
     (align_corners=False) to `occ_size` = (Z,Y,X), class merge, arg-max, gate -> uint8 [B,X,Y,Z]."""
-    _cuda_only(sem_occ_lr, bin_occ_lr, prompt_class)
+    require_cuda(sem_occ_lr, bin_occ_lr, prompt_class)
     lib = _lib.load()
     sem = sem_occ_lr.detach().contiguous().float()
     gate = bin_occ_lr.detach().contiguous().float()
@@ -215,7 +203,7 @@ def upsample_classify(sem_occ_lr, bin_occ_lr, prompt_class, occ_size, free_label
         rc = lib.veon_upsample_classify(
             ctypes.c_void_p(sem.data_ptr()), ctypes.c_void_p(gate.data_ptr()),
             ctypes.c_void_p(cls.data_ptr()), B, Q, Zi, Yi, Xi, Z, Y, X, int(free_label),
-            ctypes.c_void_p(labels.data_ptr()), _stream(dev))
+            ctypes.c_void_p(labels.data_ptr()), stream_ptr(dev))
     _lib.check(rc, "veon_upsample_classify")
     return labels
 
@@ -226,7 +214,7 @@ def voxel_text_argmax_lowres(feat_occ_lr, ov_classifier_weight, prompt_class, bi
     the merge and label rule): feat_occ_lr [B,C,Zi,Yi,Xi], bin_occ_lr [B,2,Zi,Yi,Xi] ->
     uint8 labels [B,X,Y,Z] on the `occ_size` grid.  `workspace`: optional float32 CUDA tensor of
     at least B*Q*Zi*Yi*Xi elements to hold the low-resolution logits (allocated if absent)."""
-    _cuda_only(feat_occ_lr, ov_classifier_weight, prompt_class, bin_occ_lr)
+    require_cuda(feat_occ_lr, ov_classifier_weight, prompt_class, bin_occ_lr)
     lib = _lib.load()
     feat = feat_occ_lr.detach().contiguous().float()
     w = ov_classifier_weight.detach().contiguous().float()
@@ -249,7 +237,7 @@ def voxel_text_argmax_lowres(feat_occ_lr, ov_classifier_weight, prompt_class, bi
             ctypes.c_void_p(cls.data_ptr()), ctypes.c_void_p(gate.data_ptr()),
             B, C, Q, Zi, Yi, Xi, Z, Y, X, int(free_label), ctypes.c_void_p(labels.data_ptr()),
             ctypes.c_void_p(workspace.data_ptr()), ws_bytes, _classifier_image(lib, w, dev),
-            _stream(dev))
+            stream_ptr(dev))
     _lib.check(rc, "veon_voxel_text_argmax_lowres")
     return labels
 
@@ -270,7 +258,7 @@ def point_text_argmax(pred_feat, ov_classifier_weight, class_reflection):
     How: the point rows are turned into a [C, N] operand (own transpose kernel), the logits come
     from the tcgen05 3xTF32 kernel of the inference tail, one pass over them takes both
     arg-maxes."""
-    _cuda_only(pred_feat, ov_classifier_weight)
+    require_cuda(pred_feat, ov_classifier_weight)
     lib = _lib.load()
     f = pred_feat.detach().contiguous().float()
     w = ov_classifier_weight.detach()[:-1].contiguous().float()
@@ -290,7 +278,7 @@ def point_text_argmax(pred_feat, ov_classifier_weight, class_reflection):
             torch.empty((C, ldn), dtype=torch.float32, device=dev)
         if ldn == N:
             rc = lib.veon_transpose_batched(ctypes.c_void_p(f.data_ptr()), 1, N, C,
-                                            ctypes.c_void_p(ft.data_ptr()), _stream(dev))
+                                            ctypes.c_void_p(ft.data_ptr()), stream_ptr(dev))
             _lib.check(rc, "veon_transpose_batched")
         else:
             ft[:, :N] = f.t()
@@ -298,6 +286,6 @@ def point_text_argmax(pred_feat, ov_classifier_weight, class_reflection):
         rc = lib.veon_point_text_argmax(ctypes.c_void_p(logits.data_ptr()),
                                         ctypes.c_void_p(cls.data_ptr()), Q, N, ldn,
                                         ctypes.c_void_p(p_idx.data_ptr()),
-                                        ctypes.c_void_p(c_idx.data_ptr()), _stream(dev))
+                                        ctypes.c_void_p(c_idx.data_ptr()), stream_ptr(dev))
     _lib.check(rc, "veon_point_text_argmax")
     return p_idx, c_idx

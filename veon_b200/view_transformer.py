@@ -239,26 +239,31 @@ class LSSViewTransformer(nn.Module):
         logit 0..Q-1, padding] (veon_b200.pipeline.lift_classify): uint8 labels [B,X,Y,Z], or None
         when the fused kernel does not take the shape.  Inference only."""
         with torch.no_grad():
-            prep = self._prepare_calib(calib, depth, backward_tables=False)
-            prep.plan.sync_free = self.sync_free
-            if self.prepared_hook is not None:
-                self.prepared_hook()
+            prep = self._prepared(self._prepare_calib(calib, depth, backward_tables=False))
             gs = self.grid_size
             return _bp.lift_classify_prepared(depth, pix, prep, Q, prompt_class,
                                               (int(gs[2]), int(gs[1]), int(gs[0])), free_label)
 
+    def _prepared(self, prep):
+        """A freshly prepared rank set on its way to the pooling kernels: a sync-free plan's
+        backward sizes its scratch by a bound; `prepared_hook` (see __init__) runs here."""
+        prep.plan.sync_free = self.sync_free
+        if self.prepared_hook is not None:
+            self.prepared_hook()
+        return prep
+
+    def _no_points(self, prep):
+        """The reference's empty-input case: no interval at all.  Read back after the pooling
+        has been queued, so the host read-back (the reference syncs at the same place in its
+        boolean-mask indexing) overlaps the forward kernel; never asked when sync_free."""
+        return not self.sync_free and prep.plan.n_intervals == 0
+
     def _pool_prepared(self, prep, depth, feat):
         feat_last = feat.permute(0, 1, 3, 4, 2)
         shape = self._bev_shape(depth, feat_last.shape[-1])
-        # The pooling is queued BEFORE the point / interval counts are read back, so
-        # the host read-back (the reference syncs at the same place in its
-        # boolean-mask indexing) overlaps the forward kernel instead of draining
-        # the GPU; it only decides about the reference's empty-input result.
-        prep.plan.sync_free = self.sync_free   # the backward then sizes its scratch by a bound
-        if self.prepared_hook is not None:
-            self.prepared_hook()               # see __init__: lets a caller time its transfers
-        bev_feat = _bp.pool_prepared(depth, feat_last, prep, shape, self.memory_format)
-        if not self.sync_free and prep.plan.n_intervals == 0:
+        bev_feat = _bp.pool_prepared(depth, feat_last, self._prepared(prep), shape,
+                                     self.memory_format)
+        if self._no_points(prep):
             return self._no_points_dummy(feat)
         if self.collapse_z:
             bev_feat = torch.cat(bev_feat.unbind(dim=2), 1)
@@ -395,18 +400,14 @@ class LSSViewTransformerRaw(LSSViewTransformer):
             return None
         B, N, C, H, W = tran_feat.shape
         sensor2ego, _e2g, cam2imgs, post_rots, post_trans, bda = input[1:7]
-        prep = _bp.prepare_ranks_calib(self._frustum_on(sensor2ego.device), sensor2ego, cam2imgs,
-                                       post_rots, post_trans, bda, self.grid_lower_bound,
-                                       self.grid_interval, self.grid_size)
-        prep.plan.sync_free = self.sync_free
-        if self.prepared_hook is not None:
-            self.prepared_hook()
+        prep = self._prepared(_bp.prepare_ranks_calib(
+            self._frustum_on(sensor2ego.device), sensor2ego, cam2imgs, post_rots, post_trans, bda,
+            self.grid_lower_bound, self.grid_interval, self.grid_size))
         feat_last = tran_feat.reshape(B, N, C, H, W).permute(0, 1, 3, 4, 2)
         d5 = depth.reshape(B, N, self.D, H, W)
         out = _bp.pool_prepared_maxdown(d5, feat_last, prep, self._bev_shape(d5, C))
-        if out is not None and not self.sync_free and prep.plan.n_intervals == 0:
-            return None     # let the plain route reproduce the reference's empty-input behaviour
-        return out
+        # None also lets the plain route reproduce the reference's empty-input behaviour
+        return None if out is None or self._no_points(prep) else out
 
     def _forward_downsampled(self, input, depth):
         """Inference path: pooling and the 2x2x2 maximum in one kernel, the full-resolution
@@ -422,15 +423,10 @@ class LSSViewTransformerRaw(LSSViewTransformer):
         coor = self.get_lidar_coor(*input[1:7])
         if coor.numel() == 0:
             return None
-        prep = _bp.prepare_ranks(coor, self.grid_lower_bound, self.grid_interval, self.grid_size)
-        prep.plan.sync_free = self.sync_free
-        if self.prepared_hook is not None:
-            self.prepared_hook()
+        prep = self._prepared(_bp.prepare_ranks(coor, self.grid_lower_bound, self.grid_interval,
+                                                self.grid_size))
         feat_last = tran_feat.reshape(B, N, C, H, W).permute(0, 1, 3, 4, 2)
         d5 = depth.reshape(B, N, self.D, H, W)
         out = _bp.pool_prepared_downsampled(d5, feat_last, prep, self._bev_shape(d5, C))
-        if out is None:
-            return None
-        if not self.sync_free and prep.plan.n_intervals == 0:
-            return None     # let the plain route reproduce the reference's empty-input behaviour
-        return out
+        # None also lets the plain route reproduce the reference's empty-input behaviour
+        return None if out is None or self._no_points(prep) else out
