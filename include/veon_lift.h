@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define VEON_ABI_VERSION 9
+#define VEON_ABI_VERSION 10
 
 #define VEON_E_BADARG    (-1)  /* NULL pointer / non-positive dimension          */
 #define VEON_E_WORKSPACE (-2)  /* workspace smaller than *_workspace_bytes()     */
@@ -294,6 +294,38 @@ int veon_bev_pool_v2_fwd_planar_cl(const float* depth, const float* feat,
                                    int64_t n_feat_rows /* B*N*H*W rows of feat */,
                                    float* out, void* stream);
 
+/* bfloat16 volumes.  The same pooling as veon_bev_pool_v2_fwd_planar / _cl (same arguments, same
+ * checks and error codes, same kernel selection), but `out` holds bfloat16 bit patterns: every
+ * sum is accumulated in float32 exactly as the float32 twin does and rounded once, when it is
+ * stored, to nearest even (as `cvt.rn.bf16.f32` does, which is what torch's device-side cast to
+ * bfloat16 uses).  So the result is, bit for bit, the float32 twin's volume cast to bfloat16.
+ * out must be 8-byte aligned for the vector stores (an unaligned one takes scalar stores).  The
+ * channels-first one never takes the streaming kernel: its workspace arguments are accepted and
+ * ignored. */
+int veon_bev_pool_v2_fwd_planar_bf16(const float* depth, const float* feat,
+                                     const int32_t* ranks_depth,
+                                     const int32_t* ranks_feat,
+                                     const int32_t* ranks_bev,
+                                     const int32_t* tile_start,
+                                     const int32_t* tile_istart /* may be NULL */,
+                                     const uint32_t* tile_occ /* may be NULL */,
+                                     const int32_t* tile_heavy /* may be NULL */,
+                                     int64_t tile_heavy_ints /* its size in int32 */,
+                                     int B, int C, int64_t voxels_per_sample,
+                                     int64_t n_feat_rows /* B*N*H*W rows of feat */,
+                                     uint16_t* out /* bfloat16 [B,C,Z,Y,X] */,
+                                     void* workspace, size_t workspace_bytes, void* stream);
+int veon_bev_pool_v2_fwd_planar_cl_bf16(const float* depth, const float* feat,
+                                        const int32_t* ranks_depth,
+                                        const int32_t* ranks_feat,
+                                        const int32_t* ranks_bev,
+                                        const int32_t* tile_start,
+                                        const int32_t* tile_heavy /* may be NULL */,
+                                        int64_t tile_heavy_ints /* its size in int32 */,
+                                        int B, int C, int64_t voxels_per_sample,
+                                        int64_t n_feat_rows /* B*N*H*W rows of feat */,
+                                        uint16_t* out /* bfloat16 [B,Z,Y,X,C] */, void* stream);
+
 /* Pooling fused with the 2x2x2 max-downsample VEON's neck applies next
  * (view_transformer_raw.py:549-553), forward only: out is [B, C, Z/2, Y/2, X/2], bit-identical
  * to that maximum over the volume veon_bev_pool_v2_fwd_planar would write (never materialised).
@@ -374,6 +406,31 @@ int veon_bev_pool_v2_bwd_planar_cl(const float* out_grad,
                                    int B, int N, int D, int H, int W, int C,
                                    int64_t voxels_per_sample,
                                    float* depth_grad, float* feat_grad, void* stream);
+
+/* The two backward routes above for a bfloat16 out_grad (uint16_t bit patterns; same arguments,
+ * checks and error codes as the float32 twins; rows_ws is the same float32 scratch, sized by
+ * veon_bev_pool_v2_bwd_workspace_floats).  Every gradient value is widened to float32 exactly
+ * where it is read, and everything after that is the float32 twin's arithmetic: depth_grad /
+ * feat_grad (float32) are the same bits as the twin's given the widened gradient. */
+int veon_bev_pool_v2_bwd_planar_bf16(const uint16_t* out_grad /* bfloat16 [B,C,Z,Y,X] */,
+                                     const float* depth, const float* feat,
+                                     const int32_t* tile_istart,
+                                     const uint32_t* tile_occ,
+                                     const int32_t* point_interval,
+                                     int64_t n_intervals,
+                                     int B, int N, int D, int H, int W, int C,
+                                     int64_t voxels_per_sample,
+                                     float* rows_ws, int64_t rows_ws_floats,
+                                     float* depth_grad, float* feat_grad,
+                                     void* stream);
+int veon_bev_pool_v2_bwd_planar_cl_bf16(const uint16_t* out_grad /* bfloat16 [B,Z,Y,X,C] */,
+                                        const float* depth, const float* feat,
+                                        const int32_t* ranks_bev,
+                                        const int32_t* interval_starts,
+                                        const int32_t* point_interval,
+                                        int B, int N, int D, int H, int W, int C,
+                                        int64_t voxels_per_sample,
+                                        float* depth_grad, float* feat_grad, void* stream);
 
 /* QuickCumsumCuda.backward for a gradient that arrives BEHIND the 2x2x2 max-downsample:
  * grad_ds [B,C,Z/2,Y/2,X/2] and the mask of veon_maxdown2_fwd_mask replace out_grad; the

@@ -21,6 +21,12 @@ tensors.  Everything runs in CUDA through the C ABI; there is no CPU path.
 same [B,C,Z,Y,X] values stored channels-last ([B,Z,Y,X,C] underneath), written
 that way by the kernels; a channels-last gradient is consumed in place by a
 single-pass backward, whichever layout the forward produced.
+
+`dtype=torch.bfloat16` (bev_pool_v2 / pool_prepared, either memory format) returns
+the volume in bfloat16, written so by the kernels: float32 sums rounded once, at
+the store, so the result is bit for bit the float32 volume cast to bfloat16.  Its
+bfloat16 gradient is read in place and widened exactly (depth / feat gradients
+stay float32).
 """
 import collections
 import functools
@@ -50,6 +56,17 @@ def _channels_last(memory_format):
         raise ValueError("memory_format must be torch.contiguous_format or torch.channels_last_3d, "
                          f"got {memory_format!r}")
     return memory_format is torch.channels_last_3d
+
+
+_DTYPES = (torch.float32, torch.bfloat16)
+
+
+def _bf16(dtype):
+    """True for torch.bfloat16, False for torch.float32; ValueError otherwise (float16 overflows
+    where the float32 sums do not: another contract)."""
+    if not isinstance(dtype, torch.dtype) or dtype not in _DTYPES:
+        raise ValueError(f"dtype must be torch.float32 or torch.bfloat16, got {dtype!r}")
+    return dtype is torch.bfloat16
 
 
 # Opt-in device timing of the library calls (bench.py / profiling only): CUDA
@@ -661,29 +678,34 @@ def _fwd_workspace(lib, dev, B, C, V):
     return ws
 
 
-def _fwd_planar(depth, feat, rd, rf, rb, plan, B, C, V, shape5, channels_last=False):
-    """Planar forward of a valid plan into a new volume `shape5`: [B,C,Z,Y,X], or [B,Z,Y,X,C]
-    with channels_last (the streaming kernel and its workspace are channels-first only)."""
+def _fwd_planar(depth, feat, rd, rf, rb, plan, B, C, V, shape5, channels_last=False,
+                dtype=torch.float32):
+    """Planar forward of a valid plan into a new volume `shape5` of `dtype` (float32 or
+    bfloat16): [B,C,Z,Y,X], or [B,Z,Y,X,C] with channels_last (the streaming kernel and its
+    workspace are float32 channels-first only)."""
     lib = _lib.load()
     dev = feat.device
+    bf16 = dtype is torch.bfloat16
+    suffix = "_bf16" if bf16 else ""
     with torch.cuda.device(dev):
-        out = torch.empty(shape5, dtype=torch.float32, device=dev)
+        out = torch.empty(shape5, dtype=dtype, device=dev)
         if channels_last:
-            what = "veon_bev_pool_v2_fwd_planar_cl"
-            with _timed("pool_fwd_cl", dev):
-                rc = lib.veon_bev_pool_v2_fwd_planar_cl(
+            what = "veon_bev_pool_v2_fwd_planar_cl" + suffix
+            with _timed("pool_fwd_cl" + suffix, dev):
+                rc = getattr(lib, what)(
                     _ptr(depth), _ptr(feat), _ptr(rd), _ptr(rf), _ptr(rb), _ptr(plan.tile_start),
                     _ptr(plan.tile_heavy), plan.tile_heavy.numel(), B, C, V, feat.numel() // C,
                     _ptr(out), _stream_ptr(dev))
         else:
-            what = "veon_bev_pool_v2_fwd_planar"
-            ws = _fwd_workspace(lib, dev, B, C, V)
-            with _timed("pool_fwd", dev):
-                rc = lib.veon_bev_pool_v2_fwd_planar(
+            what = "veon_bev_pool_v2_fwd_planar" + suffix
+            ws = None if bf16 else _fwd_workspace(lib, dev, B, C, V)
+            with _timed("pool_fwd" + suffix, dev):
+                rc = getattr(lib, what)(
                     _ptr(depth), _ptr(feat), _ptr(rd), _ptr(rf), _ptr(rb), _ptr(plan.tile_start),
                     _ptr(plan.tile_istart), _ptr(plan.tile_occ),
                     _ptr(plan.tile_heavy), plan.tile_heavy.numel(),
-                    B, C, V, feat.numel() // C, _ptr(out), _ptr(ws), ws.numel(), _stream_ptr(dev))
+                    B, C, V, feat.numel() // C, _ptr(out), None if bf16 else _ptr(ws),
+                    0 if bf16 else ws.numel(), _stream_ptr(dev))
     _lib.check(rc, what)
     return out
 
@@ -708,17 +730,20 @@ def _bwd_rows(lib, plan, C, dev):
 
 def _pool_bwd(out_grad, depth, feat, rd, rf, rb, ist, plan):
     """(depth_grad, feat_grad) for the gradient of a [B,Z,Y,X,C] volume, routed by its storage:
-    float32 channels-last (out_grad contiguous, its [B,C,Z,Y,X] view not) with a valid plan ->
-    the single pass, which reads the gradient rows in place; otherwise a valid plan -> the two
-    passes on a float32 channels-first copy; a rejected plan -> the generic kernel."""
+    float32 or bfloat16 channels-last (out_grad contiguous, its [B,C,Z,Y,X] view not) with a
+    valid plan -> the single pass, which reads the gradient rows in place; otherwise a valid plan
+    -> the two passes on a channels-first copy (bfloat16 stays bfloat16, anything else becomes
+    float32); a rejected plan -> the generic kernel on a float32 copy."""
     lib = _lib.load()
     dev = feat.device
     _, Z, Y, X, C = out_grad.shape
     g = out_grad.permute(0, 4, 1, 2, 3)  # back to the channels-first storage order
-    single = (out_grad.dtype == torch.float32 and not g.is_contiguous()
+    bf16 = out_grad.dtype == torch.bfloat16 and plan.ok
+    suffix = "_bf16" if bf16 else ""
+    single = ((out_grad.dtype == torch.float32 or bf16) and not g.is_contiguous()
               and out_grad.is_contiguous() and plan.ok)
     if not single:
-        g = g.float().contiguous()
+        g = g.contiguous() if bf16 else g.float().contiguous()
     with torch.cuda.device(dev):
         if not plan.ok:
             what = "veon_bev_pool_v2_grad_generic"
@@ -731,17 +756,17 @@ def _pool_bwd(out_grad, depth, feat, rd, rf, rb, ist, plan):
             B, N, D, H, W = plan.dims
             depth_grad, feat_grad = torch.empty_like(depth), torch.empty_like(feat)
             if single:
-                what = "veon_bev_pool_v2_bwd_planar_cl"
-                with _timed("pool_bwd_cl", dev):
-                    rc = lib.veon_bev_pool_v2_bwd_planar_cl(
+                what = "veon_bev_pool_v2_bwd_planar_cl" + suffix
+                with _timed("pool_bwd_cl" + suffix, dev):
+                    rc = getattr(lib, what)(
                         _ptr(out_grad), _ptr(depth), _ptr(feat), _ptr(rb), _ptr(ist),
                         _ptr(plan.point_interval), B, N, D, H, W, C, plan.V, _ptr(depth_grad),
                         _ptr(feat_grad), _stream_ptr(dev))
             else:
-                what = "veon_bev_pool_v2_bwd_planar"
+                what = "veon_bev_pool_v2_bwd_planar" + suffix
                 n_int, rows = _bwd_rows(lib, plan, C, dev)
-                with _timed("pool_bwd", dev):
-                    rc = lib.veon_bev_pool_v2_bwd_planar(
+                with _timed("pool_bwd" + suffix, dev):
+                    rc = getattr(lib, what)(
                         _ptr(g), _ptr(depth), _ptr(feat), _ptr(plan.tile_istart),
                         _ptr(plan.tile_occ), _ptr(plan.point_interval), n_int, B, N, D, H, W, C,
                         plan.V, _ptr(rows), rows.numel(), _ptr(depth_grad), _ptr(feat_grad),
@@ -761,15 +786,17 @@ class QuickCumsumCuda(torch.autograd.Function):
     storage -> the two-pass kernels; channels-last storage (a contiguous
     [B,Z,Y,X,C] gradient) with a valid plan -> the single-pass kernel, which reads
     the gradient rows in place; anything else is copied to channels-first first.
-    All routes give the same bits."""
+    All routes give the same bits.  With the extra `dtype` torch.bfloat16 the volume is
+    bfloat16 (the float32 one rounded once), and so is the gradient the backward reads."""
 
     @staticmethod
     def forward(ctx, depth, feat, ranks_depth, ranks_feat, ranks_bev,
                 bev_feat_shape, interval_starts, interval_lengths, *extra):
-        # `extra` = (PoolPlan or None[, channels_last]) when called from this package; the
-        # reference's 8-argument call is accepted unchanged
+        # `extra` = (PoolPlan or None[, channels_last[, dtype]]) when called from this package;
+        # the reference's 8-argument call is accepted unchanged
         plan = extra[0] if extra else None
         channels_last = bool(extra[1]) if len(extra) > 1 else False
+        dtype = extra[2] if len(extra) > 2 else torch.float32
         ctx.n_extra = len(extra)
         _require_cuda(depth, feat, ranks_depth, ranks_feat, ranks_bev,
                      interval_starts, interval_lengths)
@@ -798,7 +825,7 @@ class QuickCumsumCuda(torch.autograd.Function):
         shape5 = (B, Z, Y, X, C) if channels_last else (B, C, Z, Y, X)
         if plan.ok:
             out = _fwd_planar(depth, feat, ranks_depth, ranks_feat, ranks_bev, plan, B, C, V,
-                              shape5, channels_last)
+                              shape5, channels_last, dtype)
         else:
             # the interval-driven generic kernel adds into a zeroed volume
             lib = _lib.load()
@@ -810,6 +837,7 @@ class QuickCumsumCuda(torch.autograd.Function):
                     _ptr(interval_starts), _ptr(interval_lengths), _ptr(out),
                     _stream_ptr(feat.device))
             _lib.check(rc, "veon_bev_pool_v2_generic")
+            out = out.to(dtype)     # bfloat16: the same single rounding of the float32 sums
         ctx.save_for_backward(ranks_bev, depth, feat, ranks_feat, ranks_depth, interval_starts)
         ctx.plan = plan
         return out if channels_last else out.permute(0, 2, 3, 4, 1)
@@ -825,16 +853,19 @@ class QuickCumsumCuda(torch.autograd.Function):
 
 def bev_pool_v2(depth, feat, ranks_depth, ranks_feat, ranks_bev,
                 bev_feat_shape, interval_starts, interval_lengths, *,
-                memory_format=torch.contiguous_format):
+                memory_format=torch.contiguous_format, dtype=torch.float32):
     """Drop-in for the reference `bev_pool_v2` (bev_pool.py:86-92).
 
     depth [B,N,D,H,W]; feat [B,N,H,W,C] (any strides); int32 rank / interval
     tensors; bev_feat_shape = (B,Z,Y,X,C).  Returns [B,C,Z,Y,X] float32,
     differentiable w.r.t. depth and feat: contiguous, or with
     memory_format=torch.channels_last_3d the same values stored channels-last
-    (written so by the kernels, not copied)."""
+    (written so by the kernels, not copied).  dtype=torch.bfloat16 returns the
+    volume in bfloat16: the float32 result rounded to nearest even, bit for bit,
+    with no float32 volume in between."""
     cl = _channels_last(memory_format)
-    extra = (None, True) if cl else ()
+    bf16 = _bf16(dtype)
+    extra = (None, cl, dtype) if bf16 else ((None, True) if cl else ())
     x = QuickCumsumCuda.apply(depth, feat, ranks_depth, ranks_feat, ranks_bev,
                               bev_feat_shape, interval_starts, interval_lengths, *extra)
     x = x.permute(0, 4, 1, 2, 3)
@@ -842,12 +873,14 @@ def bev_pool_v2(depth, feat, ranks_depth, ranks_feat, ranks_bev,
     return x if cl else x.contiguous()
 
 
-def pool_prepared(depth, feat, prep, bev_feat_shape, memory_format=torch.contiguous_format):
+def pool_prepared(depth, feat, prep, bev_feat_shape, memory_format=torch.contiguous_format, *,
+                  dtype=torch.float32):
     """bev_pool_v2 on a `PreparedRanks` without any host synchronisation in the
     forward (the counts are only needed, and by then long available, when the
-    backward sizes its scratch).  memory_format as in bev_pool_v2."""
+    backward sizes its scratch).  memory_format and dtype as in bev_pool_v2."""
     cl = _channels_last(memory_format)
-    extra = (prep.plan, True) if cl else (prep.plan,)
+    bf16 = _bf16(dtype)
+    extra = (prep.plan, cl, dtype) if bf16 else ((prep.plan, True) if cl else (prep.plan,))
     x = QuickCumsumCuda.apply(depth, feat, prep.ranks_depth, prep.ranks_feat, prep.ranks_bev,
                               bev_feat_shape, prep.interval_starts, prep.interval_lengths, *extra)
     x = x.permute(0, 4, 1, 2, 3)

@@ -1,5 +1,6 @@
 // Shared helpers for libveonlift (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdlib.h>
@@ -126,6 +127,51 @@ __device__ __forceinline__ float ld_stream(const float* p) {
   float v;
   asm volatile("ld.global.cs.f32 %0, [%1];" : "=f"(v) : "l"(p));
   return v;
+}
+
+// bfloat16 volumes and gradients.  Sums stay float32; a stored value is rounded once, to nearest
+// even (cvt.rn.bf16.f32, as torch's device-side cast), and a loaded one is widened exactly.  The
+// overloads take the float32 helpers' element counts: st_stream4 / ld_stream4 move four elements,
+// which for bfloat16 is one 8-byte access (8-byte aligned).
+using bf16 = __nv_bfloat16;
+__device__ __forceinline__ uint32_t bf16x2_bits(float lo, float hi) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);   // .x = lo at the lower address
+  return (uint32_t)__bfloat16_as_ushort(h.x) | ((uint32_t)__bfloat16_as_ushort(h.y) << 16);
+}
+__device__ __forceinline__ void st_stream(bf16* p, float v) {
+  asm volatile("st.global.cs.b16 [%0], %1;" ::"l"(p), "h"(__bfloat16_as_ushort(__float2bfloat16_rn(v)))
+               : "memory");
+}
+__device__ __forceinline__ void st_stream4(bf16* p, float4 v) {
+  asm volatile("st.global.cs.v2.b32 [%0], {%1, %2};" ::"l"(p), "r"(bf16x2_bits(v.x, v.y)),
+               "r"(bf16x2_bits(v.z, v.w))
+               : "memory");
+}
+__device__ __forceinline__ float widen(float v) { return v; }
+__device__ __forceinline__ float widen(bf16 v) {
+  return __uint_as_float((uint32_t)__bfloat16_as_ushort(v) << 16);
+}
+__device__ __forceinline__ float4 ld_stream4(const bf16* p) {
+  uint32_t a, b;
+  asm volatile("ld.global.cs.v2.b32 {%0, %1}, [%2];" : "=r"(a), "=r"(b) : "l"(p));
+  // (not make_float4: another caller of it changes how the float kernels around it are inlined,
+  //  and their code must stay as it is)
+  float4 r;
+  r.x = __uint_as_float(a << 16);
+  r.y = __uint_as_float(a & 0xffff0000u);
+  r.z = __uint_as_float(b << 16);
+  r.w = __uint_as_float(b & 0xffff0000u);
+  return r;
+}
+__device__ __forceinline__ float ld_stream(const bf16* p) {
+  unsigned short h;
+  asm volatile("ld.global.cs.b16 %0, [%1];" : "=h"(h) : "l"(p));
+  return __uint_as_float((uint32_t)h << 16);
+}
+// read-only path, widened
+__device__ __forceinline__ float ldg_widen(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ldg_widen(const bf16* p) {
+  return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
 }
 
 __device__ __forceinline__ float warp_sum(float v) {

@@ -25,6 +25,8 @@
 // (ascending depth bin) => bitwise run-to-run deterministic.
 // A channels-last out_grad [B,Z,Y,X,C] already holds every occupied voxel's gradient as one
 // contiguous row: k_bwd_pixels<KCH, true> reads those rows in place (no row pass, no scratch).
+// A bfloat16 out_grad (template parameter T = bf16) is widened exactly where it is read: into the
+// float compact rows (row pass) or into registers (single pass); all arithmetic stays float.
 #include "common.cuh"
 
 namespace veon {
@@ -37,8 +39,8 @@ constexpr int kRowWarps = VEON_ROW_WARPS;   // row pass
 constexpr int kPitch = kTileVoxels + 1;
 
 // one warp: tile t, channel chunk starting at cbase -> compact rows
-template <int KCH>
-__device__ __forceinline__ void rows_tile(float* tile, int lane, const float* __restrict__ out_grad,
+template <int KCH, typename T>
+__device__ __forceinline__ void rows_tile(float* tile, int lane, const T* __restrict__ out_grad,
                                           const int32_t* __restrict__ tile_istart,
                                           const uint32_t* __restrict__ tile_occ, int64_t t,
                                           int cbase, int64_t tiles_per_sample, int64_t V, int C,
@@ -57,7 +59,7 @@ __device__ __forceinline__ void rows_tile(float* tile, int lane, const float* __
   const int q4 = (lane & 7) * 4, r = lane >> 3;
   const bool want = ((occ >> (q4 & 24)) & 0xffu) != 0u;
   if (vec_ok && v0 + kTileVoxels <= V) {
-    const float* g = out_grad + ((int64_t)b * C + cbase + r) * V + v0 + q4;
+    const T* g = out_grad + ((int64_t)b * C + cbase + r) * V + v0 + q4;
     float* trow = tile + r * kPitch + q4;
     if (cmax == CC) {  // all CC/4 loads of the lane in flight at once
       float4 v[CC / 4];
@@ -78,7 +80,7 @@ __device__ __forceinline__ void rows_tile(float* tile, int lane, const float* __
     }
   } else {
     const bool wants = ((occ >> (lane & 24)) & 0xffu) != 0u && (v0 + lane < V);
-    const float* g = out_grad + ((int64_t)b * C + cbase) * V + v0 + lane;
+    const T* g = out_grad + ((int64_t)b * C + cbase) * V + v0 + lane;
     for (int cl = 0; cl < cmax; ++cl)
       tile[cl * kPitch + lane] = wants ? ld_stream(g + (int64_t)cl * V) : 0.f;
   }
@@ -96,9 +98,9 @@ __device__ __forceinline__ void rows_tile(float* tile, int lane, const float* __
   }
 }
 
-template <int KCH>
+template <int KCH, typename T = float>
 __global__ void __launch_bounds__(kRowWarps * 32)
-k_bwd_rows(const float* __restrict__ out_grad, const int32_t* __restrict__ tile_istart,
+k_bwd_rows(const T* __restrict__ out_grad, const int32_t* __restrict__ tile_istart,
            const uint32_t* __restrict__ tile_occ, int64_t tile_begin, int64_t tile_end,
            int64_t tiles_per_sample, int64_t V, int C, int n_chunks, int vec_ok,
            float* __restrict__ rows) {
@@ -126,10 +128,19 @@ __device__ __forceinline__ void cp_async16_cg(void* smem_dst, const void* gsrc) 
   const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
 }
+// four voxels of a channel plane: 16 bytes of float, 8 of bf16 (cp.async.cg copies 16 bytes only)
+__device__ __forceinline__ void cp_async_4(float* smem_dst, const float* gsrc) {
+  cp_async16_cg(smem_dst, gsrc);
+}
+__device__ __forceinline__ void cp_async_4(bf16* smem_dst, const bf16* gsrc) {
+  const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(d), "l"(gsrc) : "memory");
+}
 
-template <int KCH>
+// T = bf16: the shared tiles hold the gradient's own bf16 values, widened as the rows are extracted.
+template <int KCH, typename T = float>
 __global__ void __launch_bounds__(kRowWarps * 32)
-k_bwd_rows_persistent(const float* __restrict__ out_grad, const int32_t* __restrict__ tile_istart,
+k_bwd_rows_persistent(const T* __restrict__ out_grad, const int32_t* __restrict__ tile_istart,
                       const uint32_t* __restrict__ tile_occ, int64_t n_items,
                       int64_t tiles_per_sample, int64_t V, int C, int n_chunks,
                       float* __restrict__ rows) {
@@ -137,7 +148,7 @@ k_bwd_rows_persistent(const float* __restrict__ out_grad, const int32_t* __restr
   constexpr int kBuf = CC * kRowPitchP;
   extern __shared__ __align__(16) float smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  float* buf = smem + warp * 2 * kBuf;
+  T* buf = reinterpret_cast<T*>(smem) + warp * 2 * kBuf;
   const int64_t TW = (int64_t)gridDim.x * kRowWarps;
   const int64_t first = (int64_t)blockIdx.x * kRowWarps + warp;
   if (first >= n_items) return;
@@ -155,7 +166,7 @@ k_bwd_rows_persistent(const float* __restrict__ out_grad, const int32_t* __restr
     }
   };
   // rows of the tile sitting in `tile`: j-th occupied voxel -> interval i0 + j
-  auto extract = [&](const float* tile, uint32_t occ, int32_t i0, int cbase) {
+  auto extract = [&](const T* tile, uint32_t occ, int32_t i0, int cbase) {
     const int cmax = min(CC, C - cbase);
     float* row = rows + (int64_t)i0 * C + cbase + lane;
     uint32_t rest = occ;
@@ -164,7 +175,7 @@ k_bwd_rows_persistent(const float* __restrict__ out_grad, const int32_t* __restr
       rest &= rest - 1;
 #pragma unroll
       for (int k = 0; k < KCH; ++k)
-        if (lane + 32 * k < cmax) row[32 * k] = tile[(lane + 32 * k) * kRowPitchP + vj];
+        if (lane + 32 * k < cmax) row[32 * k] = widen(tile[(lane + 32 * k) * kRowPitchP + vj]);
       row += C;
     }
   };
@@ -188,11 +199,11 @@ k_bwd_rows_persistent(const float* __restrict__ out_grad, const int32_t* __restr
       const int cmax = min(CC, C - cbase);
       // only the 32-byte sectors (8 voxels) that contain an occupied voxel
       if (((occ >> (q4 & 24)) & 0xffu) != 0u) {
-        const float* g = out_grad + ((int64_t)b * C + cbase + r) * V + v0 + q4;
-        float* dst = buf + cur * kBuf + r * kRowPitchP + q4;
+        const T* g = out_grad + ((int64_t)b * C + cbase + r) * V + v0 + q4;
+        T* dst = buf + cur * kBuf + r * kRowPitchP + q4;
 #pragma unroll
         for (int it = 0; it < CC / 4; ++it)
-          if (4 * it + r < cmax) cp_async16_cg(dst + it * 4 * kRowPitchP, g + (int64_t)it * 4 * V);
+          if (4 * it + r < cmax) cp_async_4(dst + it * 4 * kRowPitchP, g + (int64_t)it * 4 * V);
       }
       asm volatile("cp.async.commit_group;" ::: "memory");
       if (p_occ) {
@@ -396,8 +407,9 @@ __device__ __forceinline__ float reduce_many(float (&d)[U], int lane, int& which
 // CL: `rows` is a channels-last out_grad [B*V, C] itself; a kept point's row is that of its
 // voxel, ranks_bev[interval_starts[interval]] (only intervals a kept point names are read, so a
 // capacity-sized interval_starts is never read past the device-side interval count).
-template <int KCH, bool COHERENT, bool CL = false>
-__device__ __forceinline__ void pixel_warp(float* wsm, int lane, const float* __restrict__ rows,
+// T = bf16 (CL only): the gradient rows are bf16, widened in registers.
+template <int KCH, bool COHERENT, bool CL = false, typename T = float>
+__device__ __forceinline__ void pixel_warp(float* wsm, int lane, const T* __restrict__ rows,
                                            const float* __restrict__ depth,
                                            const float* __restrict__ feat,
                                            const int32_t* __restrict__ point_interval,
@@ -454,11 +466,14 @@ __device__ __forceinline__ void pixel_warp(float* wsm, int lane, const float* __
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int j = min(j0 + u, nk - 1);
-        const float* row = rows + (int64_t)iis[j] * C + cbase + lane;
+        const T* row = rows + (int64_t)iis[j] * C + cbase + lane;
 #pragma unroll
-        for (int k = 0; k < KCH; ++k)
-          g[u][k] = (cbase + lane + 32 * k < C) ? (COHERENT ? __ldcg(row + 32 * k) : __ldg(row + 32 * k))
-                                                : 0.f;
+        for (int k = 0; k < KCH; ++k) {
+          if constexpr (COHERENT)
+            g[u][k] = (cbase + lane + 32 * k < C) ? __ldcg(row + 32 * k) : 0.f;
+          else
+            g[u][k] = (cbase + lane + 32 * k < C) ? ldg_widen(row + 32 * k) : 0.f;
+        }
       }
       float dot[U];
 #pragma unroll
@@ -492,9 +507,9 @@ __device__ __forceinline__ void pixel_warp(float* wsm, int lane, const float* __
 // CL: the single-pass channels-last backward (rows = out_grad [B,Z,Y,X,C], no row pass).  (Its
 // KCH = 8 instance spills 24 bytes at the register count ptxas picks on its own; the minimum of
 // one CTA per SM lets it keep everything in registers.)
-template <int KCH, bool CL = false>
+template <int KCH, bool CL = false, typename T = float>
 __global__ void __launch_bounds__(kBwdWarps * 32, CL ? 1 : 0)
-k_bwd_pixels(const float* __restrict__ rows, const float* __restrict__ depth,
+k_bwd_pixels(const T* __restrict__ rows, const float* __restrict__ depth,
              const float* __restrict__ feat, const int32_t* __restrict__ point_interval,
              const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ interval_starts,
              int64_t pix_begin, int64_t pix_end, int D, int HW, int C,
@@ -503,7 +518,7 @@ k_bwd_pixels(const float* __restrict__ rows, const float* __restrict__ depth,
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t pix = pix_begin + (int64_t)blockIdx.x * kBwdWarps + warp;
   if (pix >= pix_end) return;
-  pixel_warp<KCH, false, CL>(smem + (size_t)warp * 4 * D, lane, rows, depth, feat, point_interval,
+  pixel_warp<KCH, false, CL, T>(smem + (size_t)warp * 4 * D, lane, rows, depth, feat, point_interval,
                              ranks_bev, interval_starts, pix, D, HW, C, depth_grad, feat_grad);
 }
 
@@ -514,33 +529,33 @@ k_bwd_pixels(const float* __restrict__ rows, const float* __restrict__ depth,
 // in L2 next to the 120 MB of out_grad a sample streams, evict-first / evict-last hints or not:
 // 491 us against 324 us for the two launches below.  profiles/README.md has the role timeline.)
 
-template <int KCH>
-static int launch_rows(const float* out_grad, const int32_t* tile_istart, const uint32_t* tile_occ,
+template <int KCH, typename T>
+static int launch_rows(const T* out_grad, const int32_t* tile_istart, const uint32_t* tile_occ,
                        int64_t tile_begin, int64_t tile_end, int64_t tps, int64_t V, int C,
                        float* rows, cudaStream_t stream) {
   constexpr int CC = 32 * KCH;
   const size_t smem = sizeof(float) * kRowWarps * CC * kPitch;
-  const size_t psmem = sizeof(float) * kRowWarps * 2 * CC * kRowPitchP;
+  const size_t psmem = sizeof(T) * kRowWarps * 2 * CC * kRowPitchP;
   static int ctas_per_sm[kMaxDevices] = {};
   const int dev = current_device();
   if (ctas_per_sm[dev] == 0) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_rows<KCH>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_rows<KCH, T>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_rows_persistent<KCH>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_rows_persistent<KCH, T>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem));
     int n = 0;
     VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
-        &n, k_bwd_rows_persistent<KCH>, kRowWarps * 32, psmem));
+        &n, k_bwd_rows_persistent<KCH, T>, kRowWarps * 32, psmem));
     ctas_per_sm[dev] = n < 1 ? 1 : n;
   }
   const int n_chunks = (C + CC - 1) / CC;
-  const int vec_ok = ((V & 3) == 0) && (((uintptr_t)out_grad & 15) == 0);
+  const int vec_ok = ((V & 3) == 0) && (((uintptr_t)out_grad & (4 * sizeof(T) - 1)) == 0);
   if (vec_ok && (V % kTileVoxels) == 0 && tile_begin == 0) {
     const int64_t n_items = tile_end * n_chunks;
     if (n_items <= 0) return 0;
     int64_t pblocks = (int64_t)ctas_per_sm[dev] * sm_count();
     if (pblocks > ceil_div64(n_items, kRowWarps)) pblocks = ceil_div64(n_items, kRowWarps);
-    k_bwd_rows_persistent<KCH><<<(unsigned)pblocks, kRowWarps * 32, psmem, stream>>>(
+    k_bwd_rows_persistent<KCH, T><<<(unsigned)pblocks, kRowWarps * 32, psmem, stream>>>(
         out_grad, tile_istart, tile_occ, n_items, tps, V, C, n_chunks, rows);
     VEON_LAUNCH_CHECK();
     return 0;
@@ -548,14 +563,14 @@ static int launch_rows(const float* out_grad, const int32_t* tile_istart, const 
   const int64_t blocks = ceil_div64(tile_end - tile_begin, kRowWarps) * n_chunks;
   if (blocks <= 0) return 0;
   if (blocks > 0x7fffffffLL) return VEON_E_RANGE;
-  k_bwd_rows<KCH><<<(unsigned)blocks, kRowWarps * 32, smem, stream>>>(
+  k_bwd_rows<KCH, T><<<(unsigned)blocks, kRowWarps * 32, smem, stream>>>(
       out_grad, tile_istart, tile_occ, tile_begin, tile_end, tps, V, C, n_chunks, vec_ok, rows);
   VEON_LAUNCH_CHECK();
   return 0;
 }
 
-template <int KCH, bool CL>
-static int launch_pixels(const float* rows, const float* depth, const float* feat,
+template <int KCH, bool CL, typename T>
+static int launch_pixels(const T* rows, const float* depth, const float* feat,
                          const int32_t* point_interval, const int32_t* ranks_bev,
                          const int32_t* interval_starts, int64_t pix_begin, int64_t pix_end,
                          int D, int HW, int C, float* depth_grad, float* feat_grad,
@@ -566,14 +581,14 @@ static int launch_pixels(const float* rows, const float* depth, const float* fea
   const int dev = current_device();
   if (attr_smem[dev] == 0) attr_smem[dev] = 48 * 1024;
   if (smem > attr_smem[dev]) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_pixels<KCH, CL>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_pixels<KCH, CL, T>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_smem[dev] = smem;
   }
   const int64_t blocks = ceil_div64(pix_end - pix_begin, kBwdWarps);
   if (blocks <= 0) return 0;
   if (blocks > 0x7fffffffLL) return VEON_E_RANGE;
-  k_bwd_pixels<KCH, CL><<<(unsigned)blocks, kBwdWarps * 32, smem, stream>>>(
+  k_bwd_pixels<KCH, CL, T><<<(unsigned)blocks, kBwdWarps * 32, smem, stream>>>(
       rows, depth, feat, point_interval, ranks_bev, interval_starts, pix_begin, pix_end, D, HW, C,
       depth_grad, feat_grad);
   VEON_LAUNCH_CHECK();
@@ -581,7 +596,8 @@ static int launch_pixels(const float* rows, const float* depth, const float* fea
 }
 
 // the compact rows of tiles [0, n_tiles)
-static int row_pass(const float* out_grad, const int32_t* tile_istart, const uint32_t* tile_occ,
+template <typename T>
+static int row_pass(const T* out_grad, const int32_t* tile_istart, const uint32_t* tile_occ,
                     int64_t n_tiles, int64_t tps, int64_t V, int C, float* rows,
                     cudaStream_t stream) {
   return C <= 32 ? launch_rows<1>(out_grad, tile_istart, tile_occ, 0, n_tiles, tps, V, C, rows, stream)
@@ -589,12 +605,12 @@ static int row_pass(const float* out_grad, const int32_t* tile_istart, const uin
 }
 
 // ranks_bev / interval_starts: the channels-last pass (rows = out_grad), else NULL
-template <bool CL = false>
-static int pixel_pass(const float* rows, const float* depth, const float* feat,
+template <bool CL = false, typename T = float>
+static int pixel_pass(const T* rows, const float* depth, const float* feat,
                       const int32_t* point_interval, int64_t pixels, int D, int HW, int C,
                       float* depth_grad, float* feat_grad, cudaStream_t stream,
                       const int32_t* ranks_bev = nullptr, const int32_t* interval_starts = nullptr) {
-#define VEON_PIX(K_) launch_pixels<K_, CL>(rows, depth, feat, point_interval, ranks_bev, interval_starts, 0, pixels, D, HW, C, depth_grad, feat_grad, stream)
+#define VEON_PIX(K_) launch_pixels<K_, CL, T>(rows, depth, feat, point_interval, ranks_bev, interval_starts, 0, pixels, D, HW, C, depth_grad, feat_grad, stream)
   switch (C <= 32 ? 1 : (C <= 64 ? 2 : (C <= 256 ? 4 : 8))) {   // channels per lane
     case 1: return VEON_PIX(1);
     case 2: return VEON_PIX(2);
@@ -618,12 +634,13 @@ extern "C" size_t veon_bev_pool_v2_bwd_workspace_floats(int64_t n_intervals, int
   return (size_t)(n_intervals > 0 ? n_intervals : 1) * (size_t)C;
 }
 
-extern "C" int veon_bev_pool_v2_bwd_planar(
-    const float* out_grad, const float* depth, const float* feat, const int32_t* tile_istart,
-    const uint32_t* tile_occ, const int32_t* point_interval, int64_t n_intervals, int B, int N,
-    int D, int H, int W, int C, int64_t V, float* rows_ws, int64_t rows_ws_floats,
-    float* depth_grad, float* feat_grad, void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
+// The two passes on a channels-first out_grad of float or bf16 elements T (the rows are float).
+template <typename T>
+static int bwd_planar(const T* out_grad, const float* depth, const float* feat,
+                      const int32_t* tile_istart, const uint32_t* tile_occ,
+                      const int32_t* point_interval, int64_t n_intervals, int B, int N, int D,
+                      int H, int W, int C, int64_t V, float* rows_ws, int64_t rows_ws_floats,
+                      float* depth_grad, float* feat_grad, cudaStream_t stream) {
   if (!out_grad || !depth || !feat || !tile_istart || !tile_occ || !point_interval || !rows_ws ||
       !depth_grad || !feat_grad || B <= 0 || N <= 0 || D <= 0 || H <= 0 || W <= 0 || C <= 0 ||
       V <= 0 || n_intervals < 0)
@@ -640,13 +657,35 @@ extern "C" int veon_bev_pool_v2_bwd_planar(
                     depth_grad, feat_grad, stream);
 }
 
+extern "C" int veon_bev_pool_v2_bwd_planar(
+    const float* out_grad, const float* depth, const float* feat, const int32_t* tile_istart,
+    const uint32_t* tile_occ, const int32_t* point_interval, int64_t n_intervals, int B, int N,
+    int D, int H, int W, int C, int64_t V, float* rows_ws, int64_t rows_ws_floats,
+    float* depth_grad, float* feat_grad, void* stream) {
+  return bwd_planar(out_grad, depth, feat, tile_istart, tile_occ, point_interval, n_intervals, B,
+                    N, D, H, W, C, V, rows_ws, rows_ws_floats, depth_grad, feat_grad,
+                    (cudaStream_t)stream);
+}
+
+// bf16 out_grad: the row pass widens it into the same float rows, the pixel pass is unchanged.
+extern "C" int veon_bev_pool_v2_bwd_planar_bf16(
+    const uint16_t* out_grad, const float* depth, const float* feat, const int32_t* tile_istart,
+    const uint32_t* tile_occ, const int32_t* point_interval, int64_t n_intervals, int B, int N,
+    int D, int H, int W, int C, int64_t V, float* rows_ws, int64_t rows_ws_floats,
+    float* depth_grad, float* feat_grad, void* stream) {
+  return bwd_planar(reinterpret_cast<const bf16*>(out_grad), depth, feat, tile_istart, tile_occ,
+                    point_interval, n_intervals, B, N, D, H, W, C, V, rows_ws, rows_ws_floats,
+                    depth_grad, feat_grad, (cudaStream_t)stream);
+}
+
 // Single pass for a channels-last out_grad [B,Z,Y,X,C]: its occupied rows are already contiguous,
 // so the pixel pass reads them in place -- no row pass, no scratch.  Same rows, same order of
 // operations: the same bits as veon_bev_pool_v2_bwd_planar on the channels-first copy.
-extern "C" int veon_bev_pool_v2_bwd_planar_cl(
-    const float* out_grad, const float* depth, const float* feat, const int32_t* ranks_bev,
-    const int32_t* interval_starts, const int32_t* point_interval, int B, int N, int D, int H,
-    int W, int C, int64_t V, float* depth_grad, float* feat_grad, void* stream_) {
+template <typename T>
+static int bwd_planar_cl(const T* out_grad, const float* depth, const float* feat,
+                         const int32_t* ranks_bev, const int32_t* interval_starts,
+                         const int32_t* point_interval, int B, int N, int D, int H, int W, int C,
+                         int64_t V, float* depth_grad, float* feat_grad, void* stream_) {
   if (!out_grad || !depth || !feat || !ranks_bev || !interval_starts || !point_interval ||
       !depth_grad || !feat_grad || B <= 0 || N <= 0 || D <= 0 || H <= 0 || W <= 0 || C <= 0 ||
       V <= 0)
@@ -655,6 +694,24 @@ extern "C" int veon_bev_pool_v2_bwd_planar_cl(
   return pixel_pass<true>(out_grad, depth, feat, point_interval, (int64_t)B * N * H * W, D, H * W,
                           C, depth_grad, feat_grad, (cudaStream_t)stream_, ranks_bev,
                           interval_starts);
+}
+
+extern "C" int veon_bev_pool_v2_bwd_planar_cl(
+    const float* out_grad, const float* depth, const float* feat, const int32_t* ranks_bev,
+    const int32_t* interval_starts, const int32_t* point_interval, int B, int N, int D, int H,
+    int W, int C, int64_t V, float* depth_grad, float* feat_grad, void* stream) {
+  return bwd_planar_cl(out_grad, depth, feat, ranks_bev, interval_starts, point_interval, B, N, D,
+                       H, W, C, V, depth_grad, feat_grad, stream);
+}
+
+// bf16 out_grad rows, read in place and widened in registers: the same float fma chain.
+extern "C" int veon_bev_pool_v2_bwd_planar_cl_bf16(
+    const uint16_t* out_grad, const float* depth, const float* feat, const int32_t* ranks_bev,
+    const int32_t* interval_starts, const int32_t* point_interval, int B, int N, int D, int H,
+    int W, int C, int64_t V, float* depth_grad, float* feat_grad, void* stream) {
+  return bwd_planar_cl(reinterpret_cast<const bf16*>(out_grad), depth, feat, ranks_bev,
+                       interval_starts, point_interval, B, N, D, H, W, C, V, depth_grad,
+                       feat_grad, stream);
 }
 
 extern "C" int veon_bev_pool_v2_bwd_planar_ds(

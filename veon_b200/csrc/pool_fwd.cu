@@ -29,6 +29,8 @@
 //   k_pool_ds_fwd      opt-in: pooling fused with the neck's 2x2x2 max-downsample
 // The first three also write channels-last volumes out[B,Z,Y,X,C] (template flag CL,
 // veon_bev_pool_v2_fwd_planar_cl): same sums, rows instead of channel planes.
+#include <type_traits>
+
 #include "common.cuh"
 #include "pool_fwd.cuh"
 
@@ -73,10 +75,11 @@ __device__ __forceinline__ void cp_async_wait_dist() {
 // Channels-last zeros: voxels [va, vb) of the tile whose first voxel has the global index g0,
 // channels [c0, c0 + cw) of each row.  Whole rows are one contiguous span (16-byte stores when
 // aligned); a channel chunk of a row is one span per voxel.  Warp-wide.
-__device__ __forceinline__ void zero_rows_cl(float* __restrict__ out, int64_t g0, int va, int vb,
+template <typename T>
+__device__ __forceinline__ void zero_rows_cl(T* __restrict__ out, int64_t g0, int va, int vb,
                                              int c0, int cw, int C, int lane) {
-  auto span = [&](float* p, int64_t n) {
-    if ((((uintptr_t)p | (uintptr_t)(n * 4)) & 15) == 0) {
+  auto span = [&](T* p, int64_t n) {
+    if ((((uintptr_t)p | (uintptr_t)(n * (int64_t)sizeof(T))) & (4 * sizeof(T) - 1)) == 0) {
       for (int64_t i = 4 * lane; i < n; i += 128) st_stream4(p + i, make_float4(0.f, 0.f, 0.f, 0.f));
     } else {
       for (int64_t i = lane; i < n; i += 32) st_stream(p + i, 0.f);
@@ -118,13 +121,14 @@ __device__ __forceinline__ void zero_rows_cl(float* __restrict__ out, int64_t g0
 // channel -- with 16-byte loads and stores (vec_ok: C % 4 == 0 and a 16-byte aligned volume).
 // Nothing is transposed.  (Storing the rows straight from the registers, with zeros for the
 // empty voxels between them, was measured at 578 us at C2: short scattered stores.)
-template <int KCH, bool FULLC, bool LOOPC = false, bool CL = false>
+// T: the volume's element type, float or bf16 (rounded once, at the store; the tiles stay float).
+template <int KCH, bool FULLC, bool LOOPC = false, bool CL = false, typename T = float>
 __global__ void __launch_bounds__(kFwdWarps * 32)
 k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
            const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
            const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ tile_start,
            const int32_t* __restrict__ heavy, uint32_t n_items, uint32_t tiles_per_sample,
-           int64_t V, int C, uint32_t n_chunks, int vec_ok, float* __restrict__ out,
+           int64_t V, int C, uint32_t n_chunks, int vec_ok, T* __restrict__ out,
            uint32_t loop_chunks) {
   constexpr int CC = 32 * KCH;
   constexpr int U = (KCH <= 2) ? 16 : 8;  // feature rows in flight per warp
@@ -252,7 +256,7 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
     if (!CL && e0 <= s0 && fast) {  // empty tile
       const int c_lo = LOOPC ? 0 : (h.w & 0xffff) * CC;
       const int c_hi = LOOPC ? C : min(c_lo + CC, C);
-      float* o = out + (int64_t)(b * (uint32_t)(C - 1) + (uint32_t)(c_lo + r)) * V + g0 + q4;
+      T* o = out + (int64_t)(b * (uint32_t)(C - 1) + (uint32_t)(c_lo + r)) * V + g0 + q4;
 #ifndef VEON_FWD_X_NOSTORE
 #pragma unroll 4
       for (int c = c_lo + r; c < c_hi; c += 4, o += ostep) st_stream4(o, make_float4(0.f, 0.f, 0.f, 0.f));
@@ -292,7 +296,7 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
       const int cbase = LOOPC ? (int)ch * CC : (h.w & 0xffff) * CC;
       const int cmax = FULLC ? CC : min(CC, C - cbase);
       // (b*C + cbase + r)*V + v0 + q4  with  v0 = g0 - b*V
-      float* o = out + (int64_t)(b * (uint32_t)(C - 1) + (uint32_t)(cbase + r)) * V + g0 + q4;
+      T* o = out + (int64_t)(b * (uint32_t)(C - 1) + (uint32_t)(cbase + r)) * V + g0 + q4;
       const char* const feat_ch = feat_lane + (LOOPC ? (uint32_t)cbase * 4u : 0u);
 
       __syncwarp();
@@ -384,10 +388,10 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
         const int per_row = cmax / w;
         int v = 0, q = lane;
         while (q >= per_row) { q -= per_row; ++v; }
-        float* const obase = out + (int64_t)g0 * C + cbase;
+        T* const obase = out + (int64_t)g0 * C + cbase;
         for (; v < v_end;) {
           const float* t = tile + v * kClPitch + q * w;
-          float* o = obase + (int64_t)v * C + q * w;
+          T* o = obase + (int64_t)v * C + q * w;
           if (vec_ok) st_stream4(o, *reinterpret_cast<const float4*>(t));
           else st_stream(o, *t);
           q += 32;
@@ -455,13 +459,13 @@ __device__ __forceinline__ void store_label(const ClsArgs& ca, uint32_t b, uint3
 }
 
 // CL: channels-last write-out (warp = voxel, lanes = channels), see k_pool_fwd
-template <int KCH, bool CLS = false, bool CL = false>
+template <int KCH, bool CLS = false, bool CL = false, typename T = float>
 __global__ void __launch_bounds__(kHeavyThreads)
 k_pool_fwd_heavy(const float* __restrict__ depth, const float* __restrict__ feat,
                  const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
                  const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ tile_start,
                  const int32_t* __restrict__ heavy, int heavy_cap, uint32_t tiles_per_sample,
-                 int64_t V, int C, uint32_t n_chunks, int vec_ok, float* __restrict__ out,
+                 int64_t V, int C, uint32_t n_chunks, int vec_ok, T* __restrict__ out,
                  int join, int min_points, ClsArgs ca = ClsArgs()) {
   constexpr int CC = 32 * KCH;
   constexpr int kSegs = CC / 4;  // 16-byte segments per staged row
@@ -586,14 +590,14 @@ k_pool_fwd_heavy(const float* __restrict__ depth, const float* __restrict__ feat
       }
     } else if constexpr (CL) {  // rows of the empty voxels are the tile's zeros
       for (int v = warp; v < kTileVoxels && v0 + v < V; v += kHeavyThreads / 32) {
-        float* o = out + ((int64_t)g0 + v) * C + cbase;
+        T* o = out + ((int64_t)g0 + v) * C + cbase;
         for (int c = lane; c < cmax; c += 32) st_stream(o + c, tile[c * kRowPitch + v]);
       }
     } else {  // write-out: thread (row = tid/8, q = tid%8) moves voxels 4q..4q+3 of channel row (+32j)
       const int q4 = (tid & 7) * 4;
       const bool fast = vec_ok && (v0 + kTileVoxels <= V);
       for (int c = tid >> 3; c < cmax; c += kHeavyThreads / 8) {
-        float* o = out + ((int64_t)b * C + cbase + c) * V + v0 + q4;
+        T* o = out + ((int64_t)b * C + cbase + c) * V + v0 + q4;
         const float* trow = tile + c * kRowPitch + q4;
         if (fast) {
           st_stream4(o, make_float4(trow[0], trow[1], trow[2], trow[3]));
@@ -818,13 +822,13 @@ constexpr int kNarrowHeavyMin = 512;
 // rows in order), so Q + 2 <= 96 channels need no more registers than 32 do.
 // CL: channels-last output; a lane's voxel row is NV 16-byte stores and the warp's 32 rows are one
 // contiguous 32 * C * 4-byte block.
-template <int NV, bool CLS = false, int NP = 1, bool CL = false>  // 16-byte pieces per pass: C = 4 * NV * NP
+template <int NV, bool CLS = false, int NP = 1, bool CL = false, typename T = float>  // 16-byte pieces per pass: C = 4 * NV * NP
 __global__ void __launch_bounds__(kNarrowWarps * 32, (NV <= 5) ? 3 : 2)
 k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ feat,
                   const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
                   const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ tile_start,
                   const int32_t* __restrict__ heavy, uint32_t n_tiles, uint32_t tiles_per_sample,
-                  int64_t V, float* __restrict__ out, uint32_t zero, int heavy_min, int join,
+                  int64_t V, T* __restrict__ out, uint32_t zero, int heavy_min, int join,
                   ClsArgs ca) {
   static_assert(CLS || NP == 1, "several passes only make sense when the sums are consumed here");
   constexpr int CP = 4 * NV;        // channels per pass
@@ -991,12 +995,12 @@ k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ fea
           cur_q = head ? q : cur_q;
         }
       } else if constexpr (CL) {
-        float* o = out + ((int64_t)g0 + lane) * C;
+        T* o = out + ((int64_t)g0 + lane) * C;
 #pragma unroll
         for (int k = 0; k < NV; ++k)
           st_stream4(o + 4 * k, make_float4(acc[4 * k], acc[4 * k + 1], acc[4 * k + 2], acc[4 * k + 3]));
       } else {
-        float* o = out + (int64_t)b * C * V + v0 + lane;
+        T* o = out + (int64_t)b * C * V + v0 + lane;
 #pragma unroll
         for (int c = 0; c < CP; ++c) st_stream(o + (int64_t)c * V, acc[c]);
       }
@@ -1015,17 +1019,17 @@ k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ fea
 
 
 // ---- launchers ---------------------------------------------------------------------------------
-template <int KCH, bool CLS = false, bool CL = false>
+template <int KCH, bool CLS = false, bool CL = false, typename T = float>
 static int heavy_config(size_t& smem, int& ctas_per_sm) {
   constexpr int CC = 32 * KCH;
   smem = sizeof(float) * (kHeavyChunk * CC + CC * kRowPitch + 2 * kHeavyChunk + 128);
   static int cached[kMaxDevices] = {};
   const int dev = current_device();
   if (cached[dev] == 0) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd_heavy<KCH, CLS, CL>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd_heavy<KCH, CLS, CL, T>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_heavy<KCH, CLS, CL>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_heavy<KCH, CLS, CL, T>,
                                                                 kHeavyThreads, smem));
     cached[dev] = n < 1 ? 1 : (n > 8 ? 8 : n);
   }
@@ -1034,29 +1038,29 @@ static int heavy_config(size_t& smem, int& ctas_per_sm) {
 }
 
 // the heavy-tile grid; pdl: queued as a programmatic dependent of the previous launch (joins it)
-template <int KCH, bool CLS = false, bool CL = false>
+template <int KCH, bool CLS = false, bool CL = false, typename T = float>
 static int launch_heavy(const float* depth, const float* feat, const int32_t* rd, const int32_t* rf,
                         const int32_t* rb, const int32_t* tile_start, const int32_t* heavy,
-                        int64_t heavy_ints, int B, int C, int64_t V, float* out, bool pdl,
+                        int64_t heavy_ints, int B, int C, int64_t V, T* out, bool pdl,
                         int min_points, cudaStream_t stream, ClsArgs ca = ClsArgs()) {
   constexpr int CC = 32 * KCH;
   size_t smem;
   int per_sm;
-  int rc = heavy_config<KCH, CLS, CL>(smem, per_sm);
+  int rc = heavy_config<KCH, CLS, CL, T>(smem, per_sm);
   if (rc) return rc;
   const int64_t tps = ceil_div64(V, kTileVoxels);
   const int n_chunks = (C + CC - 1) / CC;
-  const int vec_ok = ((V & 3) == 0) && (((uintptr_t)out & 15) == 0);
+  const int vec_ok = ((V & 3) == 0) && (((uintptr_t)out & (4 * sizeof(T) - 1)) == 0);
   const int heavy_cap = (int)(heavy_ints - 2);
   int64_t blocks = (int64_t)heavy_cap * n_chunks;
   if (blocks > (int64_t)per_sm * sm_count()) blocks = (int64_t)per_sm * sm_count();
   if (blocks <= 0) return 0;
   if (pdl) {
-    VEON_CUDA_TRY(launch_pdl(k_pool_fwd_heavy<KCH, CLS, CL>, dim3((unsigned)blocks), dim3(kHeavyThreads),
+    VEON_CUDA_TRY(launch_pdl(k_pool_fwd_heavy<KCH, CLS, CL, T>, dim3((unsigned)blocks), dim3(kHeavyThreads),
                              smem, stream, depth, feat, rd, rf, rb, tile_start, heavy, heavy_cap,
                              (uint32_t)tps, V, C, (uint32_t)n_chunks, vec_ok, out, 1, min_points, ca));
   } else {
-    k_pool_fwd_heavy<KCH, CLS, CL><<<(unsigned)blocks, kHeavyThreads, smem, stream>>>(
+    k_pool_fwd_heavy<KCH, CLS, CL, T><<<(unsigned)blocks, kHeavyThreads, smem, stream>>>(
         depth, feat, rd, rf, rb, tile_start, heavy, heavy_cap, (uint32_t)tps, V, C,
         (uint32_t)n_chunks, vec_ok, out, 0, min_points, ca);
   }
@@ -1077,11 +1081,11 @@ int launch_heavy_behind(const float* depth, const float* feat, const int32_t* rd
 }
 
 // general route: k_pool_fwd over every (tile, channel chunk), the heavy tiles queued behind it
-template <int KCH, bool FULLC, bool LOOPC, bool CL>
+template <int KCH, bool FULLC, bool LOOPC, bool CL, typename T>
 static int launch_fwd_impl(const float* depth, const float* feat, const int32_t* rd,
                            const int32_t* rf, const int32_t* rb, const int32_t* tile_start,
                            const int32_t* heavy, int64_t heavy_ints, int B, int C, int64_t V,
-                           bool feat_rows_fit_32bit, float* out, cudaStream_t stream) {
+                           bool feat_rows_fit_32bit, T* out, cudaStream_t stream) {
   constexpr int CC = 32 * KCH;
   constexpr int kExtInts = LOOPC ? ((kHeavyDefaultThreshold + 31) / 32 - 1) * 128 : 0;
   const size_t smem = sizeof(float) * kFwdWarps *
@@ -1089,10 +1093,10 @@ static int launch_fwd_impl(const float* depth, const float* feat, const int32_t*
   static int ctas_per_sm[kMaxDevices] = {};
   const int dev = current_device();
   if (ctas_per_sm[dev] == 0) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd<KCH, FULLC, LOOPC, CL>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd<KCH, FULLC, LOOPC, CL, T>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd<KCH, FULLC, LOOPC, CL>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd<KCH, FULLC, LOOPC, CL, T>,
                                                                 kFwdWarps * 32, smem));
     ctas_per_sm[dev] = n < 1 ? 1 : n;
   }
@@ -1100,16 +1104,16 @@ static int launch_fwd_impl(const float* depth, const float* feat, const int32_t*
   const int n_chunks = (C + CC - 1) / CC;
   if (n_tiles * n_chunks > 0x7fffffffLL || (int64_t)B * V > 0x7fffffffLL) return VEON_E_RANGE;
   if (!feat_rows_fit_32bit) return VEON_E_RANGE;   // the gather uses 32-bit byte offsets
-  // 16-byte stores: channel planes of 4-voxel pieces (channels-first) or rows of 4-channel
-  // pieces (channels-last)
-  const int vec_ok = (((CL ? C : V) & 3) == 0) && (((uintptr_t)out & 15) == 0);
+  // 4-element (16-byte float, 8-byte bf16) stores: channel planes of 4-voxel pieces
+  // (channels-first) or rows of 4-channel pieces (channels-last)
+  const int vec_ok = (((CL ? C : V) & 3) == 0) && (((uintptr_t)out & (4 * sizeof(T) - 1)) == 0);
   const int64_t n_items = LOOPC ? n_tiles : n_tiles * n_chunks;   // LOOPC: chunks looped per tile
   int64_t blocks = ceil_div64(n_items, kFwdWarps);
   const int64_t resident = (int64_t)ctas_per_sm[dev] * sm_count();  // persistent grid
   if (blocks > resident) blocks = resident;
   // the heavy-tile kernel stages feature rows with 16-byte copies
   if (heavy && ((C & 3) != 0 || ((uintptr_t)feat & 15) != 0)) heavy = nullptr;
-  k_pool_fwd<KCH, FULLC, LOOPC, CL><<<(unsigned)blocks, kFwdWarps * 32, smem, stream>>>(
+  k_pool_fwd<KCH, FULLC, LOOPC, CL, T><<<(unsigned)blocks, kFwdWarps * 32, smem, stream>>>(
       depth, feat, rd, rf, rb, tile_start, heavy, (uint32_t)n_items, (uint32_t)tps,
       V, C, (uint32_t)(LOOPC ? 1 : n_chunks), vec_ok, out, (uint32_t)n_chunks);
   VEON_LAUNCH_CHECK();
@@ -1118,17 +1122,17 @@ static int launch_fwd_impl(const float* depth, const float* feat, const int32_t*
   // grid before they complete.
 #ifndef VEON_FWD_X_NOHEAVY
   if (heavy)
-    return launch_heavy<(KCH > 2 ? 2 : KCH), false, CL>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints,
+    return launch_heavy<(KCH > 2 ? 2 : KCH), false, CL, T>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints,
                                              B, C, V, out, true, 0, stream);
 #endif
   return 0;
 }
 
-template <int KCH, bool CL = false>
+template <int KCH, bool CL, typename T>
 static int launch_fwd(const float* depth, const float* feat, const int32_t* rd,
                       const int32_t* rf, const int32_t* rb, const int32_t* tile_start,
                       const int32_t* heavy, int64_t heavy_ints, int B, int C, int64_t V,
-                      bool feat_rows_fit_32bit, float* out, cudaStream_t stream) {
+                      bool feat_rows_fit_32bit, T* out, cudaStream_t stream) {
   // rows of several chunks: one item per tile (needs the heavy list: it bounds a tile's points)
 #ifndef VEON_FWD_X_NOLOOPC
   const bool loopc = heavy && C > 32 * KCH && (C & 3) == 0 && ((uintptr_t)feat & 15) == 0;
@@ -1136,7 +1140,7 @@ static int launch_fwd(const float* depth, const float* feat, const int32_t* rd,
   const bool loopc = false;
 #endif
 #define VEON_FWD_GO(FULLC_, LOOPC_)                                                            \
-  return launch_fwd_impl<KCH, FULLC_, LOOPC_, CL>(depth, feat, rd, rf, rb, tile_start, heavy,      \
+  return launch_fwd_impl<KCH, FULLC_, LOOPC_, CL, T>(depth, feat, rd, rf, rb, tile_start, heavy,      \
                                               heavy_ints, B, C, V, feat_rows_fit_32bit, out, stream)
   if (C % (32 * KCH) == 0) {
     if (loopc) VEON_FWD_GO(true, true);
@@ -1151,11 +1155,11 @@ static int launch_fwd(const float* depth, const float* feat, const int32_t* rd,
 // CTA works ~100 us on one 1 000-point tile at C3 density: behind the persistent main grid the
 // two nearly serialise, 344 vs 295 us); k_pool_fwd_narrow moves in beside it as its programmatic
 // dependent and joins it at the end
-template <int NV, bool CLS = false, int NP = 1, bool CL = false>
+template <int NV, bool CLS = false, int NP = 1, bool CL = false, typename T = float>
 static int launch_fwd_narrow(const float* depth, const float* feat, const int32_t* rd,
                              const int32_t* rf, const int32_t* rb, const int32_t* tile_start,
                              const int32_t* heavy, int64_t heavy_ints, int B, int64_t V,
-                             float* out, cudaStream_t stream, ClsArgs ca = ClsArgs()) {
+                             T* out, cudaStream_t stream, ClsArgs ca = ClsArgs()) {
   constexpr int C = 4 * NV * NP;
   constexpr int KCH = (C + 31) / 32;   // the heavy CTA holds every channel of its tile
   const int64_t tps = V / kTileVoxels, n_tiles = (int64_t)B * tps;
@@ -1163,16 +1167,16 @@ static int launch_fwd_narrow(const float* depth, const float* feat, const int32_
   const int dev = current_device();
   if (ctas_per_sm[dev] == 0) {
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_narrow<NV, CLS, NP, CL>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_narrow<NV, CLS, NP, CL, T>,
                                                                 kNarrowWarps * 32, 0));
     ctas_per_sm[dev] = n < 1 ? 1 : n;
   }
   int64_t blocks = ceil_div64(n_tiles, kNarrowWarps);
   if (blocks > (int64_t)ctas_per_sm[dev] * sm_count()) blocks = (int64_t)ctas_per_sm[dev] * sm_count();
-  int rc = launch_heavy<KCH, CLS, CL>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C, V,
+  int rc = launch_heavy<KCH, CLS, CL, T>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C, V,
                                   out, false, kNarrowHeavyMin, stream, ca);
   if (rc) return rc;
-  VEON_CUDA_TRY(launch_pdl(k_pool_fwd_narrow<NV, CLS, NP, CL>, dim3((unsigned)blocks),
+  VEON_CUDA_TRY(launch_pdl(k_pool_fwd_narrow<NV, CLS, NP, CL, T>, dim3((unsigned)blocks),
                            dim3(kNarrowWarps * 32), 0, stream, depth, feat, rd, rf, rb, tile_start,
                            heavy, (uint32_t)n_tiles, (uint32_t)tps, V, out, 0u, kNarrowHeavyMin, 1,
                            ca));
@@ -1195,15 +1199,16 @@ extern "C" size_t veon_bev_pool_v2_fwd_workspace_bytes(int B, int C, int64_t V) 
   return fwd_stream_workspace_bytes(C);
 }
 
-// Both planar entry points: out is [B,C,Z,Y,X], or [B,Z,Y,X,C] with CL (the same kernels with a
-// row write-out: same sums, same bits, another layout).  Routes in order: narrow rows, the
-// streaming kernel (channels-first only; needs tile_occ and a workspace), the general kernel.
-template <bool CL>
+// All four planar entry points: out is [B,C,Z,Y,X], or [B,Z,Y,X,C] with CL (the same kernels with a
+// row write-out: same sums, same bits, another layout), of float or bf16 elements T.  Routes in
+// order: narrow rows, the streaming kernel (channels-first float only; needs tile_occ and a
+// workspace), the general kernel.
+template <bool CL, typename T>
 static int fwd_planar(const float* depth, const float* feat, const int32_t* ranks_depth,
                       const int32_t* ranks_feat, const int32_t* ranks_bev,
                       const int32_t* tile_start, const uint32_t* tile_occ,
                       const int32_t* tile_heavy, int64_t tile_heavy_ints, int B, int C, int64_t V,
-                      int64_t n_feat_rows, float* out, void* workspace, size_t workspace_bytes,
+                      int64_t n_feat_rows, T* out, void* workspace, size_t workspace_bytes,
                       cudaStream_t stream) {
   if (!depth || !feat || !ranks_depth || !ranks_feat || !ranks_bev || !tile_start || !out ||
       B <= 0 || C <= 0 || V <= 0 || n_feat_rows <= 0 || (tile_heavy && tile_heavy_ints < 2))
@@ -1216,9 +1221,9 @@ static int fwd_planar(const float* depth, const float* feat, const int32_t* rank
      // arbitrarily long voxels; rank arithmetic is exact only while B*V <= 2^24
     const bool ok = C <= 32 && (C & 3) == 0 && tile_heavy && fit32 && V % kTileVoxels == 0 &&
                     (int64_t)B * V <= (1 << 24) &&
-                    (((uintptr_t)feat | (uintptr_t)out) & 15) == 0;
+                    ((uintptr_t)feat & 15) == 0 && ((uintptr_t)out & (4 * sizeof(T) - 1)) == 0;
     if (ok) {
-#define VEON_NARROW_CASE(NV_) case NV_: return launch_fwd_narrow<NV_, false, 1, CL>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy, tile_heavy_ints, B, V, out, stream);
+#define VEON_NARROW_CASE(NV_) case NV_: return launch_fwd_narrow<NV_, false, 1, CL, T>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy, tile_heavy_ints, B, V, out, stream);
       switch (C / 4) {
         VEON_NARROW_CASE(1) VEON_NARROW_CASE(2) VEON_NARROW_CASE(3) VEON_NARROW_CASE(4)
         VEON_NARROW_CASE(5) VEON_NARROW_CASE(6) VEON_NARROW_CASE(7) VEON_NARROW_CASE(8)
@@ -1228,7 +1233,7 @@ static int fwd_planar(const float* depth, const float* feat, const int32_t* rank
     }
   }
   // aligned volumes, whole 64-channel chunks: the two-role streaming kernel
-  if constexpr (!CL) {
+  if constexpr (!CL && std::is_same<T, float>::value) {
     if (workspace && tile_occ && tile_heavy &&
         fwd_stream_supported(B, C, V, feat, out, n_feat_rows)) {
       const int rc = launch_fwd_stream(depth, feat, ranks_depth, ranks_feat, ranks_bev,
@@ -1238,9 +1243,9 @@ static int fwd_planar(const float* depth, const float* feat, const int32_t* rank
     }
   }
   if (C <= 32)
-    return launch_fwd<1, CL>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
+    return launch_fwd<1, CL, T>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
                              tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
-  return launch_fwd<2, CL>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
+  return launch_fwd<2, CL, T>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
                            tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
 }
 
@@ -1273,6 +1278,40 @@ extern "C" int veon_bev_pool_v2_fwd_planar_cl(const float* depth, const float* f
                           (cudaStream_t)stream);
 }
 
+// bfloat16 volumes: the same kernels with a bf16 write-out (float sums, one rounding per element
+// at the store).  The channels-first one never takes the streaming kernel, so it needs no
+// workspace; it accepts the float twin's arguments all the same.
+extern "C" int veon_bev_pool_v2_fwd_planar_bf16(const float* depth, const float* feat,
+                                                const int32_t* ranks_depth,
+                                                const int32_t* ranks_feat,
+                                                const int32_t* ranks_bev,
+                                                const int32_t* tile_start,
+                                                const int32_t* tile_istart,
+                                                const uint32_t* tile_occ,
+                                                const int32_t* tile_heavy, int64_t tile_heavy_ints,
+                                                int B, int C, int64_t V, int64_t n_feat_rows,
+                                                uint16_t* out, void* workspace,
+                                                size_t workspace_bytes, void* stream) {
+  return fwd_planar<false>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_occ,
+                           tile_heavy, tile_heavy_ints, B, C, V, n_feat_rows,
+                           reinterpret_cast<bf16*>(out), workspace, workspace_bytes,
+                           (cudaStream_t)stream);
+}
+
+extern "C" int veon_bev_pool_v2_fwd_planar_cl_bf16(const float* depth, const float* feat,
+                                                   const int32_t* ranks_depth,
+                                                   const int32_t* ranks_feat,
+                                                   const int32_t* ranks_bev,
+                                                   const int32_t* tile_start,
+                                                   const int32_t* tile_heavy,
+                                                   int64_t tile_heavy_ints, int B, int C, int64_t V,
+                                                   int64_t n_feat_rows, uint16_t* out,
+                                                   void* stream) {
+  return fwd_planar<true>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, nullptr,
+                          tile_heavy, tile_heavy_ints, B, C, V, n_feat_rows,
+                          reinterpret_cast<bf16*>(out), nullptr, 0, (cudaStream_t)stream);
+}
+
 // Fused lift + classify: pools the [gate 0, gate 1, logit 0..Q-1, pad] rows and ends every tile
 // as 32 labels -- the pooled logit volume is never written (SURVEY 8f-4).
 extern "C" int veon_lift_classify_fwd(const float* depth, const float* pix,
@@ -1302,7 +1341,7 @@ extern "C" int veon_lift_classify_fwd(const float* depth, const float* pix,
   if (C == 4 * NV_ * NP_)                                                                         \
     return launch_fwd_narrow<NV_, true, NP_>(depth, pix, ranks_depth, ranks_feat, ranks_bev,      \
                                              tile_start, tile_heavy, tile_heavy_ints, B, V,       \
-                                             nullptr, stream, ca);
+                                             (float*)nullptr, stream, ca);
   if (C <= 32) {
     VEON_CLS_CASE(1, 1) VEON_CLS_CASE(2, 1) VEON_CLS_CASE(3, 1) VEON_CLS_CASE(4, 1)
     VEON_CLS_CASE(5, 1) VEON_CLS_CASE(6, 1) VEON_CLS_CASE(7, 1) VEON_CLS_CASE(8, 1)

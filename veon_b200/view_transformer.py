@@ -38,15 +38,23 @@ class LSSViewTransformer(nn.Module):
     channels-last, written that way by the pooling kernels (the layout a
     channels-last 3D encoder wants; its channels-last gradient is consumed
     without a copy).  The default, torch.contiguous_format, is the reference's.
+
+    Extra: `dtype` -- torch.bfloat16 makes every pooling route return the
+    volume in bfloat16 (the float32 volume rounded once, bit for bit, written
+    so by the kernels; the layout a bfloat16 3D encoder under autocast wants),
+    combined with either memory format.  Its bfloat16 gradient is read as it
+    arrives; the depth / feature gradients stay float32.
     """
 
     def __init__(self, grid_config, input_size, downsample=16, in_channels=512,
                  out_channels=64, accelerate=False, sid=False, collapse_z=True,
                  sync_free=False, rank_cache=0, depth_eps=None,
-                 memory_format=torch.contiguous_format):
+                 memory_format=torch.contiguous_format, dtype=torch.float32):
         super().__init__()
         _bp._channels_last(memory_format)     # ValueError for anything but the two formats
+        _bp._bf16(dtype)                      # ValueError for anything but float32 / bfloat16
         self.memory_format = memory_format
+        self.dtype = dtype
         self.grid_config = grid_config
         self.downsample = downsample
         self.create_grid_infos(**grid_config)
@@ -262,7 +270,7 @@ class LSSViewTransformer(nn.Module):
         feat_last = feat.permute(0, 1, 3, 4, 2)
         shape = self._bev_shape(depth, feat_last.shape[-1])
         bev_feat = _bp.pool_prepared(depth, feat_last, self._prepared(prep), shape,
-                                     self.memory_format)
+                                     self.memory_format, dtype=self.dtype)
         if self._no_points(prep):
             return self._no_points_dummy(feat)
         if self.collapse_z:
@@ -275,6 +283,8 @@ class LSSViewTransformer(nn.Module):
         gs = self.grid_size
         dummy = torch.zeros(size=[feat.shape[0], feat.shape[2], int(gs[2]), int(gs[0]),
                                   int(gs[1])]).to(feat)
+        if self.dtype is torch.bfloat16:
+            dummy = dummy.to(torch.bfloat16)
         return torch.cat(dummy.unbind(dim=2), 1)
 
     # -- a10 -----------------------------------------------------------------
@@ -293,7 +303,7 @@ class LSSViewTransformer(nn.Module):
             bev_feat = _bp.bev_pool_v2(depth, feat, self.ranks_depth, self.ranks_feat,
                                        self.ranks_bev, self._bev_shape(depth, feat.shape[-1]),
                                        self.interval_starts, self.interval_lengths,
-                                       memory_format=self.memory_format)
+                                       memory_format=self.memory_format, dtype=self.dtype)
             bev_feat = bev_feat.squeeze(2)
         elif self.fuse_geometry and input[1].is_cuda:
             # get_lidar_coor folded into the index preparation: same ranks, no coor tensor
@@ -327,11 +337,16 @@ class LSSViewTransformerRaw(LSSViewTransformer):
     max-pools the volume 2x2x2.  With memory_format=torch.channels_last_3d it
     pools channels-last and reduces with the channels-last 2x2x2 kernels (the
     fused `fuse_ds` kernel and the one-node PoolMaxDown training route are
-    channels-first only and are not taken); the result is channels-last-3d."""
+    channels-first only and are not taken); the result is channels-last-3d.
+    Float32 only: its 2x2x2 maximum, `PoolMaxDown`, `fuse_ds` and the fused lift + classify
+    have no bfloat16 form (a bfloat16 maximum may pick another first arg-max than the float32
+    one), so any other `dtype` raises ValueError."""
 
     def __init__(self, *args, use_ds=True, ds=(2, 2, 2), fuse_ds=False, **kwargs):
         kwargs.setdefault("collapse_z", False)
         super().__init__(*args, **kwargs)
+        if self.dtype is not torch.float32:
+            raise ValueError(f"LSSViewTransformerRaw is float32 only, got dtype={self.dtype!r}")
         self.use_ds = use_ds
         self.ds = tuple(ds)
         # Extra (not in the reference): pool and max-reduce in ONE kernel on the no-grad path,
