@@ -546,6 +546,34 @@ int veon_voxel_text_argmax_lowres(const float* feat_occ_lr, const float* text_w,
                                   void* workspace, size_t ws_bytes, const void* w_image,
                                   void* stream);
 
+/* The three tail entry points on a bfloat16 feature volume (feat_occ / feat_occ_lr: bfloat16
+ * [B,C,Z,Y,X], as the pooling's _bf16 entries write it or a 3D decoder under autocast returns
+ * it).  Every result equals the float32 twin's on the volume widened to float32: the same
+ * labels byte for byte and the same logits value for value (NaN where it has NaN; only the sign
+ * of an exact zero may differ).  A widened bfloat16 value is exactly TF32-representable, so the
+ * tensor-core kernel reads the volume as it is (half the bytes) and drops the third product of
+ * the 3xTF32 sum, which is exactly zero.  text_w, bin_occ / bin_occ_lr, w_image and every
+ * output are the float32 twins'; so are the arguments, checks and error codes.  The route is
+ * the one the float32 twin would take: the fp32 FFMA kernel reading bfloat16 where that one
+ * takes it (C % 32 != 0, V % 4 != 0, Q > 128), else tcgen05, which here needs V % 8 == 0 and a
+ * 16-byte aligned feat_occ; where it cannot have them the entry returns VEON_E_UNSUPPORTED and
+ * the caller widens the volume and calls the float32 twin.  The workspace of the low-resolution
+ * entry is sized by veon_voxel_text_argmax_lowres_workspace_bytes. */
+int veon_voxel_text_argmax_bf16(const uint16_t* feat_occ, const float* text_w,
+                                const int32_t* class_of_prompt, const float* bin_occ,
+                                int B, int C, int Q, int Z, int Y, int X,
+                                int free_label, uint8_t* labels, const void* w_image,
+                                void* stream);
+int veon_semantic_inference_3d_bf16(const float* text_w, const uint16_t* feat_occ,
+                                    int B, int C, int Q, int Z, int Y, int X,
+                                    float* sem_occ, const void* w_image, void* stream);
+int veon_voxel_text_argmax_lowres_bf16(const uint16_t* feat_occ_lr, const float* text_w,
+                                       const int32_t* class_of_prompt, const float* bin_occ_lr,
+                                       int B, int C, int Q, int Zi, int Yi, int Xi,
+                                       int Z, int Y, int X, int free_label, uint8_t* labels,
+                                       void* workspace, size_t ws_bytes, const void* w_image,
+                                       void* stream);
+
 /* Multi-GPU callers that overlap a collective (NCCL on another stream) with the path: the
  * persistent grids here fill every SM, so the collective's CTAs wait for a kernel boundary.
  * veon_reserve_sms(n) makes every persistent grid of the library launch on (SM count - n) SMs;

@@ -106,9 +106,17 @@ _SIGNATURES = {
     "veon_voxel_text_argmax_lowres": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
                                               c_int, c_int, c_int, c_int, c_int, _P, _P, c_size_t,
                                               _P, _P]),
+    "veon_voxel_text_argmax_bf16": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int,
+                                            c_int, _P, _P, _P]),
+    "veon_semantic_inference_3d_bf16": (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, c_int, _P,
+                                                _P, _P]),
+    "veon_voxel_text_argmax_lowres_bf16": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
+                                                   c_int, c_int, c_int, c_int, c_int, _P, _P, c_size_t,
+                                                   _P, _P]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
+E_UNSUPPORTED = -4   # VEON_E_UNSUPPORTED: the shape does not fit this entry point
 _lib = None
 
 

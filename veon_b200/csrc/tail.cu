@@ -11,6 +11,8 @@
 // path (tail_tc.cu: tcgen05 3xTF32, TMEM accumulators) does not take (C % 32 != 0,
 // V % 4 != 0, more than 128 prompt rows) -- one thread per voxel, text rows staged in
 // shared memory per prompt tile, everything after the dot products fused in registers.
+// Features are float32 or bfloat16 (T); a bfloat16 value is widened exactly on load, so the
+// bfloat16 instances give the float32 ones' bits on x.float().
 #include <math.h>
 
 #include "common.cuh"
@@ -21,9 +23,9 @@ constexpr int kTailThreads = 128;
 constexpr int kTailQT = 24;  // prompts held in registers per pass
 
 // LOGITS: store sem_occ [B,Q,V] (semantic_inference_3d alone) instead of the labels.
-template <bool LOGITS>
+template <bool LOGITS, typename T>
 __global__ void __launch_bounds__(kTailThreads)
-k_voxel_text_argmax(const float* __restrict__ feat_occ, const float* __restrict__ text_w,
+k_voxel_text_argmax(const T* __restrict__ feat_occ, const float* __restrict__ text_w,
                     const int32_t* __restrict__ class_of_prompt,
                     const float* __restrict__ bin_occ, int C, int Q, int Z, int Y, int X,
                     int free_label, uint8_t* __restrict__ labels, float* __restrict__ logits) {
@@ -32,7 +34,7 @@ k_voxel_text_argmax(const float* __restrict__ feat_occ, const float* __restrict_
   const int b = blockIdx.y;
   const int64_t v = (int64_t)blockIdx.x * kTailThreads + threadIdx.x;
   const bool live = v < V;
-  const float* f = feat_occ + (int64_t)b * C * V + (live ? v : 0);
+  const T* f = feat_occ + (int64_t)b * C * V + (live ? v : 0);
 
   float best = 0.f, cur = 0.f;
   int best_cls = -1, cur_cls = -1;
@@ -48,8 +50,8 @@ k_voxel_text_argmax(const float* __restrict__ feat_occ, const float* __restrict_
     for (int q = 0; q < kTailQT; ++q) acc[q] = 0.f;
     int c = 0;
     for (; c + 4 <= C; c += 4) {
-      const float f0 = __ldg(f + (int64_t)(c + 0) * V), f1 = __ldg(f + (int64_t)(c + 1) * V);
-      const float f2 = __ldg(f + (int64_t)(c + 2) * V), f3 = __ldg(f + (int64_t)(c + 3) * V);
+      const float f0 = ldg_widen(f + (int64_t)(c + 0) * V), f1 = ldg_widen(f + (int64_t)(c + 1) * V);
+      const float f2 = ldg_widen(f + (int64_t)(c + 2) * V), f3 = ldg_widen(f + (int64_t)(c + 3) * V);
 #pragma unroll
       for (int q = 0; q < kTailQT; ++q) {
         if (q < nq) {
@@ -62,7 +64,7 @@ k_voxel_text_argmax(const float* __restrict__ feat_occ, const float* __restrict_
       }
     }
     for (; c < C; ++c) {
-      const float f0 = __ldg(f + (int64_t)c * V);
+      const float f0 = ldg_widen(f + (int64_t)c * V);
 #pragma unroll
       for (int q = 0; q < kTailQT; ++q)
         if (q < nq) acc[q] = fmaf(w_s[q * C + c], f0, acc[q]);
@@ -113,20 +115,27 @@ k_voxel_text_argmax(const float* __restrict__ feat_occ, const float* __restrict_
 using namespace veon;
 
 // tensor-core path (tail_tc.cu); VEON_E_UNSUPPORTED when the shape does not fit it
-int veon_tail_tc_launch(const float* feat_occ, const float* text_w, const int32_t* cls,
+bool veon_tail_tc_takes(int C, int Q, int64_t V, const float* text_w);
+template <typename T>
+int veon_tail_tc_launch(const T* feat_occ, const float* text_w, const int32_t* cls,
                         const float* bin_occ, int B, int C, int Q, int Z, int Y, int X,
                         int free_label, uint8_t* labels, float* logits, const void* w_image,
                         cudaStream_t stream);
 
-// labels (logits == nullptr) or raw logits (labels == nullptr) of B volumes
-static int tail_dispatch(const float* feat_occ, const float* text_w,
+// labels (logits == nullptr) or raw logits (labels == nullptr) of B volumes.  bfloat16 features
+// take the route the float32 call would take on x.float(): the FFMA kernel where it takes that,
+// else tcgen05 -- and VEON_E_UNSUPPORTED where its bfloat16 loader cannot (V % 8 == 4 or an
+// 8- but not 16-byte aligned feat_occ), so that the caller widens instead of getting other bits.
+template <typename T>
+static int tail_dispatch(const T* feat_occ, const float* text_w,
                          const int32_t* class_of_prompt, const float* bin_occ, int B, int C,
                          int Q, int Z, int Y, int X, int free_label, uint8_t* labels,
                          float* logits, const void* w_image, cudaStream_t stream) {
   {  // tcgen05 path unless the shape does not fit it (C % 32, V % 4, Q > 128)
-    const int rc = veon_tail_tc_launch(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y, X,
-                                       free_label, labels, logits, w_image, stream);
+    const int rc = veon_tail_tc_launch<T>(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y,
+                                          X, free_label, labels, logits, w_image, stream);
     if (rc != VEON_E_UNSUPPORTED) return rc;
+    if (sizeof(T) == 2 && veon_tail_tc_takes(C, Q, (int64_t)Z * Y * X, text_w)) return rc;
   }
   const size_t smem = sizeof(float) * (size_t)kTailQT * C;
   if (smem > 200 * 1024) return VEON_E_UNSUPPORTED;
@@ -134,28 +143,29 @@ static int tail_dispatch(const float* feat_occ, const float* text_w,
   size_t& attr_smem = attr_smem_dev[current_device()];
   if (attr_smem == 0) attr_smem = 48 * 1024;
   if (smem > attr_smem) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_voxel_text_argmax<false>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_voxel_text_argmax<false, T>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_voxel_text_argmax<true>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_voxel_text_argmax<true, T>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_smem = smem;
   }
   const int64_t V = (int64_t)Z * Y * X;
   dim3 grid((unsigned)ceil_div64(V, kTailThreads), (unsigned)B);
   if (logits)
-    k_voxel_text_argmax<true><<<grid, kTailThreads, smem, stream>>>(
+    k_voxel_text_argmax<true, T><<<grid, kTailThreads, smem, stream>>>(
         feat_occ, text_w, class_of_prompt, bin_occ, C, Q, Z, Y, X, free_label, labels, logits);
   else
-    k_voxel_text_argmax<false><<<grid, kTailThreads, smem, stream>>>(
+    k_voxel_text_argmax<false, T><<<grid, kTailThreads, smem, stream>>>(
         feat_occ, text_w, class_of_prompt, bin_occ, C, Q, Z, Y, X, free_label, labels, logits);
   VEON_LAUNCH_CHECK();
   return 0;
 }
 
-extern "C" int veon_voxel_text_argmax(const float* feat_occ, const float* text_w,
-                                      const int32_t* class_of_prompt, const float* bin_occ,
-                                      int B, int C, int Q, int Z, int Y, int X, int free_label,
-                                      uint8_t* labels, const void* w_image, void* stream) {
+template <typename T>
+static int voxel_text_argmax(const T* feat_occ, const float* text_w,
+                             const int32_t* class_of_prompt, const float* bin_occ, int B, int C,
+                             int Q, int Z, int Y, int X, int free_label, uint8_t* labels,
+                             const void* w_image, void* stream) {
   if (!feat_occ || !text_w || !class_of_prompt || !bin_occ || !labels || B <= 0 || C <= 0 ||
       Q <= 0 || Z <= 0 || Y <= 0 || X <= 0 || B > 65535)
     return VEON_E_BADARG;
@@ -163,14 +173,45 @@ extern "C" int veon_voxel_text_argmax(const float* feat_occ, const float* text_w
                        labels, nullptr, w_image, (cudaStream_t)stream);
 }
 
-extern "C" int veon_semantic_inference_3d(const float* text_w, const float* feat_occ, int B, int C,
-                                          int Q, int Z, int Y, int X, float* sem_occ,
-                                          const void* w_image, void* stream) {
+template <typename T>
+static int semantic_inference_3d(const float* text_w, const T* feat_occ, int B, int C, int Q,
+                                 int Z, int Y, int X, float* sem_occ, const void* w_image,
+                                 void* stream) {
   if (!feat_occ || !text_w || !sem_occ || B <= 0 || C <= 0 || Q <= 0 || Z <= 0 || Y <= 0 ||
       X <= 0 || B > 65535)
     return VEON_E_BADARG;
   return tail_dispatch(feat_occ, text_w, nullptr, nullptr, B, C, Q, Z, Y, X, 0, nullptr, sem_occ,
                        w_image, (cudaStream_t)stream);
+}
+
+extern "C" int veon_voxel_text_argmax(const float* feat_occ, const float* text_w,
+                                      const int32_t* class_of_prompt, const float* bin_occ,
+                                      int B, int C, int Q, int Z, int Y, int X, int free_label,
+                                      uint8_t* labels, const void* w_image, void* stream) {
+  return voxel_text_argmax(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y, X,
+                           free_label, labels, w_image, stream);
+}
+
+extern "C" int veon_voxel_text_argmax_bf16(const uint16_t* feat_occ, const float* text_w,
+                                           const int32_t* class_of_prompt, const float* bin_occ,
+                                           int B, int C, int Q, int Z, int Y, int X,
+                                           int free_label, uint8_t* labels, const void* w_image,
+                                           void* stream) {
+  return voxel_text_argmax(reinterpret_cast<const bf16*>(feat_occ), text_w, class_of_prompt,
+                           bin_occ, B, C, Q, Z, Y, X, free_label, labels, w_image, stream);
+}
+
+extern "C" int veon_semantic_inference_3d(const float* text_w, const float* feat_occ, int B, int C,
+                                          int Q, int Z, int Y, int X, float* sem_occ,
+                                          const void* w_image, void* stream) {
+  return semantic_inference_3d(text_w, feat_occ, B, C, Q, Z, Y, X, sem_occ, w_image, stream);
+}
+
+extern "C" int veon_semantic_inference_3d_bf16(const float* text_w, const uint16_t* feat_occ,
+                                               int B, int C, int Q, int Z, int Y, int X,
+                                               float* sem_occ, const void* w_image, void* stream) {
+  return semantic_inference_3d(text_w, reinterpret_cast<const bf16*>(feat_occ), B, C, Q, Z, Y, X,
+                               sem_occ, w_image, stream);
 }
 
 // ---- training-time voxel x text arg-max over a POINT LIST (SURVEY 8f-4) ----------------------

@@ -27,7 +27,15 @@
 //     tensor-memory addresses stay in uniform registers (see the note in that role).
 // Warp roles (23 warps): 0-15 converters, 16 MMA issuer (+TMEM alloc), 17-20 epilogue,
 // 21-22 loaders.
+//
+// bfloat16 features (T = bf16): a widened bfloat16 value is exactly TF32-representable, so
+// a_hi = a and a_lo = 0 and the third product of every 3xTF32 sum is exactly zero.  That
+// instance reads half the bytes ([KC][TM] bf16 raw tiles, twice as many in flight), writes one
+// tensor-memory column per channel (no lo half) and issues a*w_hi + a*w_lo per K-step: the
+// float32 instance's sums on x.float(), bit for bit.
 #include <math.h>
+
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -44,9 +52,13 @@ constexpr int kMmaWarp = 16;
 constexpr int kLoadWarp0 = 21;  // 21, 22: loaders
 constexpr int kLoadWarps = 2;
 constexpr int kWarps = 23;
-constexpr int kRaw = 7;                        // raw tiles in flight per SM
-constexpr uint32_t kRawBytes = KC * TM * 4;    // 16 KB
 constexpr int kMaxStages = 6;
+// per element type T of the features: raw tiles [KC][TM] of T, ~112 KB in flight per SM either way
+template <typename T> constexpr int kRawOf = 7 * 4 / (int)sizeof(T);            // 7 (f32), 14 (bf16)
+template <typename T> constexpr uint32_t kRawBytesOf = KC * TM * sizeof(T);     // 16 KB, 8 KB
+template <typename T> constexpr int kVec = 16 / (int)sizeof(T);   // voxels per 16-byte copy
+// tensor-memory columns of one operand slot: a_hi and a_lo (f32), a alone (bf16)
+template <typename T> constexpr int kSlotCols = sizeof(T) == 4 ? 2 * KC : KC;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return (uint32_t)__cvta_generic_to_shared(p);
@@ -160,7 +172,7 @@ __device__ __forceinline__ float tf32_hi(float x) {  // exactly TF32-representab
 }
 
 struct Params {
-  const float* feat;     // [B,C,V]
+  const void* feat;      // [B,C,V] of T
   const float* w_image;  // k_w_image's output
   const int32_t* cls;    // [Q]
   const float* bin_occ;  // [B,2,V]
@@ -229,18 +241,30 @@ __device__ __forceinline__ void tc_mma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a,
       : "memory");
 }
 
+// a bfloat16 feature widened for the A operand.  The float32 route splits an infinite a into
+// hi = a, lo = a - a = NaN, so every logit it touches is NaN; without a lo half the same
+// logits would be +-inf, so an infinity is widened to a NaN instead (same NaN positions).
+__device__ __forceinline__ float widen_operand(uint16_t h) {
+  const uint32_t x = (uint32_t)h << 16;
+  return __uint_as_float((x << 1) == 0xff000000u ? 0x7fc00000u : x);
+}
+
 // Tensor-memory map (all 512 columns): [0, 2*npad) two accumulator buffers of npad columns
 // (every (voxel, prompt) sum lives in ONE column: a_hi*w_hi + a_hi*w_lo + a_lo*w_hi), then
-// `stages` operand slots of 2*KC columns: a_hi (KC columns, one per channel) and a_lo.
+// `stages` operand slots of kSlotCols<T> columns: a_hi (KC columns, one per channel) and a_lo,
+// or for bfloat16 features a alone.
 // Shared memory holds only the W ring: one [W_hi ; W_lo] block per stage.
 // LOGITS: the epilogue stores the raw logits (semantic_inference_3d alone) instead of labels.
-template <bool LOGITS>
+template <bool LOGITS, typename T>
 __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
+  constexpr int kRaw = kRawOf<T>;
+  constexpr uint32_t kRawBytes = kRawBytesOf<T>;
+  constexpr uint32_t kSlot = (uint32_t)kSlotCols<T>;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int npad = p.npad, stages = p.stages;
   const uint32_t w_bytes = 2 * npad * KC * 4;    // [W_hi ; W_lo] chunk
-  uint8_t* raw_base = smem_raw;                                  // [kRaw] raw tiles [KC][TM] f32
+  uint8_t* raw_base = smem_raw;                                  // [kRaw] raw tiles [KC][TM] of T
   uint8_t* stage_base = smem_raw + (size_t)kRaw * kRawBytes;     // [stages] W blocks
   uint64_t* bars = reinterpret_cast<uint64_t*>(stage_base + (size_t)stages * w_bytes);
   uint64_t* full = bars;                  // [stages]   converters + W copy -> MMA
@@ -291,26 +315,33 @@ __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
   if (warp >= kLoadWarp0) {
     // ============================ LOADERS ============================
     // 16-byte cp.async copies, a warp-instruction per 512-byte row segment (128 voxels of one
-    // channel plane), completion reported to the raw slot's barrier.  Nothing passes through
-    // registers, so the bytes in flight are bounded only by the raw ring (kRaw x 16 KB per SM).
+    // channel plane; for bfloat16 two rows of 256 bytes, 16 lanes each), completion reported to
+    // the raw slot's barrier.  Nothing passes through registers, so the bytes in flight are
+    // bounded only by the raw ring (kRaw x kRawBytes, ~112 KB per SM).
     // (One 512-byte bulk copy per row instead: 77 cycles per copy, 1.9 TB/s in all.)
-    const int lw = warp - kLoadWarp0;                       // rows lw, lw + kLoadWarps, ...
+    constexpr int kRowLanes = TM / kVec<T>;                  // lanes per channel row: 32, 16
+    constexpr int kRowsPerCopy = 32 / kRowLanes;             // channel rows per warp-instruction
+    constexpr int kRowStep = kLoadWarps * kRowsPerCopy;
+    const int lw = warp - kLoadWarp0;
+    const int row = lw * kRowsPerCopy + lane / kRowLanes;    // rows row, row + kRowStep, ...
+    const int seg = lane % kRowLanes;                        // 16-byte piece of the row
     uint32_t rs = 0, rphase = 0;
     bool first_round = true;
     for (int64_t tile = tile_begin; tile < tile_end; tile += tile_step) {
       const int64_t b = tile / vtiles;
-      const int64_t v = (tile - b * vtiles) * TM + 4 * lane;
-      const uint32_t nbytes = v < p.V ? 16u : 0u;           // V % 4 == 0; past the end: zero-fill
-      const float* src = p.feat + ((int64_t)b * p.C + lw) * p.V + (v < p.V ? v : 0);
+      const int64_t v = (tile - b * vtiles) * TM + kVec<T> * seg;
+      const uint32_t nbytes = v < p.V ? 16u : 0u;           // V % kVec == 0; past the end: zero-fill
+      const T* src = static_cast<const T*>(p.feat) + ((int64_t)b * p.C + row) * p.V + (v < p.V ? v : 0);
       for (int ch = 0; ch < n_chunks; ++ch, src += (int64_t)KC * p.V) {
         if (!first_round) mbar_wait(raw_empty + rs, rphase);
-        const uint32_t dst = smem_u32(raw_base + (size_t)rs * kRawBytes) + (uint32_t)(lw * TM * 4 + lane * 16);
+        const uint32_t dst = smem_u32(raw_base + (size_t)rs * kRawBytes) +
+                             (uint32_t)(row * TM * (int)sizeof(T) + seg * 16);
 #ifndef VEON_TAIL_X_NOLOAD
 #pragma unroll
-        for (int r = 0; r < KC / kLoadWarps; ++r)
+        for (int r = 0; r < KC / kRowStep; ++r)
           asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(
-                           dst + (uint32_t)(r * kLoadWarps * TM * 4)),
-                       "l"(src + (int64_t)r * kLoadWarps * p.V), "r"(nbytes)
+                           dst + (uint32_t)(r * kRowStep * TM * (int)sizeof(T))),
+                       "l"(src + (int64_t)r * kRowStep * p.V), "r"(nbytes)
                        : "memory");
 #endif
         asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(raw_full + rs))
@@ -326,11 +357,13 @@ __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
     // ============================ CONVERTERS ============================
     // thread <-> voxel (TMEM lane 32*quarter + lane; a warp reaches only the lanes of warp % 4),
     // warp / 4 = which 8 of the stage's 32 channels.  Column reads of the raw tile are
-    // conflict-free (lanes = consecutive voxels); the values go hi/lo-split from registers
-    // straight into tensor memory, so the tensor core never reads A from shared memory.
+    // conflict-free (lanes = consecutive voxels); the values go hi/lo-split (bfloat16: widened)
+    // from registers straight into tensor memory, so the tensor core never reads A from shared
+    // memory.
     const int quarter = warp & 3, grp = warp >> 2;
     const uint32_t lane_field = (uint32_t)(32 * quarter) << 16;
-    const float* raw_col = reinterpret_cast<const float*>(raw_base) + (kRows * grp) * TM + 32 * quarter + lane;
+    using Raw = typename std::conditional<sizeof(T) == 4, float, uint16_t>::type;
+    const Raw* raw_col = reinterpret_cast<const Raw*>(raw_base) + (kRows * grp) * TM + 32 * quarter + lane;
     uint32_t s = 0, phase = 0;     // operand slot and the parity its `empty` barrier completes next
     uint32_t rs = 0, rphase = 0;   // raw slot and the parity its `raw_full` barrier completes next
     bool first_round = true;
@@ -340,12 +373,16 @@ __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
       mbar_wait(raw_full + rs, rphase);
       VEON_TACC(0)
       float hi[kRows], lo[kRows];
-      const float* col = raw_col + (size_t)rs * (kRawBytes / 4);
+      const Raw* col = raw_col + (size_t)rs * (kRawBytes / sizeof(Raw));
 #pragma unroll
       for (int i = 0; i < kRows; ++i) {
-        const float a = col[i * TM];
-        hi[i] = tf32_hi(a);
-        lo[i] = a - hi[i];
+        if constexpr (sizeof(T) == 4) {
+          const float a = col[i * TM];
+          hi[i] = tf32_hi(a);
+          lo[i] = a - hi[i];
+        } else {
+          hi[i] = widen_operand(col[i * TM]);
+        }
       }
       __syncwarp();
       if (lane == 0) mbar_arrive(raw_empty + rs);   // the values are in registers
@@ -367,9 +404,9 @@ __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
             : "memory");
       }
       if (++sch == n_chunks) sch = 0;
-      const uint32_t slot = a_base + s * (2 * KC) + lane_field + (uint32_t)(kRows * grp);
+      const uint32_t slot = a_base + s * kSlot + lane_field + (uint32_t)(kRows * grp);
       tc_st8(slot, hi);
-      tc_st8(slot + KC, lo);
+      if constexpr (sizeof(T) == 4) tc_st8(slot + KC, lo);
       asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
       tc_fence_before();
       __syncwarp();
@@ -408,7 +445,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
           tc_fence_after();
           VEON_TACC(1)
           const uint32_t sw = sw0 + s * w_bytes;
-          const uint32_t a_hi = a0 + s * (2 * KC), a_lo = a_hi + KC;
+          const uint32_t a_hi = a0 + s * kSlot, a_lo = a_hi + KC;
 #ifndef VEON_TAIL_X_NOMMA
 #pragma unroll
           for (int k = 0; k < KC / 8; ++k) {
@@ -417,7 +454,8 @@ __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
             if (leader) {
               tc_mma_tf32_ts(d, a_hi + 8 * k, w_hi, idesc, (ch > 0 || k > 0) ? 1u : 0u);
               tc_mma_tf32_ts(d, a_hi + 8 * k, w_lo, idesc, 1u);
-              tc_mma_tf32_ts(d, a_lo + 8 * k, w_hi, idesc, 1u);
+              // bfloat16: a_lo = 0, every product of the third MMA is zero and it is not issued
+              if constexpr (sizeof(T) == 4) tc_mma_tf32_ts(d, a_lo + 8 * k, w_hi, idesc, 1u);
             }
           }
 #endif
@@ -542,16 +580,16 @@ extern "C" int veon_internal_tail_trace(unsigned long long* host_out, int clear)
 
 // returns 0 when launched, VEON_E_UNSUPPORTED when the shape does not fit this path.
 // logits != nullptr: write sem_occ [B,Q,V] (cls / bin_occ / labels unused).
-template <bool LOGITS>
+template <bool LOGITS, typename T>
 static int launch_variant(const tc::Params& p, unsigned grid, size_t smem, cudaStream_t stream) {
   static size_t attr_smem_dev[kMaxDevices] = {};   // per device: one process may drive several GPUs
   size_t& attr_smem = attr_smem_dev[current_device()];
   if (smem > attr_smem) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(tc::k_tail_tc<LOGITS>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(tc::k_tail_tc<LOGITS, T>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_smem = smem;
   }
-  tc::k_tail_tc<LOGITS><<<grid, tc::kWarps * 32, smem, stream>>>(p);
+  tc::k_tail_tc<LOGITS, T><<<grid, tc::kWarps * 32, smem, stream>>>(p);
   VEON_LAUNCH_CHECK();
   return 0;
 }
@@ -576,19 +614,28 @@ extern "C" int veon_text_classifier_image(const float* text_w, int Q, int C, voi
   return 0;
 }
 
-int veon_tail_tc_launch(const float* feat_occ, const float* text_w, const int32_t* cls,
+// The shapes the float32 instance takes.  The bfloat16 one also needs V % 8 == 0 (a 16-byte copy
+// carries 8 voxels); both need a 16-byte aligned feat_occ.
+bool veon_tail_tc_takes(int C, int Q, int64_t V, const float* text_w) {
+  const int npad = ((Q + 15) / 16) * 16;
+  return C % tc::KC == 0 && (V & 3) == 0 && V < (int64_t(1) << 31) && npad <= 128 &&
+         ((uintptr_t)text_w & 15) == 0;
+}
+
+template <typename T>
+int veon_tail_tc_launch(const T* feat_occ, const float* text_w, const int32_t* cls,
                         const float* bin_occ, int B, int C, int Q, int Z, int Y, int X,
                         int free_label, uint8_t* labels, float* logits, const void* w_image,
                         cudaStream_t stream) {
   const int64_t V = (int64_t)Z * Y * X;
   const int npad = ((Q + 15) / 16) * 16;
-  if (C % tc::KC != 0 || (V & 3) != 0 || V >= (int64_t(1) << 31) || npad > 128 || (((uintptr_t)feat_occ | (uintptr_t)text_w) & 15))
+  if (!veon_tail_tc_takes(C, Q, V, text_w) || V % tc::kVec<T> != 0 || ((uintptr_t)feat_occ & 15))
     return VEON_E_UNSUPPORTED;
   const size_t w_bytes = 2 * (size_t)npad * tc::KC * 4;
   const size_t tail = 1024;  // barriers + tmem slot
-  int stages = (int)((tc::kTmemCols - 2 * npad) / (2 * tc::KC));   // operand slots in tensor memory
+  int stages = (int)((tc::kTmemCols - 2 * npad) / tc::kSlotCols<T>);   // operand slots in tensor memory
   if (stages > tc::kMaxStages) stages = tc::kMaxStages;
-  const size_t raw = (size_t)tc::kRaw * tc::kRawBytes;
+  const size_t raw = (size_t)tc::kRawOf<T> * tc::kRawBytesOf<T>;
   if (raw + (size_t)stages * w_bytes + tail > 227 * 1024) stages = (int)((227 * 1024 - tail - raw) / w_bytes);
   if (stages < 2) return VEON_E_UNSUPPORTED;
   const size_t smem = raw + stages * w_bytes + tail;
@@ -603,8 +650,8 @@ int veon_tail_tc_launch(const float* feat_occ, const float* text_w, const int32_
   if (w_image) {
     if ((uintptr_t)w_image & 15) return VEON_E_BADARG;
     p.w_image = static_cast<const float*>(w_image);
-    return logits ? launch_variant<true>(p, grid, smem, stream)
-                  : launch_variant<false>(p, grid, smem, stream);
+    return logits ? launch_variant<true, T>(p, grid, smem, stream)
+                  : launch_variant<false, T>(p, grid, smem, stream);
   }
   // no prepared image: build one for the duration of the call in a stream-ordered allocation
   float* image = nullptr;
@@ -613,8 +660,14 @@ int veon_tail_tc_launch(const float* feat_occ, const float* text_w, const int32_
   int rc = veon_text_classifier_image(text_w, Q, C, image, image_bytes, stream);
   p.w_image = image;
   if (rc == 0)
-    rc = logits ? launch_variant<true>(p, grid, smem, stream)
-                : launch_variant<false>(p, grid, smem, stream);
+    rc = logits ? launch_variant<true, T>(p, grid, smem, stream)
+                : launch_variant<false, T>(p, grid, smem, stream);
   cudaFreeAsync(image, stream);
   return rc;
 }
+template int veon_tail_tc_launch<float>(const float*, const float*, const int32_t*, const float*,
+                                        int, int, int, int, int, int, int, uint8_t*, float*,
+                                        const void*, cudaStream_t);
+template int veon_tail_tc_launch<bf16>(const bf16*, const float*, const int32_t*, const float*,
+                                       int, int, int, int, int, int, int, uint8_t*, float*,
+                                       const void*, cudaStream_t);

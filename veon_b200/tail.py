@@ -10,6 +10,11 @@ and, for the decoder-resolution route (SURVEY.md 8f-4), the two up-samplings in 
 (san_in_veon_temporal.py:196-207): `voxel_text_argmax_lowres` classifies the low-resolution
 volume and interpolates the Q logit channels instead of the C feature channels.
 `semantic_inference_3d` is the reference method of that name on its own (logits out).
+
+The three feature-volume entries read a bfloat16 volume as it is (the pooling's bfloat16 output,
+or a 3D decoder's under autocast): half the bytes of the float32 copy they used to make, and the
+same results as that float32 route, byte for byte for the labels and value for value for the
+logits.  Other dtypes are widened to float32; the classifier and the gate always are.
 """
 import ctypes
 
@@ -73,13 +78,35 @@ def prepare_vocabulary(text_embeddings, bg_embed, logit_scale):
     return (scale * emb).clone().detach()
 
 
+def _features(t):
+    """(volume, entry-point suffix): a bfloat16 volume is read as it is (contiguous bfloat16,
+    the `_bf16` entries), anything else as float32"""
+    t = t.detach()
+    if t.dtype == torch.bfloat16:
+        return t.contiguous(), "_bf16"
+    return t.contiguous().float(), ""
+
+
+def _call_features(lib, name, feat, call):
+    """call(entry, volume) on the volume's own dtype; where the bfloat16 entry returns
+    VEON_E_UNSUPPORTED (the float32 route would take the tensor cores, whose bfloat16 loader
+    needs V % 8 == 0 and a 16-byte aligned volume) the volume is widened and the float32 entry
+    called, which is what the bfloat16 entry stands in for."""
+    feat, suffix = _features(feat)
+    rc = call(getattr(lib, name + suffix), feat)
+    if suffix and rc == _lib.E_UNSUPPORTED:
+        suffix = ""
+        rc = call(getattr(lib, name), feat.float())
+    _lib.check(rc, name + suffix)
+
+
 def voxel_text_argmax(feat_occ, ov_classifier_weight, prompt_class, bin_occ, free_label=17):
-    """feat_occ [B,C,Z,Y,X] f32, ov_classifier_weight [Q,C] f32, prompt_class
+    """feat_occ [B,C,Z,Y,X] f32 or bf16, ov_classifier_weight [Q,C] f32, prompt_class
     [Q] int32 (from `class_of_prompt`), bin_occ [B,2,Z,Y,X] f32 ->
-    uint8 occupancy labels [B,X,Y,Z] (free voxels = `free_label`)."""
+    uint8 occupancy labels [B,X,Y,Z] (free voxels = `free_label`).  A bfloat16 feat_occ is read
+    without a float32 copy and gives the labels of `feat_occ.float()`."""
     require_cuda(feat_occ, ov_classifier_weight, prompt_class, bin_occ)
     lib = _lib.load()
-    feat_occ = feat_occ.detach().contiguous().float()
     w = ov_classifier_weight.detach().contiguous().float()
     cls = prompt_class.contiguous().int()
     bin_occ = bin_occ.detach().contiguous().float()
@@ -90,12 +117,12 @@ def voxel_text_argmax(feat_occ, ov_classifier_weight, prompt_class, bin_occ, fre
     dev = feat_occ.device
     with torch.cuda.device(dev):
         labels = torch.empty((B, X, Y, Z), dtype=torch.uint8, device=dev)
-        rc = lib.veon_voxel_text_argmax(
-            ctypes.c_void_p(feat_occ.data_ptr()), ctypes.c_void_p(w.data_ptr()),
+        image = _classifier_image(lib, w, dev)
+        _call_features(lib, "veon_voxel_text_argmax", feat_occ, lambda fn, feat: fn(
+            ctypes.c_void_p(feat.data_ptr()), ctypes.c_void_p(w.data_ptr()),
             ctypes.c_void_p(cls.data_ptr()), ctypes.c_void_p(bin_occ.data_ptr()),
             B, C, Q, Z, Y, X, int(free_label), ctypes.c_void_p(labels.data_ptr()),
-            _classifier_image(lib, w, dev), stream_ptr(dev))
-    _lib.check(rc, "veon_voxel_text_argmax")
+            image, stream_ptr(dev)))
     return labels
 
 
@@ -127,22 +154,22 @@ def semantic_inference_3d(ov_classifier_weight, mask_pred):
     """`SANInVeonTemporal.semantic_inference_3d` (san_in_veon_temporal.py:257-259):
     einsum("qc,bczhw->bqzhw") of the [Q,C] classifier and a [B,C,Z,Y,X] volume -> [B,Q,Z,Y,X]
     f32 (no gradient: the reference's weight is a detached constant and this entry serves the
-    inference route)."""
+    inference route).  A bfloat16 volume is read without a float32 copy and gives the logits of
+    `mask_pred.float()` (NaN where those are NaN; only the sign of an exact zero may differ)."""
     require_cuda(ov_classifier_weight, mask_pred)
     lib = _lib.load()
     w = ov_classifier_weight.detach().contiguous().float()
-    feat = mask_pred.detach().contiguous().float()
-    B, C, Z, Y, X = feat.shape
+    B, C, Z, Y, X = mask_pred.shape
     Q = w.shape[0]
     if w.shape[1] != C:
         raise ValueError("inconsistent tail shapes")
-    dev = feat.device
+    dev = mask_pred.device
     with torch.cuda.device(dev):
         sem = torch.empty((B, Q, Z, Y, X), dtype=torch.float32, device=dev)
-        rc = lib.veon_semantic_inference_3d(
+        image = _classifier_image(lib, w, dev)
+        _call_features(lib, "veon_semantic_inference_3d", mask_pred, lambda fn, feat: fn(
             ctypes.c_void_p(w.data_ptr()), ctypes.c_void_p(feat.data_ptr()), B, C, Q, Z, Y, X,
-            ctypes.c_void_p(sem.data_ptr()), _classifier_image(lib, w, dev), stream_ptr(dev))
-    _lib.check(rc, "veon_semantic_inference_3d")
+            ctypes.c_void_p(sem.data_ptr()), image, stream_ptr(dev)))
     return sem
 
 
@@ -213,32 +240,32 @@ def voxel_text_argmax_lowres(feat_occ_lr, ov_classifier_weight, prompt_class, bi
     """The whole inference tail from the decoder's outputs (san_in_veon_temporal.py:196-208 +
     the merge and label rule): feat_occ_lr [B,C,Zi,Yi,Xi], bin_occ_lr [B,2,Zi,Yi,Xi] ->
     uint8 labels [B,X,Y,Z] on the `occ_size` grid.  `workspace`: optional float32 CUDA tensor of
-    at least B*Q*Zi*Yi*Xi elements to hold the low-resolution logits (allocated if absent)."""
+    at least B*Q*Zi*Yi*Xi elements to hold the low-resolution logits (allocated if absent).
+    A bfloat16 feat_occ_lr is read without a float32 copy and gives the labels of
+    `feat_occ_lr.float()`; bin_occ_lr is taken as float32."""
     require_cuda(feat_occ_lr, ov_classifier_weight, prompt_class, bin_occ_lr)
     lib = _lib.load()
-    feat = feat_occ_lr.detach().contiguous().float()
     w = ov_classifier_weight.detach().contiguous().float()
     cls = prompt_class.contiguous().int()
     gate = bin_occ_lr.detach().contiguous().float()
-    B, C, Zi, Yi, Xi = feat.shape
+    B, C, Zi, Yi, Xi = feat_occ_lr.shape
     Q = w.shape[0]
     Z, Y, X = (int(v) for v in occ_size)
     if w.shape[1] != C or cls.numel() != Q or tuple(gate.shape) != (B, 2, Zi, Yi, Xi):
         raise ValueError("inconsistent tail shapes")
-    dev = feat.device
+    dev = feat_occ_lr.device
     need = lib.veon_voxel_text_argmax_lowres_workspace_bytes(B, Q, Zi, Yi, Xi)
     with torch.cuda.device(dev):
         if workspace is None:
             workspace = torch.empty(need // 4, dtype=torch.float32, device=dev)
         ws_bytes = workspace.numel() * workspace.element_size()
         labels = torch.empty((B, X, Y, Z), dtype=torch.uint8, device=dev)
-        rc = lib.veon_voxel_text_argmax_lowres(
+        image = _classifier_image(lib, w, dev)
+        _call_features(lib, "veon_voxel_text_argmax_lowres", feat_occ_lr, lambda fn, feat: fn(
             ctypes.c_void_p(feat.data_ptr()), ctypes.c_void_p(w.data_ptr()),
             ctypes.c_void_p(cls.data_ptr()), ctypes.c_void_p(gate.data_ptr()),
             B, C, Q, Zi, Yi, Xi, Z, Y, X, int(free_label), ctypes.c_void_p(labels.data_ptr()),
-            ctypes.c_void_p(workspace.data_ptr()), ws_bytes, _classifier_image(lib, w, dev),
-            stream_ptr(dev))
-    _lib.check(rc, "veon_voxel_text_argmax_lowres")
+            ctypes.c_void_p(workspace.data_ptr()), ws_bytes, image, stream_ptr(dev)))
     return labels
 
 
