@@ -574,6 +574,49 @@ int veon_voxel_text_argmax_lowres_bf16(const uint16_t* feat_occ_lr, const float*
                                        void* workspace, size_t ws_bytes, const void* w_image,
                                        void* stream);
 
+/* The three tail entry points, float32 and bfloat16, on a channels-last feature volume:
+ * feat_occ / feat_occ_lr hold
+ * [B,Z,Y,X,C] (float32, or bfloat16 for _cl_bf16), as a channels_last_3d [B,C,Z,Y,X] tensor
+ * stores it, e.g. a 3D decoder running cuDNN's conv3d in that layout, or the pooling's _cl
+ * entries.  Every result equals the channels-first twin's on the same volume made contiguous, bit
+ * for bit: the tensor-core kernel reads each voxel's 32-channel segments into the same
+ * tensor-memory lanes and columns and issues the same MMAs.  Only that kernel has a channels-last
+ * loader, so these entries run exactly where the channels-first call on the contiguous volume
+ * takes tcgen05 (C % 32 == 0, Q <= 128, V % 4 == 0) and feat_occ is 16-byte aligned; elsewhere
+ * they return VEON_E_UNSUPPORTED and the caller makes the volume contiguous.  A bfloat16 volume
+ * with V % 8 == 4 runs here although its channels-first twin widens it: the bits are the same.
+ * Arguments, checks and error codes are the channels-first twins'; text_w, bin_occ /
+ * bin_occ_lr, w_image and every output keep their layout. */
+int veon_voxel_text_argmax_cl(const float* feat_occ, const float* text_w,
+                              const int32_t* class_of_prompt, const float* bin_occ,
+                              int B, int C, int Q, int Z, int Y, int X,
+                              int free_label, uint8_t* labels, const void* w_image,
+                              void* stream);
+int veon_voxel_text_argmax_cl_bf16(const uint16_t* feat_occ, const float* text_w,
+                                   const int32_t* class_of_prompt, const float* bin_occ,
+                                   int B, int C, int Q, int Z, int Y, int X,
+                                   int free_label, uint8_t* labels, const void* w_image,
+                                   void* stream);
+int veon_semantic_inference_3d_cl(const float* text_w, const float* feat_occ,
+                                  int B, int C, int Q, int Z, int Y, int X,
+                                  float* sem_occ, const void* w_image, void* stream);
+int veon_semantic_inference_3d_cl_bf16(const float* text_w, const uint16_t* feat_occ,
+                                       int B, int C, int Q, int Z, int Y, int X,
+                                       float* sem_occ, const void* w_image, void* stream);
+int veon_voxel_text_argmax_lowres_cl(const float* feat_occ_lr, const float* text_w,
+                                     const int32_t* class_of_prompt, const float* bin_occ_lr,
+                                     int B, int C, int Q, int Zi, int Yi, int Xi,
+                                     int Z, int Y, int X, int free_label, uint8_t* labels,
+                                     void* workspace, size_t ws_bytes, const void* w_image,
+                                     void* stream);
+int veon_voxel_text_argmax_lowres_cl_bf16(const uint16_t* feat_occ_lr, const float* text_w,
+                                          const int32_t* class_of_prompt,
+                                          const float* bin_occ_lr,
+                                          int B, int C, int Q, int Zi, int Yi, int Xi,
+                                          int Z, int Y, int X, int free_label, uint8_t* labels,
+                                          void* workspace, size_t ws_bytes,
+                                          const void* w_image, void* stream);
+
 /* Multi-GPU callers that overlap a collective (NCCL on another stream) with the path: the
  * persistent grids here fill every SM, so the collective's CTAs wait for a kernel boundary.
  * veon_reserve_sms(n) makes every persistent grid of the library launch on (SM count - n) SMs;

@@ -1,7 +1,8 @@
 """Where the roles of k_tail_tc (CTA 0) spend their cycles on one call; needs a build with
 -DVEON_TAIL_TRACE (tools/build_variant.sh) loaded through VEON_LIB.
 
-    python tools/tail_trace.py [q67] [bf16]     (bf16: a bfloat16 feature volume)"""
+    python tools/tail_trace.py [q67] [bf16] [cl]     (bf16: a bfloat16 feature volume;
+                                                      cl: a channels_last_3d one)"""
 import ctypes
 import os
 import sys
@@ -24,6 +25,8 @@ w = torch.randn(len(refl) + 1, C, device=dev, generator=g)
 bo = torch.randn(B, 2, 16, 200, 200, device=dev, generator=g)
 if "bf16" in sys.argv[1:]:
     feat = feat.to(torch.bfloat16)
+if "cl" in sys.argv[1:]:
+    feat = feat.contiguous(memory_format=torch.channels_last_3d)
 cls = class_of_prompt(refl).to(dev)
 lib = ctypes.CDLL(_lib.LIB_PATH)
 for _ in range(3):

@@ -113,6 +113,20 @@ _SIGNATURES = {
     "veon_voxel_text_argmax_lowres_bf16": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
                                                    c_int, c_int, c_int, c_int, c_int, _P, _P, c_size_t,
                                                    _P, _P]),
+    "veon_voxel_text_argmax_cl": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int,
+                                          c_int, _P, _P, _P]),
+    "veon_voxel_text_argmax_cl_bf16": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
+                                               c_int, c_int, _P, _P, _P]),
+    "veon_semantic_inference_3d_cl": (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, c_int, _P,
+                                              _P, _P]),
+    "veon_semantic_inference_3d_cl_bf16": (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, c_int,
+                                                   _P, _P, _P]),
+    "veon_voxel_text_argmax_lowres_cl": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
+                                                 c_int, c_int, c_int, c_int, c_int, _P, _P, c_size_t,
+                                                 _P, _P]),
+    "veon_voxel_text_argmax_lowres_cl_bf16": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int,
+                                                      c_int, c_int, c_int, c_int, c_int, c_int, _P, _P,
+                                                      c_size_t, _P, _P]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

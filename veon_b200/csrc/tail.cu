@@ -12,7 +12,8 @@
 // V % 4 != 0, more than 128 prompt rows) -- one thread per voxel, text rows staged in
 // shared memory per prompt tile, everything after the dot products fused in registers.
 // Features are float32 or bfloat16 (T); a bfloat16 value is widened exactly on load, so the
-// bfloat16 instances give the float32 ones' bits on x.float().
+// bfloat16 instances give the float32 ones' bits on x.float().  Channels-last volumes
+// ([B,Z,Y,X,C], the _cl entries) take the tensor-core path alone.
 #include <math.h>
 
 #include "common.cuh"
@@ -114,9 +115,10 @@ k_voxel_text_argmax(const T* __restrict__ feat_occ, const float* __restrict__ te
 
 using namespace veon;
 
-// tensor-core path (tail_tc.cu); VEON_E_UNSUPPORTED when the shape does not fit it
+// tensor-core path (tail_tc.cu); VEON_E_UNSUPPORTED when the shape does not fit it.
+// CL: feat_occ is channels-last [B,Z,Y,X,C].
 bool veon_tail_tc_takes(int C, int Q, int64_t V, const float* text_w);
-template <typename T>
+template <typename T, bool CL>
 int veon_tail_tc_launch(const T* feat_occ, const float* text_w, const int32_t* cls,
                         const float* bin_occ, int B, int C, int Q, int Z, int Y, int X,
                         int free_label, uint8_t* labels, float* logits, const void* w_image,
@@ -132,7 +134,7 @@ static int tail_dispatch(const T* feat_occ, const float* text_w,
                          int Q, int Z, int Y, int X, int free_label, uint8_t* labels,
                          float* logits, const void* w_image, cudaStream_t stream) {
   {  // tcgen05 path unless the shape does not fit it (C % 32, V % 4, Q > 128)
-    const int rc = veon_tail_tc_launch<T>(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y,
+    const int rc = veon_tail_tc_launch<T, false>(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y,
                                           X, free_label, labels, logits, w_image, stream);
     if (rc != VEON_E_UNSUPPORTED) return rc;
     if (sizeof(T) == 2 && veon_tail_tc_takes(C, Q, (int64_t)Z * Y * X, text_w)) return rc;
@@ -161,7 +163,24 @@ static int tail_dispatch(const T* feat_occ, const float* text_w,
   return 0;
 }
 
-template <typename T>
+// A channels-last volume (CL) takes tcgen05 exactly where the channels-first call on its
+// contiguous copy does, so both give the same bits; everywhere else (C % 32 != 0, V % 4 != 0,
+// Q > 128, a feat_occ that is not 16-byte aligned) VEON_E_UNSUPPORTED, and the caller makes the
+// volume contiguous.  There is no channels-last FFMA kernel.
+template <bool CL, typename T>
+static int tail_route(const T* feat_occ, const float* text_w, const int32_t* class_of_prompt,
+                      const float* bin_occ, int B, int C, int Q, int Z, int Y, int X,
+                      int free_label, uint8_t* labels, float* logits, const void* w_image,
+                      cudaStream_t stream) {
+  if constexpr (CL)
+    return veon_tail_tc_launch<T, true>(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y,
+                                        X, free_label, labels, logits, w_image, stream);
+  else
+    return tail_dispatch(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y, X, free_label,
+                         labels, logits, w_image, stream);
+}
+
+template <bool CL = false, typename T>
 static int voxel_text_argmax(const T* feat_occ, const float* text_w,
                              const int32_t* class_of_prompt, const float* bin_occ, int B, int C,
                              int Q, int Z, int Y, int X, int free_label, uint8_t* labels,
@@ -169,19 +188,19 @@ static int voxel_text_argmax(const T* feat_occ, const float* text_w,
   if (!feat_occ || !text_w || !class_of_prompt || !bin_occ || !labels || B <= 0 || C <= 0 ||
       Q <= 0 || Z <= 0 || Y <= 0 || X <= 0 || B > 65535)
     return VEON_E_BADARG;
-  return tail_dispatch(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y, X, free_label,
-                       labels, nullptr, w_image, (cudaStream_t)stream);
+  return tail_route<CL>(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y, X, free_label,
+                        labels, nullptr, w_image, (cudaStream_t)stream);
 }
 
-template <typename T>
+template <bool CL = false, typename T>
 static int semantic_inference_3d(const float* text_w, const T* feat_occ, int B, int C, int Q,
                                  int Z, int Y, int X, float* sem_occ, const void* w_image,
                                  void* stream) {
   if (!feat_occ || !text_w || !sem_occ || B <= 0 || C <= 0 || Q <= 0 || Z <= 0 || Y <= 0 ||
       X <= 0 || B > 65535)
     return VEON_E_BADARG;
-  return tail_dispatch(feat_occ, text_w, nullptr, nullptr, B, C, Q, Z, Y, X, 0, nullptr, sem_occ,
-                       w_image, (cudaStream_t)stream);
+  return tail_route<CL>(feat_occ, text_w, nullptr, nullptr, B, C, Q, Z, Y, X, 0, nullptr, sem_occ,
+                        w_image, (cudaStream_t)stream);
 }
 
 extern "C" int veon_voxel_text_argmax(const float* feat_occ, const float* text_w,
@@ -212,6 +231,38 @@ extern "C" int veon_semantic_inference_3d_bf16(const float* text_w, const uint16
                                                float* sem_occ, const void* w_image, void* stream) {
   return semantic_inference_3d(text_w, reinterpret_cast<const bf16*>(feat_occ), B, C, Q, Z, Y, X,
                                sem_occ, w_image, stream);
+}
+
+// channels-last feat_occ [B,Z,Y,X,C]
+extern "C" int veon_voxel_text_argmax_cl(const float* feat_occ, const float* text_w,
+                                         const int32_t* class_of_prompt, const float* bin_occ,
+                                         int B, int C, int Q, int Z, int Y, int X, int free_label,
+                                         uint8_t* labels, const void* w_image, void* stream) {
+  return voxel_text_argmax<true>(feat_occ, text_w, class_of_prompt, bin_occ, B, C, Q, Z, Y, X,
+                                 free_label, labels, w_image, stream);
+}
+
+extern "C" int veon_voxel_text_argmax_cl_bf16(const uint16_t* feat_occ, const float* text_w,
+                                              const int32_t* class_of_prompt, const float* bin_occ,
+                                              int B, int C, int Q, int Z, int Y, int X,
+                                              int free_label, uint8_t* labels,
+                                              const void* w_image, void* stream) {
+  return voxel_text_argmax<true>(reinterpret_cast<const bf16*>(feat_occ), text_w, class_of_prompt,
+                                 bin_occ, B, C, Q, Z, Y, X, free_label, labels, w_image, stream);
+}
+
+extern "C" int veon_semantic_inference_3d_cl(const float* text_w, const float* feat_occ, int B,
+                                             int C, int Q, int Z, int Y, int X, float* sem_occ,
+                                             const void* w_image, void* stream) {
+  return semantic_inference_3d<true>(text_w, feat_occ, B, C, Q, Z, Y, X, sem_occ, w_image, stream);
+}
+
+extern "C" int veon_semantic_inference_3d_cl_bf16(const float* text_w, const uint16_t* feat_occ,
+                                                  int B, int C, int Q, int Z, int Y, int X,
+                                                  float* sem_occ, const void* w_image,
+                                                  void* stream) {
+  return semantic_inference_3d<true>(text_w, reinterpret_cast<const bf16*>(feat_occ), B, C, Q, Z,
+                                     Y, X, sem_occ, w_image, stream);
 }
 
 // ---- training-time voxel x text arg-max over a POINT LIST (SURVEY 8f-4) ----------------------

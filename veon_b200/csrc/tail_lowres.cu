@@ -299,9 +299,9 @@ extern "C" size_t veon_voxel_text_argmax_lowres_workspace_bytes(int B, int Q, in
   return sizeof(float) * (size_t)B * Q * Zi * Yi * Xi;
 }
 
-// T = float or uint16_t (bfloat16): the logits pass of that element type, then the same
-// interpolation and classification of the float32 logits
-template <typename T>
+// T = float or uint16_t (bfloat16), CL = channels-last [B,Zi,Yi,Xi,C]: the logits pass of that
+// element type and layout, then the same interpolation and classification of the float32 logits
+template <bool CL = false, typename T>
 static int voxel_text_argmax_lowres(const T* feat_occ_lr, const float* text_w,
                                     const int32_t* class_of_prompt, const float* bin_occ_lr, int B,
                                     int C, int Q, int Zi, int Yi, int Xi, int Z, int Y, int X,
@@ -312,7 +312,13 @@ static int voxel_text_argmax_lowres(const T* feat_occ_lr, const float* text_w,
     return VEON_E_WORKSPACE;
   float* sem_lr = static_cast<float*>(workspace);
   int rc;
-  if constexpr (sizeof(T) == 4)
+  if constexpr (CL && sizeof(T) == 4)
+    rc = veon_semantic_inference_3d_cl(text_w, feat_occ_lr, B, C, Q, Zi, Yi, Xi, sem_lr, w_image,
+                                       stream);
+  else if constexpr (CL)
+    rc = veon_semantic_inference_3d_cl_bf16(text_w, feat_occ_lr, B, C, Q, Zi, Yi, Xi, sem_lr,
+                                            w_image, stream);
+  else if constexpr (sizeof(T) == 4)
     rc = veon_semantic_inference_3d(text_w, feat_occ_lr, B, C, Q, Zi, Yi, Xi, sem_lr, w_image, stream);
   else
     rc = veon_semantic_inference_3d_bf16(text_w, feat_occ_lr, B, C, Q, Zi, Yi, Xi, sem_lr, w_image,
@@ -343,4 +349,29 @@ extern "C" int veon_voxel_text_argmax_lowres_bf16(const uint16_t* feat_occ_lr, c
   return voxel_text_argmax_lowres(feat_occ_lr, text_w, class_of_prompt, bin_occ_lr, B, C, Q, Zi,
                                   Yi, Xi, Z, Y, X, free_label, labels, workspace, ws_bytes,
                                   w_image, stream);
+}
+
+extern "C" int veon_voxel_text_argmax_lowres_cl(const float* feat_occ_lr, const float* text_w,
+                                                const int32_t* class_of_prompt,
+                                                const float* bin_occ_lr, int B, int C, int Q,
+                                                int Zi, int Yi, int Xi, int Z, int Y, int X,
+                                                int free_label, uint8_t* labels, void* workspace,
+                                                size_t ws_bytes, const void* w_image,
+                                                void* stream) {
+  return voxel_text_argmax_lowres<true>(feat_occ_lr, text_w, class_of_prompt, bin_occ_lr, B, C, Q,
+                                        Zi, Yi, Xi, Z, Y, X, free_label, labels, workspace,
+                                        ws_bytes, w_image, stream);
+}
+
+extern "C" int veon_voxel_text_argmax_lowres_cl_bf16(const uint16_t* feat_occ_lr,
+                                                     const float* text_w,
+                                                     const int32_t* class_of_prompt,
+                                                     const float* bin_occ_lr, int B, int C, int Q,
+                                                     int Zi, int Yi, int Xi, int Z, int Y, int X,
+                                                     int free_label, uint8_t* labels,
+                                                     void* workspace, size_t ws_bytes,
+                                                     const void* w_image, void* stream) {
+  return voxel_text_argmax_lowres<true>(feat_occ_lr, text_w, class_of_prompt, bin_occ_lr, B, C, Q,
+                                        Zi, Yi, Xi, Z, Y, X, free_label, labels, workspace,
+                                        ws_bytes, w_image, stream);
 }

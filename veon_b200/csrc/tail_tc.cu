@@ -33,6 +33,13 @@
 // instance reads half the bytes ([KC][TM] bf16 raw tiles, twice as many in flight), writes one
 // tensor-memory column per channel (no lo half) and issues a*w_hi + a*w_lo per K-step: the
 // float32 instance's sums on x.float(), bit for bit.
+//
+// Channels-last features (CL = true, feat_occ [B,Z,Y,X,C]): a voxel's 32 channels of a stage are
+// one contiguous 128-byte (bfloat16: 64-byte) segment.  The loaders copy those segments into a
+// voxel-major raw tile [TM][KC] of T whose 16-byte pieces are XOR-swizzled by voxel, and a
+// converter thread reads its voxel's kRows channels with 16-byte loads, conflict-free.  From the
+// registers on nothing changes: the same values go to the same tensor-memory lanes and columns and
+// the MMAs are the same, so a channels-last volume gives the bits of its contiguous copy.
 #include <math.h>
 
 #include <type_traits>
@@ -59,6 +66,14 @@ template <typename T> constexpr uint32_t kRawBytesOf = KC * TM * sizeof(T);     
 template <typename T> constexpr int kVec = 16 / (int)sizeof(T);   // voxels per 16-byte copy
 // tensor-memory columns of one operand slot: a_hi and a_lo (f32), a alone (bf16)
 template <typename T> constexpr int kSlotCols = sizeof(T) == 4 ? 2 * KC : KC;
+// channels-last raw tiles: one row of KC channels per voxel, kPieces 16-byte pieces (8 f32, 4 bf16)
+template <typename T> constexpr int kPieces = KC * (int)sizeof(T) / 16;
+// where piece j of voxel row v sits in its row: the 8 lanes of a quarter-warp phase (8 consecutive
+// voxels, one piece index) land on 8 distinct 16-byte positions of a 128-byte line.  f32: one row
+// per line, j ^ (v & 7); bf16: two rows per line, j ^ ((v >> 1) & 3).
+template <typename T> __device__ __forceinline__ uint32_t cl_piece(int j, int v) {
+  return (uint32_t)(j ^ ((v / (8 / kPieces<T>)) & (kPieces<T> - 1)));
+}
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return (uint32_t)__cvta_generic_to_shared(p);
@@ -172,7 +187,7 @@ __device__ __forceinline__ float tf32_hi(float x) {  // exactly TF32-representab
 }
 
 struct Params {
-  const void* feat;      // [B,C,V] of T
+  const void* feat;      // [B,C,V] of T; channels-last instances: [B,V,C]
   const float* w_image;  // k_w_image's output
   const int32_t* cls;    // [Q]
   const float* bin_occ;  // [B,2,V]
@@ -255,7 +270,9 @@ __device__ __forceinline__ float widen_operand(uint16_t h) {
 // or for bfloat16 features a alone.
 // Shared memory holds only the W ring: one [W_hi ; W_lo] block per stage.
 // LOGITS: the epilogue stores the raw logits (semantic_inference_3d alone) instead of labels.
-template <bool LOGITS, typename T>
+// CL: feat is channels-last [B,V,C]; only the loaders and the converters' shared-memory reads
+// differ (raw tiles [TM][KC] of T, swizzled by cl_piece).
+template <bool LOGITS, typename T, bool CL = false>
 __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
   constexpr int kRaw = kRawOf<T>;
   constexpr uint32_t kRawBytes = kRawBytesOf<T>;
@@ -319,40 +336,82 @@ __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
     // the raw slot's barrier.  Nothing passes through registers, so the bytes in flight are
     // bounded only by the raw ring (kRaw x kRawBytes, ~112 KB per SM).
     // (One 512-byte bulk copy per row instead: 77 cycles per copy, 1.9 TB/s in all.)
-    constexpr int kRowLanes = TM / kVec<T>;                  // lanes per channel row: 32, 16
-    constexpr int kRowsPerCopy = 32 / kRowLanes;             // channel rows per warp-instruction
-    constexpr int kRowStep = kLoadWarps * kRowsPerCopy;
-    const int lw = warp - kLoadWarp0;
-    const int row = lw * kRowsPerCopy + lane / kRowLanes;    // rows row, row + kRowStep, ...
-    const int seg = lane % kRowLanes;                        // 16-byte piece of the row
-    uint32_t rs = 0, rphase = 0;
-    bool first_round = true;
-    for (int64_t tile = tile_begin; tile < tile_end; tile += tile_step) {
-      const int64_t b = tile / vtiles;
-      const int64_t v = (tile - b * vtiles) * TM + kVec<T> * seg;
-      const uint32_t nbytes = v < p.V ? 16u : 0u;           // V % kVec == 0; past the end: zero-fill
-      const T* src = static_cast<const T*>(p.feat) + ((int64_t)b * p.C + row) * p.V + (v < p.V ? v : 0);
-      for (int ch = 0; ch < n_chunks; ++ch, src += (int64_t)KC * p.V) {
-        if (!first_round) mbar_wait(raw_empty + rs, rphase);
-        const uint32_t dst = smem_u32(raw_base + (size_t)rs * kRawBytes) +
-                             (uint32_t)(row * TM * (int)sizeof(T) + seg * 16);
+    if constexpr (CL) {
+      // channels-last: kPieces lanes per voxel segment (KC channels of one voxel), 32 / kPieces
+      // voxels per warp-instruction, so the instruction count per stage is the channels-first one
+      constexpr int kVoxPerCopy = 32 / kPieces<T>;
+      constexpr int kVoxStep = kLoadWarps * kVoxPerCopy;
+      constexpr int kRowBytes = KC * (int)sizeof(T);
+      const int lw = warp - kLoadWarp0;
+      const int vox = lw * kVoxPerCopy + lane / kPieces<T>;  // voxels vox, vox + kVoxStep, ...
+      const int piece = lane % kPieces<T>;
+      const T* feat = static_cast<const T*>(p.feat) + piece * kVec<T>;
+      uint32_t rs = 0, rphase = 0;
+      bool first_round = true;
+      for (int64_t tile = tile_begin; tile < tile_end; tile += tile_step) {
+        const int64_t b = tile / vtiles;
+        const int64_t v0 = (tile - b * vtiles) * TM + vox;
+        for (int ch = 0; ch < n_chunks; ++ch) {
+          if (!first_round) mbar_wait(raw_empty + rs, rphase);
+          const uint32_t dst = smem_u32(raw_base + (size_t)rs * kRawBytes);
 #ifndef VEON_TAIL_X_NOLOAD
 #pragma unroll
-        for (int r = 0; r < KC / kRowStep; ++r)
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(
-                           dst + (uint32_t)(r * kRowStep * TM * (int)sizeof(T))),
-                       "l"(src + (int64_t)r * kRowStep * p.V), "r"(nbytes)
-                       : "memory");
+          for (int r = 0; r < TM / kVoxStep; ++r) {
+            const int vl = vox + r * kVoxStep;
+            const int64_t v = v0 + r * kVoxStep;
+            const uint32_t nbytes = v < p.V ? 16u : 0u;   // past the end: zero-fill
+            const T* src = feat + ((int64_t)b * p.V + (v < p.V ? v : 0)) * p.C + ch * KC;
+            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(
+                             dst + (uint32_t)(vl * kRowBytes) + (cl_piece<T>(piece, vl) << 4)),
+                         "l"(src), "r"(nbytes)
+                         : "memory");
+          }
 #endif
-        asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(raw_full + rs))
-                     : "memory");
-        if (++rs == kRaw) {
-          rs = 0;
-          if (first_round) first_round = false; else rphase ^= 1;
+          asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(raw_full + rs))
+                       : "memory");
+          if (++rs == kRaw) {
+            rs = 0;
+            if (first_round) first_round = false; else rphase ^= 1;
+          }
         }
       }
+      asm volatile("cp.async.wait_all;" ::: "memory");
+    } else {
+      constexpr int kRowLanes = TM / kVec<T>;                  // lanes per channel row: 32, 16
+      constexpr int kRowsPerCopy = 32 / kRowLanes;             // channel rows per warp-instruction
+      constexpr int kRowStep = kLoadWarps * kRowsPerCopy;
+      const int lw = warp - kLoadWarp0;
+      const int row = lw * kRowsPerCopy + lane / kRowLanes;    // rows row, row + kRowStep, ...
+      const int seg = lane % kRowLanes;                        // 16-byte piece of the row
+      uint32_t rs = 0, rphase = 0;
+      bool first_round = true;
+      for (int64_t tile = tile_begin; tile < tile_end; tile += tile_step) {
+        const int64_t b = tile / vtiles;
+        const int64_t v = (tile - b * vtiles) * TM + kVec<T> * seg;
+        const uint32_t nbytes = v < p.V ? 16u : 0u;           // V % kVec == 0; past the end: zero-fill
+        const T* src = static_cast<const T*>(p.feat) + ((int64_t)b * p.C + row) * p.V + (v < p.V ? v : 0);
+        for (int ch = 0; ch < n_chunks; ++ch, src += (int64_t)KC * p.V) {
+          if (!first_round) mbar_wait(raw_empty + rs, rphase);
+          const uint32_t dst = smem_u32(raw_base + (size_t)rs * kRawBytes) +
+                               (uint32_t)(row * TM * (int)sizeof(T) + seg * 16);
+#ifndef VEON_TAIL_X_NOLOAD
+#pragma unroll
+          for (int r = 0; r < KC / kRowStep; ++r)
+            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(
+                             dst + (uint32_t)(r * kRowStep * TM * (int)sizeof(T))),
+                         "l"(src + (int64_t)r * kRowStep * p.V), "r"(nbytes)
+                         : "memory");
+#endif
+          asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(raw_full + rs))
+                       : "memory");
+          if (++rs == kRaw) {
+            rs = 0;
+            if (first_round) first_round = false; else rphase ^= 1;
+          }
+        }
+      }
+      asm volatile("cp.async.wait_all;" ::: "memory");
     }
-    asm volatile("cp.async.wait_all;" ::: "memory");
   } else if (warp < kProdWarps) {
     // ============================ CONVERTERS ============================
     // thread <-> voxel (TMEM lane 32*quarter + lane; a warp reaches only the lanes of warp % 4),
@@ -364,6 +423,12 @@ __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
     const uint32_t lane_field = (uint32_t)(32 * quarter) << 16;
     using Raw = typename std::conditional<sizeof(T) == 4, float, uint16_t>::type;
     const Raw* raw_col = reinterpret_cast<const Raw*>(raw_base) + (kRows * grp) * TM + 32 * quarter + lane;
+    // channels-last: this voxel's row of the [TM][KC] tile and the pieces holding its kRows
+    // channels (two for f32, one for bf16)
+    const int cl_vox = 32 * quarter + lane;
+    const uint32_t cl_row = (uint32_t)(cl_vox * KC * (int)sizeof(T));
+    const uint32_t cl_off0 = cl_row + (cl_piece<T>(kRows * grp * (int)sizeof(T) / 16, cl_vox) << 4);
+    const uint32_t cl_off1 = cl_row + (cl_piece<T>(kRows * grp * (int)sizeof(T) / 16 + 1, cl_vox) << 4);
     uint32_t s = 0, phase = 0;     // operand slot and the parity its `empty` barrier completes next
     uint32_t rs = 0, rphase = 0;   // raw slot and the parity its `raw_full` barrier completes next
     bool first_round = true;
@@ -373,15 +438,34 @@ __global__ void __launch_bounds__(kWarps * 32, 1) k_tail_tc(const Params p) {
       mbar_wait(raw_full + rs, rphase);
       VEON_TACC(0)
       float hi[kRows], lo[kRows];
-      const Raw* col = raw_col + (size_t)rs * (kRawBytes / sizeof(Raw));
-#pragma unroll
-      for (int i = 0; i < kRows; ++i) {
+      if constexpr (CL) {
+        const uint8_t* tile = raw_base + (size_t)rs * kRawBytes;
         if constexpr (sizeof(T) == 4) {
-          const float a = col[i * TM];
-          hi[i] = tf32_hi(a);
-          lo[i] = a - hi[i];
+          const float4 x0 = *reinterpret_cast<const float4*>(tile + cl_off0);
+          const float4 x1 = *reinterpret_cast<const float4*>(tile + cl_off1);
+          const float a[kRows] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
+#pragma unroll
+          for (int i = 0; i < kRows; ++i) {
+            hi[i] = tf32_hi(a[i]);
+            lo[i] = a[i] - hi[i];
+          }
         } else {
-          hi[i] = widen_operand(col[i * TM]);
+          const uint4 x = *reinterpret_cast<const uint4*>(tile + cl_off0);
+          const uint32_t w[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+          for (int i = 0; i < kRows; ++i) hi[i] = widen_operand((uint16_t)(w[i / 2] >> (16 * (i & 1))));
+        }
+      } else {
+        const Raw* col = raw_col + (size_t)rs * (kRawBytes / sizeof(Raw));
+#pragma unroll
+        for (int i = 0; i < kRows; ++i) {
+          if constexpr (sizeof(T) == 4) {
+            const float a = col[i * TM];
+            hi[i] = tf32_hi(a);
+            lo[i] = a - hi[i];
+          } else {
+            hi[i] = widen_operand(col[i * TM]);
+          }
         }
       }
       __syncwarp();
@@ -580,16 +664,16 @@ extern "C" int veon_internal_tail_trace(unsigned long long* host_out, int clear)
 
 // returns 0 when launched, VEON_E_UNSUPPORTED when the shape does not fit this path.
 // logits != nullptr: write sem_occ [B,Q,V] (cls / bin_occ / labels unused).
-template <bool LOGITS, typename T>
+template <bool LOGITS, typename T, bool CL>
 static int launch_variant(const tc::Params& p, unsigned grid, size_t smem, cudaStream_t stream) {
   static size_t attr_smem_dev[kMaxDevices] = {};   // per device: one process may drive several GPUs
   size_t& attr_smem = attr_smem_dev[current_device()];
   if (smem > attr_smem) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(tc::k_tail_tc<LOGITS, T>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(tc::k_tail_tc<LOGITS, T, CL>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_smem = smem;
   }
-  tc::k_tail_tc<LOGITS, T><<<grid, tc::kWarps * 32, smem, stream>>>(p);
+  tc::k_tail_tc<LOGITS, T, CL><<<grid, tc::kWarps * 32, smem, stream>>>(p);
   VEON_LAUNCH_CHECK();
   return 0;
 }
@@ -615,21 +699,25 @@ extern "C" int veon_text_classifier_image(const float* text_w, int Q, int C, voi
 }
 
 // The shapes the float32 instance takes.  The bfloat16 one also needs V % 8 == 0 (a 16-byte copy
-// carries 8 voxels); both need a 16-byte aligned feat_occ.
+// carries 8 voxels); both need a 16-byte aligned feat_occ.  The channels-last instances need
+// neither V % 4 nor V % 8 (a copy carries channels of one voxel), but they keep V % 4 == 0: the
+// channels-first call takes the FFMA kernel otherwise, whose sums differ from tcgen05's, and a
+// channels-last volume must give its contiguous copy's bits.
 bool veon_tail_tc_takes(int C, int Q, int64_t V, const float* text_w) {
   const int npad = ((Q + 15) / 16) * 16;
   return C % tc::KC == 0 && (V & 3) == 0 && V < (int64_t(1) << 31) && npad <= 128 &&
          ((uintptr_t)text_w & 15) == 0;
 }
 
-template <typename T>
+// CL: feat_occ is channels-last [B,Z,Y,X,C]
+template <typename T, bool CL>
 int veon_tail_tc_launch(const T* feat_occ, const float* text_w, const int32_t* cls,
                         const float* bin_occ, int B, int C, int Q, int Z, int Y, int X,
                         int free_label, uint8_t* labels, float* logits, const void* w_image,
                         cudaStream_t stream) {
   const int64_t V = (int64_t)Z * Y * X;
   const int npad = ((Q + 15) / 16) * 16;
-  if (!veon_tail_tc_takes(C, Q, V, text_w) || V % tc::kVec<T> != 0 || ((uintptr_t)feat_occ & 15))
+  if (!veon_tail_tc_takes(C, Q, V, text_w) || (!CL && V % tc::kVec<T> != 0) || ((uintptr_t)feat_occ & 15))
     return VEON_E_UNSUPPORTED;
   const size_t w_bytes = 2 * (size_t)npad * tc::KC * 4;
   const size_t tail = 1024;  // barriers + tmem slot
@@ -650,8 +738,8 @@ int veon_tail_tc_launch(const T* feat_occ, const float* text_w, const int32_t* c
   if (w_image) {
     if ((uintptr_t)w_image & 15) return VEON_E_BADARG;
     p.w_image = static_cast<const float*>(w_image);
-    return logits ? launch_variant<true, T>(p, grid, smem, stream)
-                  : launch_variant<false, T>(p, grid, smem, stream);
+    return logits ? launch_variant<true, T, CL>(p, grid, smem, stream)
+                  : launch_variant<false, T, CL>(p, grid, smem, stream);
   }
   // no prepared image: build one for the duration of the call in a stream-ordered allocation
   float* image = nullptr;
@@ -660,14 +748,16 @@ int veon_tail_tc_launch(const T* feat_occ, const float* text_w, const int32_t* c
   int rc = veon_text_classifier_image(text_w, Q, C, image, image_bytes, stream);
   p.w_image = image;
   if (rc == 0)
-    rc = logits ? launch_variant<true, T>(p, grid, smem, stream)
-                : launch_variant<false, T>(p, grid, smem, stream);
+    rc = logits ? launch_variant<true, T, CL>(p, grid, smem, stream)
+                : launch_variant<false, T, CL>(p, grid, smem, stream);
   cudaFreeAsync(image, stream);
   return rc;
 }
-template int veon_tail_tc_launch<float>(const float*, const float*, const int32_t*, const float*,
-                                        int, int, int, int, int, int, int, uint8_t*, float*,
-                                        const void*, cudaStream_t);
-template int veon_tail_tc_launch<bf16>(const bf16*, const float*, const int32_t*, const float*,
-                                       int, int, int, int, int, int, int, uint8_t*, float*,
-                                       const void*, cudaStream_t);
+#define VEON_TAIL_TC_INSTANCE(T, CL)                                                              \
+  template int veon_tail_tc_launch<T, CL>(const T*, const float*, const int32_t*, const float*, int, \
+                                          int, int, int, int, int, int, uint8_t*, float*,            \
+                                          const void*, cudaStream_t);
+VEON_TAIL_TC_INSTANCE(float, false)
+VEON_TAIL_TC_INSTANCE(bf16, false)
+VEON_TAIL_TC_INSTANCE(float, true)
+VEON_TAIL_TC_INSTANCE(bf16, true)

@@ -15,6 +15,10 @@ The three feature-volume entries read a bfloat16 volume as it is (the pooling's 
 or a 3D decoder's under autocast): half the bytes of the float32 copy they used to make, and the
 same results as that float32 route, byte for byte for the labels and value for value for the
 logits.  Other dtypes are widened to float32; the classifier and the gate always are.
+
+A float32 or bfloat16 volume in `torch.channels_last_3d` (a 3D decoder running its conv3d in that
+layout, or the pooling's channels-last output) is read as it is too, with the bits of the same
+call on its contiguous copy; shapes the channels-last kernel does not take are copied first.
 """
 import ctypes
 
@@ -87,11 +91,29 @@ def _features(t):
     return t.contiguous().float(), ""
 
 
+def _channels_last(t):
+    """a 5-D float32 / bfloat16 volume stored [B,Z,Y,X,C] (channels_last_3d, not contiguous)"""
+    return (t.dim() == 5 and t.dtype in (torch.float32, torch.bfloat16) and not t.is_contiguous()
+            and t.is_contiguous(memory_format=torch.channels_last_3d))
+
+
 def _call_features(lib, name, feat, call):
     """call(entry, volume) on the volume's own dtype; where the bfloat16 entry returns
     VEON_E_UNSUPPORTED (the float32 route would take the tensor cores, whose bfloat16 loader
     needs V % 8 == 0 and a 16-byte aligned volume) the volume is widened and the float32 entry
-    called, which is what the bfloat16 entry stands in for."""
+    called, which is what the bfloat16 entry stands in for.
+
+    A channels-last volume goes as it is to the `_cl` / `_cl_bf16` entry, which gives the bits of
+    the contiguous route; where that entry returns VEON_E_UNSUPPORTED (a shape the channels-first
+    call runs on the FFMA kernel, or a volume that is not 16-byte aligned) the volume is made
+    contiguous in its own dtype and takes the route above."""
+    feat = feat.detach()
+    if _channels_last(feat):
+        suffix = "_cl_bf16" if feat.dtype == torch.bfloat16 else "_cl"
+        rc = call(getattr(lib, name + suffix), feat)
+        if rc != _lib.E_UNSUPPORTED:
+            _lib.check(rc, name + suffix)
+            return
     feat, suffix = _features(feat)
     rc = call(getattr(lib, name + suffix), feat)
     if suffix and rc == _lib.E_UNSUPPORTED:
@@ -104,7 +126,9 @@ def voxel_text_argmax(feat_occ, ov_classifier_weight, prompt_class, bin_occ, fre
     """feat_occ [B,C,Z,Y,X] f32 or bf16, ov_classifier_weight [Q,C] f32, prompt_class
     [Q] int32 (from `class_of_prompt`), bin_occ [B,2,Z,Y,X] f32 ->
     uint8 occupancy labels [B,X,Y,Z] (free voxels = `free_label`).  A bfloat16 feat_occ is read
-    without a float32 copy and gives the labels of `feat_occ.float()`."""
+    without a float32 copy and gives the labels of `feat_occ.float()`.  A channels_last_3d
+    feat_occ (float32 or bfloat16) is read without a contiguous copy where the tensor cores take
+    the shape, and gives the labels of `feat_occ.contiguous()`."""
     require_cuda(feat_occ, ov_classifier_weight, prompt_class, bin_occ)
     lib = _lib.load()
     w = ov_classifier_weight.detach().contiguous().float()
@@ -155,7 +179,10 @@ def semantic_inference_3d(ov_classifier_weight, mask_pred):
     einsum("qc,bczhw->bqzhw") of the [Q,C] classifier and a [B,C,Z,Y,X] volume -> [B,Q,Z,Y,X]
     f32 (no gradient: the reference's weight is a detached constant and this entry serves the
     inference route).  A bfloat16 volume is read without a float32 copy and gives the logits of
-    `mask_pred.float()` (NaN where those are NaN; only the sign of an exact zero may differ)."""
+    `mask_pred.float()` (NaN where those are NaN; only the sign of an exact zero may differ).
+    A channels_last_3d volume (float32 or bfloat16) is read without a contiguous copy where the
+    tensor cores take the shape, and gives the logits of `mask_pred.contiguous()` bit for bit;
+    the logits are contiguous [B,Q,Z,Y,X] either way."""
     require_cuda(ov_classifier_weight, mask_pred)
     lib = _lib.load()
     w = ov_classifier_weight.detach().contiguous().float()
@@ -242,7 +269,9 @@ def voxel_text_argmax_lowres(feat_occ_lr, ov_classifier_weight, prompt_class, bi
     uint8 labels [B,X,Y,Z] on the `occ_size` grid.  `workspace`: optional float32 CUDA tensor of
     at least B*Q*Zi*Yi*Xi elements to hold the low-resolution logits (allocated if absent).
     A bfloat16 feat_occ_lr is read without a float32 copy and gives the labels of
-    `feat_occ_lr.float()`; bin_occ_lr is taken as float32."""
+    `feat_occ_lr.float()`; bin_occ_lr is taken as float32.  A channels_last_3d feat_occ_lr
+    (float32 or bfloat16) is read without a contiguous copy where the tensor cores take the shape,
+    and gives the labels of `feat_occ_lr.contiguous()`; bin_occ_lr is made contiguous."""
     require_cuda(feat_occ_lr, ov_classifier_weight, prompt_class, bin_occ_lr)
     lib = _lib.load()
     w = ov_classifier_weight.detach().contiguous().float()
