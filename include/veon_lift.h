@@ -444,6 +444,98 @@ int veon_bev_pool_v2_bwd_planar_ds(const float* grad_ds, const uint8_t* mask,
                                    float* rows_ws, float* depth_grad, float* feat_grad,
                                    void* stream);
 
+/* bfloat16 feature rows.  The planar forwards and backwards above for feat given as bfloat16
+ * [B*N*H*W, C] rows (uint16_t bit patterns), the input a network running under bfloat16 autocast
+ * hands the lift.  Same arguments, checks and error codes as the twin without `_bf16feat`.
+ * Every feature value is widened to float32 exactly where it is loaded, and everything after the
+ * load is the twin's float32 arithmetic in the same order: each volume (float32 or bfloat16) is,
+ * bit for bit, the twin's volume on the widened rows, and depth_grad (float32) is the twin's
+ * depth_grad.  feat_grad is bfloat16 [B*N*H*W, C]: the twin's float32 feat_grad rounded once, to
+ * nearest even.  The vectorised kernels need C % 4 == 0 and 8-byte aligned rows (else the
+ * lane-per-channel kernel, which reads any alignment).  The feature-row range check is the
+ * float32 one.  veon_bev_pool_v2_fwd_planar_bf16feat returns VEON_E_UNSUPPORTED where its twin
+ * would take the two-role streaming kernel, which reads float32 rows only: the caller then widens
+ * the rows and calls veon_bev_pool_v2_fwd_planar. */
+int veon_bev_pool_v2_fwd_planar_bf16feat(const float* depth, const uint16_t* feat,
+                                         const int32_t* ranks_depth, const int32_t* ranks_feat,
+                                         const int32_t* ranks_bev, const int32_t* tile_start,
+                                         const int32_t* tile_istart /* may be NULL */,
+                                         const uint32_t* tile_occ /* may be NULL */,
+                                         const int32_t* tile_heavy /* may be NULL */,
+                                         int64_t tile_heavy_ints, int B, int C,
+                                         int64_t voxels_per_sample, int64_t n_feat_rows,
+                                         float* out, void* workspace, size_t workspace_bytes,
+                                         void* stream);
+int veon_bev_pool_v2_fwd_planar_bf16_bf16feat(const float* depth, const uint16_t* feat,
+                                              const int32_t* ranks_depth,
+                                              const int32_t* ranks_feat,
+                                              const int32_t* ranks_bev,
+                                              const int32_t* tile_start,
+                                              const int32_t* tile_istart /* may be NULL */,
+                                              const uint32_t* tile_occ /* may be NULL */,
+                                              const int32_t* tile_heavy /* may be NULL */,
+                                              int64_t tile_heavy_ints, int B, int C,
+                                              int64_t voxels_per_sample, int64_t n_feat_rows,
+                                              uint16_t* out /* bfloat16 [B,C,Z,Y,X] */,
+                                              void* workspace, size_t workspace_bytes,
+                                              void* stream);
+int veon_bev_pool_v2_fwd_planar_cl_bf16feat(const float* depth, const uint16_t* feat,
+                                            const int32_t* ranks_depth, const int32_t* ranks_feat,
+                                            const int32_t* ranks_bev, const int32_t* tile_start,
+                                            const int32_t* tile_heavy /* may be NULL */,
+                                            int64_t tile_heavy_ints, int B, int C,
+                                            int64_t voxels_per_sample, int64_t n_feat_rows,
+                                            float* out /* [B,Z,Y,X,C] */, void* stream);
+int veon_bev_pool_v2_fwd_planar_cl_bf16_bf16feat(const float* depth, const uint16_t* feat,
+                                                 const int32_t* ranks_depth,
+                                                 const int32_t* ranks_feat,
+                                                 const int32_t* ranks_bev,
+                                                 const int32_t* tile_start,
+                                                 const int32_t* tile_heavy /* may be NULL */,
+                                                 int64_t tile_heavy_ints, int B, int C,
+                                                 int64_t voxels_per_sample, int64_t n_feat_rows,
+                                                 uint16_t* out /* bfloat16 [B,Z,Y,X,C] */,
+                                                 void* stream);
+int veon_bev_pool_v2_bwd_planar_bf16feat(const float* out_grad, const float* depth,
+                                         const uint16_t* feat, const int32_t* tile_istart,
+                                         const uint32_t* tile_occ, const int32_t* point_interval,
+                                         int64_t n_intervals, int B, int N, int D, int H, int W,
+                                         int C, int64_t voxels_per_sample, float* rows_ws,
+                                         int64_t rows_ws_floats, float* depth_grad,
+                                         uint16_t* feat_grad, void* stream);
+int veon_bev_pool_v2_bwd_planar_bf16_bf16feat(const uint16_t* out_grad, const float* depth,
+                                              const uint16_t* feat, const int32_t* tile_istart,
+                                              const uint32_t* tile_occ,
+                                              const int32_t* point_interval, int64_t n_intervals,
+                                              int B, int N, int D, int H, int W, int C,
+                                              int64_t voxels_per_sample, float* rows_ws,
+                                              int64_t rows_ws_floats, float* depth_grad,
+                                              uint16_t* feat_grad, void* stream);
+int veon_bev_pool_v2_bwd_planar_cl_bf16feat(const float* out_grad, const float* depth,
+                                            const uint16_t* feat, const int32_t* ranks_bev,
+                                            const int32_t* interval_starts,
+                                            const int32_t* point_interval, int B, int N, int D,
+                                            int H, int W, int C, int64_t voxels_per_sample,
+                                            float* depth_grad, uint16_t* feat_grad, void* stream);
+int veon_bev_pool_v2_bwd_planar_cl_bf16_bf16feat(const uint16_t* out_grad, const float* depth,
+                                                 const uint16_t* feat, const int32_t* ranks_bev,
+                                                 const int32_t* interval_starts,
+                                                 const int32_t* point_interval, int B, int N,
+                                                 int D, int H, int W, int C,
+                                                 int64_t voxels_per_sample, float* depth_grad,
+                                                 uint16_t* feat_grad, void* stream);
+int veon_bev_pool_v2_bwd_planar_ds_bf16feat(const float* grad_ds, const uint8_t* mask,
+                                            const float* depth, const uint16_t* feat,
+                                            const int32_t* tile_istart, const uint32_t* tile_occ,
+                                            const int32_t* point_interval, int64_t n_intervals,
+                                            int B, int N, int D, int H, int W, int C, int Z, int Y,
+                                            int X, float* rows_ws, float* depth_grad,
+                                            uint16_t* feat_grad, void* stream);
+/* veon_transpose_batched for 2-byte elements (bfloat16 maps and feature gradients): the same
+ * tiles and checks, the bits moved unchanged. */
+int veon_transpose_batched_u16(const uint16_t* src, int64_t batch, int R, int S, uint16_t* dst,
+                               void* stream);
+
 /* ------------------------------------------------------------------------
  * (4) Open-vocabulary tail: voxel-feature x text-embedding logits, per-class
  *     max over prompts, argmax, occupancy gate, uint8 labels.

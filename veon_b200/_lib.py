@@ -84,6 +84,33 @@ _SIGNATURES = {
                                                  _P, c_int64, _P, _P, _P]),
     "veon_bev_pool_v2_bwd_planar_cl_bf16": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int,
                                                     c_int, c_int, c_int, c_int64, _P, _P, _P]),
+    "veon_bev_pool_v2_fwd_planar_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, c_int64,
+                                                     c_int, c_int, c_int64, c_int64, _P, _P,
+                                                     c_size_t, _P]),
+    "veon_bev_pool_v2_fwd_planar_bf16_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P,
+                                                          c_int64, c_int, c_int, c_int64, c_int64,
+                                                          _P, _P, c_size_t, _P]),
+    "veon_bev_pool_v2_fwd_planar_cl_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64,
+                                                        c_int, c_int, c_int64, c_int64, _P, _P]),
+    "veon_bev_pool_v2_fwd_planar_cl_bf16_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64,
+                                                             c_int, c_int, c_int64, c_int64, _P,
+                                                             _P]),
+    "veon_bev_pool_v2_bwd_planar_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, c_int64,
+                                                     c_int, c_int, c_int, c_int, c_int, c_int,
+                                                     c_int64, _P, c_int64, _P, _P, _P]),
+    "veon_bev_pool_v2_bwd_planar_bf16_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, c_int64,
+                                                          c_int, c_int, c_int, c_int, c_int, c_int,
+                                                          c_int64, _P, c_int64, _P, _P, _P]),
+    "veon_bev_pool_v2_bwd_planar_cl_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int,
+                                                        c_int, c_int, c_int, c_int, c_int64, _P,
+                                                        _P, _P]),
+    "veon_bev_pool_v2_bwd_planar_cl_bf16_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int,
+                                                             c_int, c_int, c_int, c_int, c_int64,
+                                                             _P, _P, _P]),
+    "veon_bev_pool_v2_bwd_planar_ds_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64,
+                                                        c_int, c_int, c_int, c_int, c_int, c_int,
+                                                        c_int, c_int, c_int, _P, _P, _P, _P]),
+    "veon_transpose_batched_u16": (c_int, [_P, c_int64, c_int, c_int, _P, _P]),
     "veon_bev_pool_v2_bwd_workspace_floats": (c_size_t, [c_int64, c_int, c_int, c_int, c_int, c_int,
                                                          c_int, c_int64]),
     "veon_bev_pool_v2_bwd_planar": (c_int, [_P, _P, _P, _P, _P, _P, c_int64,

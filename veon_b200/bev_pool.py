@@ -27,6 +27,11 @@ the volume in bfloat16, written so by the kernels: float32 sums rounded once, at
 the store, so the result is bit for bit the float32 volume cast to bfloat16.  Its
 bfloat16 gradient is read in place and widened exactly (depth / feat gradients
 stay float32).
+
+A bfloat16 `feat` (what a network under bfloat16 autocast hands the lift) is read as it is: the
+kernels widen each value exactly where they load it, so every volume is bit for bit the one the
+same call makes from `feat.float()`, depth_grad is that call's, and feat_grad comes back in
+bfloat16, that call's feat_grad rounded once.  Only the bfloat16 rows are kept for the backward.
 """
 import collections
 import functools
@@ -447,7 +452,7 @@ def pool_prepared_downsampled(depth, feat, prep, bev_feat_shape):
     lib = _lib.load()
     dev = feat.device
     depth = depth.detach().contiguous().float()
-    feat, _ = _feat_rows(feat.detach())
+    feat = _feat_rows(feat.detach())[0].float()     # the fused kernel reads float32 rows
     with torch.cuda.device(dev):
         out = torch.empty((B, C, Z // 2, Y // 2, X // 2), dtype=torch.float32, device=dev)
         with _timed("pool_ds_fwd", dev):
@@ -585,16 +590,17 @@ class PoolMaxDown(torch.autograd.Function):
         dev = feat.device
         g = grad_ds.contiguous().float()
         _need_backward_tables(plan)
+        suffix = "_bf16feat" if feat.dtype == torch.bfloat16 else ""
         with torch.cuda.device(dev):
             depth_grad = torch.empty_like(depth)
-            feat_grad = torch.empty_like(feat)
+            feat_grad = torch.empty_like(feat)          # in the rows' dtype
             n_int, rows = _bwd_rows(lib, plan, C, dev)
-            with _timed("pool_bwd_ds", dev):
-                rc = lib.veon_bev_pool_v2_bwd_planar_ds(
+            with _timed("pool_bwd_ds" + suffix, dev):
+                rc = getattr(lib, "veon_bev_pool_v2_bwd_planar_ds" + suffix)(
                     _ptr(g), _ptr(mask), _ptr(depth), _ptr(feat), _ptr(plan.tile_istart),
                     _ptr(plan.tile_occ), _ptr(plan.point_interval), n_int, B, N, D, H, W, C,
                     Z, Y, X, _ptr(rows), _ptr(depth_grad), _ptr(feat_grad), _stream_ptr(dev))
-        _lib.check(rc, "veon_bev_pool_v2_bwd_planar_ds")
+        _lib.check(rc, "veon_bev_pool_v2_bwd_planar_ds" + suffix)
         return depth_grad, _feat_grad_back(feat_grad, ctx.feat_transposed), None, None
 
 
@@ -628,25 +634,30 @@ def voxel_pooling_prepare_v2(coor, grid_lower_bound, grid_interval, grid_size):
 
 # ------------------------------------------------------------------ pooling
 def _transpose_batched(src, batch, R, S, out_shape):
-    """[batch][R][S] -> [batch][S][R] of a contiguous float32 tensor, returned as `out_shape`."""
+    """[batch][R][S] -> [batch][S][R] of a contiguous float32 or bfloat16 tensor (bfloat16 bits
+    are moved, not rounded), returned as `out_shape` in the same dtype."""
     lib = _lib.load()
     dev = src.device
+    what = "veon_transpose_batched_u16" if src.dtype == torch.bfloat16 else "veon_transpose_batched"
     with torch.cuda.device(dev):
-        dst = torch.empty(out_shape, dtype=torch.float32, device=dev)
-        rc = lib.veon_transpose_batched(_ptr(src), batch, R, S, _ptr(dst), _stream_ptr(dev))
-    _lib.check(rc, "veon_transpose_batched")
+        dst = torch.empty(out_shape, dtype=src.dtype, device=dev)
+        rc = getattr(lib, what)(_ptr(src), batch, R, S, _ptr(dst), _stream_ptr(dev))
+    _lib.check(rc, what)
     return dst
 
 
 def _feat_rows(feat):
-    """feat [B,N,H,W,C] as contiguous float32 rows, and whether they were transposed: the necks
-    hand over a channels-last VIEW of channels-first maps, which our own transpose kernel turns
-    into rows instead of a strided copy."""
-    if (feat.dtype == torch.float32 and not feat.is_contiguous()
+    """feat [B,N,H,W,C] as contiguous rows, and whether they were transposed: float32 and bfloat16
+    rows keep their dtype, any other dtype is widened to float32.  The necks hand over a
+    channels-last VIEW of channels-first maps, which our own transpose kernel turns into rows
+    instead of a strided copy."""
+    if (feat.dtype in _DTYPES and not feat.is_contiguous()
             and feat.permute(0, 1, 4, 2, 3).is_contiguous()):
         B, N, H, W, C = feat.shape
         return _transpose_batched(feat.permute(0, 1, 4, 2, 3), B * N, C, H * W,
                                   (B, N, H, W, C)), True
+    if feat.dtype == torch.bfloat16:
+        return feat.contiguous(), False
     return feat.contiguous().float(), False
 
 
@@ -680,13 +691,15 @@ def _fwd_workspace(lib, dev, B, C, V):
 
 def _fwd_planar(depth, feat, rd, rf, rb, plan, B, C, V, shape5, channels_last=False,
                 dtype=torch.float32):
-    """Planar forward of a valid plan into a new volume `shape5` of `dtype` (float32 or
-    bfloat16): [B,C,Z,Y,X], or [B,Z,Y,X,C] with channels_last (the streaming kernel and its
-    workspace are float32 channels-first only)."""
+    """Planar forward of a valid plan from float32 or bfloat16 rows `feat` into a new volume
+    `shape5` of `dtype` (float32 or bfloat16): [B,C,Z,Y,X], or [B,Z,Y,X,C] with channels_last
+    (the streaming kernel and its workspace are float32 channels-first only, from float32 rows:
+    where it would run, bfloat16 rows are widened first)."""
     lib = _lib.load()
     dev = feat.device
     bf16 = dtype is torch.bfloat16
-    suffix = "_bf16" if bf16 else ""
+    bf16feat = feat.dtype == torch.bfloat16
+    suffix = ("_bf16" if bf16 else "") + ("_bf16feat" if bf16feat else "")
     with torch.cuda.device(dev):
         out = torch.empty(shape5, dtype=dtype, device=dev)
         if channels_last:
@@ -706,6 +719,10 @@ def _fwd_planar(depth, feat, rd, rf, rb, plan, B, C, V, shape5, channels_last=Fa
                     _ptr(plan.tile_heavy), plan.tile_heavy.numel(),
                     B, C, V, feat.numel() // C, _ptr(out), None if bf16 else _ptr(ws),
                     0 if bf16 else ws.numel(), _stream_ptr(dev))
+    if bf16feat and rc == _lib.E_UNSUPPORTED:
+        # a 64-channel float32 channels-first volume: the streaming kernel, on widened rows
+        return _fwd_planar(depth, feat.float(), rd, rf, rb, plan, B, C, V, shape5, channels_last,
+                           dtype)
     _lib.check(rc, what)
     return out
 
@@ -733,13 +750,14 @@ def _pool_bwd(out_grad, depth, feat, rd, rf, rb, ist, plan):
     float32 or bfloat16 channels-last (out_grad contiguous, its [B,C,Z,Y,X] view not) with a
     valid plan -> the single pass, which reads the gradient rows in place; otherwise a valid plan
     -> the two passes on a channels-first copy (bfloat16 stays bfloat16, anything else becomes
-    float32); a rejected plan -> the generic kernel on a float32 copy."""
+    float32); a rejected plan -> the generic kernel on a float32 copy.  feat_grad has the dtype of
+    the rows `feat` (float32 or bfloat16)."""
     lib = _lib.load()
     dev = feat.device
     _, Z, Y, X, C = out_grad.shape
     g = out_grad.permute(0, 4, 1, 2, 3)  # back to the channels-first storage order
     bf16 = out_grad.dtype == torch.bfloat16 and plan.ok
-    suffix = "_bf16" if bf16 else ""
+    suffix = ("_bf16" if bf16 else "") + ("_bf16feat" if feat.dtype == torch.bfloat16 else "")
     single = ((out_grad.dtype == torch.float32 or bf16) and not g.is_contiguous()
               and out_grad.is_contiguous() and plan.ok)
     if not single:
@@ -747,10 +765,13 @@ def _pool_bwd(out_grad, depth, feat, rd, rf, rb, ist, plan):
     with torch.cuda.device(dev):
         if not plan.ok:
             what = "veon_bev_pool_v2_grad_generic"
-            depth_grad, feat_grad = torch.zeros_like(depth), torch.zeros_like(feat)
+            featf = feat.float()                 # the generic kernels read float32 rows
+            depth_grad, feat_grad = torch.zeros_like(depth), torch.zeros_like(featf)
             rc = lib.veon_bev_pool_v2_grad_generic(
-                C, rb.numel(), LAYOUT_BCZYX, Z * Y * X, _ptr(g), _ptr(depth), _ptr(feat), _ptr(rd),
-                _ptr(rf), _ptr(rb), _ptr(depth_grad), _ptr(feat_grad), _stream_ptr(dev))
+                C, rb.numel(), LAYOUT_BCZYX, Z * Y * X, _ptr(g), _ptr(depth), _ptr(featf),
+                _ptr(rd), _ptr(rf), _ptr(rb), _ptr(depth_grad), _ptr(feat_grad), _stream_ptr(dev))
+            _lib.check(rc, what)
+            return depth_grad, feat_grad.to(feat.dtype)
         else:
             _need_backward_tables(plan)
             B, N, D, H, W = plan.dims
@@ -787,7 +808,8 @@ class QuickCumsumCuda(torch.autograd.Function):
     [B,Z,Y,X,C] gradient) with a valid plan -> the single-pass kernel, which reads
     the gradient rows in place; anything else is copied to channels-first first.
     All routes give the same bits.  With the extra `dtype` torch.bfloat16 the volume is
-    bfloat16 (the float32 one rounded once), and so is the gradient the backward reads."""
+    bfloat16 (the float32 one rounded once), and so is the gradient the backward reads.  A
+    bfloat16 `feat` is pooled and saved as bfloat16 rows; its gradient is bfloat16."""
 
     @staticmethod
     def forward(ctx, depth, feat, ranks_depth, ranks_feat, ranks_bev,
@@ -827,13 +849,14 @@ class QuickCumsumCuda(torch.autograd.Function):
             out = _fwd_planar(depth, feat, ranks_depth, ranks_feat, ranks_bev, plan, B, C, V,
                               shape5, channels_last, dtype)
         else:
-            # the interval-driven generic kernel adds into a zeroed volume
+            # the interval-driven generic kernel adds float32 rows into a zeroed volume
             lib = _lib.load()
-            out = feat.new_zeros(shape5)
+            featf = feat.float()
+            out = featf.new_zeros(shape5)
             with torch.cuda.device(feat.device):
                 rc = lib.veon_bev_pool_v2_generic(
                     C, interval_starts.numel(), LAYOUT_BZYXC if channels_last else LAYOUT_BCZYX, V,
-                    _ptr(depth), _ptr(feat), _ptr(ranks_depth), _ptr(ranks_feat), _ptr(ranks_bev),
+                    _ptr(depth), _ptr(featf), _ptr(ranks_depth), _ptr(ranks_feat), _ptr(ranks_bev),
                     _ptr(interval_starts), _ptr(interval_lengths), _ptr(out),
                     _stream_ptr(feat.device))
             _lib.check(rc, "veon_bev_pool_v2_generic")

@@ -174,6 +174,35 @@ __device__ __forceinline__ float ldg_widen(const bf16* p) {
   return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
 }
 
+// bfloat16 feature rows (the pooling's input under autocast): four channels are one 16-byte
+// (float) or 8-byte (bf16, 8-byte aligned) read-only load, widened exactly in registers; a
+// feature gradient stored as bf16 is rounded once, to nearest even.
+__device__ __forceinline__ float4 ldg_widen4(const float* p) {
+  return __ldg(reinterpret_cast<const float4*>(p));
+}
+__device__ __forceinline__ float4 ldg_widen4(const bf16* p) {
+  const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+  float4 r;
+  r.x = __uint_as_float(u.x << 16);
+  r.y = __uint_as_float(u.x & 0xffff0000u);
+  r.z = __uint_as_float(u.y << 16);
+  r.w = __uint_as_float(u.y & 0xffff0000u);
+  return r;
+}
+__device__ __forceinline__ void store_rn(float* p, float v) { *p = v; }
+__device__ __forceinline__ void store_rn(bf16* p, float v) { *p = __float2bfloat16_rn(v); }
+
+// four elements of a row or a channel plane into shared memory: 16 bytes of float, 8 of bf16
+// (cp.async.cg copies 16 bytes only)
+__device__ __forceinline__ void cp_async_4(float* smem_dst, const float* gsrc) {
+  const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
+}
+__device__ __forceinline__ void cp_async_4(bf16* smem_dst, const bf16* gsrc) {
+  const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(d), "l"(gsrc) : "memory");
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -82,10 +82,12 @@ int launch_cam_xforms(const float* sensor2ego, const float* cam2imgs, const floa
 // view_transformer.py:279-285 views + permutes it) and the pooling kernels gather
 // channel-contiguous rows; the reference lets `.contiguous()` do the copy
 // (bev_pool.py:88).  Batched tiled transpose [batch][R][S] -> [batch][S][R], used in
-// both directions (feat forward, feat_grad backward).
+// both directions (feat forward, feat_grad backward).  E = uint16_t moves bfloat16 maps and
+// gradients as bits: nothing is rounded.
+template <typename E>
 __global__ void __launch_bounds__(256)
-k_transpose(const float* __restrict__ src, int R, int S, float* __restrict__ dst) {
-  __shared__ float t[32][33];
+k_transpose(const E* __restrict__ src, int R, int S, E* __restrict__ dst) {
+  __shared__ E t[32][33];
   const int64_t base = (int64_t)blockIdx.z * R * S;
   const int s0 = blockIdx.x * 32, r0 = blockIdx.y * 32;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
@@ -130,15 +132,25 @@ extern "C" int veon_lidar_coor(const float* frustum, const float* sensor2ego,
   return 0;
 }
 
-extern "C" int veon_transpose_batched(const float* src, int64_t batch, int R, int S, float* dst,
-                                      void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
+template <typename E>
+static int transpose_batched(const E* src, int64_t batch, int R, int S, E* dst,
+                             cudaStream_t stream) {
   if (!src || !dst || batch <= 0 || R <= 0 || S <= 0) return VEON_E_BADARG;
   if (batch > 65535) return VEON_E_RANGE;
   const dim3 grid((unsigned)((S + 31) / 32), (unsigned)((R + 31) / 32), (unsigned)batch);
   k_transpose<<<grid, 256, 0, stream>>>(src, R, S, dst);
   VEON_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int veon_transpose_batched(const float* src, int64_t batch, int R, int S, float* dst,
+                                      void* stream) {
+  return transpose_batched(src, batch, R, S, dst, (cudaStream_t)stream);
+}
+
+extern "C" int veon_transpose_batched_u16(const uint16_t* src, int64_t batch, int R, int S,
+                                          uint16_t* dst, void* stream) {
+  return transpose_batched(src, batch, R, S, dst, (cudaStream_t)stream);
 }
 
 // ---- calibration hash (SURVEY 8f-3: rank cache keyed on the calibration) ------------------------

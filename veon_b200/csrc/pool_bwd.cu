@@ -124,19 +124,6 @@ k_bwd_rows(const T* __restrict__ out_grad, const int32_t* __restrict__ tile_ista
 // nor the transposition/row write sits between two tiles' loads.
 constexpr int kRowPitchP = kTileVoxels + 4;  // 16-byte aligned rows for cp.async
 
-__device__ __forceinline__ void cp_async16_cg(void* smem_dst, const void* gsrc) {
-  const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
-}
-// four voxels of a channel plane: 16 bytes of float, 8 of bf16 (cp.async.cg copies 16 bytes only)
-__device__ __forceinline__ void cp_async_4(float* smem_dst, const float* gsrc) {
-  cp_async16_cg(smem_dst, gsrc);
-}
-__device__ __forceinline__ void cp_async_4(bf16* smem_dst, const bf16* gsrc) {
-  const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(d), "l"(gsrc) : "memory");
-}
-
 // T = bf16: the shared tiles hold the gradient's own bf16 values, widened as the rows are extracted.
 template <int KCH, typename T = float>
 __global__ void __launch_bounds__(kRowWarps * 32)
@@ -408,16 +395,18 @@ __device__ __forceinline__ float reduce_many(float (&d)[U], int lane, int& which
 // voxel, ranks_bev[interval_starts[interval]] (only intervals a kept point names are read, so a
 // capacity-sized interval_starts is never read past the device-side interval count).
 // T = bf16 (CL only): the gradient rows are bf16, widened in registers.
-template <int KCH, bool COHERENT, bool CL = false, typename T = float>
+// TF = bf16: the pixel's feature row is read as bf16 and widened; feat_grad is stored as bf16,
+// each float sum rounded once.
+template <int KCH, bool COHERENT, bool CL = false, typename T = float, typename TF = float>
 __device__ __forceinline__ void pixel_warp(float* wsm, int lane, const T* __restrict__ rows,
                                            const float* __restrict__ depth,
-                                           const float* __restrict__ feat,
+                                           const TF* __restrict__ feat,
                                            const int32_t* __restrict__ point_interval,
                                            const int32_t* __restrict__ ranks_bev,
                                            const int32_t* __restrict__ interval_starts,
                                            int64_t pix, int D, int HW, int C,
                                            float* __restrict__ depth_grad,
-                                           float* __restrict__ feat_grad) {
+                                           TF* __restrict__ feat_grad) {
   constexpr int CC = 32 * KCH;
   constexpr int U = (KCH <= 2) ? 8 : 4;  // gradient rows in flight per warp
   // per warp: dots[D] | dep[D] | iis[D] (row index: interval, CL: voxel) | kd[D]
@@ -458,7 +447,7 @@ __device__ __forceinline__ void pixel_warp(float* wsm, int lane, const T* __rest
 #pragma unroll
     for (int k = 0; k < KCH; ++k) {
       const int c = cbase + lane + 32 * k;
-      f[k] = c < C ? __ldg(feat + pix * C + c) : 0.f;
+      f[k] = c < C ? ldg_widen(feat + pix * C + c) : 0.f;
       acc[k] = 0.f;
     }
     for (int j0 = 0; j0 < nk; j0 += U) {
@@ -496,7 +485,7 @@ __device__ __forceinline__ void pixel_warp(float* wsm, int lane, const T* __rest
 #pragma unroll
     for (int k = 0; k < KCH; ++k) {
       const int c = cbase + lane + 32 * k;
-      if (c < C) feat_grad[pix * C + c] = acc[k];
+      if (c < C) store_rn(feat_grad + pix * C + c, acc[k]);
     }
   }
   __syncwarp();
@@ -507,18 +496,18 @@ __device__ __forceinline__ void pixel_warp(float* wsm, int lane, const T* __rest
 // CL: the single-pass channels-last backward (rows = out_grad [B,Z,Y,X,C], no row pass).  (Its
 // KCH = 8 instance spills 24 bytes at the register count ptxas picks on its own; the minimum of
 // one CTA per SM lets it keep everything in registers.)
-template <int KCH, bool CL = false, typename T = float>
+template <int KCH, bool CL = false, typename T = float, typename TF = float>
 __global__ void __launch_bounds__(kBwdWarps * 32, CL ? 1 : 0)
 k_bwd_pixels(const T* __restrict__ rows, const float* __restrict__ depth,
-             const float* __restrict__ feat, const int32_t* __restrict__ point_interval,
+             const TF* __restrict__ feat, const int32_t* __restrict__ point_interval,
              const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ interval_starts,
              int64_t pix_begin, int64_t pix_end, int D, int HW, int C,
-             float* __restrict__ depth_grad, float* __restrict__ feat_grad) {
+             float* __restrict__ depth_grad, TF* __restrict__ feat_grad) {
   extern __shared__ float smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t pix = pix_begin + (int64_t)blockIdx.x * kBwdWarps + warp;
   if (pix >= pix_end) return;
-  pixel_warp<KCH, false, CL, T>(smem + (size_t)warp * 4 * D, lane, rows, depth, feat, point_interval,
+  pixel_warp<KCH, false, CL, T, TF>(smem + (size_t)warp * 4 * D, lane, rows, depth, feat, point_interval,
                              ranks_bev, interval_starts, pix, D, HW, C, depth_grad, feat_grad);
 }
 
@@ -569,11 +558,11 @@ static int launch_rows(const T* out_grad, const int32_t* tile_istart, const uint
   return 0;
 }
 
-template <int KCH, bool CL, typename T>
-static int launch_pixels(const T* rows, const float* depth, const float* feat,
+template <int KCH, bool CL, typename T, typename TF>
+static int launch_pixels(const T* rows, const float* depth, const TF* feat,
                          const int32_t* point_interval, const int32_t* ranks_bev,
                          const int32_t* interval_starts, int64_t pix_begin, int64_t pix_end,
-                         int D, int HW, int C, float* depth_grad, float* feat_grad,
+                         int D, int HW, int C, float* depth_grad, TF* feat_grad,
                          cudaStream_t stream) {
   const size_t smem = sizeof(float) * kBwdWarps * 4 * (size_t)D;
   if (smem > 200 * 1024) return VEON_E_UNSUPPORTED;
@@ -581,14 +570,14 @@ static int launch_pixels(const T* rows, const float* depth, const float* feat,
   const int dev = current_device();
   if (attr_smem[dev] == 0) attr_smem[dev] = 48 * 1024;
   if (smem > attr_smem[dev]) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_pixels<KCH, CL, T>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_bwd_pixels<KCH, CL, T, TF>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_smem[dev] = smem;
   }
   const int64_t blocks = ceil_div64(pix_end - pix_begin, kBwdWarps);
   if (blocks <= 0) return 0;
   if (blocks > 0x7fffffffLL) return VEON_E_RANGE;
-  k_bwd_pixels<KCH, CL, T><<<(unsigned)blocks, kBwdWarps * 32, smem, stream>>>(
+  k_bwd_pixels<KCH, CL, T, TF><<<(unsigned)blocks, kBwdWarps * 32, smem, stream>>>(
       rows, depth, feat, point_interval, ranks_bev, interval_starts, pix_begin, pix_end, D, HW, C,
       depth_grad, feat_grad);
   VEON_LAUNCH_CHECK();
@@ -605,12 +594,12 @@ static int row_pass(const T* out_grad, const int32_t* tile_istart, const uint32_
 }
 
 // ranks_bev / interval_starts: the channels-last pass (rows = out_grad), else NULL
-template <bool CL = false, typename T = float>
-static int pixel_pass(const T* rows, const float* depth, const float* feat,
+template <bool CL = false, typename T = float, typename TF = float>
+static int pixel_pass(const T* rows, const float* depth, const TF* feat,
                       const int32_t* point_interval, int64_t pixels, int D, int HW, int C,
-                      float* depth_grad, float* feat_grad, cudaStream_t stream,
+                      float* depth_grad, TF* feat_grad, cudaStream_t stream,
                       const int32_t* ranks_bev = nullptr, const int32_t* interval_starts = nullptr) {
-#define VEON_PIX(K_) launch_pixels<K_, CL, T>(rows, depth, feat, point_interval, ranks_bev, interval_starts, 0, pixels, D, HW, C, depth_grad, feat_grad, stream)
+#define VEON_PIX(K_) launch_pixels<K_, CL, T, TF>(rows, depth, feat, point_interval, ranks_bev, interval_starts, 0, pixels, D, HW, C, depth_grad, feat_grad, stream)
   switch (C <= 32 ? 1 : (C <= 64 ? 2 : (C <= 256 ? 4 : 8))) {   // channels per lane
     case 1: return VEON_PIX(1);
     case 2: return VEON_PIX(2);
@@ -634,13 +623,14 @@ extern "C" size_t veon_bev_pool_v2_bwd_workspace_floats(int64_t n_intervals, int
   return (size_t)(n_intervals > 0 ? n_intervals : 1) * (size_t)C;
 }
 
-// The two passes on a channels-first out_grad of float or bf16 elements T (the rows are float).
-template <typename T>
-static int bwd_planar(const T* out_grad, const float* depth, const float* feat,
+// The two passes on a channels-first out_grad of float or bf16 elements T (the rows are float),
+// for feature rows (and their gradient) of float or bf16 elements TF.
+template <typename T, typename TF = float>
+static int bwd_planar(const T* out_grad, const float* depth, const TF* feat,
                       const int32_t* tile_istart, const uint32_t* tile_occ,
                       const int32_t* point_interval, int64_t n_intervals, int B, int N, int D,
                       int H, int W, int C, int64_t V, float* rows_ws, int64_t rows_ws_floats,
-                      float* depth_grad, float* feat_grad, cudaStream_t stream) {
+                      float* depth_grad, TF* feat_grad, cudaStream_t stream) {
   if (!out_grad || !depth || !feat || !tile_istart || !tile_occ || !point_interval || !rows_ws ||
       !depth_grad || !feat_grad || B <= 0 || N <= 0 || D <= 0 || H <= 0 || W <= 0 || C <= 0 ||
       V <= 0 || n_intervals < 0)
@@ -681,11 +671,11 @@ extern "C" int veon_bev_pool_v2_bwd_planar_bf16(
 // Single pass for a channels-last out_grad [B,Z,Y,X,C]: its occupied rows are already contiguous,
 // so the pixel pass reads them in place -- no row pass, no scratch.  Same rows, same order of
 // operations: the same bits as veon_bev_pool_v2_bwd_planar on the channels-first copy.
-template <typename T>
-static int bwd_planar_cl(const T* out_grad, const float* depth, const float* feat,
+template <typename T, typename TF = float>
+static int bwd_planar_cl(const T* out_grad, const float* depth, const TF* feat,
                          const int32_t* ranks_bev, const int32_t* interval_starts,
                          const int32_t* point_interval, int B, int N, int D, int H, int W, int C,
-                         int64_t V, float* depth_grad, float* feat_grad, void* stream_) {
+                         int64_t V, float* depth_grad, TF* feat_grad, void* stream_) {
   if (!out_grad || !depth || !feat || !ranks_bev || !interval_starts || !point_interval ||
       !depth_grad || !feat_grad || B <= 0 || N <= 0 || D <= 0 || H <= 0 || W <= 0 || C <= 0 ||
       V <= 0)
@@ -714,12 +704,12 @@ extern "C" int veon_bev_pool_v2_bwd_planar_cl_bf16(
                        feat_grad, stream);
 }
 
-extern "C" int veon_bev_pool_v2_bwd_planar_ds(
-    const float* grad_ds, const uint8_t* mask, const float* depth, const float* feat,
+template <typename TF>
+static int bwd_planar_ds(
+    const float* grad_ds, const uint8_t* mask, const float* depth, const TF* feat,
     const int32_t* tile_istart, const uint32_t* tile_occ, const int32_t* point_interval,
     int64_t n_intervals, int B, int N, int D, int H, int W, int C, int Z, int Y, int X,
-    float* rows_ws, float* depth_grad, float* feat_grad, void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
+    float* rows_ws, float* depth_grad, TF* feat_grad, cudaStream_t stream) {
   if (!grad_ds || !mask || !depth || !feat || !tile_istart || !tile_occ || !point_interval ||
       !rows_ws || !depth_grad || !feat_grad || B <= 0 || N <= 0 || D <= 0 || H <= 0 || W <= 0 ||
       C <= 0 || Z <= 0 || Y <= 0 || X <= 0 || n_intervals < 0)
@@ -743,6 +733,70 @@ extern "C" int veon_bev_pool_v2_bwd_planar_ds(
   VEON_LAUNCH_CHECK();
   return pixel_pass(rows_ws, depth, feat, point_interval, (int64_t)B * N * H * W, D, H * W, C,
                     depth_grad, feat_grad, stream);
+}
+
+extern "C" int veon_bev_pool_v2_bwd_planar_ds(
+    const float* grad_ds, const uint8_t* mask, const float* depth, const float* feat,
+    const int32_t* tile_istart, const uint32_t* tile_occ, const int32_t* point_interval,
+    int64_t n_intervals, int B, int N, int D, int H, int W, int C, int Z, int Y, int X,
+    float* rows_ws, float* depth_grad, float* feat_grad, void* stream) {
+  return bwd_planar_ds(grad_ds, mask, depth, feat, tile_istart, tile_occ, point_interval,
+                       n_intervals, B, N, D, H, W, C, Z, Y, X, rows_ws, depth_grad, feat_grad,
+                       (cudaStream_t)stream);
+}
+
+// bfloat16 feature rows [B*N*H*W, C] and their gradient: the pixel pass reads each pixel's row as
+// bf16 (widened exactly) and stores feat_grad as bf16 (the float sums rounded once, to nearest
+// even); depth_grad and the row passes are those of the float twins, bit for bit.  Arguments,
+// checks and error codes are the twins'.
+extern "C" int veon_bev_pool_v2_bwd_planar_bf16feat(
+    const float* out_grad, const float* depth, const uint16_t* feat, const int32_t* tile_istart,
+    const uint32_t* tile_occ, const int32_t* point_interval, int64_t n_intervals, int B, int N,
+    int D, int H, int W, int C, int64_t V, float* rows_ws, int64_t rows_ws_floats,
+    float* depth_grad, uint16_t* feat_grad, void* stream) {
+  return bwd_planar(out_grad, depth, reinterpret_cast<const bf16*>(feat), tile_istart, tile_occ,
+                    point_interval, n_intervals, B, N, D, H, W, C, V, rows_ws, rows_ws_floats,
+                    depth_grad, reinterpret_cast<bf16*>(feat_grad), (cudaStream_t)stream);
+}
+
+extern "C" int veon_bev_pool_v2_bwd_planar_bf16_bf16feat(
+    const uint16_t* out_grad, const float* depth, const uint16_t* feat, const int32_t* tile_istart,
+    const uint32_t* tile_occ, const int32_t* point_interval, int64_t n_intervals, int B, int N,
+    int D, int H, int W, int C, int64_t V, float* rows_ws, int64_t rows_ws_floats,
+    float* depth_grad, uint16_t* feat_grad, void* stream) {
+  return bwd_planar(reinterpret_cast<const bf16*>(out_grad), depth,
+                    reinterpret_cast<const bf16*>(feat), tile_istart, tile_occ, point_interval,
+                    n_intervals, B, N, D, H, W, C, V, rows_ws, rows_ws_floats, depth_grad,
+                    reinterpret_cast<bf16*>(feat_grad), (cudaStream_t)stream);
+}
+
+extern "C" int veon_bev_pool_v2_bwd_planar_cl_bf16feat(
+    const float* out_grad, const float* depth, const uint16_t* feat, const int32_t* ranks_bev,
+    const int32_t* interval_starts, const int32_t* point_interval, int B, int N, int D, int H,
+    int W, int C, int64_t V, float* depth_grad, uint16_t* feat_grad, void* stream) {
+  return bwd_planar_cl(out_grad, depth, reinterpret_cast<const bf16*>(feat), ranks_bev,
+                       interval_starts, point_interval, B, N, D, H, W, C, V, depth_grad,
+                       reinterpret_cast<bf16*>(feat_grad), stream);
+}
+
+extern "C" int veon_bev_pool_v2_bwd_planar_cl_bf16_bf16feat(
+    const uint16_t* out_grad, const float* depth, const uint16_t* feat, const int32_t* ranks_bev,
+    const int32_t* interval_starts, const int32_t* point_interval, int B, int N, int D, int H,
+    int W, int C, int64_t V, float* depth_grad, uint16_t* feat_grad, void* stream) {
+  return bwd_planar_cl(reinterpret_cast<const bf16*>(out_grad), depth,
+                       reinterpret_cast<const bf16*>(feat), ranks_bev, interval_starts,
+                       point_interval, B, N, D, H, W, C, V, depth_grad,
+                       reinterpret_cast<bf16*>(feat_grad), stream);
+}
+
+extern "C" int veon_bev_pool_v2_bwd_planar_ds_bf16feat(
+    const float* grad_ds, const uint8_t* mask, const float* depth, const uint16_t* feat,
+    const int32_t* tile_istart, const uint32_t* tile_occ, const int32_t* point_interval,
+    int64_t n_intervals, int B, int N, int D, int H, int W, int C, int Z, int Y, int X,
+    float* rows_ws, float* depth_grad, uint16_t* feat_grad, void* stream) {
+  return bwd_planar_ds(grad_ds, mask, depth, reinterpret_cast<const bf16*>(feat), tile_istart,
+                       tile_occ, point_interval, n_intervals, B, N, D, H, W, C, Z, Y, X, rows_ws,
+                       depth_grad, reinterpret_cast<bf16*>(feat_grad), (cudaStream_t)stream);
 }
 
 #ifdef VEON_TOOLS   // tools/build_variant.sh NAME "-DVEON_TOOLS": never in the shipped library

@@ -93,6 +93,19 @@ __device__ __forceinline__ void zero_rows_cl(T* __restrict__ out, int64_t g0, in
   }
 }
 
+// A feature element as the lane-per-channel gather carries it: a float as it is, a bf16 as its raw
+// bits, widened only at the fma (a widened copy next to each of the rows in flight made the
+// kernel spill).
+__device__ __forceinline__ float ld_feat(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_feat(const bf16* p) {
+  return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)));
+}
+template <typename TF>
+__device__ __forceinline__ float feat_value(float v) {
+  if constexpr (std::is_same<TF, float>::value) return v;
+  else return __uint_as_float(__float_as_uint(v) << 16);
+}
+
 // Persistent: every warp strides over (tile, channel-chunk) items.
 //  * index prefetch: tile bounds -> rank triple -> depth value run 3 / 2 / 1 x kDist
 //    items ahead as 4-byte cp.async copies into a per-warp ring (no registers held;
@@ -122,9 +135,12 @@ __device__ __forceinline__ void zero_rows_cl(T* __restrict__ out, int64_t g0, in
 // Nothing is transposed.  (Storing the rows straight from the registers, with zeros for the
 // empty voxels between them, was measured at 578 us at C2: short scattered stores.)
 // T: the volume's element type, float or bf16 (rounded once, at the store; the tiles stay float).
-template <int KCH, bool FULLC, bool LOOPC = false, bool CL = false, typename T = float>
+// TF: the feature rows' element type, float or bf16: a lane loads its channel's 2 or 4 bytes and
+// widens them exactly; the point records' byte offsets scale by sizeof(TF).
+template <int KCH, bool FULLC, bool LOOPC = false, bool CL = false, typename T = float,
+          typename TF = float>
 __global__ void __launch_bounds__(kFwdWarps * 32)
-k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
+k_pool_fwd(const float* __restrict__ depth, const TF* __restrict__ feat,
            const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
            const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ tile_start,
            const int32_t* __restrict__ heavy, uint32_t n_items, uint32_t tiles_per_sample,
@@ -209,7 +225,8 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
       const int2 h = *reinterpret_cast<const int2*>(sl + 2);
       const int32_t up = lane ? pt[-4] : -1;
       // byte offset of this channel chunk of the point's feature row (< 2^32, checked)
-      pt[1] = (int32_t)(((uint32_t)pt[1] * (uint32_t)C + (uint32_t)(h.y & 0xffff) * CC) * 4u);
+      pt[1] = (int32_t)(((uint32_t)pt[1] * (uint32_t)C + (uint32_t)(h.y & 0xffff) * CC) *
+                        (uint32_t)sizeof(TF));
       pt[2] = (rb - h.x) | ((rb != up) ? 0x100 : 0);  // voxel | first-of-voxel
     }
   };
@@ -227,7 +244,7 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
 
   const int q4 = (lane & 7) * 4, r = lane >> 3;  // write-out role of this lane
   float* const tlane = tile + lane * kRowPitch;   // flush base: channel = lane (+32k)
-  const char* const feat_lane = reinterpret_cast<const char*>(feat) + lane * 4;
+  const char* const feat_lane = reinterpret_cast<const char*>(feat) + lane * (int)sizeof(TF);
   const int64_t ostep = 4 * V;
 
   for (uint32_t m = 0; m < my_items; ++m) {
@@ -279,7 +296,7 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
       if (lane == 0) up = last_rb;   // first point of the block: new voxel iff it differs
       int32_t* pt = dst + 4 * lane;
       pt[0] = rb;
-      pt[1] = (int32_t)(((uint32_t)rf * (uint32_t)C + (uint32_t)cb) * 4u);
+      pt[1] = (int32_t)(((uint32_t)rf * (uint32_t)C + (uint32_t)cb) * (uint32_t)sizeof(TF));
       pt[2] = (rb - g0) | ((rb != up) ? 0x100 : 0);
       pt[3] = __float_as_int(d);
       return __shfl_sync(0xffffffffu, rb, 31);
@@ -297,7 +314,7 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
       const int cmax = FULLC ? CC : min(CC, C - cbase);
       // (b*C + cbase + r)*V + v0 + q4  with  v0 = g0 - b*V
       T* o = out + (int64_t)(b * (uint32_t)(C - 1) + (uint32_t)(cbase + r)) * V + g0 + q4;
-      const char* const feat_ch = feat_lane + (LOOPC ? (uint32_t)cbase * 4u : 0u);
+      const char* const feat_ch = feat_lane + (LOOPC ? (uint32_t)cbase * (uint32_t)sizeof(TF) : 0u);
 
       __syncwarp();
       {  // zero the tile (empty voxels must read as 0)
@@ -344,13 +361,13 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
               for (int uu = 0; uu < 4; ++uu) {
                 const int u = 4 * g + uu;
                 p[u] = pts[min(j0 + u, cnt - 1)];
-                const float* row = reinterpret_cast<const float*>(feat_ch + (uint32_t)p[u].y);
+                const TF* row = reinterpret_cast<const TF*>(feat_ch + (uint32_t)p[u].y);
 #pragma unroll
                 for (int k = 0; k < KCH; ++k)
 #ifdef VEON_FWD_X_NOGATHER   // tools only: elimination timing
                   f[u][k] = (float)p[u].y;
 #else
-                  f[u][k] = (FULLC || full_chunk || lane + 32 * k < cmax) ? __ldg(row + 32 * k) : 0.f;
+                  f[u][k] = (FULLC || full_chunk || lane + 32 * k < cmax) ? ld_feat(row + 32 * k) : 0.f;
 #endif
               }
             }
@@ -367,10 +384,10 @@ k_pool_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
                     if (acc_vl >= 0) flush();
                     acc_vl = p[u].z & 0xff;
 #pragma unroll
-                    for (int k = 0; k < KCH; ++k) acc[k] = fmaf(f[u][k], dj, 0.f);
+                    for (int k = 0; k < KCH; ++k) acc[k] = fmaf(feat_value<TF>(f[u][k]), dj, 0.f);
                   } else {
 #pragma unroll
-                    for (int k = 0; k < KCH; ++k) acc[k] = fmaf(f[u][k], dj, acc[k]);
+                    for (int k = 0; k < KCH; ++k) acc[k] = fmaf(feat_value<TF>(f[u][k]), dj, acc[k]);
                   }
                 }
               }
@@ -459,9 +476,11 @@ __device__ __forceinline__ void store_label(const ClsArgs& ca, uint32_t b, uint3
 }
 
 // CL: channels-last write-out (warp = voxel, lanes = channels), see k_pool_fwd
-template <int KCH, bool CLS = false, bool CL = false, typename T = float>
+// TF = bf16: rows are staged as they are (8-byte copies of 4-channel pieces, half the shared
+// memory) and widened in the fma chains.
+template <int KCH, bool CLS = false, bool CL = false, typename T = float, typename TF = float>
 __global__ void __launch_bounds__(kHeavyThreads)
-k_pool_fwd_heavy(const float* __restrict__ depth, const float* __restrict__ feat,
+k_pool_fwd_heavy(const float* __restrict__ depth, const TF* __restrict__ feat,
                  const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
                  const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ tile_start,
                  const int32_t* __restrict__ heavy, int heavy_cap, uint32_t tiles_per_sample,
@@ -470,8 +489,8 @@ k_pool_fwd_heavy(const float* __restrict__ depth, const float* __restrict__ feat
   constexpr int CC = 32 * KCH;
   constexpr int kSegs = CC / 4;  // 16-byte segments per staged row
   extern __shared__ __align__(16) float hsm[];
-  float* rows = hsm;                                            // [kHeavyChunk][CC]
-  float* tile = rows + kHeavyChunk * CC;                        // [CC][kRowPitch]
+  TF* rows = reinterpret_cast<TF*>(hsm);                        // [kHeavyChunk][CC]
+  float* tile = reinterpret_cast<float*>(rows + kHeavyChunk * CC);  // [CC][kRowPitch]
   float* dep = tile + CC * kRowPitch;                           // [kHeavyChunk]
   uint32_t* off = reinterpret_cast<uint32_t*>(dep + kHeavyChunk);  // [kHeavyChunk]
   int32_t* bounds = reinterpret_cast<int32_t*>(off + kHeavyChunk); // [2][start 32 | end 32]
@@ -552,7 +571,7 @@ k_pool_fwd_heavy(const float* __restrict__ depth, const float* __restrict__ feat
         const int idx = tid + kHeavyThreads * i;
         const int r = idx / kSegs, seg = (idx % kSegs) * 4;
 #ifndef VEON_FWD_X_HEAVY_NOCOPY   // tools only: elimination timing
-        if (r < cnt && seg < cmax) cp_async16(rows + r * CC + seg, feat + off[r] + cbase + seg);
+        if (r < cnt && seg < cmax) cp_async_4(rows + r * CC + seg, feat + off[r] + cbase + seg);
 #endif
       }
       cp_async_commit();
@@ -572,7 +591,7 @@ k_pool_fwd_heavy(const float* __restrict__ depth, const float* __restrict__ feat
         for (int j = a; j < e; ++j) {
           const float dj = dep[j];
 #pragma unroll
-          for (int c = 0; c < KCH; ++c) acc[c] = fmaf(rows[j * CC + lane + 32 * c], dj, acc[c]);
+          for (int c = 0; c < KCH; ++c) acc[c] = fmaf(widen(rows[j * CC + lane + 32 * c]), dj, acc[c]);
         }
 #endif
 #pragma unroll
@@ -822,9 +841,11 @@ constexpr int kNarrowHeavyMin = 512;
 // rows in order), so Q + 2 <= 96 channels need no more registers than 32 do.
 // CL: channels-last output; a lane's voxel row is NV 16-byte stores and the warp's 32 rows are one
 // contiguous 32 * C * 4-byte block.
-template <int NV, bool CLS = false, int NP = 1, bool CL = false, typename T = float>  // 16-byte pieces per pass: C = 4 * NV * NP
+// TF = bf16: a 4-channel piece is one 8-byte load, widened in registers.
+template <int NV, bool CLS = false, int NP = 1, bool CL = false, typename T = float,
+          typename TF = float>  // 4-channel pieces per pass: C = 4 * NV * NP
 __global__ void __launch_bounds__(kNarrowWarps * 32, (NV <= 5) ? 3 : 2)
-k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ feat,
+k_pool_fwd_narrow(const float* __restrict__ depth, const TF* __restrict__ feat,
                   const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
                   const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ tile_start,
                   const int32_t* __restrict__ heavy, uint32_t n_tiles, uint32_t tiles_per_sample,
@@ -924,7 +945,7 @@ k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ fea
 #pragma unroll
       for (int c = 0; c < CP; ++c) acc[c] = 0.f;
       if (st >= 0) {
-        const float* fbase = feat + pass * CP;
+        const TF* fbase = feat + pass * CP;
         int32_t i = st;
         bool two = i + 1 < en;
         int32_t r0 = __ldg(ranks_depth + i), f0 = __ldg(ranks_feat + i);
@@ -935,13 +956,13 @@ k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ fea
           // point's loads into); a missing second point is (+0) * (-0): acc + (-0) == acc bit for
           // bit, whatever acc is.
           const float d0 = __ldg(depth + r0), d1 = two ? __ldg(depth + r1) : -0.f;
-          const float4* row0 = reinterpret_cast<const float4*>(fbase + (int64_t)f0 * C);
-          const float4* row1 = reinterpret_cast<const float4*>(fbase + (int64_t)f1 * C);
+          const TF* row0 = fbase + (int64_t)f0 * C;
+          const TF* row1 = fbase + (int64_t)f1 * C;
           float4 a[NV], q[NV];
 #pragma unroll
-          for (int k = 0; k < NV; ++k) a[k] = __ldg(row0 + k);
+          for (int k = 0; k < NV; ++k) a[k] = ldg_widen4(row0 + 4 * k);
 #pragma unroll
-          for (int k = 0; k < NV; ++k) q[k] = two ? __ldg(row1 + k) : make_float4(0.f, 0.f, 0.f, 0.f);
+          for (int k = 0; k < NV; ++k) q[k] = two ? ldg_widen4(row1 + 4 * k) : make_float4(0.f, 0.f, 0.f, 0.f);
           // `zero` is a kernel argument that is always 0: making the first depth value depend
           // on every piece of the second row keeps the assembler from re-using the first row's
           // registers for the second row's loads (it otherwise issues them only after the first
@@ -1019,17 +1040,17 @@ k_pool_fwd_narrow(const float* __restrict__ depth, const float* __restrict__ fea
 
 
 // ---- launchers ---------------------------------------------------------------------------------
-template <int KCH, bool CLS = false, bool CL = false, typename T = float>
+template <int KCH, bool CLS = false, bool CL = false, typename T = float, typename TF = float>
 static int heavy_config(size_t& smem, int& ctas_per_sm) {
   constexpr int CC = 32 * KCH;
-  smem = sizeof(float) * (kHeavyChunk * CC + CC * kRowPitch + 2 * kHeavyChunk + 128);
+  smem = sizeof(TF) * kHeavyChunk * CC + sizeof(float) * (CC * kRowPitch + 2 * kHeavyChunk + 128);
   static int cached[kMaxDevices] = {};
   const int dev = current_device();
   if (cached[dev] == 0) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd_heavy<KCH, CLS, CL, T>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd_heavy<KCH, CLS, CL, T, TF>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_heavy<KCH, CLS, CL, T>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_heavy<KCH, CLS, CL, T, TF>,
                                                                 kHeavyThreads, smem));
     cached[dev] = n < 1 ? 1 : (n > 8 ? 8 : n);
   }
@@ -1038,15 +1059,15 @@ static int heavy_config(size_t& smem, int& ctas_per_sm) {
 }
 
 // the heavy-tile grid; pdl: queued as a programmatic dependent of the previous launch (joins it)
-template <int KCH, bool CLS = false, bool CL = false, typename T = float>
-static int launch_heavy(const float* depth, const float* feat, const int32_t* rd, const int32_t* rf,
+template <int KCH, bool CLS = false, bool CL = false, typename T = float, typename TF = float>
+static int launch_heavy(const float* depth, const TF* feat, const int32_t* rd, const int32_t* rf,
                         const int32_t* rb, const int32_t* tile_start, const int32_t* heavy,
                         int64_t heavy_ints, int B, int C, int64_t V, T* out, bool pdl,
                         int min_points, cudaStream_t stream, ClsArgs ca = ClsArgs()) {
   constexpr int CC = 32 * KCH;
   size_t smem;
   int per_sm;
-  int rc = heavy_config<KCH, CLS, CL, T>(smem, per_sm);
+  int rc = heavy_config<KCH, CLS, CL, T, TF>(smem, per_sm);
   if (rc) return rc;
   const int64_t tps = ceil_div64(V, kTileVoxels);
   const int n_chunks = (C + CC - 1) / CC;
@@ -1056,11 +1077,11 @@ static int launch_heavy(const float* depth, const float* feat, const int32_t* rd
   if (blocks > (int64_t)per_sm * sm_count()) blocks = (int64_t)per_sm * sm_count();
   if (blocks <= 0) return 0;
   if (pdl) {
-    VEON_CUDA_TRY(launch_pdl(k_pool_fwd_heavy<KCH, CLS, CL, T>, dim3((unsigned)blocks), dim3(kHeavyThreads),
+    VEON_CUDA_TRY(launch_pdl(k_pool_fwd_heavy<KCH, CLS, CL, T, TF>, dim3((unsigned)blocks), dim3(kHeavyThreads),
                              smem, stream, depth, feat, rd, rf, rb, tile_start, heavy, heavy_cap,
                              (uint32_t)tps, V, C, (uint32_t)n_chunks, vec_ok, out, 1, min_points, ca));
   } else {
-    k_pool_fwd_heavy<KCH, CLS, CL, T><<<(unsigned)blocks, kHeavyThreads, smem, stream>>>(
+    k_pool_fwd_heavy<KCH, CLS, CL, T, TF><<<(unsigned)blocks, kHeavyThreads, smem, stream>>>(
         depth, feat, rd, rf, rb, tile_start, heavy, heavy_cap, (uint32_t)tps, V, C,
         (uint32_t)n_chunks, vec_ok, out, 0, min_points, ca);
   }
@@ -1081,8 +1102,8 @@ int launch_heavy_behind(const float* depth, const float* feat, const int32_t* rd
 }
 
 // general route: k_pool_fwd over every (tile, channel chunk), the heavy tiles queued behind it
-template <int KCH, bool FULLC, bool LOOPC, bool CL, typename T>
-static int launch_fwd_impl(const float* depth, const float* feat, const int32_t* rd,
+template <int KCH, bool FULLC, bool LOOPC, bool CL, typename T, typename TF>
+static int launch_fwd_impl(const float* depth, const TF* feat, const int32_t* rd,
                            const int32_t* rf, const int32_t* rb, const int32_t* tile_start,
                            const int32_t* heavy, int64_t heavy_ints, int B, int C, int64_t V,
                            bool feat_rows_fit_32bit, T* out, cudaStream_t stream) {
@@ -1093,10 +1114,10 @@ static int launch_fwd_impl(const float* depth, const float* feat, const int32_t*
   static int ctas_per_sm[kMaxDevices] = {};
   const int dev = current_device();
   if (ctas_per_sm[dev] == 0) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd<KCH, FULLC, LOOPC, CL, T>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_fwd<KCH, FULLC, LOOPC, CL, T, TF>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd<KCH, FULLC, LOOPC, CL, T>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd<KCH, FULLC, LOOPC, CL, T, TF>,
                                                                 kFwdWarps * 32, smem));
     ctas_per_sm[dev] = n < 1 ? 1 : n;
   }
@@ -1111,9 +1132,9 @@ static int launch_fwd_impl(const float* depth, const float* feat, const int32_t*
   int64_t blocks = ceil_div64(n_items, kFwdWarps);
   const int64_t resident = (int64_t)ctas_per_sm[dev] * sm_count();  // persistent grid
   if (blocks > resident) blocks = resident;
-  // the heavy-tile kernel stages feature rows with 16-byte copies
-  if (heavy && ((C & 3) != 0 || ((uintptr_t)feat & 15) != 0)) heavy = nullptr;
-  k_pool_fwd<KCH, FULLC, LOOPC, CL, T><<<(unsigned)blocks, kFwdWarps * 32, smem, stream>>>(
+  // the heavy-tile kernel stages feature rows with 4-element (16- or 8-byte) copies
+  if (heavy && ((C & 3) != 0 || ((uintptr_t)feat & (4 * sizeof(TF) - 1)) != 0)) heavy = nullptr;
+  k_pool_fwd<KCH, FULLC, LOOPC, CL, T, TF><<<(unsigned)blocks, kFwdWarps * 32, smem, stream>>>(
       depth, feat, rd, rf, rb, tile_start, heavy, (uint32_t)n_items, (uint32_t)tps,
       V, C, (uint32_t)(LOOPC ? 1 : n_chunks), vec_ok, out, (uint32_t)n_chunks);
   VEON_LAUNCH_CHECK();
@@ -1122,25 +1143,26 @@ static int launch_fwd_impl(const float* depth, const float* feat, const int32_t*
   // grid before they complete.
 #ifndef VEON_FWD_X_NOHEAVY
   if (heavy)
-    return launch_heavy<(KCH > 2 ? 2 : KCH), false, CL, T>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints,
+    return launch_heavy<(KCH > 2 ? 2 : KCH), false, CL, T, TF>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints,
                                              B, C, V, out, true, 0, stream);
 #endif
   return 0;
 }
 
-template <int KCH, bool CL, typename T>
-static int launch_fwd(const float* depth, const float* feat, const int32_t* rd,
+template <int KCH, bool CL, typename T, typename TF>
+static int launch_fwd(const float* depth, const TF* feat, const int32_t* rd,
                       const int32_t* rf, const int32_t* rb, const int32_t* tile_start,
                       const int32_t* heavy, int64_t heavy_ints, int B, int C, int64_t V,
                       bool feat_rows_fit_32bit, T* out, cudaStream_t stream) {
   // rows of several chunks: one item per tile (needs the heavy list: it bounds a tile's points)
 #ifndef VEON_FWD_X_NOLOOPC
-  const bool loopc = heavy && C > 32 * KCH && (C & 3) == 0 && ((uintptr_t)feat & 15) == 0;
+  const bool loopc =
+      heavy && C > 32 * KCH && (C & 3) == 0 && ((uintptr_t)feat & (4 * sizeof(TF) - 1)) == 0;
 #else
   const bool loopc = false;
 #endif
 #define VEON_FWD_GO(FULLC_, LOOPC_)                                                            \
-  return launch_fwd_impl<KCH, FULLC_, LOOPC_, CL, T>(depth, feat, rd, rf, rb, tile_start, heavy,      \
+  return launch_fwd_impl<KCH, FULLC_, LOOPC_, CL, T, TF>(depth, feat, rd, rf, rb, tile_start, heavy,      \
                                               heavy_ints, B, C, V, feat_rows_fit_32bit, out, stream)
   if (C % (32 * KCH) == 0) {
     if (loopc) VEON_FWD_GO(true, true);
@@ -1155,8 +1177,9 @@ static int launch_fwd(const float* depth, const float* feat, const int32_t* rd,
 // CTA works ~100 us on one 1 000-point tile at C3 density: behind the persistent main grid the
 // two nearly serialise, 344 vs 295 us); k_pool_fwd_narrow moves in beside it as its programmatic
 // dependent and joins it at the end
-template <int NV, bool CLS = false, int NP = 1, bool CL = false, typename T = float>
-static int launch_fwd_narrow(const float* depth, const float* feat, const int32_t* rd,
+template <int NV, bool CLS = false, int NP = 1, bool CL = false, typename T = float,
+          typename TF = float>
+static int launch_fwd_narrow(const float* depth, const TF* feat, const int32_t* rd,
                              const int32_t* rf, const int32_t* rb, const int32_t* tile_start,
                              const int32_t* heavy, int64_t heavy_ints, int B, int64_t V,
                              T* out, cudaStream_t stream, ClsArgs ca = ClsArgs()) {
@@ -1167,16 +1190,16 @@ static int launch_fwd_narrow(const float* depth, const float* feat, const int32_
   const int dev = current_device();
   if (ctas_per_sm[dev] == 0) {
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_narrow<NV, CLS, NP, CL, T>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_pool_fwd_narrow<NV, CLS, NP, CL, T, TF>,
                                                                 kNarrowWarps * 32, 0));
     ctas_per_sm[dev] = n < 1 ? 1 : n;
   }
   int64_t blocks = ceil_div64(n_tiles, kNarrowWarps);
   if (blocks > (int64_t)ctas_per_sm[dev] * sm_count()) blocks = (int64_t)ctas_per_sm[dev] * sm_count();
-  int rc = launch_heavy<KCH, CLS, CL, T>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C, V,
+  int rc = launch_heavy<KCH, CLS, CL, T, TF>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C, V,
                                   out, false, kNarrowHeavyMin, stream, ca);
   if (rc) return rc;
-  VEON_CUDA_TRY(launch_pdl(k_pool_fwd_narrow<NV, CLS, NP, CL, T>, dim3((unsigned)blocks),
+  VEON_CUDA_TRY(launch_pdl(k_pool_fwd_narrow<NV, CLS, NP, CL, T, TF>, dim3((unsigned)blocks),
                            dim3(kNarrowWarps * 32), 0, stream, depth, feat, rd, rf, rb, tile_start,
                            heavy, (uint32_t)n_tiles, (uint32_t)tps, V, out, 0u, kNarrowHeavyMin, 1,
                            ca));
@@ -1199,12 +1222,13 @@ extern "C" size_t veon_bev_pool_v2_fwd_workspace_bytes(int B, int C, int64_t V) 
   return fwd_stream_workspace_bytes(C);
 }
 
-// All four planar entry points: out is [B,C,Z,Y,X], or [B,Z,Y,X,C] with CL (the same kernels with a
-// row write-out: same sums, same bits, another layout), of float or bf16 elements T.  Routes in
-// order: narrow rows, the streaming kernel (channels-first float only; needs tile_occ and a
-// workspace), the general kernel.
-template <bool CL, typename T>
-static int fwd_planar(const float* depth, const float* feat, const int32_t* ranks_depth,
+// All planar entry points: out is [B,C,Z,Y,X], or [B,Z,Y,X,C] with CL (the same kernels with a
+// row write-out: same sums, same bits, another layout), of float or bf16 elements T, from feature
+// rows of float or bf16 elements TF.  Routes in order: narrow rows, the streaming kernel
+// (channels-first float volumes from float rows only; needs tile_occ and a workspace), the general
+// kernel.
+template <bool CL, typename T, typename TF = float>
+static int fwd_planar(const float* depth, const TF* feat, const int32_t* ranks_depth,
                       const int32_t* ranks_feat, const int32_t* ranks_bev,
                       const int32_t* tile_start, const uint32_t* tile_occ,
                       const int32_t* tile_heavy, int64_t tile_heavy_ints, int B, int C, int64_t V,
@@ -1221,9 +1245,10 @@ static int fwd_planar(const float* depth, const float* feat, const int32_t* rank
      // arbitrarily long voxels; rank arithmetic is exact only while B*V <= 2^24
     const bool ok = C <= 32 && (C & 3) == 0 && tile_heavy && fit32 && V % kTileVoxels == 0 &&
                     (int64_t)B * V <= (1 << 24) &&
-                    ((uintptr_t)feat & 15) == 0 && ((uintptr_t)out & (4 * sizeof(T) - 1)) == 0;
+                    ((uintptr_t)feat & (4 * sizeof(TF) - 1)) == 0 &&
+                    ((uintptr_t)out & (4 * sizeof(T) - 1)) == 0;
     if (ok) {
-#define VEON_NARROW_CASE(NV_) case NV_: return launch_fwd_narrow<NV_, false, 1, CL, T>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy, tile_heavy_ints, B, V, out, stream);
+#define VEON_NARROW_CASE(NV_) case NV_: return launch_fwd_narrow<NV_, false, 1, CL, T, TF>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, tile_heavy, tile_heavy_ints, B, V, out, stream);
       switch (C / 4) {
         VEON_NARROW_CASE(1) VEON_NARROW_CASE(2) VEON_NARROW_CASE(3) VEON_NARROW_CASE(4)
         VEON_NARROW_CASE(5) VEON_NARROW_CASE(6) VEON_NARROW_CASE(7) VEON_NARROW_CASE(8)
@@ -1232,8 +1257,15 @@ static int fwd_planar(const float* depth, const float* feat, const int32_t* rank
 #undef VEON_NARROW_CASE
     }
   }
-  // aligned volumes, whole 64-channel chunks: the two-role streaming kernel
-  if constexpr (!CL && std::is_same<T, float>::value) {
+  // aligned volumes, whole 64-channel chunks: the two-role streaming kernel.  It has no bf16-row
+  // form: where it would run on float rows, bf16 rows are refused (VEON_E_UNSUPPORTED), and the
+  // caller widens them into a fresh -- aligned -- float copy and calls the float entry.
+  if constexpr (!CL && std::is_same<T, float>::value && !std::is_same<TF, float>::value) {
+    if (workspace && tile_occ && tile_heavy &&
+        fwd_stream_supported(B, C, V, out, out, n_feat_rows))
+      return VEON_E_UNSUPPORTED;
+  }
+  if constexpr (!CL && std::is_same<T, float>::value && std::is_same<TF, float>::value) {
     if (workspace && tile_occ && tile_heavy &&
         fwd_stream_supported(B, C, V, feat, out, n_feat_rows)) {
       const int rc = launch_fwd_stream(depth, feat, ranks_depth, ranks_feat, ranks_bev,
@@ -1243,9 +1275,9 @@ static int fwd_planar(const float* depth, const float* feat, const int32_t* rank
     }
   }
   if (C <= 32)
-    return launch_fwd<1, CL, T>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
+    return launch_fwd<1, CL, T, TF>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
                              tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
-  return launch_fwd<2, CL, T>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
+  return launch_fwd<2, CL, T, TF>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start,
                            tile_heavy, tile_heavy_ints, B, C, V, fit32, out, stream);
 }
 
@@ -1310,6 +1342,54 @@ extern "C" int veon_bev_pool_v2_fwd_planar_cl_bf16(const float* depth, const flo
   return fwd_planar<true>(depth, feat, ranks_depth, ranks_feat, ranks_bev, tile_start, nullptr,
                           tile_heavy, tile_heavy_ints, B, C, V, n_feat_rows,
                           reinterpret_cast<bf16*>(out), nullptr, 0, (cudaStream_t)stream);
+}
+
+// bfloat16 feature rows [n_feat_rows, C]: the same kernels reading 2-byte channels, widened exactly,
+// so every volume is the bits of the float twin on the widened rows.  Arguments, checks and error
+// codes are the twins'; the channels-first float-volume entry returns VEON_E_UNSUPPORTED where its
+// twin would take the streaming kernel (see fwd_planar).
+extern "C" int veon_bev_pool_v2_fwd_planar_bf16feat(
+    const float* depth, const uint16_t* feat, const int32_t* ranks_depth,
+    const int32_t* ranks_feat, const int32_t* ranks_bev, const int32_t* tile_start,
+    const int32_t* tile_istart, const uint32_t* tile_occ, const int32_t* tile_heavy,
+    int64_t tile_heavy_ints, int B, int C, int64_t V, int64_t n_feat_rows, float* out,
+    void* workspace, size_t workspace_bytes, void* stream) {
+  return fwd_planar<false>(depth, reinterpret_cast<const bf16*>(feat), ranks_depth, ranks_feat,
+                           ranks_bev, tile_start, tile_occ, tile_heavy, tile_heavy_ints, B, C, V,
+                           n_feat_rows, out, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int veon_bev_pool_v2_fwd_planar_bf16_bf16feat(
+    const float* depth, const uint16_t* feat, const int32_t* ranks_depth,
+    const int32_t* ranks_feat, const int32_t* ranks_bev, const int32_t* tile_start,
+    const int32_t* tile_istart, const uint32_t* tile_occ, const int32_t* tile_heavy,
+    int64_t tile_heavy_ints, int B, int C, int64_t V, int64_t n_feat_rows, uint16_t* out,
+    void* workspace, size_t workspace_bytes, void* stream) {
+  return fwd_planar<false>(depth, reinterpret_cast<const bf16*>(feat), ranks_depth, ranks_feat,
+                           ranks_bev, tile_start, tile_occ, tile_heavy, tile_heavy_ints, B, C, V,
+                           n_feat_rows, reinterpret_cast<bf16*>(out), workspace, workspace_bytes,
+                           (cudaStream_t)stream);
+}
+
+extern "C" int veon_bev_pool_v2_fwd_planar_cl_bf16feat(
+    const float* depth, const uint16_t* feat, const int32_t* ranks_depth,
+    const int32_t* ranks_feat, const int32_t* ranks_bev, const int32_t* tile_start,
+    const int32_t* tile_heavy, int64_t tile_heavy_ints, int B, int C, int64_t V,
+    int64_t n_feat_rows, float* out, void* stream) {
+  return fwd_planar<true>(depth, reinterpret_cast<const bf16*>(feat), ranks_depth, ranks_feat,
+                          ranks_bev, tile_start, nullptr, tile_heavy, tile_heavy_ints, B, C, V,
+                          n_feat_rows, out, nullptr, 0, (cudaStream_t)stream);
+}
+
+extern "C" int veon_bev_pool_v2_fwd_planar_cl_bf16_bf16feat(
+    const float* depth, const uint16_t* feat, const int32_t* ranks_depth,
+    const int32_t* ranks_feat, const int32_t* ranks_bev, const int32_t* tile_start,
+    const int32_t* tile_heavy, int64_t tile_heavy_ints, int B, int C, int64_t V,
+    int64_t n_feat_rows, uint16_t* out, void* stream) {
+  return fwd_planar<true>(depth, reinterpret_cast<const bf16*>(feat), ranks_depth, ranks_feat,
+                          ranks_bev, tile_start, nullptr, tile_heavy, tile_heavy_ints, B, C, V,
+                          n_feat_rows, reinterpret_cast<bf16*>(out), nullptr, 0,
+                          (cudaStream_t)stream);
 }
 
 // Fused lift + classify: pools the [gate 0, gate 1, logit 0..Q-1, pad] rows and ends every tile
