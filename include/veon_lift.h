@@ -367,6 +367,24 @@ int veon_maxdown2_cl_fwd(const float* in, int B, int C, int Z, int Y, int X, flo
                          void* stream);
 int veon_maxdown2_cl_bwd(const float* in, const float* out, const float* grad_out,
                          int B, int C, int Z, int Y, int X, float* grad_in, void* stream);
+/* The same operations on bfloat16 volumes (uint16_t bit patterns), with the arguments, checks and
+ * error codes of the float32 twins, except that the channels-first entries need in / grad_in
+ * 8-byte and out / grad_out 4-byte aligned (else VEON_E_UNSUPPORTED).  Values are widened exactly
+ * where they are loaded and compared as the twins compare them, so out and grad_in are, bit for
+ * bit, `rearrange + torch.max(dim=-1)` on the bfloat16 tensor and its gradient (NaN payloads
+ * aside).  veon_maxdown2_fwd_mask_bf16 reads a float32 volume (16-byte aligned, as its twin) and
+ * stores the float32 maximum rounded once to nearest even as bfloat16 out (4-byte aligned); the
+ * mask is its twin's, taken over the float32 values. */
+int veon_maxdown2_fwd_bf16(const uint16_t* in, int64_t BC, int Z, int Y, int X, uint16_t* out,
+                           void* stream);
+int veon_maxdown2_fwd_mask_bf16(const float* in, int64_t BC, int Z, int Y, int X, uint16_t* out,
+                                uint8_t* mask, void* stream);
+int veon_maxdown2_bwd_bf16(const uint16_t* in, const uint16_t* out, const uint16_t* grad_out,
+                           int64_t BC, int Z, int Y, int X, uint16_t* grad_in, void* stream);
+int veon_maxdown2_cl_fwd_bf16(const uint16_t* in, int B, int C, int Z, int Y, int X,
+                              uint16_t* out, void* stream);
+int veon_maxdown2_cl_bwd_bf16(const uint16_t* in, const uint16_t* out, const uint16_t* grad_out,
+                              int B, int C, int Z, int Y, int X, uint16_t* grad_in, void* stream);
 
 /* QuickCumsumCuda.backward (bev_pool.py:43-83) for a [B,C,Z,Y,X] out_grad.
  *   rows_ws      float scratch of at least veon_bev_pool_v2_bwd_workspace_floats() elements
@@ -531,6 +549,26 @@ int veon_bev_pool_v2_bwd_planar_ds_bf16feat(const float* grad_ds, const uint8_t*
                                             int B, int N, int D, int H, int W, int C, int Z, int Y,
                                             int X, float* rows_ws, float* depth_grad,
                                             uint16_t* feat_grad, void* stream);
+/* veon_bev_pool_v2_bwd_planar_ds (and its _bf16feat form) for a bfloat16 grad_ds, the reduced
+ * volume of veon_maxdown2_fwd_mask_bf16: every value is widened exactly where the row pass loads
+ * it, everything after is the float32 twin's, so depth_grad / feat_grad are the twin's bits given
+ * the widened gradient.  Same arguments, checks and error codes as the twins. */
+int veon_bev_pool_v2_bwd_planar_ds_bf16(const uint16_t* grad_ds, const uint8_t* mask,
+                                        const float* depth, const float* feat,
+                                        const int32_t* tile_istart, const uint32_t* tile_occ,
+                                        const int32_t* point_interval, int64_t n_intervals,
+                                        int B, int N, int D, int H, int W, int C, int Z, int Y,
+                                        int X, float* rows_ws, float* depth_grad,
+                                        float* feat_grad, void* stream);
+int veon_bev_pool_v2_bwd_planar_ds_bf16_bf16feat(const uint16_t* grad_ds, const uint8_t* mask,
+                                                 const float* depth, const uint16_t* feat,
+                                                 const int32_t* tile_istart,
+                                                 const uint32_t* tile_occ,
+                                                 const int32_t* point_interval,
+                                                 int64_t n_intervals, int B, int N, int D, int H,
+                                                 int W, int C, int Z, int Y, int X,
+                                                 float* rows_ws, float* depth_grad,
+                                                 uint16_t* feat_grad, void* stream);
 /* veon_transpose_batched for 2-byte elements (bfloat16 maps and feature gradients): the same
  * tiles and checks, the bits moved unchanged. */
 int veon_transpose_batched_u16(const uint16_t* src, int64_t batch, int R, int S, uint16_t* dst,

@@ -111,6 +111,18 @@ _SIGNATURES = {
                                                         c_int, c_int, c_int, c_int, c_int, c_int,
                                                         c_int, c_int, c_int, _P, _P, _P, _P]),
     "veon_transpose_batched_u16": (c_int, [_P, c_int64, c_int, c_int, _P, _P]),
+    "veon_maxdown2_fwd_bf16": (c_int, [_P, c_int64, c_int, c_int, c_int, _P, _P]),
+    "veon_maxdown2_fwd_mask_bf16": (c_int, [_P, c_int64, c_int, c_int, c_int, _P, _P, _P]),
+    "veon_maxdown2_bwd_bf16": (c_int, [_P, _P, _P, c_int64, c_int, c_int, c_int, _P, _P]),
+    "veon_maxdown2_cl_fwd_bf16": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
+    "veon_maxdown2_cl_bwd_bf16": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
+    "veon_bev_pool_v2_bwd_planar_ds_bf16": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64,
+                                                    c_int, c_int, c_int, c_int, c_int, c_int,
+                                                    c_int, c_int, c_int, _P, _P, _P, _P]),
+    "veon_bev_pool_v2_bwd_planar_ds_bf16_bf16feat": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64,
+                                                             c_int, c_int, c_int, c_int, c_int,
+                                                             c_int, c_int, c_int, c_int, _P, _P,
+                                                             _P, _P]),
     "veon_bev_pool_v2_bwd_workspace_floats": (c_size_t, [c_int64, c_int, c_int, c_int, c_int, c_int,
                                                          c_int, c_int64]),
     "veon_bev_pool_v2_bwd_planar": (c_int, [_P, _P, _P, _P, _P, _P, c_int64,

@@ -492,11 +492,12 @@ class MaxDown2x2x2(torch.autograd.Function):
     """The neck's 2x2x2 reduction, `rearrange(... '(dz dh dw)') -> torch.max(dim=-1).values`
     (view_transformer_raw.py:549-553), and its gradient (all of it to the first arg-max of a
     block, as max(dim) does) as two streaming kernels.  A channels-last-3d input (even Z, Y, X)
-    goes through the channels-last kernels and gives a channels-last-3d result."""
+    goes through the channels-last kernels and gives a channels-last-3d result.  A bfloat16 input
+    gives a bfloat16 result and gradient, bit for bit that expression on the bfloat16 tensor."""
 
     @staticmethod
     def supports(x):
-        if not (x.is_cuda and x.dtype == torch.float32 and x.dim() == 5
+        if not (x.is_cuda and x.dtype in _DTYPES and x.dim() == 5
                 and x.shape[2] % 2 == 0 and x.shape[3] % 2 == 0):
             return False
         if x.is_contiguous():
@@ -507,22 +508,25 @@ class MaxDown2x2x2(torch.autograd.Function):
     def forward(ctx, x):
         lib = _lib.load()
         B, C, Z, Y, X = x.shape
+        sfx = "_bf16" if x.dtype == torch.bfloat16 else ""
         ctx.channels_last = not x.is_contiguous()
         if ctx.channels_last:
+            what = "veon_maxdown2_cl_fwd" + sfx
             with torch.cuda.device(x.device):
-                out = torch.empty((B, Z // 2, Y // 2, X // 2, C), dtype=torch.float32,
+                out = torch.empty((B, Z // 2, Y // 2, X // 2, C), dtype=x.dtype,
                                   device=x.device).permute(0, 4, 1, 2, 3)
-                with _timed("maxdown_cl_fwd", x.device):
-                    rc = lib.veon_maxdown2_cl_fwd(_ptr(x), B, C, Z, Y, X, _ptr(out),
-                                                  _stream_ptr(x.device))
-            _lib.check(rc, "veon_maxdown2_cl_fwd")
+                with _timed("maxdown_cl_fwd" + sfx, x.device):
+                    rc = getattr(lib, what)(_ptr(x), B, C, Z, Y, X, _ptr(out),
+                                            _stream_ptr(x.device))
+            _lib.check(rc, what)
             ctx.save_for_backward(x, out)
             return out
+        what = "veon_maxdown2_fwd" + sfx
         with torch.cuda.device(x.device):
-            out = torch.empty((B, C, Z // 2, Y // 2, X // 2), dtype=torch.float32, device=x.device)
-            with _timed("maxdown_fwd", x.device):
-                rc = lib.veon_maxdown2_fwd(_ptr(x), B * C, Z, Y, X, _ptr(out), _stream_ptr(x.device))
-        _lib.check(rc, "veon_maxdown2_fwd")
+            out = torch.empty((B, C, Z // 2, Y // 2, X // 2), dtype=x.dtype, device=x.device)
+            with _timed("maxdown_fwd" + sfx, x.device):
+                rc = getattr(lib, what)(_ptr(x), B * C, Z, Y, X, _ptr(out), _stream_ptr(x.device))
+        _lib.check(rc, what)
         ctx.save_for_backward(x, out)
         return out
 
@@ -531,22 +535,25 @@ class MaxDown2x2x2(torch.autograd.Function):
         x, out = ctx.saved_tensors
         lib = _lib.load()
         B, C, Z, Y, X = x.shape
+        sfx = "_bf16" if x.dtype == torch.bfloat16 else ""
         if ctx.channels_last:
-            g = grad_out.float().contiguous(memory_format=torch.channels_last_3d)
+            what = "veon_maxdown2_cl_bwd" + sfx
+            g = grad_out.to(x.dtype).contiguous(memory_format=torch.channels_last_3d)
             with torch.cuda.device(x.device):
                 grad_in = torch.empty_like(x)          # channels-last, like x
-                with _timed("maxdown_cl_bwd", x.device):
-                    rc = lib.veon_maxdown2_cl_bwd(_ptr(x), _ptr(out), _ptr(g), B, C, Z, Y, X,
-                                                  _ptr(grad_in), _stream_ptr(x.device))
-            _lib.check(rc, "veon_maxdown2_cl_bwd")
+                with _timed("maxdown_cl_bwd" + sfx, x.device):
+                    rc = getattr(lib, what)(_ptr(x), _ptr(out), _ptr(g), B, C, Z, Y, X,
+                                            _ptr(grad_in), _stream_ptr(x.device))
+            _lib.check(rc, what)
             return grad_in
-        g = grad_out.contiguous().float()
+        what = "veon_maxdown2_bwd" + sfx
+        g = grad_out.contiguous().to(x.dtype)
         with torch.cuda.device(x.device):
             grad_in = torch.empty_like(x)
-            with _timed("maxdown_bwd", x.device):
-                rc = lib.veon_maxdown2_bwd(_ptr(x), _ptr(out), _ptr(g), B * C, Z, Y, X,
-                                           _ptr(grad_in), _stream_ptr(x.device))
-        _lib.check(rc, "veon_maxdown2_bwd")
+            with _timed("maxdown_bwd" + sfx, x.device):
+                rc = getattr(lib, what)(_ptr(x), _ptr(out), _ptr(g), B * C, Z, Y, X,
+                                        _ptr(grad_in), _stream_ptr(x.device))
+        _lib.check(rc, what)
         return grad_in
 
 
@@ -556,10 +563,15 @@ class PoolMaxDown(torch.autograd.Function):
     of the plain route, plus an 8-bit mask per output (one bit: which input is the arg-max,
     the first one on ties).  Backward: the gradient rows of the occupied voxels come straight
     from grad_ds and the mask (the gradient of torch.max(dim): everything to the arg-max), so
-    neither the 1.31 GB full-resolution gradient nor the volume is kept or touched."""
+    neither the 1.31 GB full-resolution gradient nor the volume is kept or touched.
+
+    dtype=torch.bfloat16: the maximum and its mask are taken over the float32 volume and the
+    reduced volume is stored in bfloat16 (the float32 result rounded once); its bfloat16 gradient
+    is read in place and widened exactly, so depth / feat gradients are those of the float32 node
+    for the widened gradient."""
 
     @staticmethod
-    def forward(ctx, depth, feat, prep, bev_feat_shape):
+    def forward(ctx, depth, feat, prep, bev_feat_shape, dtype=torch.float32):
         lib = _lib.load()
         B, Z, Y, X, C = (int(v) for v in bev_feat_shape)
         plan = prep.plan
@@ -568,15 +580,17 @@ class PoolMaxDown(torch.autograd.Function):
         vol = _fwd_planar(depth, feat, prep.ranks_depth, prep.ranks_feat, prep.ranks_bev, plan,
                           B, C, Z * Y * X, (B, C, Z, Y, X))
         dev = vol.device
+        ctx.sfx = "_bf16" if dtype is torch.bfloat16 else ""
+        what = "veon_maxdown2_fwd_mask" + ctx.sfx
         with torch.cuda.device(dev):
-            out = torch.empty((B, C, Z // 2, Y // 2, X // 2), dtype=torch.float32, device=dev)
+            out = torch.empty((B, C, Z // 2, Y // 2, X // 2), dtype=dtype, device=dev)
             mask = torch.empty(out.shape, dtype=torch.uint8, device=dev)
-            with _timed("maxdown_fwd", dev):
-                rc = lib.veon_maxdown2_fwd_mask(_ptr(vol), B * C, Z, Y, X, _ptr(out), _ptr(mask),
-                                                _stream_ptr(dev))
-        _lib.check(rc, "veon_maxdown2_fwd_mask")
+            with _timed("maxdown_fwd" + ("_mask_bf16" if ctx.sfx else ""), dev):
+                rc = getattr(lib, what)(_ptr(vol), B * C, Z, Y, X, _ptr(out), _ptr(mask),
+                                        _stream_ptr(dev))
+        _lib.check(rc, what)
         ctx.save_for_backward(depth, feat, mask)
-        ctx.plan, ctx.grid = plan, (Z, Y, X)
+        ctx.plan, ctx.grid, ctx.dtype = plan, (Z, Y, X), dtype
         return out
 
     @staticmethod
@@ -588,9 +602,9 @@ class PoolMaxDown(torch.autograd.Function):
         B, N, D, H, W = plan.dims
         C = feat.shape[-1]
         dev = feat.device
-        g = grad_ds.contiguous().float()
+        g = grad_ds.contiguous().to(ctx.dtype)
         _need_backward_tables(plan)
-        suffix = "_bf16feat" if feat.dtype == torch.bfloat16 else ""
+        suffix = ctx.sfx + ("_bf16feat" if feat.dtype == torch.bfloat16 else "")
         with torch.cuda.device(dev):
             depth_grad = torch.empty_like(depth)
             feat_grad = torch.empty_like(feat)          # in the rows' dtype
@@ -601,17 +615,19 @@ class PoolMaxDown(torch.autograd.Function):
                     _ptr(plan.tile_occ), _ptr(plan.point_interval), n_int, B, N, D, H, W, C,
                     Z, Y, X, _ptr(rows), _ptr(depth_grad), _ptr(feat_grad), _stream_ptr(dev))
         _lib.check(rc, "veon_bev_pool_v2_bwd_planar_ds" + suffix)
-        return depth_grad, _feat_grad_back(feat_grad, ctx.feat_transposed), None, None
+        return depth_grad, _feat_grad_back(feat_grad, ctx.feat_transposed), None, None, None
 
 
-def pool_prepared_maxdown(depth, feat, prep, bev_feat_shape):
+def pool_prepared_maxdown(depth, feat, prep, bev_feat_shape, *, dtype=torch.float32):
     """Pool + 2x2x2 max as one differentiable node (see PoolMaxDown); None when the grid is not
-    even / X % 4 != 0 or the plan is not a prepared one (the caller then takes the plain route)."""
+    even / X % 4 != 0 or the plan is not a prepared one (the caller then takes the plain route).
+    dtype (float32 or bfloat16) is that of the reduced volume and of the gradient it takes."""
+    _bf16(dtype)                      # ValueError for anything but float32 / bfloat16
     B, Z, Y, X, C = (int(v) for v in bev_feat_shape)
     if (Z | Y) & 1 or X & 3 or not prep.plan.ok:
         return None
     _require_cuda(depth, feat)
-    return PoolMaxDown.apply(depth, feat, prep, bev_feat_shape)
+    return PoolMaxDown.apply(depth, feat, prep, bev_feat_shape, dtype)
 
 
 def voxel_pooling_prepare_v2(coor, grid_lower_bound, grid_interval, grid_size):

@@ -10,6 +10,11 @@
 // 16-byte load from each of the four input x-rows, so every access is a full coalesced line.
 // NaN propagates like torch.max (a NaN input makes the output NaN; the first NaN takes the
 // gradient).
+// bfloat16 volumes (TIn / TOut / T = bf16) are widened exactly where they are loaded and the
+// maximum is stored rounded to nearest even: exact for a bfloat16 input, whose maximum is one of
+// its own values, and the float32 maximum rounded once for a float32 input.  The comparisons are
+// the float32 kernels' on the widened values, so the NaN rule, the first arg-max and the -0/+0
+// result do not change.
 #include "common.cuh"
 
 namespace veon {
@@ -21,10 +26,27 @@ __device__ __forceinline__ float max_nan(float a, float b) { return (b > a || b 
 // (dz*2+dy)*2+dx = the position in the reference's trailing (dz dh dw) axis, first maximum on
 // ties): all the backward needs, so the volume need not be kept for it.
 __device__ __forceinline__ bool is_max(float v, float m) { return v == m || (m != m && v != v); }
-template <bool MASK>
+
+// two neighbouring outputs: 8 bytes of float, 4 of bf16
+__device__ __forceinline__ void st_pair(float* p, float2 v) { *reinterpret_cast<float2*>(p) = v; }
+__device__ __forceinline__ void st_pair(bf16* p, float2 v) {
+  *reinterpret_cast<uint32_t*>(p) = bf16x2_bits(v.x, v.y);
+}
+__device__ __forceinline__ float2 ld_pair(const float* p) {
+  return *reinterpret_cast<const float2*>(p);
+}
+__device__ __forceinline__ float2 ld_pair(const bf16* p) {
+  const uint32_t u = *reinterpret_cast<const uint32_t*>(p);
+  float2 r;
+  r.x = __uint_as_float(u << 16);
+  r.y = __uint_as_float(u & 0xffff0000u);
+  return r;
+}
+
+template <bool MASK, typename TIn, typename TOut>
 __global__ void __launch_bounds__(256)
-k_maxdown2_fwd(const float* __restrict__ in, int64_t n_quads, int Zh, int Yh, int X4, int Y, int X,
-               float* __restrict__ out, uint8_t* __restrict__ mask) {
+k_maxdown2_fwd(const TIn* __restrict__ in, int64_t n_quads, int Zh, int Yh, int X4, int Y, int X,
+               TOut* __restrict__ out, uint8_t* __restrict__ mask) {
   for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < n_quads;
        q += (int64_t)gridDim.x * blockDim.x) {
     const int x4 = (int)(q % X4);
@@ -33,7 +55,7 @@ k_maxdown2_fwd(const float* __restrict__ in, int64_t n_quads, int Zh, int Yh, in
     r /= Yh;
     const int zo = (int)(r % Zh);
     const int64_t bc = r / Zh;
-    const float* p = in + ((bc * (2 * Zh) + 2 * zo) * Y + 2 * yo) * (int64_t)X + 4 * x4;
+    const TIn* p = in + ((bc * (2 * Zh) + 2 * zo) * Y + 2 * yo) * (int64_t)X + 4 * x4;
     const float4 a = ld_stream4(p), b = ld_stream4(p + X);
     const float4 c = ld_stream4(p + (int64_t)Y * X), d = ld_stream4(p + (int64_t)Y * X + X);
     float2 o;
@@ -42,7 +64,7 @@ k_maxdown2_fwd(const float* __restrict__ in, int64_t n_quads, int Zh, int Yh, in
     o.y = max_nan(max_nan(max_nan(a.z, a.w), max_nan(b.z, b.w)),
                   max_nan(max_nan(c.z, c.w), max_nan(d.z, d.w)));
     const int64_t oi = ((bc * Zh + zo) * Yh + yo) * (int64_t)(X / 2) + 2 * x4;
-    *reinterpret_cast<float2*>(out + oi) = o;
+    st_pair(out + oi, o);
     if (MASK) {
       uint32_t m0 = is_max(a.x, o.x) | is_max(a.y, o.x) << 1 | is_max(b.x, o.x) << 2 |
                     is_max(b.y, o.x) << 3 | is_max(c.x, o.x) << 4 | is_max(c.y, o.x) << 5 |
@@ -57,10 +79,11 @@ k_maxdown2_fwd(const float* __restrict__ in, int64_t n_quads, int Zh, int Yh, in
   }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(256)
-k_maxdown2_bwd(const float* __restrict__ in, const float* __restrict__ out,
-               const float* __restrict__ grad_out, int64_t n_quads, int Zh, int Yh, int X4, int Y,
-               int X, float* __restrict__ grad_in) {
+k_maxdown2_bwd(const T* __restrict__ in, const T* __restrict__ out,
+               const T* __restrict__ grad_out, int64_t n_quads, int Zh, int Yh, int X4, int Y,
+               int X, T* __restrict__ grad_in) {
   for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < n_quads;
        q += (int64_t)gridDim.x * blockDim.x) {
     const int x4 = (int)(q % X4);
@@ -75,8 +98,8 @@ k_maxdown2_bwd(const float* __restrict__ in, const float* __restrict__ out,
     float4 v[4];
 #pragma unroll
     for (int k = 0; k < 4; ++k) v[k] = ld_stream4(in + ibase + step[k]);
-    const float2 m = *reinterpret_cast<const float2*>(out + obase);
-    const float2 g = *reinterpret_cast<const float2*>(grad_out + obase);
+    const float2 m = ld_pair(out + obase);
+    const float2 g = ld_pair(grad_out + obase);
     // the whole gradient to the FIRST maximum in (dz, dy, dx) order = k-major, then x
     // (the backward of torch.max(dim).values: index_put of the arg-max)
     bool open0 = true, open1 = true;
@@ -119,9 +142,10 @@ __device__ __forceinline__ void cl_block(int64_t e, int C, int Zh, int Yh, int X
   step[3] = (int64_t)Y * row + row;
 }
 
+template <typename T>
 __global__ void __launch_bounds__(256)
-k_maxdown2_cl_fwd(const float* __restrict__ in, int64_t n_out, int C, int Zh, int Yh, int Xh, int Y,
-                  int X, float* __restrict__ out) {
+k_maxdown2_cl_fwd(const T* __restrict__ in, int64_t n_out, int C, int Zh, int Yh, int Xh, int Y,
+                  int X, T* __restrict__ out) {
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n_out;
        e += (int64_t)gridDim.x * blockDim.x) {
     int64_t ib, st[4];
@@ -129,18 +153,19 @@ k_maxdown2_cl_fwd(const float* __restrict__ in, int64_t n_out, int C, int Zh, in
     float a[4][2];
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-      a[k][0] = __ldcs(in + ib + st[k]);
-      a[k][1] = __ldcs(in + ib + st[k] + C);
+      a[k][0] = widen(__ldcs(in + ib + st[k]));
+      a[k][1] = widen(__ldcs(in + ib + st[k] + C));
     }
-    out[e] = max_nan(max_nan(max_nan(a[0][0], a[0][1]), max_nan(a[1][0], a[1][1])),
-                     max_nan(max_nan(a[2][0], a[2][1]), max_nan(a[3][0], a[3][1])));
+    store_rn(out + e, max_nan(max_nan(max_nan(a[0][0], a[0][1]), max_nan(a[1][0], a[1][1])),
+                              max_nan(max_nan(a[2][0], a[2][1]), max_nan(a[3][0], a[3][1]))));
   }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(256)
-k_maxdown2_cl_bwd(const float* __restrict__ in, const float* __restrict__ out,
-                  const float* __restrict__ grad_out, int64_t n_out, int C, int Zh, int Yh, int Xh,
-                  int Y, int X, float* __restrict__ grad_in) {
+k_maxdown2_cl_bwd(const T* __restrict__ in, const T* __restrict__ out,
+                  const T* __restrict__ grad_out, int64_t n_out, int C, int Zh, int Yh, int Xh,
+                  int Y, int X, T* __restrict__ grad_in) {
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n_out;
        e += (int64_t)gridDim.x * blockDim.x) {
     int64_t ib, st[4];
@@ -148,10 +173,10 @@ k_maxdown2_cl_bwd(const float* __restrict__ in, const float* __restrict__ out,
     float v[4][2];
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-      v[k][0] = __ldcs(in + ib + st[k]);
-      v[k][1] = __ldcs(in + ib + st[k] + C);
+      v[k][0] = widen(__ldcs(in + ib + st[k]));
+      v[k][1] = widen(__ldcs(in + ib + st[k] + C));
     }
-    const float m = out[e], g = grad_out[e];
+    const float m = widen(out[e]), g = widen(grad_out[e]);
     bool open = true;   // the whole gradient to the FIRST maximum in (dz, dy, dx) order
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
@@ -172,10 +197,73 @@ static int check_cl(const void* a, const void* b, int B, int C, int Z, int Y, in
   return 0;
 }
 
-static int check(const void* a, const void* b, int64_t BC, int Z, int Y, int X) {
+// a: the [BC,Z,Y,X] volume (four-element loads), b: the reduced one (two-element stores); the
+// alignments are those of TIn / TOut: 16 and 8 bytes for float, 8 and 4 for bf16
+template <typename TIn, typename TOut>
+static int check(const TIn* a, const TOut* b, int64_t BC, int Z, int Y, int X) {
   if (!a || !b || BC <= 0 || Z <= 0 || Y <= 0 || X <= 0) return VEON_E_BADARG;
-  if ((Z & 1) || (Y & 1) || (X & 3) || ((uintptr_t)a & 15) || ((uintptr_t)b & 7))
+  if ((Z & 1) || (Y & 1) || (X & 3) || ((uintptr_t)a & (4 * sizeof(TIn) - 1)) ||
+      ((uintptr_t)b & (2 * sizeof(TOut) - 1)))
     return VEON_E_UNSUPPORTED;
+  return 0;
+}
+
+static int64_t grid_blocks(int64_t n) {
+  const int64_t blocks = ceil_div64(n, 256);
+  return blocks > 148 * 64 ? 148 * 64 : blocks;
+}
+
+template <bool MASK, typename TIn, typename TOut>
+static int maxdown2_fwd(const TIn* in, int64_t BC, int Z, int Y, int X, TOut* out, uint8_t* mask,
+                        cudaStream_t stream) {
+  int rc = check(in, out, BC, Z, Y, X);
+  if (rc) return rc;
+  if (MASK && !mask) return VEON_E_BADARG;
+  if (MASK && ((uintptr_t)mask & 1)) return VEON_E_UNSUPPORTED;
+  const int64_t n_quads = BC * (Z / 2) * (Y / 2) * (X / 4);
+  k_maxdown2_fwd<MASK, TIn, TOut><<<(unsigned)grid_blocks(n_quads), 256, 0, stream>>>(
+      in, n_quads, Z / 2, Y / 2, X / 4, Y, X, out, mask);
+  VEON_LAUNCH_CHECK();
+  return 0;
+}
+
+template <typename T>
+static int maxdown2_bwd(const T* in, const T* out, const T* grad_out, int64_t BC, int Z, int Y,
+                        int X, T* grad_in, cudaStream_t stream) {
+  int rc = check(in, out, BC, Z, Y, X);
+  if (rc) return rc;
+  if (!grad_out || !grad_in) return VEON_E_BADARG;
+  if (((uintptr_t)grad_in & (4 * sizeof(T) - 1)) || ((uintptr_t)grad_out & (2 * sizeof(T) - 1)))
+    return VEON_E_UNSUPPORTED;
+  const int64_t n_quads = BC * (Z / 2) * (Y / 2) * (X / 4);
+  k_maxdown2_bwd<T><<<(unsigned)grid_blocks(n_quads), 256, 0, stream>>>(
+      in, out, grad_out, n_quads, Z / 2, Y / 2, X / 4, Y, X, grad_in);
+  VEON_LAUNCH_CHECK();
+  return 0;
+}
+
+template <typename T>
+static int maxdown2_cl_fwd(const T* in, int B, int C, int Z, int Y, int X, T* out,
+                           cudaStream_t stream) {
+  int rc = check_cl(in, out, B, C, Z, Y, X);
+  if (rc) return rc;
+  const int64_t n_out = (int64_t)B * (Z / 2) * (Y / 2) * (X / 2) * C;
+  k_maxdown2_cl_fwd<T><<<(unsigned)grid_blocks(n_out), 256, 0, stream>>>(
+      in, n_out, C, Z / 2, Y / 2, X / 2, Y, X, out);
+  VEON_LAUNCH_CHECK();
+  return 0;
+}
+
+template <typename T>
+static int maxdown2_cl_bwd(const T* in, const T* out, const T* grad_out, int B, int C, int Z,
+                           int Y, int X, T* grad_in, cudaStream_t stream) {
+  int rc = check_cl(in, out, B, C, Z, Y, X);
+  if (rc) return rc;
+  if (!grad_out || !grad_in) return VEON_E_BADARG;
+  const int64_t n_out = (int64_t)B * (Z / 2) * (Y / 2) * (X / 2) * C;
+  k_maxdown2_cl_bwd<T><<<(unsigned)grid_blocks(n_out), 256, 0, stream>>>(
+      in, out, grad_out, n_out, C, Z / 2, Y / 2, X / 2, Y, X, grad_in);
+  VEON_LAUNCH_CHECK();
   return 0;
 }
 
@@ -185,71 +273,60 @@ using namespace veon;
 
 extern "C" int veon_maxdown2_fwd(const float* in, int64_t BC, int Z, int Y, int X, float* out,
                                  void* stream_) {
-  int rc = check(in, out, BC, Z, Y, X);
-  if (rc) return rc;
-  const int64_t n_quads = BC * (Z / 2) * (Y / 2) * (X / 4);
-  int64_t blocks = ceil_div64(n_quads, 256);
-  if (blocks > 148 * 64) blocks = 148 * 64;
-  k_maxdown2_fwd<false><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(
-      in, n_quads, Z / 2, Y / 2, X / 4, Y, X, out, nullptr);
-  VEON_LAUNCH_CHECK();
-  return 0;
+  return maxdown2_fwd<false>(in, BC, Z, Y, X, out, nullptr, (cudaStream_t)stream_);
 }
 
 extern "C" int veon_maxdown2_fwd_mask(const float* in, int64_t BC, int Z, int Y, int X, float* out,
                                       uint8_t* mask, void* stream_) {
-  int rc = check(in, out, BC, Z, Y, X);
-  if (rc) return rc;
-  if (!mask) return VEON_E_BADARG;
-  if ((uintptr_t)mask & 1) return VEON_E_UNSUPPORTED;
-  const int64_t n_quads = BC * (Z / 2) * (Y / 2) * (X / 4);
-  int64_t blocks = ceil_div64(n_quads, 256);
-  if (blocks > 148 * 64) blocks = 148 * 64;
-  k_maxdown2_fwd<true><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(
-      in, n_quads, Z / 2, Y / 2, X / 4, Y, X, out, mask);
-  VEON_LAUNCH_CHECK();
-  return 0;
+  return maxdown2_fwd<true>(in, BC, Z, Y, X, out, mask, (cudaStream_t)stream_);
 }
 
 extern "C" int veon_maxdown2_bwd(const float* in, const float* out, const float* grad_out,
                                  int64_t BC, int Z, int Y, int X, float* grad_in, void* stream_) {
-  int rc = check(in, out, BC, Z, Y, X);
-  if (rc) return rc;
-  if (!grad_out || !grad_in) return VEON_E_BADARG;
-  if (((uintptr_t)grad_in & 15) || ((uintptr_t)grad_out & 7)) return VEON_E_UNSUPPORTED;
-  const int64_t n_quads = BC * (Z / 2) * (Y / 2) * (X / 4);
-  int64_t blocks = ceil_div64(n_quads, 256);
-  if (blocks > 148 * 64) blocks = 148 * 64;
-  k_maxdown2_bwd<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(
-      in, out, grad_out, n_quads, Z / 2, Y / 2, X / 4, Y, X, grad_in);
-  VEON_LAUNCH_CHECK();
-  return 0;
+  return maxdown2_bwd(in, out, grad_out, BC, Z, Y, X, grad_in, (cudaStream_t)stream_);
 }
 
 extern "C" int veon_maxdown2_cl_fwd(const float* in, int B, int C, int Z, int Y, int X, float* out,
                                     void* stream_) {
-  int rc = check_cl(in, out, B, C, Z, Y, X);
-  if (rc) return rc;
-  const int64_t n_out = (int64_t)B * (Z / 2) * (Y / 2) * (X / 2) * C;
-  int64_t blocks = ceil_div64(n_out, 256);
-  if (blocks > 148 * 64) blocks = 148 * 64;
-  k_maxdown2_cl_fwd<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(
-      in, n_out, C, Z / 2, Y / 2, X / 2, Y, X, out);
-  VEON_LAUNCH_CHECK();
-  return 0;
+  return maxdown2_cl_fwd(in, B, C, Z, Y, X, out, (cudaStream_t)stream_);
 }
 
 extern "C" int veon_maxdown2_cl_bwd(const float* in, const float* out, const float* grad_out,
                                     int B, int C, int Z, int Y, int X, float* grad_in,
                                     void* stream_) {
-  int rc = check_cl(in, out, B, C, Z, Y, X);
-  if (rc) return rc;
-  if (!grad_out || !grad_in) return VEON_E_BADARG;
-  const int64_t n_out = (int64_t)B * (Z / 2) * (Y / 2) * (X / 2) * C;
-  int64_t blocks = ceil_div64(n_out, 256);
-  if (blocks > 148 * 64) blocks = 148 * 64;
-  k_maxdown2_cl_bwd<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(
-      in, out, grad_out, n_out, C, Z / 2, Y / 2, X / 2, Y, X, grad_in);
-  VEON_LAUNCH_CHECK();
-  return 0;
+  return maxdown2_cl_bwd(in, out, grad_out, B, C, Z, Y, X, grad_in, (cudaStream_t)stream_);
+}
+
+// bfloat16 volumes (uint16_t bit patterns), the arguments of the float32 twins
+static const bf16* as_bf16(const uint16_t* p) { return reinterpret_cast<const bf16*>(p); }
+static bf16* as_bf16(uint16_t* p) { return reinterpret_cast<bf16*>(p); }
+
+extern "C" int veon_maxdown2_fwd_bf16(const uint16_t* in, int64_t BC, int Z, int Y, int X,
+                                      uint16_t* out, void* stream_) {
+  return maxdown2_fwd<false>(as_bf16(in), BC, Z, Y, X, as_bf16(out), nullptr,
+                             (cudaStream_t)stream_);
+}
+
+extern "C" int veon_maxdown2_fwd_mask_bf16(const float* in, int64_t BC, int Z, int Y, int X,
+                                           uint16_t* out, uint8_t* mask, void* stream_) {
+  return maxdown2_fwd<true>(in, BC, Z, Y, X, as_bf16(out), mask, (cudaStream_t)stream_);
+}
+
+extern "C" int veon_maxdown2_bwd_bf16(const uint16_t* in, const uint16_t* out,
+                                      const uint16_t* grad_out, int64_t BC, int Z, int Y, int X,
+                                      uint16_t* grad_in, void* stream_) {
+  return maxdown2_bwd(as_bf16(in), as_bf16(out), as_bf16(grad_out), BC, Z, Y, X, as_bf16(grad_in),
+                      (cudaStream_t)stream_);
+}
+
+extern "C" int veon_maxdown2_cl_fwd_bf16(const uint16_t* in, int B, int C, int Z, int Y, int X,
+                                         uint16_t* out, void* stream_) {
+  return maxdown2_cl_fwd(as_bf16(in), B, C, Z, Y, X, as_bf16(out), (cudaStream_t)stream_);
+}
+
+extern "C" int veon_maxdown2_cl_bwd_bf16(const uint16_t* in, const uint16_t* out,
+                                         const uint16_t* grad_out, int B, int C, int Z, int Y,
+                                         int X, uint16_t* grad_in, void* stream_) {
+  return maxdown2_cl_bwd(as_bf16(in), as_bf16(out), as_bf16(grad_out), B, C, Z, Y, X,
+                         as_bf16(grad_in), (cudaStream_t)stream_);
 }

@@ -224,8 +224,13 @@ k_bwd_rows_persistent(const T* __restrict__ out_grad, const int32_t* __restrict_
 // and neither the full-resolution gradient nor the volume itself is ever read: 0.2 GB instead
 // of 2.9 + 1.2 GB for the down-sample backward followed by the plain row pass.
 // One warp per occupied tile, lanes = channels, four voxels' loads in flight.
-__global__ void __launch_bounds__(256)
-k_bwd_rows_ds(const float* __restrict__ grad_ds, const uint8_t* __restrict__ mask,
+// A bfloat16 grad_ds (TG = bf16) is widened exactly where it is loaded; the rows stay float.
+// ptxas gives either instance 64 registers; asked for 4 CTAs per SM (the same 64), it allocates
+// the bf16 one without the 20-byte spill the float one has.  (0 = no minimum: the float kernel
+// compiles as it did.)
+template <typename TG>
+__global__ void __launch_bounds__(256, sizeof(TG) == 2 ? 4 : 0)
+k_bwd_rows_ds(const TG* __restrict__ grad_ds, const uint8_t* __restrict__ mask,
               const int32_t* __restrict__ tile_istart, const uint32_t* __restrict__ tile_occ,
               int64_t n_tiles, int64_t tiles_per_sample, int Z, int Y, int X, int C,
               float* __restrict__ rows) {
@@ -267,7 +272,7 @@ k_bwd_rows_ds(const float* __restrict__ grad_ds, const uint8_t* __restrict__ mas
           g[q] = 0.f;
           m[q] = 0u;
           if (q < nv) {
-            g[q] = __ldg(grad_ds + base + blk[q]);
+            g[q] = ldg_widen(grad_ds + base + blk[q]);
             m[q] = __ldg(mask + base + blk[q]);
           }
         }
@@ -286,10 +291,11 @@ k_bwd_rows_ds(const float* __restrict__ grad_ds, const uint8_t* __restrict__ mas
 // lengths are then multiples of 8, so every aligned group of 8 voxels of a tile lies in one
 // x-row = 4 consecutive blocks of one (z/2, y/2) row of the down-sampled volume.  Lane
 // (cs = lane / 4, q = lane % 4) owns voxels 8q..8q+7 of the tile for channels cs, cs + 8, ...:
-// one 16-byte load of grad_ds and one 4-byte load of the mask per channel, then up to 8
-// predicated 4-byte row stores; the 8 lanes of a q write 32 consecutive bytes of a row.
+// one 16-byte (bf16: 8-byte) load of grad_ds and one 4-byte load of the mask per channel, then up
+// to 8 predicated 4-byte row stores; the 8 lanes of a q write 32 consecutive bytes of a row.
+template <typename TG>
 __global__ void __launch_bounds__(256)
-k_bwd_rows_ds_direct(const float* __restrict__ grad_ds, const uint8_t* __restrict__ mask,
+k_bwd_rows_ds_direct(const TG* __restrict__ grad_ds, const uint8_t* __restrict__ mask,
                      const int32_t* __restrict__ tile_istart,
                      const uint32_t* __restrict__ tile_occ, int64_t n_tiles,
                      int64_t tiles_per_sample, int Z, int Y, int X, int C,
@@ -315,7 +321,7 @@ k_bwd_rows_ds_direct(const float* __restrict__ grad_ds, const uint8_t* __restric
     const int ibase = i0 + __popc(occ & ((1u << (8 * q)) - 1u));   // interval of the first set bit
     for (int c = cs; c < C; c += 8) {
       const int64_t src = ((int64_t)b * C + c) * plane + blk0;
-      const float4 g4 = __ldg(reinterpret_cast<const float4*>(grad_ds + src));
+      const float4 g4 = ldg_widen4(grad_ds + src);
       const uchar4 m4 = __ldg(reinterpret_cast<const uchar4*>(mask + src));
       const float gv[4] = {g4.x, g4.y, g4.z, g4.w};
       const uint32_t mv[4] = {m4.x, m4.y, m4.z, m4.w};
@@ -704,9 +710,9 @@ extern "C" int veon_bev_pool_v2_bwd_planar_cl_bf16(
                        feat_grad, stream);
 }
 
-template <typename TF>
+template <typename TG, typename TF>
 static int bwd_planar_ds(
-    const float* grad_ds, const uint8_t* mask, const float* depth, const TF* feat,
+    const TG* grad_ds, const uint8_t* mask, const float* depth, const TF* feat,
     const int32_t* tile_istart, const uint32_t* tile_occ, const int32_t* point_interval,
     int64_t n_intervals, int B, int N, int D, int H, int W, int C, int Z, int Y, int X,
     float* rows_ws, float* depth_grad, TF* feat_grad, cudaStream_t stream) {
@@ -720,16 +726,17 @@ static int bwd_planar_ds(
   if ((int64_t)B * V > 0x7fffffffLL) return VEON_E_RANGE;
   const int sms = sm_count();
   const int64_t plane = (int64_t)(Z / 2) * (Y / 2) * (X / 2);
-  const bool direct = (X % 8) == 0 && (plane % 4) == 0 && ((uintptr_t)grad_ds & 15) == 0 &&
+  const bool direct = (X % 8) == 0 && (plane % 4) == 0 &&
+                      ((uintptr_t)grad_ds & (4 * sizeof(TG) - 1)) == 0 &&
                       ((uintptr_t)mask & 3) == 0;
   int64_t blocks = ceil_div64(n_tiles, 8);
   if (blocks > (int64_t)sms * 8) blocks = (int64_t)sms * 8;
   if (direct)
-    k_bwd_rows_ds_direct<<<(unsigned)blocks, 256, 0, stream>>>(grad_ds, mask, tile_istart, tile_occ,
-                                                               n_tiles, tps, Z, Y, X, C, rows_ws);
+    k_bwd_rows_ds_direct<TG><<<(unsigned)blocks, 256, 0, stream>>>(
+        grad_ds, mask, tile_istart, tile_occ, n_tiles, tps, Z, Y, X, C, rows_ws);
   else
-    k_bwd_rows_ds<<<(unsigned)blocks, 256, 0, stream>>>(grad_ds, mask, tile_istart, tile_occ,
-                                                        n_tiles, tps, Z, Y, X, C, rows_ws);
+    k_bwd_rows_ds<TG><<<(unsigned)blocks, 256, 0, stream>>>(grad_ds, mask, tile_istart, tile_occ,
+                                                            n_tiles, tps, Z, Y, X, C, rows_ws);
   VEON_LAUNCH_CHECK();
   return pixel_pass(rows_ws, depth, feat, point_interval, (int64_t)B * N * H * W, D, H * W, C,
                     depth_grad, feat_grad, stream);
@@ -797,6 +804,29 @@ extern "C" int veon_bev_pool_v2_bwd_planar_ds_bf16feat(
   return bwd_planar_ds(grad_ds, mask, depth, reinterpret_cast<const bf16*>(feat), tile_istart,
                        tile_occ, point_interval, n_intervals, B, N, D, H, W, C, Z, Y, X, rows_ws,
                        depth_grad, reinterpret_cast<bf16*>(feat_grad), (cudaStream_t)stream);
+}
+
+// bfloat16 grad_ds [B,C,Z/2,Y/2,X/2] (the reduced volume of veon_maxdown2_fwd_mask_bf16): widened
+// exactly where the row pass loads it, everything after is the float32 twin's.
+extern "C" int veon_bev_pool_v2_bwd_planar_ds_bf16(
+    const uint16_t* grad_ds, const uint8_t* mask, const float* depth, const float* feat,
+    const int32_t* tile_istart, const uint32_t* tile_occ, const int32_t* point_interval,
+    int64_t n_intervals, int B, int N, int D, int H, int W, int C, int Z, int Y, int X,
+    float* rows_ws, float* depth_grad, float* feat_grad, void* stream) {
+  return bwd_planar_ds(reinterpret_cast<const bf16*>(grad_ds), mask, depth, feat, tile_istart,
+                       tile_occ, point_interval, n_intervals, B, N, D, H, W, C, Z, Y, X, rows_ws,
+                       depth_grad, feat_grad, (cudaStream_t)stream);
+}
+
+extern "C" int veon_bev_pool_v2_bwd_planar_ds_bf16_bf16feat(
+    const uint16_t* grad_ds, const uint8_t* mask, const float* depth, const uint16_t* feat,
+    const int32_t* tile_istart, const uint32_t* tile_occ, const int32_t* point_interval,
+    int64_t n_intervals, int B, int N, int D, int H, int W, int C, int Z, int Y, int X,
+    float* rows_ws, float* depth_grad, uint16_t* feat_grad, void* stream) {
+  return bwd_planar_ds(reinterpret_cast<const bf16*>(grad_ds), mask, depth,
+                       reinterpret_cast<const bf16*>(feat), tile_istart, tile_occ, point_interval,
+                       n_intervals, B, N, D, H, W, C, Z, Y, X, rows_ws, depth_grad,
+                       reinterpret_cast<bf16*>(feat_grad), (cudaStream_t)stream);
 }
 
 #ifdef VEON_TOOLS   // tools/build_variant.sh NAME "-DVEON_TOOLS": never in the shipped library

@@ -338,15 +338,39 @@ class LSSViewTransformerRaw(LSSViewTransformer):
     pools channels-last and reduces with the channels-last 2x2x2 kernels (the
     fused `fuse_ds` kernel and the one-node PoolMaxDown training route are
     channels-first only and are not taken); the result is channels-last-3d.
-    Float32 only: its 2x2x2 maximum, `PoolMaxDown`, `fuse_ds` and the fused lift + classify
-    have no bfloat16 form (a bfloat16 maximum may pick another first arg-max than the float32
-    one), so any other `dtype` raises ValueError."""
 
-    def __init__(self, *args, use_ds=True, ds=(2, 2, 2), fuse_ds=False, **kwargs):
+    `dtype` (the pooled full-resolution volume) is float32 only: any other raises ValueError.
+
+    Extra: `ds_dtype` -- the dtype of the 2x2x2-reduced output, torch.float32 (the default) or
+    torch.bfloat16 (what a 3D decoder under bfloat16 autocast reads; needs use_ds).  With bfloat16:
+    - a gradient wanted: the output is, bit for bit, the float32 neck's output cast to bfloat16,
+      and the depth / feature gradients are the float32 neck's for the widened output gradient.
+      The maximum and its first arg-max are taken over the float32 sums, as the reference's are
+      under autocast.  Channels-first 2x2x2 takes the one-node PoolMaxDown route, which stores a
+      bfloat16 result and reads its bfloat16 gradient in place; channels-last takes the float32
+      route followed by a cast (which keeps the layout).
+    - no gradient (2x2x2, even grid, fused geometry): the neck pools straight into a bfloat16
+      volume (either layout) and takes the maximum in bfloat16, so no float32 full-resolution
+      volume is written; this replaces `fuse_ds`.  Rounding to nearest even is monotone, so every
+      value equals the float32 route cast (==), and so do the bits, except that a zero result
+      may carry the other sign: a window whose float32 sums include a nonzero one of magnitude
+      below 2^-134, which bfloat16 rounds to a signed zero, may then return the zero of another
+      element.  Which element is the arg-max is not observable without a gradient.
+    - any other case (other `ds`, odd grids, `accelerate`, `collapse_z`, the empty-input dummy):
+      the float32 route, then one cast."""
+
+    def __init__(self, *args, use_ds=True, ds=(2, 2, 2), fuse_ds=False, ds_dtype=torch.float32,
+                 **kwargs):
+        if not isinstance(ds_dtype, torch.dtype) or ds_dtype not in _bp._DTYPES:
+            raise ValueError(f"ds_dtype must be torch.float32 or torch.bfloat16, got {ds_dtype!r}")
+        if ds_dtype is torch.bfloat16 and not use_ds:
+            raise ValueError("ds_dtype=torch.bfloat16 is the dtype of the 2x2x2-reduced volume "
+                             "and needs use_ds=True")
         kwargs.setdefault("collapse_z", False)
         super().__init__(*args, **kwargs)
         if self.dtype is not torch.float32:
             raise ValueError(f"LSSViewTransformerRaw is float32 only, got dtype={self.dtype!r}")
+        self.ds_dtype = ds_dtype
         self.use_ds = use_ds
         self.ds = tuple(ds)
         # Extra (not in the reference): pool and max-reduce in ONE kernel on the no-grad path,
@@ -384,7 +408,10 @@ class LSSViewTransformerRaw(LSSViewTransformer):
     def forward(self, input, depth, stereo_metas=None):
         tran_feat = input[0]
         B, N, C, H, W = tran_feat.shape
-        fused = self._forward_downsampled(input, depth)
+        if self.ds_dtype is torch.bfloat16:
+            fused = self._forward_bf16_inference(input, depth)
+        else:
+            fused = self._forward_downsampled(input, depth)
         if fused is None:
             fused = self._forward_pool_maxdown(input, depth)
         if fused is not None:
@@ -402,7 +429,7 @@ class LSSViewTransformerRaw(LSSViewTransformer):
                 bev_feat = bev_feat.view(b, c, z // dz, dz, y // dy, dy, x // dx, dx) \
                     .permute(0, 1, 2, 4, 6, 3, 5, 7).reshape(b, c, z // dz, y // dy, x // dx, -1)
                 bev_feat = torch.max(bev_feat, dim=-1).values
-        return bev_feat
+        return bev_feat.to(self.ds_dtype)      # (float32: the tensor itself)
 
     def _forward_pool_maxdown(self, input, depth):
         """Training path: pooling and the 2x2x2 maximum as ONE autograd node whose backward never
@@ -420,7 +447,8 @@ class LSSViewTransformerRaw(LSSViewTransformer):
             self.grid_lower_bound, self.grid_interval, self.grid_size))
         feat_last = tran_feat.reshape(B, N, C, H, W).permute(0, 1, 3, 4, 2)
         d5 = depth.reshape(B, N, self.D, H, W)
-        out = _bp.pool_prepared_maxdown(d5, feat_last, prep, self._bev_shape(d5, C))
+        out = _bp.pool_prepared_maxdown(d5, feat_last, prep, self._bev_shape(d5, C),
+                                        dtype=self.ds_dtype)
         # None also lets the plain route reproduce the reference's empty-input behaviour
         return None if out is None or self._no_points(prep) else out
 
@@ -445,3 +473,27 @@ class LSSViewTransformerRaw(LSSViewTransformer):
         out = _bp.pool_prepared_downsampled(d5, feat_last, prep, self._bev_shape(d5, C))
         # None also lets the plain route reproduce the reference's empty-input behaviour
         return None if out is None or self._no_points(prep) else out
+
+    def _forward_bf16_inference(self, input, depth):
+        """ds_dtype=bfloat16 without a gradient: pool into a bfloat16 volume in the neck's memory
+        format and take the 2x2x2 maximum of it in bfloat16 (see the class docstring for what
+        that returns).  Same ranks as the plain route (fused geometry, rank cache, depth_eps).
+        None -> another route."""
+        tran_feat = input[0]
+        if (self.ds != (2, 2, 2) or self.accelerate or self.collapse_z or not self.fuse_geometry
+                or not tran_feat.is_cuda or not input[1].is_cuda
+                or (torch.is_grad_enabled() and (tran_feat.requires_grad or depth.requires_grad))):
+            return None
+        B, N, C, H, W = tran_feat.shape
+        d5 = depth.reshape(B, N, self.D, H, W)
+        shape = self._bev_shape(d5, C)
+        _, Z, Y, X, _ = shape
+        cl = self.memory_format is torch.channels_last_3d
+        if (Z | Y) & 1 or X % (2 if cl else 4):     # what MaxDown2x2x2 takes
+            return None
+        feat_last = tran_feat.reshape(B, N, C, H, W).permute(0, 1, 3, 4, 2)
+        prep = self._prepare_calib(input[1:7], d5)
+        vol = _bp.pool_prepared(d5, feat_last, self._prepared(prep), shape, self.memory_format,
+                                dtype=torch.bfloat16)
+        # None also lets the plain route reproduce the reference's empty-input behaviour
+        return None if self._no_points(prep) else _bp.MaxDown2x2x2.apply(vol)
