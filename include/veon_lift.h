@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define VEON_ABI_VERSION 10
+#define VEON_ABI_VERSION 11
 
 #define VEON_E_BADARG    (-1)  /* NULL pointer / non-positive dimension          */
 #define VEON_E_WORKSPACE (-2)  /* workspace smaller than *_workspace_bytes()     */
@@ -153,11 +153,6 @@ int veon_lidar_coor(const float* frustum, const float* sensor2ego, const float* 
 size_t veon_prepare_v2_workspace_bytes(int B, int N, int D, int H, int W,
                                        const float* grid_size /*[host]*/);
 int64_t veon_pool_num_tiles(int B, int64_t voxels_per_sample);
-/* Byte offset, inside the veon_prepare_v2 workspace, of `voxel_start`: int32[B*V + 1], first
- * point of every voxel (an exclusive prefix of the per-voxel point counts, valid after the call
- * for B*V < 2^24).  Consumed by veon_bev_pool_v2_ds_fwd.  (size_t)-1 on bad arguments. */
-size_t veon_prepare_v2_voxel_start_offset(int B, int N, int D, int H, int W,
-                                          const float* grid_size /*[host]*/);
 /* int32 elements a tile_heavy buffer needs for a plan over at most n_points points */
 int64_t veon_pool_heavy_list_ints(int64_t n_points, int64_t n_tiles);
 
@@ -245,16 +240,17 @@ int veon_transpose_batched(const float* src, int64_t batch, int R, int S, float*
  *     The result is bit-identical to the reference kernel for every C.
  *     Kernel selection: rows of at most 32 channels (C % 4 == 0, tile_heavy
  *     given, B*V <= 2^24) take a lane-per-voxel kernel; aligned volumes
- *     (V % 32 == 0) with C a multiple of 64 (of 128 above 128, up to 1024), a
- *     complete plan (tile_istart, tile_occ, tile_heavy) and a workspace take the
- *     two-role streaming kernel (compact rows through an L2-resident ring, the
- *     volume written as a pure store stream); everything else the general
- *     lane-per-channel kernel.
+ *     (V % 32 == 0) with C == 64, a complete plan (tile_istart, tile_occ,
+ *     tile_heavy) and a workspace take the two-role streaming kernel (compact
+ *     rows through an L2-resident ring, the volume written as a pure store
+ *     stream); everything else the general lane-per-channel kernel.
  *   workspace   optional scratch of veon_bev_pool_v2_fwd_workspace_bytes()
  *               bytes, 256-byte aligned (a larger or smaller buffer is legal: it
  *               sizes the ring; too small a one selects the general kernel);
  *               contents need not be preserved between calls, but one buffer
- *               must not be shared by calls that may run concurrently.
+ *               must not be shared by calls that may run concurrently.  The
+ *               size is 0 for every C other than 64: no kernel needs a
+ *               workspace there, and NULL with workspace_bytes = 0 is correct.
  * ------------------------------------------------------------------------ */
 size_t veon_bev_pool_v2_fwd_workspace_bytes(int B, int C, int64_t voxels_per_sample);
 int veon_bev_pool_v2_fwd_planar(const float* depth, const float* feat,
@@ -325,16 +321,6 @@ int veon_bev_pool_v2_fwd_planar_cl_bf16(const float* depth, const float* feat,
                                         int B, int C, int64_t voxels_per_sample,
                                         int64_t n_feat_rows /* B*N*H*W rows of feat */,
                                         uint16_t* out /* bfloat16 [B,Z,Y,X,C] */, void* stream);
-
-/* Pooling fused with the 2x2x2 max-downsample VEON's neck applies next
- * (view_transformer_raw.py:549-553), forward only: out is [B, C, Z/2, Y/2, X/2], bit-identical
- * to that maximum over the volume veon_bev_pool_v2_fwd_planar would write (never materialised).
- * Needs even Z, Y, X, C % 64 == 0 and the `voxel_start` array of the prepare workspace. */
-int veon_bev_pool_v2_ds_fwd(const float* depth, const float* feat,
-                            const int32_t* ranks_depth, const int32_t* ranks_feat,
-                            const int32_t* ranks_bev, const int32_t* voxel_start,
-                            int B, int C, int Z, int Y, int X, int64_t n_feat_rows,
-                            float* out, void* stream);
 
 /* Depth-distribution producer in front of the path: LSSViewTransformerRaw.downsample_depth +
  * get_two_hot_depth (view_transformer_raw.py:393-429).  depths [BN, H_out*s, W_out*s] metric

@@ -12,9 +12,9 @@ def _buf():
     return ctypes.cast((ctypes.c_float * 64)(), ctypes.c_void_p)
 
 
-def test_abi_version_is_10():
+def test_abi_version_is_11():
     from veon_b200 import _lib
-    assert _lib.load().veon_abi_version() == 10
+    assert _lib.load().veon_abi_version() == 11
 
 
 @pytest.mark.parametrize("suffix", ["", "_bf16"])

@@ -350,9 +350,9 @@ def test_raw_neck_channels_last_equals_default_bit_for_bit():
         return t.contiguous().view(torch.int32)
     assert torch.equal(bits(a), bits(b))
     assert torch.equal(bits(da), bits(db)) and torch.equal(bits(fa), bits(fb))
-    # inference (no gradient): the plain channels-last route as well, fuse_ds skipped
+    # inference (no gradient): the plain channels-last route as well
     neck = LSSViewTransformerRaw(cfg.grid_config, cfg.input_size, cfg.downsample, 8, C,
-                                 fuse_ds=True, memory_format=CL)
+                                 memory_format=CL)
     with torch.no_grad():
         c = neck([feat5] + metas, depth5)
     assert _is_cl_view(c) and torch.equal(bits(c), bits(a))

@@ -27,7 +27,7 @@ def test_every_new_entry_is_declared_and_bound():
         # the same arguments as the twin without `_bf16feat`
         twin = name.replace("_bf16feat", "").replace("_u16", "")
         assert _lib._SIGNATURES[name] == _lib._SIGNATURES[twin], name
-    assert re.search(r"#define\s+VEON_ABI_VERSION\s+10\b", open(os.path.join(
+    assert re.search(r"#define\s+VEON_ABI_VERSION\s+11\b", open(os.path.join(
         ROOT, "include", "veon_lift.h")).read())
 
 

@@ -318,7 +318,7 @@ def test_lss_neck_forward_under_autocast():
 
 def test_raw_neck_bf16_features():
     """the Raw neck pools bfloat16 features into its float32 volume: the one-node training route
-    (native `_ds` backward), the channels-last plain route, and fuse_ds inference (widened)"""
+    (native `_ds` backward), the channels-last plain route, and no-grad inference (widened)"""
     from veon_b200 import bev_pool as BP
     from veon_b200.view_transformer import LSSViewTransformerRaw
     cfg = S.CONFIGS["small"]
@@ -350,8 +350,7 @@ def test_raw_neck_bf16_features():
         same_bits(da, db)
         assert fa.dtype == BF
         same_bits(fa, fb.to(BF))
-    neck = LSSViewTransformerRaw(cfg.grid_config, cfg.input_size, cfg.downsample, 8, C,
-                                 fuse_ds=True)
+    neck = LSSViewTransformerRaw(cfg.grid_config, cfg.input_size, cfg.downsample, 8, C)
     with torch.no_grad():
         a = neck([feat5] + metas, depth5)
         b = neck([feat5.float()] + metas, depth5)

@@ -148,13 +148,14 @@ def test_no_point_in_grid_matches_reference_dummy():
 
 
 @pytest.mark.parametrize("C", [64, 128])
-def test_raw_neck_fused_downsample_is_bit_identical(C):
-    """SURVEY 8f-1: the no-grad Raw neck pools and max-reduces 2x2x2 in one kernel; the result
-    must equal pool (bit-exact forward) + amax exactly, and the gradient route must be untouched."""
+def test_raw_neck_inference_equals_gradient_route(C):
+    """The no-grad Raw neck pools, then max-reduces 2x2x2 with its own kernel; the result must
+    equal the gradient route's (the one-node pool + maximum) bit for bit, and that route must still
+    give a gradient."""
     from veon_b200.view_transformer import LSSViewTransformerRaw
     cfg = S.CONFIGS["small"]
     B = 2
-    neck = LSSViewTransformerRaw(cfg.grid_config, cfg.input_size, cfg.downsample, 8, C, fuse_ds=True)
+    neck = LSSViewTransformerRaw(cfg.grid_config, cfg.input_size, cfg.downsample, 8, C)
     img, metas, depth, feat = inputs(cfg, B, C, seed=4)
     H, W = cfg.feat_hw
     feat5 = feat.view(B, cfg.n_cams, C, H, W)
@@ -165,7 +166,7 @@ def test_raw_neck_fused_downsample_is_bit_identical(C):
         fused = neck([feat5] + metas, depth5)
     used = BP.kernel_timings_ms()
     BP.enable_kernel_timing(False)
-    assert "pool_ds_fwd" in used and "pool_fwd" not in used      # the fused kernel really ran
+    assert {"pool_fwd", "maxdown_fwd"} <= set(used), used
     assert fused.shape == (B, C, 8, 100, 100)
     f = feat5.detach().clone().requires_grad_()                   # gradient wanted -> plain route
     plain = neck([f] + metas, depth5)

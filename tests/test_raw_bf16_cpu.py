@@ -36,8 +36,8 @@ def test_new_entries_are_declared_bound_and_take_the_twins_arguments():
     for name, twin in TWINS.items():
         assert name in declared and name in _lib.EXPORTED_SYMBOLS and hasattr(lib, name), name
         assert _lib._SIGNATURES[name] == _lib._SIGNATURES[twin], name
-    assert re.search(r"#define\s+VEON_ABI_VERSION\s+10\b", header)
-    assert lib.veon_abi_version() == 10
+    assert re.search(r"#define\s+VEON_ABI_VERSION\s+11\b", header)
+    assert lib.veon_abi_version() == 11
 
 
 @pytest.mark.parametrize("suffix", ["", "_bf16"])

@@ -200,14 +200,13 @@ def test_raw_neck_bf16_training_channels_last(feat_dtype):
 @pytest.mark.parametrize("feat_dtype", [torch.float32, BF])
 def test_raw_neck_bf16_inference(fmt, feat_dtype):
     feat5, depth5, metas, _ = _small_inputs(feat_dtype)
-    for fuse_ds in (False, True):                 # the bfloat16 route replaces fuse_ds
-        used, out = _check_inference(fmt, 64, feat5, depth5, metas, fuse_ds=fuse_ds)
-        sfx = "_bf16feat" if feat_dtype == BF else ""
-        cl = "_cl" if fmt is CL else ""
-        assert _is_cl_view(out) if fmt is CL else out.is_contiguous()
-        assert {f"pool_fwd{cl}_bf16{sfx}", f"maxdown{cl}_fwd_bf16"} <= used, used
-        # no float32 full-resolution volume
-        assert not used & {f"pool_fwd{cl}{sfx}", f"maxdown{cl}_fwd", "pool_ds_fwd"}, used
+    used, out = _check_inference(fmt, 64, feat5, depth5, metas)
+    sfx = "_bf16feat" if feat_dtype == BF else ""
+    cl = "_cl" if fmt is CL else ""
+    assert _is_cl_view(out) if fmt is CL else out.is_contiguous()
+    assert {f"pool_fwd{cl}_bf16{sfx}", f"maxdown{cl}_fwd_bf16"} <= used, used
+    # no float32 full-resolution volume
+    assert not used & {f"pool_fwd{cl}{sfx}", f"maxdown{cl}_fwd"}, used
 
 
 def test_raw_neck_bf16_fallbacks_are_the_float32_route_cast():

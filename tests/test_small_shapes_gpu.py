@@ -15,10 +15,11 @@ def test_small_and_ragged_shapes(capsys):
     assert "ALL OK" in capsys.readouterr().out
 
 
-def test_streaming_forward_kernel_is_bit_exact_at_every_width():
-    """tools/fwd_check.py pushes C = 64 ... 768 through the two-role streaming kernel (wide rows
-    are normally left to the general kernel: it is faster there) and compares the volumes with
-    the general kernel's bit for bit, three calls each (the ring and its barriers are reused)."""
+def test_streaming_forward_kernel_is_bit_exact_at_every_ring_size():
+    """tools/fwd_check.py runs 64-channel volumes of several geometries and batches through the
+    two-role streaming kernel with rings of 2, 4, 8 and 16 slots per SM (slots are reused across
+    generations) and compares them with the general kernel's bit for bit, three calls each (the
+    ring and its barriers are reused)."""
     import subprocess
     import sys
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "fwd_check.py"), "check"],

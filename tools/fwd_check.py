@@ -1,4 +1,5 @@
-"""Forward pooling: streaming two-role kernel vs the general kernel (bit-exact) + timings.
+"""Forward pooling: streaming two-role kernel vs the general kernel (bit-exact) + timings, at
+C = 64 (the only width the streaming kernel takes) and over ring sizes of 2 ... 16 slots per SM.
     python tools/fwd_check.py [check] [time]
 Run under `timeout`: the streaming kernel spins on flags, a bug there hangs instead of failing."""
 import sys
@@ -11,6 +12,8 @@ sys.path.insert(0, ".")
 from veon_b200 import _lib, bev_pool as BP, synthetic as S  # noqa: E402
 if os.environ.get("VEON_LIB"):          # an experimental build of tools/build_variant.sh
     _lib.LIB_PATH = os.environ["VEON_LIB"]
+
+RING_SLOTS = (2, 4, 8, 16)              # ring slots per SM (the library's default is 8)
 
 
 def setup(cfg_name, B, C, seed=0):
@@ -25,20 +28,34 @@ def setup(cfg_name, B, C, seed=0):
     return prep, depth, feat, (B, C, 16, 200, 200)
 
 
-def general(prep, depth, feat, shape, out=None):
+def ring(ns):
+    """A streaming-forward workspace of `ns` slots (512 rows x 64 channels) per SM."""
+    sms = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+    return torch.empty(sms * ns * 512 * 64 * 4, dtype=torch.uint8, device="cuda")
+
+
+def planar(prep, depth, feat, shape, ws=None, out=None):
+    """veon_bev_pool_v2_fwd_planar: without a workspace the general kernel; with the whole plan and
+    a workspace (C = 64) the streaming kernel, its ring sized by the workspace."""
     lib = _lib.load()
     B, C = shape[0], shape[1]
     V = 640000
     if out is None:
         out = torch.full(shape, float("nan"), device="cuda")
     p = prep.plan
+    stream = ws is not None
     rc = lib.veon_bev_pool_v2_fwd_planar(
         BP._ptr(depth), BP._ptr(feat), BP._ptr(prep.ranks_depth), BP._ptr(prep.ranks_feat),
-        BP._ptr(prep.ranks_bev), BP._ptr(p.tile_start), None, None, BP._ptr(p.tile_heavy),
-        p.tile_heavy.numel(), B, C, V, feat.numel() // C, BP._ptr(out), None, 0,
-        BP._stream_ptr(depth.device))
+        BP._ptr(prep.ranks_bev), BP._ptr(p.tile_start), BP._ptr(p.tile_istart) if stream else None,
+        BP._ptr(p.tile_occ) if stream else None, BP._ptr(p.tile_heavy), p.tile_heavy.numel(), B, C,
+        V, feat.numel() // C, BP._ptr(out), BP._ptr(ws) if stream else None,
+        ws.numel() if stream else 0, BP._stream_ptr(depth.device))
     assert rc == 0, rc
     return out
+
+
+def general(prep, depth, feat, shape, out=None):
+    return planar(prep, depth, feat, shape, out=out)
 
 
 def ev_ms(fn, n=20, warm=3):
@@ -56,48 +73,43 @@ def ev_ms(fn, n=20, warm=3):
 
 def main():
     what = sys.argv[1:] or ["check", "time"]
-    import ctypes
-    ctypes.CDLL(_lib.LIB_PATH).veon_internal_fwd_stream_force(1)   # wide rows too
     if "check" in what:
-        for cfg, B, C in (("C1", 1, 64), ("C1", 2, 64), ("small", 3, 128), ("C1", 1, 256),
-                          ("C3", 1, 512), ("C1", 1, 768), ("C2", 8, 64)):
-            prep, depth, feat, shape = setup(cfg, B, C)
-            t0 = time.time()
-            a = BP._fwd_planar(depth, feat, prep.ranks_depth, prep.ranks_feat, prep.ranks_bev,
-                               prep.plan, B, C, 640000, shape)
-            torch.cuda.synchronize()
+        for cfg, B in (("C1", 1), ("C1", 2), ("C1", 4), ("small", 3), ("C3", 1), ("C3", 2),
+                       ("C2", 8)):
+            prep, depth, feat, shape = setup(cfg, B, 64)
             b = general(prep, depth, feat, shape)
-            torch.cuda.synchronize()
-            same = torch.equal(a, b)
-            print(f"check {cfg} B={B} C={C}: equal={same} ({time.time() - t0:.2f}s)", flush=True)
-            if not same:
-                d = (a != b) | (a.isnan() != b.isnan())
-                idx = d.nonzero()
-                print("  mismatches:", int(d.sum()), "first:", idx[:5].tolist())
-            # twice more: the ring / control block are reused
-            for _ in range(2):
-                a2 = BP._fwd_planar(depth, feat, prep.ranks_depth, prep.ranks_feat,
-                                    prep.ranks_bev, prep.plan, B, C, 640000, shape)
-                assert torch.equal(a2, b) == same
-            del a, b, prep, depth, feat
+            for ns in RING_SLOTS:
+                t0 = time.time()
+                ws = ring(ns)
+                a = planar(prep, depth, feat, shape, ws)
+                torch.cuda.synchronize()
+                same = torch.equal(a, b)
+                print(f"check {cfg} B={B} C=64 ring={ns} slots/SM: equal={same} "
+                      f"({time.time() - t0:.2f}s)", flush=True)
+                if not same:
+                    d = (a != b) | (a.isnan() != b.isnan())
+                    idx = d.nonzero()
+                    print("  mismatches:", int(d.sum()), "first:", idx[:5].tolist())
+                # twice more: the ring and its barriers are reused
+                for _ in range(2):
+                    assert torch.equal(planar(prep, depth, feat, shape, ws), b) == same
+                del a, ws
+            del b, prep, depth, feat
     if "time" in what:
-        for cfg, B, C in (("C2", 8, 64), ("C3", 2, 512), ("C3", 4, 256), ("C3", 8, 128)):
-            prep, depth, feat, shape = setup(cfg, B, C)
+        for cfg, B in (("C2", 8), ("C3", 4)):
+            prep, depth, feat, shape = setup(cfg, B, 64)
             scratch = torch.empty(shape, device="cuda")
             tg = ev_ms(lambda: general(prep, depth, feat, shape, scratch), n=10)
-            del scratch
-            line = f"time {cfg} B={B} C={C}: general {tg * 1e3:.1f} us"
-            slot = 512 * min(C, 128) * 4
-            for ns in (4, 8, 16) if C <= 512 else (8, 16):
-                BP.FWD_RING_BYTES = 148 * ns * slot
-                ts = ev_ms(lambda: BP._fwd_planar(depth, feat, prep.ranks_depth, prep.ranks_feat,
-                                                  prep.ranks_bev, prep.plan, B, C, 640000, shape), n=10)
+            line = f"time {cfg} B={B} C=64: general {tg * 1e3:.1f} us"
+            for ns in RING_SLOTS:
+                ws = ring(ns)
+                ts = ev_ms(lambda: planar(prep, depth, feat, shape, ws, scratch), n=10)
                 line += f" | {ns} slots/SM: {ts * 1e3:.1f} us"
-            BP.FWD_RING_BYTES = None
-            gb = 4.0 * 640000 * C * B / 1e9
+                del ws
+            gb = 4.0 * 640000 * 64 * B / 1e9
             line += f"   (volume {gb:.2f} GB)"
             print(line, flush=True)
-            del prep, depth, feat
+            del scratch, prep, depth, feat
 
 
 if __name__ == "__main__":

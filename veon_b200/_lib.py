@@ -50,9 +50,6 @@ _SIGNATURES = {
     "veon_maxdown2_bwd": (c_int, [_P, _P, _P, c_int64, c_int, c_int, c_int, _P, _P]),
     "veon_maxdown2_cl_fwd": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     "veon_maxdown2_cl_bwd": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
-    "veon_prepare_v2_voxel_start_offset": (c_size_t, [c_int, c_int, c_int, c_int, c_int, _P]),
-    "veon_bev_pool_v2_ds_fwd": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
-                                        c_int64, _P, _P]),
     "veon_pool_heavy_list_ints": (c_int64, [c_int64, c_int64]),
     "veon_prepare_v2": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P,
                                 _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t, _P]),

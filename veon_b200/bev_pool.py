@@ -130,19 +130,18 @@ def lidar_coor(frustum, sensor2ego, cam2imgs, post_rots, post_trans, bda):
 
 class PoolPlan:
     """By-products of the index preparation used by the planar kernels."""
-    __slots__ = ("__weakref__", "tile_start", "tile_istart", "tile_occ", "tile_heavy", "voxel_start",
+    __slots__ = ("__weakref__", "tile_start", "tile_istart", "tile_occ", "tile_heavy",
                  "point_interval", "dims", "V",
                  "flags", "_n_intervals", "_n_points", "counts_dev", "counts_host",
                  "counts_event", "keepalive", "sync_free")
 
-    def __init__(self, tiles, heavy, point_interval, dims, V, flags=0, voxel_start=None,
+    def __init__(self, tiles, heavy, point_interval, dims, V, flags=0,
                  counts=(None, None, None), n_points=None, n_intervals=None):
         """tiles: the [3, n_tiles + 1] start / interval-start / occupancy table; counts: the
         (device, pinned host, event) of counts still in flight, else n_points / n_intervals."""
         self.tile_start, self.tile_istart, self.tile_occ = tiles[0], tiles[1], tiles[2]
         self.tile_heavy = heavy
         self.point_interval = point_interval
-        self.voxel_start = voxel_start
         self.dims, self.V, self.flags = dims, V, flags
         self.counts_dev, self.counts_host, self.counts_event = counts
         self._n_points, self._n_intervals = n_points, n_intervals
@@ -324,10 +323,9 @@ def _prepare(coor, calib, dims, dev, grid_lower_bound, grid_interval, grid_size,
         if len(_GEOMETRY_CACHE) > 64:
             _GEOMETRY_CACHE.clear()
         geo = (_lib.float3(lower), _lib.float3(interval), c_size, V, ws_bytes, n_tiles,
-               lib.veon_pool_heavy_list_ints(P, n_tiles),
-               lib.veon_prepare_v2_voxel_start_offset(B, N, D, H, W, c_size))
+               lib.veon_pool_heavy_list_ints(P, n_tiles))
         _GEOMETRY_CACHE[key] = geo
-    c_lower, c_interval, c_size, V, ws_bytes, n_tiles, nh, vs_off = geo
+    c_lower, c_interval, c_size, V, ws_bytes, n_tiles, nh = geo
     with torch.cuda.device(dev):
         # one allocation for every int32 output + the kernel workspace (fewer allocator
         # round-trips per call); the pieces below are views of it
@@ -374,11 +372,8 @@ def _prepare(coor, calib, dims, dev, grid_lower_bound, grid_interval, grid_size,
         _lib.check(rc, "veon_prepare_v2")
         ev = torch.cuda.Event()
         ev.record(launch_on)
-    # first point of every voxel: lives in the preparation workspace (kept alive by this view)
-    voxel_start = (ws[vs_off // 4: vs_off // 4 + B * V + 1]
-                   if B * V < (1 << 24) and vs_off % 4 == 0 else None)
     plan = PoolPlan(tiles, heavy, point_interval if backward_tables else None, (B, N, D, H, W), V,
-                    voxel_start=voxel_start, counts=(counts, counts_host, ev))
+                    counts=(counts, counts_host, ev))
     _COUNTS_RING[dev.index][1][slot] = (ev, weakref.ref(plan))
     out = PreparedRanks()
     out.ranks_bev, out.ranks_depth, out.ranks_feat = ranks[0], ranks[1], ranks[2]
@@ -435,35 +430,6 @@ def _plan_for(rd, rf, rb, ist, iln, dims, V):
                         n_points=rd.numel(), n_intervals=ist.numel())
     _remember_plan(key, plan, (rd, rf, rb, ist, iln))
     return plan
-
-
-def pool_prepared_downsampled(depth, feat, prep, bev_feat_shape):
-    """bev_pool_v2 fused with the neck's 2x2x2 max-downsample (view_transformer_raw.py:549-553),
-    forward only: returns [B, C, Z/2, Y/2, X/2] without materialising the full volume, or None
-    when the shape is outside what the fused kernel takes (the caller then pools and reduces).
-
-    depth [B,N,D,H,W]; feat [B,N,H,W,C] (a permuted view of channels-first maps is fine);
-    prep from `prepare_ranks` (its workspace holds the per-voxel point prefix)."""
-    B, Z, Y, X, C = (int(v) for v in bev_feat_shape)
-    vs = prep.plan.voxel_start
-    if vs is None or (Z | Y | X) & 1 or C % 64 != 0:
-        return None
-    _require_cuda(depth, feat)
-    lib = _lib.load()
-    dev = feat.device
-    depth = depth.detach().contiguous().float()
-    feat = _feat_rows(feat.detach())[0].float()     # the fused kernel reads float32 rows
-    with torch.cuda.device(dev):
-        out = torch.empty((B, C, Z // 2, Y // 2, X // 2), dtype=torch.float32, device=dev)
-        with _timed("pool_ds_fwd", dev):
-            rc = lib.veon_bev_pool_v2_ds_fwd(
-                _ptr(depth), _ptr(feat), _ptr(prep.ranks_depth), _ptr(prep.ranks_feat),
-                _ptr(prep.ranks_bev), _ptr(vs), B, C, Z, Y, X, feat.numel() // C, _ptr(out),
-                _stream_ptr(dev))
-    if rc == -4:        # VEON_E_UNSUPPORTED: shape outside the fused kernel
-        return None
-    _lib.check(rc, "veon_bev_pool_v2_ds_fwd")
-    return out
 
 
 def two_hot_depth(depths, depth_cfg, D, gamma=4.0, downsample=0):
@@ -686,18 +652,16 @@ def _feat_grad_back(feat_grad, transposed):
     return _transpose_batched(feat_grad, B * N, H * W, C, (B, N, C, H, W)).permute(0, 1, 3, 4, 2)
 
 
-# Scratch of the streaming forward (control block + the L2-resident ring of compact rows):
-# one buffer per (device, stream) -- calls on one stream are ordered, calls on different
-# streams may overlap and must not share it.  FWD_RING_BYTES: None = the library's default size
-# (tools/fwd_check.py sweeps it: the buffer size decides how many ring slots an SM gets).
+# Scratch of the streaming forward (the L2-resident ring of compact rows): one buffer per
+# (device, stream) -- calls on one stream are ordered, calls on different streams may overlap and
+# must not share it.  None where the library asks for none (every width but C == 64).
 _FWD_WS = {}
-FWD_RING_BYTES = None
 
 
 def _fwd_workspace(lib, dev, B, C, V):
     need = lib.veon_bev_pool_v2_fwd_workspace_bytes(B, C, V)
-    if FWD_RING_BYTES is not None:
-        need = int(FWD_RING_BYTES)
+    if need == 0:
+        return None
     key = (dev.index, torch.cuda.current_stream(dev).cuda_stream)
     ws = _FWD_WS.get(key)
     if ws is None or ws.numel() != need:
@@ -733,8 +697,8 @@ def _fwd_planar(depth, feat, rd, rf, rb, plan, B, C, V, shape5, channels_last=Fa
                     _ptr(depth), _ptr(feat), _ptr(rd), _ptr(rf), _ptr(rb), _ptr(plan.tile_start),
                     _ptr(plan.tile_istart), _ptr(plan.tile_occ),
                     _ptr(plan.tile_heavy), plan.tile_heavy.numel(),
-                    B, C, V, feat.numel() // C, _ptr(out), None if bf16 else _ptr(ws),
-                    0 if bf16 else ws.numel(), _stream_ptr(dev))
+                    B, C, V, feat.numel() // C, _ptr(out), None if ws is None else _ptr(ws),
+                    0 if ws is None else ws.numel(), _stream_ptr(dev))
     if bf16feat and rc == _lib.E_UNSUPPORTED:
         # a 64-channel float32 channels-first volume: the streaming kernel, on widened rows
         return _fwd_planar(depth, feat.float(), rd, rf, rb, plan, B, C, V, shape5, channels_last,

@@ -21,13 +21,12 @@
 //
 // Kernels in this file:
 //   k_pool_fwd         the warp-per-tile kernel above: the general route (any C, ragged volumes,
-//                      no workspace).  Aligned volumes with C % 64 == 0 take the two-role
+//                      no workspace).  Aligned volumes with C == 64 take the two-role
 //                      streaming kernel of pool_fwd_stream.cu instead (see there).
 //   k_pool_fwd_heavy   a CTA per heavy tile (rows staged by cp.async), queued behind the main grid
 //   k_pool_fwd_narrow  C <= 32 (C % 4 == 0): a LANE per voxel instead of a lane per channel, all
 //                      channels of the voxel in registers, same fma order; heavy grid first
-//   k_pool_ds_fwd      opt-in: pooling fused with the neck's 2x2x2 max-downsample
-// The first three also write channels-last volumes out[B,Z,Y,X,C] (template flag CL,
+// All three also write channels-last volumes out[B,Z,Y,X,C] (template flag CL,
 // veon_bev_pool_v2_fwd_planar_cl): same sums, rows instead of channel planes.
 #include <type_traits>
 
@@ -457,11 +456,6 @@ k_pool_fwd(const float* __restrict__ depth, const TF* __restrict__ feat,
 constexpr int kHeavyThreads = 256;
 constexpr int kHeavyChunk = 128;  // points per round; one index record per thread < 128
 
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
-  const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
-}
-
 // Fused lift + classify (veon_lift_classify_fwd): the pooled channels are
 // [gate 0, gate 1, logit 0 .. Q-1, padding] and a tile ends as 32 labels instead of C planes.
 struct ClsArgs {
@@ -637,189 +631,6 @@ k_pool_fwd_heavy(const float* __restrict__ depth, const TF* __restrict__ feat,
   if (join) pdl_wait();
 }
 
-
-// ---- fused pooling + 2x2x2 max-downsample, forward (SURVEY 8f-1) ------------------------
-// VEON's neck reduces the pooled volume 8x right away (view_transformer_raw.py:549-553:
-// rearrange to [..., (dz dh dw)] + torch.max(dim=-1).values).  Here the full-resolution volume is never written: a CTA
-// takes one output row (b, z/2, y/2), pools its four input x-rows one after the other into a
-// shared [c][X] tile -- points of a row are one contiguous slice of the sorted rank arrays,
-// found through the per-voxel prefix `voxel_start` the preparation leaves in its workspace;
-// rows staged by cp.async, rank-ordered fma chains as in k_pool_fwd_heavy -- and folds each
-// into a running [c][X/2] maximum.  Sums are the same bits as the unfused kernel's and max is
-// exact, so the result equals pool + that reduction bit for bit.  Forward only (inference path).
-__device__ __forceinline__ float ds_max(float a, float b) { return (b > a || b != b) ? b : a; }
-constexpr int kDsThreads = 256;
-constexpr int kDsRound = 96;   // points staged per round (thread per point)
-
-template <int KCH>
-__global__ void __launch_bounds__(kDsThreads)
-k_pool_ds_fwd(const float* __restrict__ depth, const float* __restrict__ feat,
-              const int32_t* __restrict__ ranks_depth, const int32_t* __restrict__ ranks_feat,
-              const int32_t* __restrict__ ranks_bev, const int32_t* __restrict__ voxel_start,
-              uint32_t n_items, uint32_t n_chunks, int Z, int Y, int Xfull, int xsplit,
-              int C, float* __restrict__ out) {
-  constexpr int CC = 32 * KCH;
-  constexpr int kSegs = CC / 4;
-  const int X = Xfull / xsplit;              // voxels of the x-run one item covers
-  const int Xp = (X + 3) / 4 * 4 + 4;        // pitch of the full-resolution row tile
-  const int Xh = X / 2, Xhp = Xh + 1;        // pitch of the running maximum
-  extern __shared__ __align__(16) float dsm[];
-  float* rows = dsm;                                                // [kDsRound][CC]
-  float* stage = rows + kDsRound * CC;                              // [CC][Xp]
-  float* outb = stage + CC * Xp;                                    // [CC][Xhp]
-  float* dep = outb + CC * Xhp;                                     // [kDsRound]
-  uint32_t* off = reinterpret_cast<uint32_t*>(dep + kDsRound);      // [kDsRound]
-  int32_t* bounds = reinterpret_cast<int32_t*>(off + kDsRound);     // [2][start Xp | end Xp]
-  int32_t* rs = bounds + 4 * Xp;                                    // [4] first point of a row
-  int32_t* rn = rs + 4;                                             // [4] points in the row
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int Zh = Z / 2, Yh = Y / 2;
-  const int64_t V = (int64_t)Z * Y * Xfull;
-
-  struct Rec { int32_t rb, rp, rf, rd; float d; };
-  struct Rnd { int sub, base; };
-  auto first_round = [&]() -> Rnd {
-    for (int q = 0; q < 4; ++q) if (rn[q] > 0) return Rnd{q, 0};
-    return Rnd{4, 0};
-  };
-  auto next_round = [&](Rnd r) -> Rnd {
-    if (r.base + kDsRound < rn[r.sub]) return Rnd{r.sub, r.base + kDsRound};
-    for (int q = r.sub + 1; q < 4; ++q) if (rn[q] > 0) return Rnd{q, 0};
-    return Rnd{4, 0};
-  };
-  auto stage_a = [&](Rnd r, Rec& c) {
-    c.rb = -1;
-    c.rp = -1;
-    const int q = r.base + tid;
-    if (tid < kDsRound && q < rn[r.sub]) {
-      const int32_t i = rs[r.sub] + q;
-      c.rb = __ldg(ranks_bev + i);
-      c.rf = __ldg(ranks_feat + i);
-      c.rd = __ldg(ranks_depth + i);
-      if (q > 0) c.rp = __ldg(ranks_bev + i - 1);
-    }
-  };
-  auto stage_b = [&](Rec& c) {
-    c.d = 0.f;
-    if (c.rb >= 0) c.d = __ldg(depth + c.rd);
-  };
-
-  for (uint32_t item = blockIdx.x; item < n_items; item += gridDim.x) {
-    const uint32_t piece = item / n_chunks, chunk = item - piece * n_chunks;
-    const uint32_t cell = piece / (uint32_t)xsplit;
-    const int x0 = (int)(piece - cell * (uint32_t)xsplit) * X;   // first input voxel of the run
-    const int yo = (int)(cell % (uint32_t)Yh);
-    const int zo = (int)((cell / (uint32_t)Yh) % (uint32_t)Zh);
-    const int64_t b = cell / ((uint32_t)Yh * (uint32_t)Zh);
-    const int cbase = (int)chunk * CC;
-    __syncthreads();   // previous item fully written out
-    if (tid < 4) {
-      const int64_t g = b * V + ((int64_t)(2 * zo + (tid >> 1)) * Y + 2 * yo + (tid & 1)) * Xfull + x0;
-      const int32_t s0 = __ldg(voxel_start + g);
-      rs[tid] = s0;
-      rn[tid] = __ldg(voxel_start + g + X) - s0;
-    }
-    for (int i = tid; i < 4 * Xp; i += kDsThreads) bounds[i] = 0;
-    __syncthreads();
-
-    Rnd cur = first_round();
-    Rec rec;
-    rec.rb = -1;
-    if (cur.sub < 4) {
-      stage_a(cur, rec);
-      stage_b(rec);
-    }
-    int parity = 0;
-    for (int sub = 0; sub < 4; ++sub) {
-      if (rn[sub] == 0) {   // empty input row: contributes zeros
-        for (int c = warp; c < CC; c += kDsThreads / 32)
-          for (int xo = lane; xo < Xh; xo += 32)
-            outb[c * Xhp + xo] = sub == 0 ? 0.f : ds_max(outb[c * Xhp + xo], 0.f);
-        continue;
-      }
-      const int32_t g_row = (int32_t)(b * V + ((int64_t)(2 * zo + (sub >> 1)) * Y + 2 * yo + (sub & 1)) * Xfull + x0);
-      {
-        float4* s4 = reinterpret_cast<float4*>(stage);
-        for (int i = tid; i < CC * Xp / 4; i += kDsThreads) s4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-      while (cur.sub == sub) {
-        const int cnt = min(kDsRound, rn[sub] - cur.base);
-        int32_t* cstart = bounds + parity * 2 * Xp;
-        int32_t* cend = cstart + Xp;
-        if (rec.rb >= 0) {   // publish the round's records and voxel [start, end) ranges
-          const int vox = rec.rb - g_row;
-          off[tid] = ((uint32_t)rec.rf * (uint32_t)C + chunk * CC) * 4u;
-          dep[tid] = rec.d;
-          const bool starts = (tid == 0) || (rec.rb != rec.rp);
-          if (starts) cstart[vox] = tid;
-          if (tid > 0 && rec.rb != rec.rp) cend[rec.rp - g_row] = tid;
-          if (tid == cnt - 1) cend[vox] = cnt;
-        }
-        const Rnd nx = next_round(cur);
-        __syncthreads();
-        {
-          const char* fbase = reinterpret_cast<const char*>(feat);
-#pragma unroll
-          for (int i = 0; i < kDsRound * kSegs / kDsThreads; ++i) {
-            const int idx = tid + kDsThreads * i;
-            const int r = idx / kSegs, seg = (idx % kSegs) * 4;
-            if (r < cnt) cp_async16(rows + r * CC + seg, fbase + off[r] + seg * 4);
-          }
-          cp_async_commit();
-        }
-        Rec nrec;
-        nrec.rb = -1;
-        if (nx.sub < 4) stage_a(nx, nrec);
-        for (int i = tid; i < 2 * Xp; i += kDsThreads) bounds[(parity ^ 1) * 2 * Xp + i] = 0;
-        cp_async_wait_all();
-        __syncthreads();
-        if (nx.sub < 4) stage_b(nrec);
-        // fma chains: voxel block k (32 voxels) belongs to warp k % 8; lanes = channels
-        for (int vb = warp * 32; vb < X; vb += kDsThreads) {
-          const int vv = vb + lane;
-          const int a_l = vv < X ? cstart[vv] : 0, e_l = vv < X ? cend[vv] : 0;
-          uint32_t m = __ballot_sync(0xffffffffu, e_l > a_l);
-          while (m) {
-            const int v = __ffs(m) - 1;
-            m &= m - 1;
-            const int a = __shfl_sync(0xffffffffu, a_l, v), e = __shfl_sync(0xffffffffu, e_l, v);
-            float* sp = stage + lane * Xp + vb + v;
-            float acc[KCH];
-#pragma unroll
-            for (int c = 0; c < KCH; ++c) acc[c] = sp[32 * c * Xp];
-#pragma unroll 4
-            for (int j = a; j < e; ++j) {
-              const float dj = dep[j];
-#pragma unroll
-              for (int c = 0; c < KCH; ++c) acc[c] = fmaf(rows[j * CC + lane + 32 * c], dj, acc[c]);
-            }
-#pragma unroll
-            for (int c = 0; c < KCH; ++c) sp[32 * c * Xp] = acc[c];
-          }
-        }
-        parity ^= 1;
-        rec = nrec;
-        cur = nx;
-        __syncthreads();
-      }
-      // fold the finished row into the running maximum (pairs along x)
-      // (warp w: channels w, w+8, ...; lanes along x -- the same element-to-thread map in
-      //  every fold and in the write-out, so outb needs no barrier of its own)
-      for (int c = warp; c < CC; c += kDsThreads / 32)
-        for (int xo = lane; xo < Xh; xo += 32) {
-          const float2 p2 = *reinterpret_cast<const float2*>(stage + c * Xp + 2 * xo);
-          const float m2 = ds_max(p2.x, p2.y);
-          outb[c * Xhp + xo] = sub == 0 ? m2 : ds_max(outb[c * Xhp + xo], m2);
-        }
-      __syncthreads();
-    }
-    // out[b, cbase + c, zo, yo, :]
-    for (int c = warp; c < CC; c += kDsThreads / 32) {
-      float* o = out + (((b * C + cbase + c) * Zh + zo) * Yh + yo) * (int64_t)(Xfull / 2) + x0 / 2;
-      for (int xo = lane; xo < Xh; xo += 32) o[xo] = outb[c * Xhp + xo];
-    }
-  }
-}
 
 // ---- narrow rows (C <= 32): lane = voxel ---------------------------------------------------
 // With few channels a lane-per-channel warp leaves lanes idle and pays one row-load latency
@@ -1095,10 +906,8 @@ int launch_heavy_behind(const float* depth, const float* feat, const int32_t* rd
                         float* out, int min_points, cudaStream_t stream) {
   if (!heavy || heavy_ints < 2 || (C & 3) != 0 || ((uintptr_t)feat & 15) != 0)
     return VEON_E_BADARG;
-  return C <= 32 ? launch_heavy<1>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C, V,
-                                   out, true, min_points, stream)
-                 : launch_heavy<2>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C, V,
-                                   out, true, min_points, stream);
+  return launch_heavy<2>(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C, V, out,
+                         true, min_points, stream);
 }
 
 // general route: k_pool_fwd over every (tile, channel chunk), the heavy tiles queued behind it
@@ -1211,14 +1020,10 @@ static int launch_fwd_narrow(const float* depth, const TF* feat, const int32_t* 
 
 using namespace veon;
 
-// Not part of the ABI in include/veon_lift.h: lets tools/fwd_check.py push wide rows through the
-// streaming kernel for its parity sweep and timing comparison.
-extern "C" void veon_internal_fwd_stream_force(int on) { stream_force = on != 0; }
-
 extern "C" size_t veon_bev_pool_v2_fwd_workspace_bytes(int B, int C, int64_t V) {
   if (B <= 0 || C <= 0 || V <= 0) return 0;
-  // the ring of compact rows (a few slots per SM; only their occupied prefix is ever touched,
-  // so the part that lives in L2 is a fraction of this)
+  // the streaming kernel's ring of compact rows (a few slots per SM; only their occupied prefix
+  // is ever touched, so the part that lives in L2 is a fraction of this); 0 unless C == 64
   return fwd_stream_workspace_bytes(C);
 }
 
@@ -1257,7 +1062,7 @@ static int fwd_planar(const float* depth, const TF* feat, const int32_t* ranks_d
 #undef VEON_NARROW_CASE
     }
   }
-  // aligned volumes, whole 64-channel chunks: the two-role streaming kernel.  It has no bf16-row
+  // aligned volumes, 64-channel rows: the two-role streaming kernel.  It has no bf16-row
   // form: where it would run on float rows, bf16 rows are refused (VEON_E_UNSUPPORTED), and the
   // caller widens them into a fresh -- aligned -- float copy and calls the float entry.
   if constexpr (!CL && std::is_same<T, float>::value && !std::is_same<TF, float>::value) {
@@ -1432,47 +1237,4 @@ extern "C" int veon_lift_classify_fwd(const float* depth, const float* pix,
   }
 #undef VEON_CLS_CASE
   return VEON_E_UNSUPPORTED;
-}
-
-extern "C" int veon_bev_pool_v2_ds_fwd(const float* depth, const float* feat,
-                                       const int32_t* ranks_depth, const int32_t* ranks_feat,
-                                       const int32_t* ranks_bev, const int32_t* voxel_start,
-                                       int B, int C, int Z, int Y, int X, int64_t n_feat_rows,
-                                       float* out, void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  if (!depth || !feat || !ranks_depth || !ranks_feat || !ranks_bev || !voxel_start || !out ||
-      B <= 0 || C <= 0 || Z <= 0 || Y <= 0 || X <= 0 || n_feat_rows <= 0)
-    return VEON_E_BADARG;
-  constexpr int KCH = 2, CC = 64;
-  // even grid, whole 64-channel chunks, 16-byte feature rows, exact float32 voxel ranks
-  if ((Z | Y | X) & 1 || C % CC != 0 || ((uintptr_t)feat & 15) != 0) return VEON_E_UNSUPPORTED;
-  const int64_t V = (int64_t)Z * Y * X;
-  if ((int64_t)B * V >= (1 << 24) || n_feat_rows * (int64_t)C > 0x3fffffffLL) return VEON_E_RANGE;
-  const int xsplit = 1;   // (halving the x-rows per item was measured slower: per-item overheads)
-  const int Xs = X / xsplit;
-  const int Xp = (Xs + 3) / 4 * 4 + 4, Xhp = Xs / 2 + 1;
-  const size_t smem = sizeof(float) * ((size_t)kDsRound * CC + (size_t)CC * Xp + (size_t)CC * Xhp +
-                                       2 * kDsRound + 4 * (size_t)Xp + 8);
-  if (smem > 220 * 1024) return VEON_E_UNSUPPORTED;
-  static size_t attr_smem[kMaxDevices] = {};
-  const int dev = current_device();
-  if (smem > attr_smem[dev]) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_pool_ds_fwd<KCH>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_smem[dev] = smem;
-  }
-  int per_sm = 1;
-  VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_pool_ds_fwd<KCH>,
-                                                              kDsThreads, smem));
-  if (per_sm < 1) per_sm = 1;
-  const int n_chunks = C / CC;
-  const int64_t n_items = (int64_t)B * (Z / 2) * (Y / 2) * xsplit * n_chunks;
-  if (n_items > 0x7fffffffLL) return VEON_E_RANGE;
-  int64_t blocks = (int64_t)per_sm * sm_count();
-  if (blocks > n_items) blocks = n_items;
-  k_pool_ds_fwd<KCH><<<(unsigned)blocks, kDsThreads, smem, stream>>>(
-      depth, feat, ranks_depth, ranks_feat, ranks_bev, voxel_start, (uint32_t)n_items,
-      (uint32_t)n_chunks, Z, Y, X, xsplit, C, out);
-  VEON_LAUNCH_CHECK();
-  return 0;
 }

@@ -8,7 +8,6 @@ namespace veon {
 bool fwd_stream_supported(int B, int C, int64_t V, const void* feat, const void* out,
                           int64_t n_feat_rows);
 size_t fwd_stream_workspace_bytes(int C);
-extern bool stream_force;
 int launch_fwd_stream(const float* depth, const float* feat, const int32_t* rd, const int32_t* rf,
                       const int32_t* rb, const int32_t* tile_start, const uint32_t* tile_occ,
                       const int32_t* heavy, int64_t heavy_ints, int B, int C, int64_t V,

@@ -15,9 +15,7 @@
 //                     flight, lanes = channels, acc = fma(feat, depth, acc) starting from 0: the
 //                     reference kernel's rounding sequence, so the result stays bit-identical --
 //                     and stores ONE channel-contiguous row per occupied voxel into the CTA's
-//                     ring.  Wide rows are produced in passes of 128 channels from the same index
-//                     records: the index work is done once per point, not once per 64-channel
-//                     chunk.  No tile buffer, no zero fill, no transposition.
+//                     ring.  No tile buffer, no zero fill, no transposition.
 //   role E, 16 warps  Two groups of 8 warps; a group's item is 8 consecutive tiles x a
 //                     64-channel chunk (an aligned 1 KB run of every channel plane).  A warp
 //                     copies its tile's rows out of the ring into shared memory (16-byte
@@ -28,14 +26,17 @@
 //                     reads nothing from DRAM: its only long-latency traffic is the store stream.
 //
 // Work is dealt in ROUNDS of 16 consecutive tiles (round r -> CTA r mod grid: every CTA samples
-// the whole volume, so the point density averages out).  A unit = (round, 128-channel pass) is
-// produced by the 16 A warps of a CTA and consumed by the 16 E warps of the SAME CTA, through one
-// of the CTA's own NS ring slots (512 rows x <=128 channels; rows of the round's tiles packed
-// by the running count of occupied voxels).  All flow control is two shared-memory counters per
+// the whole volume, so the point density averages out).  A round is produced by the 16 A warps
+// of a CTA and consumed by the 16 E warps of the SAME CTA, through one of the CTA's own NS ring
+// slots (512 rows x 64 channels; rows of the round's tiles packed by the running count of
+// occupied voxels).  All flow control is two shared-memory counters per
 // slot (filled by A, drained by E): no global flags, no atomics on global memory, no dependence
 // between CTAs.  The ring (grid x NS slots, only the occupied prefix of a slot is ever touched)
 // is a few tens of MB: its lines are rewritten while still dirty in L2 and never reach DRAM;
 // DRAM sees the inputs once and the volume once.
+//
+// Rows are 64 channels wide, the only width at which this kernel beats k_pool_fwd (pool_fwd.cu);
+// every other width takes that kernel.
 //
 // Tiles at or above the plan's heavy threshold are left to k_pool_fwd_heavy (pool_fwd.cu),
 // which writes them straight into the volume, queued behind this grid.
@@ -47,6 +48,7 @@ namespace veon {
 constexpr int kRoundTiles = 16;         // tiles per round
 constexpr int kAWarps = 16;             // role A warps per CTA: a tile each
 constexpr int kEWarps = 16;             // role E warps per CTA: a tile each, two groups of 8
+constexpr int CU = 64;                  // channels of a row
 constexpr int kEGroup = 8;
 constexpr int kStreamWarps = kAWarps + kEWarps;
 // Registers are re-dealt between the warpgroups at role entry (setmaxnreg).  The pool is what
@@ -100,20 +102,6 @@ __device__ unsigned long long veon_fwd_trace[32 * 8];
 #define VEON_TACC(slotid)
 #endif
 
-template <int VEC> struct VecT;
-template <> struct VecT<2> { using T = float2; };
-template <> struct VecT<4> { using T = float4; };
-
-template <int VEC>
-__device__ __forceinline__ void vec_fma(float (&acc)[VEC], const typename VecT<VEC>::T& f, float d,
-                                        bool first) {
-  const float* fv = reinterpret_cast<const float*>(&f);
-#pragma unroll
-  for (int i = 0; i < VEC; ++i) acc[i] = fmaf(fv[i], d, first ? 0.f : acc[i]);
-}
-
-bool stream_force = false;   // tools only: also take wide rows (veon_fwd_stream_force)
-
 struct FwdStreamParams {
   const float *depth, *feat;
   const int32_t *ranks_depth, *ranks_feat, *ranks_bev;
@@ -124,12 +112,12 @@ struct FwdStreamParams {
   float* out;
   int64_t V;
   uint32_t n_tiles, n_rounds, tiles_per_sample;
-  int C, n_pass, ns_log2;    // n_pass = C / CU passes per round; 2^ns_log2 ring slots per CTA
+  int C, ns_log2;            // 2^ns_log2 ring slots per CTA
 };
 
-// Per ring slot: `full`, an mbarrier on which every tile of a round arrives when its rows of the
-// unit are in the slot (a generation of the slot = one phase; the E warps, which visit every
-// unit in order, wait on it suspended by the hardware, not spinning through the issue slots);
+// Per ring slot: `full`, an mbarrier on which every tile of a round arrives when its rows are in
+// the slot (a generation of the slot = one phase; the E warps, which visit every round in order,
+// wait on it suspended by the hardware, not spinning through the issue slots);
 // and `drained`, a plain counter every E warp bumps when it has copied its rows out.  The
 // way back is a COUNTER, not an mbarrier phase, on purpose: role A claims its tiles
 // dynamically, so a warp may meet a slot it has not touched for several generations, and a
@@ -138,7 +126,7 @@ struct StreamShared {
   uint64_t full[kMaxSlots];
   volatile uint32_t drained[kMaxSlots];   // + 1 per E warp per use of the slot
   uint32_t next_item;   // role A: next (round, tile) of this CTA's sequence to be claimed
-  // what role E needs to know about tile w of the unit in slot s, published by the A warp that
+  // what role E needs to know about tile w of the round in slot s, published by the A warp that
   // produced it (before its arrival on `full`): .x = occupancy mask, .y = first slot row of the
   // tile | kMetaMine when the tile is this kernel's (inside the volume, not heavy)
   uint2 meta[kMaxSlots][kRoundTiles];
@@ -173,22 +161,18 @@ __device__ __forceinline__ int rows_before(int32_t ts, uint32_t occ, int lane, i
 }
 
 // ------------------------------------------------------------------------------------------
-// role A: rows of the occupied voxels -> the CTA's ring.  CU = 32 * VEC channels per pass; a
-// lane owns VEC consecutive channels.
+// role A: rows of the occupied voxels -> the CTA's ring.  A lane owns 2 consecutive channels.
 // The tiles of the CTA's rounds are CLAIMED one by one from a shared counter (three stages
 // ahead, when their index records start to travel), not dealt statically: a warp that draws a
 // 90-point tile simply claims fewer, so a round is not held up by its slowest tile any longer
-// than the ring's slack allows.  A tile's arrival on its unit's `full` barrier is per tile.
+// than the ring's slack allows.  A tile's arrival on its round's `full` barrier is per tile.
 // ------------------------------------------------------------------------------------------
 constexpr int kHdrItem = 33;   // header word: the claimed item (round-in-CTA * 16 + tile-in-round)
 
-template <int VEC>
 __device__ __forceinline__ void role_rows(const FwdStreamParams& p, int32_t* ring_idx,
                                           StreamShared* sh, int lane) {
-  using V = typename VecT<VEC>::T;
-  constexpr int CU = 32 * VEC;
   __builtin_assume(__isShared(ring_idx));   // LDS/STS instead of generic accesses
-  constexpr int U = VEC == 2 ? 12 : 8;   // feature-row pieces in flight per lane (3 / 4 KB per warp)
+  constexpr int U = 12;   // feature-row pieces in flight per lane (3 KB per warp)
   if (blockIdx.x >= p.n_rounds) return;
   const uint32_t my_rounds = (p.n_rounds - blockIdx.x + gridDim.x - 1) / gridDim.x;
   const uint32_t my_items = my_rounds * kRoundTiles;
@@ -263,7 +247,7 @@ __device__ __forceinline__ void role_rows(const FwdStreamParams& p, int32_t* rin
   for (int i = 0; i < kADist; ++i) issue_depth(i);
   cpa_commit(); cpa_wait<0>(); __syncwarp();
 
-  const uint32_t lane_off = (uint32_t)lane * (VEC * 4);
+  const uint32_t lane_off = (uint32_t)lane * 8u;
 
   VEON_T0
   for (uint32_t k = 0;; ++k) {
@@ -287,95 +271,88 @@ __device__ __forceinline__ void role_rows(const FwdStreamParams& p, int32_t* rin
     issue_depth(k + kADist);
     cpa_commit();
 
-    for (int pass = 0; pass < p.n_pass; ++pass) {
-      const uint32_t unit = m * (uint32_t)p.n_pass + pass;
-      const uint32_t slot = unit & ns_mask;
-      const uint32_t gen = unit >> p.ns_log2;
-      // every earlier use of the slot has been read out by all E warps
-      VEON_TACC(1)
-      while (sh->drained[slot] < kEWarps * gen) __nanosleep(256);
-      VEON_TACC(2)
-      if (e0 > s0) {
-        char* const slotb = reinterpret_cast<char*>(cta_ring + (size_t)slot * (kSlotRows * CU));
-        const char* const featb = reinterpret_cast<const char*>(p.feat) + pass * (CU * 4);
-        // byte offset, inside the slot, of this lane's piece of the row being accumulated; the
-        // first point always opens a voxel, so the -1 row is stepped over before any store
-        uint32_t rowoff = (uint32_t)(base_row - 1) * (CU * 4) + lane_off;
-        float acc[VEC];
-#pragma unroll
-        for (int i = 0; i < VEC; ++i) acc[i] = 0.f;
-        for (int32_t base = s0; base < e0; base += 32) {
-          const int cnt = min(32, e0 - base);
-          if (base != s0 || (pass > 0 && e0 - s0 > 32)) {
-            // more than 32 points: the records of every 32-point piece but the prefetched
-            // first one (of the first pass) are fetched synchronously
-            const int32_t i = base + lane;
-            __syncwarp();
-            int32_t rb = -1, rf = 0;
-            float d = 0.f;
-            if (i < e0) {
-              rb = __ldg(p.ranks_bev + i);
-              rf = __ldg(p.ranks_feat + i);
-              d = __ldg(p.depth + __ldg(p.ranks_depth + i));
-            }
-            int32_t up = __shfl_up_sync(0xffffffffu, rb, 1);
-            int32_t* pt = sl + kAHdr + 4 * lane;
-            if (lane == 0) up = base == s0 ? -1 : sl[kAHdr + 4 * 31 + 0];   // last point before
-            __syncwarp();
-            pt[0] = rb;
-            pt[2] = (int32_t)(((uint32_t)rf * row_bytes) | (rb != up ? 1u : 0u));
-            pt[3] = __float_as_int(d);
-            __syncwarp();
+    const uint32_t slot = m & ns_mask;
+    const uint32_t gen = m >> p.ns_log2;
+    // every earlier use of the slot has been read out by all E warps
+    VEON_TACC(1)
+    while (sh->drained[slot] < kEWarps * gen) __nanosleep(256);
+    VEON_TACC(2)
+    if (e0 > s0) {
+      char* const slotb = reinterpret_cast<char*>(cta_ring + (size_t)slot * (kSlotRows * CU));
+      const char* const featb = reinterpret_cast<const char*>(p.feat);
+      // byte offset, inside the slot, of this lane's piece of the row being accumulated; the
+      // first point always opens a voxel, so the -1 row is stepped over before any store
+      uint32_t rowoff = (uint32_t)(base_row - 1) * (CU * 4) + lane_off;
+      float acc[2] = {0.f, 0.f};
+      for (int32_t base = s0; base < e0; base += 32) {
+        const int cnt = min(32, e0 - base);
+        if (base != s0) {
+          // more than 32 points: the records of every 32-point piece but the prefetched
+          // first one are fetched synchronously
+          const int32_t i = base + lane;
+          __syncwarp();
+          int32_t rb = -1, rf = 0;
+          float d = 0.f;
+          if (i < e0) {
+            rb = __ldg(p.ranks_bev + i);
+            rf = __ldg(p.ranks_feat + i);
+            d = __ldg(p.depth + __ldg(p.ranks_depth + i));
           }
-          const int32_t* pts = sl + kAHdr + 2;   // record j: {row offset | first, depth} at pts[4 j]
-          // Branch-free body: loads in groups of four (a group past the last point is skipped
-          // as a whole, warp-uniformly), then one predicated fma chain per point; the running
-          // sum is stored after EVERY point (the last store of a voxel leaves its total), which
-          // costs L2 some repeated row writes and saves the flush branches.
-          for (int j0 = 0; j0 < cnt; j0 += U) {
-            int2 q[U];
-            V f[U];
+          int32_t up = __shfl_up_sync(0xffffffffu, rb, 1);
+          int32_t* pt = sl + kAHdr + 4 * lane;
+          if (lane == 0) up = base == s0 ? -1 : sl[kAHdr + 4 * 31 + 0];   // last point before
+          __syncwarp();
+          pt[0] = rb;
+          pt[2] = (int32_t)(((uint32_t)rf * row_bytes) | (rb != up ? 1u : 0u));
+          pt[3] = __float_as_int(d);
+          __syncwarp();
+        }
+        const int32_t* pts = sl + kAHdr + 2;   // record j: {row offset | first, depth} at pts[4 j]
+        // Branch-free body: loads in groups of four (a group past the last point is skipped
+        // as a whole, warp-uniformly), then one predicated fma chain per point; the running
+        // sum is stored after EVERY point (the last store of a voxel leaves its total), which
+        // costs L2 some repeated row writes and saves the flush branches.
+        for (int j0 = 0; j0 < cnt; j0 += U) {
+          int2 q[U];
+          float2 f[U];
 #pragma unroll
-            for (int gq = 0; gq < U; gq += 4) {
-              if (j0 + gq < cnt) {
+          for (int gq = 0; gq < U; gq += 4) {
+            if (j0 + gq < cnt) {
 #pragma unroll
-                for (int uu = 0; uu < 4; ++uu) {
-                  const int u = gq + uu;
-                  q[u] = *reinterpret_cast<const int2*>(pts + 4 * min(j0 + u, cnt - 1));
-                  f[u] = __ldg(reinterpret_cast<const V*>(featb + (((uint32_t)q[u].x & ~1u) + lane_off)));
-                }
+              for (int uu = 0; uu < 4; ++uu) {
+                const int u = gq + uu;
+                q[u] = *reinterpret_cast<const int2*>(pts + 4 * min(j0 + u, cnt - 1));
+                f[u] = __ldg(reinterpret_cast<const float2*>(featb + (((uint32_t)q[u].x & ~1u) + lane_off)));
               }
             }
+          }
 #pragma unroll
-            for (int gq = 0; gq < U; gq += 4) {
-              if (j0 + gq < cnt) {
+          for (int gq = 0; gq < U; gq += 4) {
+            if (j0 + gq < cnt) {
 #pragma unroll
-                for (int uu = 0; uu < 4; ++uu) {
-                  const int u = gq + uu;
-                  const bool ok = j0 + u < cnt;
-                  const bool first = q[u].x & 1;
-                  const float dj = __int_as_float(q[u].y);
-                  rowoff += (ok && first) ? (uint32_t)(CU * 4) : 0u;
-                  const float* fv = reinterpret_cast<const float*>(&f[u]);
-#pragma unroll
-                  for (int i = 0; i < VEC; ++i)
-                    acc[i] = ok ? fmaf(fv[i], dj, first ? 0.f : acc[i]) : acc[i];
-                  if (ok) *reinterpret_cast<V*>(slotb + rowoff) = *reinterpret_cast<const V*>(acc);
-                }
+              for (int uu = 0; uu < 4; ++uu) {
+                const int u = gq + uu;
+                const bool ok = j0 + u < cnt;
+                const bool first = q[u].x & 1;
+                const float dj = __int_as_float(q[u].y);
+                rowoff += (ok && first) ? (uint32_t)(CU * 4) : 0u;
+                acc[0] = ok ? fmaf(f[u].x, dj, first ? 0.f : acc[0]) : acc[0];
+                acc[1] = ok ? fmaf(f[u].y, dj, first ? 0.f : acc[1]) : acc[1];
+                if (ok) *reinterpret_cast<float2*>(slotb + rowoff) = make_float2(acc[0], acc[1]);
               }
             }
           }
         }
       }
-      // this tile's rows of the unit are in the slot
-      __syncwarp();
-      VEON_TACC(3)
-      if (lane == 0) {
-        const uint32_t t = (blockIdx.x + m * gridDim.x) * kRoundTiles + w;
-        sh->meta[slot][w] = make_uint2((uint32_t)sl[17 + w],
-                                       (uint32_t)base_row | ((live_w && t < p.n_tiles) ? kMetaMine : 0u));
-        mbar_arrive(&sh->full[slot]);   // release: the rows and the meta word are visible with it
-      }
+    }
+    // this tile's rows of the round are in the slot
+    __syncwarp();
+    VEON_TACC(3)
+    if (lane == 0) {
+      const uint32_t t = (blockIdx.x + m * gridDim.x) * kRoundTiles + w;
+      sh->meta[slot][w] = make_uint2((uint32_t)sl[17 + w],
+                                     (uint32_t)base_row | ((live_w && t < p.n_tiles) ? kMetaMine : 0u));
+      mbar_arrive(&sh->full[slot]);   // release: the rows and the meta word are visible with it
     }
   }
   cpa_wait<0>();
@@ -388,21 +365,19 @@ __device__ __forceinline__ void role_rows(const FwdStreamParams& p, int32_t* rin
 // eight lanes of a store quad-row (eight different rows, same channel) hit different banks
 __device__ __forceinline__ uint32_t e_swz(uint32_t j) { return (j ^ (j >> 2)) & 7u; }
 
-// One E step = (unit, 32-channel sub-chunk).  The steps are software-pipelined over two staging
+// One E step = (round, 32-channel sub-chunk).  The steps are software-pipelined over two staging
 // buffers: the copies of step i+1 (ring -> shared memory, L2 latency) are in flight while step i is
-// written out, and the wait for role A's next unit happens a step early.
+// written out, and the wait for role A's next round happens a step early.
 struct ECursor {
-  uint32_t m, pass, sub;      // round of this CTA, channel pass, sub-chunk
+  uint32_t m, sub;            // round of this CTA, sub-chunk
   uint32_t b, vt;             // sample and tile inside the sample of this warp's tile
   uint32_t occ;
   int base, n;
   bool mine;
 };
 
-template <int VEC>
 __device__ __forceinline__ void role_expand(const FwdStreamParams& p, float* stage,
                                             StreamShared* sh, int lane, int ew) {
-  constexpr int CU = 32 * VEC;
   constexpr int kSub = CU / kEChunk;
   constexpr uint32_t kBufBytes = kERows * kEChunk * 4;
   __builtin_assume(__isShared(stage));
@@ -423,7 +398,7 @@ __device__ __forceinline__ void role_expand(const FwdStreamParams& p, float* sta
   __syncwarp();
 
   auto start = [&](ECursor& c) {
-    c.m = 0; c.pass = 0; c.sub = 0;
+    c.m = 0; c.sub = 0;
     const uint32_t t = blockIdx.x * kRoundTiles + ew;
     c.b = t / p.tiles_per_sample;
     c.vt = t - c.b * p.tiles_per_sample;
@@ -432,8 +407,6 @@ __device__ __forceinline__ void role_expand(const FwdStreamParams& p, float* sta
   auto advance = [&](ECursor& c) {
     if (++c.sub < (uint32_t)kSub) return;
     c.sub = 0;
-    if (++c.pass < (uint32_t)p.n_pass) return;
-    c.pass = 0;
     ++c.m;
     c.vt += t_step;
     while (c.vt >= p.tiles_per_sample) {
@@ -443,20 +416,18 @@ __device__ __forceinline__ void role_expand(const FwdStreamParams& p, float* sta
   };
   // start the copies of the cursor's step into buffer `buf`
   auto issue = [&](ECursor& c, uint32_t buf) {
-    const uint32_t unit = c.m * (uint32_t)p.n_pass + c.pass;
-    const uint32_t slot = unit & ns_mask;
+    const uint32_t slot = c.m & ns_mask;
     if (c.sub == 0) {
-      // Role A has put the unit's rows into the slot.  EVERY E warp waits here, also one whose
+      // Role A has put the round's rows into the slot.  EVERY E warp waits here, also one whose
       // tile is empty: no E warp may run a slot generation ahead of the others (its tick on
       // `drained` would be taken for a slower warp's).
-      mbar_wait(&sh->full[slot], (unit >> p.ns_log2) & 1u);
-      if (c.pass == 0) {   // what role A published about this warp's tile (the same for every pass)
-        const uint2 mt = sh->meta[slot][ew];
-        c.occ = mt.x;
-        c.base = (int)(mt.y & ~kMetaMine);
-        c.mine = (mt.y & kMetaMine) != 0u;
-        c.n = __popc(c.occ);
-      }
+      mbar_wait(&sh->full[slot], (c.m >> p.ns_log2) & 1u);
+      // what role A published about this warp's tile
+      const uint2 mt = sh->meta[slot][ew];
+      c.occ = mt.x;
+      c.base = (int)(mt.y & ~kMetaMine);
+      c.mine = (mt.y & kMetaMine) != 0u;
+      c.n = __popc(c.occ);
     }
     if (c.mine && c.n > 0) {
       const float* src = cta_ring + (size_t)slot * (kSlotRows * CU) + (size_t)c.base * CU +
@@ -469,7 +440,7 @@ __device__ __forceinline__ void role_expand(const FwdStreamParams& p, float* sta
     cpa_commit();
   };
 
-  const uint32_t n_steps = my_rounds * (uint32_t)p.n_pass * kSub;
+  const uint32_t n_steps = my_rounds * kSub;
   ECursor wc, ic;     // step being written, step whose copies are issued next
   start(wc);
   start(ic);
@@ -482,13 +453,12 @@ __device__ __forceinline__ void role_expand(const FwdStreamParams& p, float* sta
     const uint32_t buf = st & 1u;
     VEON_TACC(0)
     // this step's copies (issued a step ago) have landed; the slot is released BEFORE the wait
-    // for role A's next unit: an A warp may be blocked on exactly this slot while other tiles
-    // of the next unit are still unclaimed (tiles are claimed dynamically)
+    // for role A's next round: an A warp may be blocked on exactly this slot while other tiles
+    // of the next round are still unclaimed (tiles are claimed dynamically)
     cpa_wait<0>();
     __syncwarp();
-    const uint32_t unit = wc.m * (uint32_t)p.n_pass + wc.pass;
     if (wc.sub == (uint32_t)kSub - 1 && lane == 0)   // slot needed no more
-      atomicAdd(const_cast<uint32_t*>(&sh->drained[unit & ns_mask]), 1u);
+      atomicAdd(const_cast<uint32_t*>(&sh->drained[wc.m & ns_mask]), 1u);
     VEON_TACC(2)
     if (st + 1 < n_steps) {   // the next step's copies fly during the barrier and the write-out
       advance(ic);
@@ -501,7 +471,7 @@ __device__ __forceinline__ void role_expand(const FwdStreamParams& p, float* sta
     else asm volatile("bar.sync 2, %0;" ::"n"(kEGroup * 32) : "memory");
 #endif
     VEON_TACC(3)
-    if (wc.sub == 0 && wc.pass == 0) {
+    if (wc.sub == 0) {
       // offset of channel r of the staged row of each of this lane's four voxels inside a
       // buffer, the row's swizzle folded in; the zero row for empty voxels
 #pragma unroll
@@ -514,7 +484,7 @@ __device__ __forceinline__ void role_expand(const FwdStreamParams& p, float* sta
       }
     }
     if (wc.mine) {
-      float* o = p.out + ((int64_t)wc.b * p.C + wc.pass * CU + wc.sub * kEChunk + r) * p.V +
+      float* o = p.out + ((int64_t)wc.b * p.C + wc.sub * kEChunk + r) * p.V +
                  wc.vt * kTileVoxels + q4;
       const int64_t ostep = 4 * p.V;
       if (wc.n == 0) {
@@ -543,11 +513,10 @@ __device__ __forceinline__ void role_expand(const FwdStreamParams& p, float* sta
     VEON_TACC(4)
     // move the write cursor; a new tile takes over the meta the issue cursor has read
     advance(wc);
-    if (wc.sub == 0 && wc.pass == 0) { wc.occ = ic.occ; wc.base = ic.base; wc.n = ic.n; wc.mine = ic.mine; }
+    if (wc.sub == 0) { wc.occ = ic.occ; wc.base = ic.base; wc.n = ic.n; wc.mine = ic.mine; }
   }
 }
 
-template <int VEC>
 __global__ void __launch_bounds__(kStreamWarps * 32, 1)
 k_fwd_stream(const FwdStreamParams p) {
   extern __shared__ __align__(16) float fs_smem_raw[];
@@ -567,40 +536,37 @@ k_fwd_stream(const FwdStreamParams p) {
   constexpr int kEStageFloats = kEWarps * 2 * kERows * kEChunk;
   if (warp < kAWarps) {
     reg_inc<kARegs>();
-    role_rows<VEC>(p, reinterpret_cast<int32_t*>(fs_smem + kEStageFloats) +
-                          warp * (kASlots * kASlotInts), &sh, lane);
+    role_rows(p, reinterpret_cast<int32_t*>(fs_smem + kEStageFloats) + warp * (kASlots * kASlotInts),
+              &sh, lane);
   } else {
     reg_dec<kERegs>();
     const int ew = warp - kAWarps;
-    role_expand<VEC>(p, fs_smem + ew * 2 * kERows * kEChunk, &sh, lane, ew);
+    role_expand(p, fs_smem + ew * 2 * kERows * kEChunk, &sh, lane, ew);
   }
 }
 
 bool fwd_stream_supported(int B, int C, int64_t V, const void* feat, const void* out,
                           int64_t n_feat_rows) {
   if (V % kTileVoxels != 0) return false;
-  // The kernel handles C = 64 and every multiple of 128 (bit-identical; tools/fwd_check.py runs
-  // them all through stream_force), but it only WINS for 64-channel rows (318 vs 337 us at C2);
-  // wider rows at VEON's point density are faster through the general kernel (B200, round 2:
-  // 1.15-1.5 ms vs 1.10 ms for a 2.6 GB volume), so they stay there.
-  if (C != 64 && !(stream_force && C % 128 == 0)) return false;
+  // 64-channel rows only: there the kernel wins (318 vs 337 us at C2); wider rows at VEON's point
+  // density were faster through the general kernel (B200, round 2: 1.15-1.5 ms vs 1.10 ms for a
+  // 2.6 GB volume)
+  if (C != 64) return false;
   if (((uintptr_t)feat | (uintptr_t)out) & 15) return false;
   if ((int64_t)B * V > 0x7fffffffLL || n_feat_rows * (int64_t)C > 0x3fffffffLL) return false;
   return true;
 }
 
-template <int VEC>
 static int launch_stream_kernel(FwdStreamParams& p, size_t ring_bytes, cudaStream_t stream) {
-  constexpr int CU = 32 * VEC;
   const size_t smem = sizeof(float) * kEWarps * 2 * kERows * kEChunk +
                       sizeof(int32_t) * kAWarps * kASlots * kASlotInts + 256;
   static int per_sm[kMaxDevices] = {};
   const int dev = current_device();
   if (per_sm[dev] == 0) {
-    VEON_CUDA_TRY(cudaFuncSetAttribute(k_fwd_stream<VEC>,
+    VEON_CUDA_TRY(cudaFuncSetAttribute(k_fwd_stream,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int n = 0;
-    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_fwd_stream<VEC>,
+    VEON_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_fwd_stream,
                                                                 kStreamWarps * 32, smem));
     per_sm[dev] = n > 0 ? n : -1;
   }
@@ -613,22 +579,15 @@ static int launch_stream_kernel(FwdStreamParams& p, size_t ring_bytes, cudaStrea
   if (ns < 2) return VEON_E_WORKSPACE;
   p.ns_log2 = 1;   // the largest power of two that fits, at most kMaxSlots
   while ((2 << p.ns_log2) <= ns && (2 << p.ns_log2) <= kMaxSlots) ++p.ns_log2;
-  p.n_pass = p.C / CU;
-  // a tile's passes must not need one slot twice: the second use would wait for the round to
-  // be consumed, i.e. for tiles the very same warp may still hold a claim on
-  if (p.n_pass > (1 << p.ns_log2)) return VEON_E_WORKSPACE;
-  k_fwd_stream<VEC><<<(unsigned)grid, kStreamWarps * 32, smem, stream>>>(p);
+  k_fwd_stream<<<(unsigned)grid, kStreamWarps * 32, smem, stream>>>(p);
   VEON_LAUNCH_CHECK();
   return 0;
 }
 
 size_t fwd_stream_workspace_bytes(int C) {
-  // (SM count of the current device) x 8 slots (C = 64) / 4 slots (wider rows, at least one per
-  // 128-channel pass) = 148 x 1 MB at least
-  const int CU = C == 64 ? 64 : 128;
-  int ns = C == 64 ? 8 : 4;
-  while (ns < C / CU) ns *= 2;
-  return (size_t)sm_count_total() * ns * sizeof(float) * kSlotRows * CU;
+  // (SM count of the current device) x 8 slots = 148 x 1 MB; no ring where the kernel is not used
+  if (C != 64) return 0;
+  return (size_t)sm_count_total() * 8 * sizeof(float) * kSlotRows * CU;
 }
 
 int launch_fwd_stream(const float* depth, const float* feat, const int32_t* rd, const int32_t* rf,
@@ -644,9 +603,8 @@ int launch_fwd_stream(const float* depth, const float* feat, const int32_t* rd, 
   p.out = out; p.V = V; p.n_tiles = (uint32_t)n_tiles;
   p.n_rounds = (uint32_t)ceil_div64(n_tiles, kRoundTiles);
   p.tiles_per_sample = (uint32_t)tps;
-  p.C = C; p.n_pass = 1; p.ns_log2 = 1;
-  int rc = C == 64 ? launch_stream_kernel<2>(p, ws_bytes, stream)
-                   : launch_stream_kernel<4>(p, ws_bytes, stream);
+  p.C = C; p.ns_log2 = 1;
+  int rc = launch_stream_kernel(p, ws_bytes, stream);
   if (rc) return rc;
   if (heavy) return launch_heavy_behind(depth, feat, rd, rf, rb, tile_start, heavy, heavy_ints, B, C,
                                         V, out, kStreamHeavyMin, stream);

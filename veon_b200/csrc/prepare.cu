@@ -637,18 +637,6 @@ extern "C" size_t veon_prepare_v2_workspace_bytes(int B, int N, int D, int H, in
   return w.total;
 }
 
-extern "C" size_t veon_prepare_v2_voxel_start_offset(int B, int N, int D, int H, int W,
-                                                     const float* grid_size) {
-  int64_t P;
-  if (!grid_size || check_dims(B, N, D, H, W, &P)) return (size_t)-1;
-  const float one[3] = {1.f, 1.f, 1.f}, zero[3] = {0.f, 0.f, 0.f};
-  GridF g = make_grid(zero, one, grid_size);
-  int64_t nbins = num_bins(B, g);
-  if (nbins < 0) return (size_t)-1;
-  PrepWs w = carve(nullptr, P, nbins, (int64_t)B * voxels_of(grid_size));
-  return (size_t)((char*)w.offset - (char*)nullptr);
-}
-
 static int prepare_impl(const float* coor, const float* frustum, const CamXform* xf, int B, int N,
                         int D, int H, int W, const float* lower, const float* interval,
                                const float* grid_size, int32_t* ranks_bev,

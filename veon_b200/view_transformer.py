@@ -336,8 +336,8 @@ class LSSViewTransformerRaw(LSSViewTransformer):
     ready-made features and a depth distribution, lifts, then (use_ds)
     max-pools the volume 2x2x2.  With memory_format=torch.channels_last_3d it
     pools channels-last and reduces with the channels-last 2x2x2 kernels (the
-    fused `fuse_ds` kernel and the one-node PoolMaxDown training route are
-    channels-first only and are not taken); the result is channels-last-3d.
+    one-node PoolMaxDown training route is channels-first only and is not
+    taken); the result is channels-last-3d.
 
     `dtype` (the pooled full-resolution volume) is float32 only: any other raises ValueError.
 
@@ -351,16 +351,14 @@ class LSSViewTransformerRaw(LSSViewTransformer):
       route followed by a cast (which keeps the layout).
     - no gradient (2x2x2, even grid, fused geometry): the neck pools straight into a bfloat16
       volume (either layout) and takes the maximum in bfloat16, so no float32 full-resolution
-      volume is written; this replaces `fuse_ds`.  Rounding to nearest even is monotone, so every
-      value equals the float32 route cast (==), and so do the bits, except that a zero result
-      may carry the other sign: a window whose float32 sums include a nonzero one of magnitude
-      below 2^-134, which bfloat16 rounds to a signed zero, may then return the zero of another
-      element.  Which element is the arg-max is not observable without a gradient.
+      volume is written.  Rounding to nearest even is monotone, so every value equals the float32
+      route cast (==), and so do the bits, except that a zero result may carry the other sign: a
+      window whose float32 sums include a nonzero one of magnitude below 2^-134, which bfloat16
+      rounds to a signed zero, may then return the zero of another element.  Which element is the arg-max is not observable without a gradient.
     - any other case (other `ds`, odd grids, `accelerate`, `collapse_z`, the empty-input dummy):
       the float32 route, then one cast."""
 
-    def __init__(self, *args, use_ds=True, ds=(2, 2, 2), fuse_ds=False, ds_dtype=torch.float32,
-                 **kwargs):
+    def __init__(self, *args, use_ds=True, ds=(2, 2, 2), ds_dtype=torch.float32, **kwargs):
         if not isinstance(ds_dtype, torch.dtype) or ds_dtype not in _bp._DTYPES:
             raise ValueError(f"ds_dtype must be torch.float32 or torch.bfloat16, got {ds_dtype!r}")
         if ds_dtype is torch.bfloat16 and not use_ds:
@@ -373,11 +371,6 @@ class LSSViewTransformerRaw(LSSViewTransformer):
         self.ds_dtype = ds_dtype
         self.use_ds = use_ds
         self.ds = tuple(ds)
-        # Extra (not in the reference): pool and max-reduce in ONE kernel on the no-grad path,
-        # never writing the full-resolution volume (SURVEY 8f-1).  Bit-identical, but the first
-        # cut of that kernel is latency-bound and currently slower than pooling followed by
-        # our streaming 2x2x2 kernel (784 vs 705 us at C2), so it is opt-in.
-        self.fuse_ds = fuse_ds
 
     # -- depth-distribution producer (SURVEY 8f-2) ------------------------------
     def downsample_depth(self, depths, downsample):
@@ -408,10 +401,9 @@ class LSSViewTransformerRaw(LSSViewTransformer):
     def forward(self, input, depth, stereo_metas=None):
         tran_feat = input[0]
         B, N, C, H, W = tran_feat.shape
+        fused = None
         if self.ds_dtype is torch.bfloat16:
             fused = self._forward_bf16_inference(input, depth)
-        else:
-            fused = self._forward_downsampled(input, depth)
         if fused is None:
             fused = self._forward_pool_maxdown(input, depth)
         if fused is not None:
@@ -449,28 +441,6 @@ class LSSViewTransformerRaw(LSSViewTransformer):
         d5 = depth.reshape(B, N, self.D, H, W)
         out = _bp.pool_prepared_maxdown(d5, feat_last, prep, self._bev_shape(d5, C),
                                         dtype=self.ds_dtype)
-        # None also lets the plain route reproduce the reference's empty-input behaviour
-        return None if out is None or self._no_points(prep) else out
-
-    def _forward_downsampled(self, input, depth):
-        """Inference path: pooling and the 2x2x2 maximum in one kernel, the full-resolution
-        volume is never written (SURVEY 8f-1).  Returns None whenever the plain route must be
-        taken: gradients wanted, cached ranks (`accelerate`), other `ds`, odd grids, ..."""
-        tran_feat = input[0]
-        if (not self.fuse_ds or not self.use_ds or self.ds != (2, 2, 2) or self.accelerate
-                or self.collapse_z or self.memory_format is not torch.contiguous_format
-                or (torch.is_grad_enabled() and (tran_feat.requires_grad or depth.requires_grad))
-                or not tran_feat.is_cuda):
-            return None
-        B, N, C, H, W = tran_feat.shape
-        coor = self.get_lidar_coor(*input[1:7])
-        if coor.numel() == 0:
-            return None
-        prep = self._prepared(_bp.prepare_ranks(coor, self.grid_lower_bound, self.grid_interval,
-                                                self.grid_size))
-        feat_last = tran_feat.reshape(B, N, C, H, W).permute(0, 1, 3, 4, 2)
-        d5 = depth.reshape(B, N, self.D, H, W)
-        out = _bp.pool_prepared_downsampled(d5, feat_last, prep, self._bev_shape(d5, C))
         # None also lets the plain route reproduce the reference's empty-input behaviour
         return None if out is None or self._no_points(prep) else out
 
